@@ -2,6 +2,7 @@
 """bench.py -- the BORE-MLP hot path (fit -> multi-start argmax) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg3]
+                    [--dump-outputs DIR]
 
 A "step" is one BO iteration on synthetic quantile-labelled data: fit the classifier (Keras
 semantics: `epochs` x ceil(N/64) Adam steps) then maximise it from S start points with the
@@ -324,11 +325,12 @@ def run_ours(args, wl, rank, local_rank, world):
                 torch.cuda.synchronize()
                 timers["fit_ms"] += ev[0].elapsed_time(ev[1])
                 timers["argmax_ms"] += ev[1].elapsed_time(ev[2])
-            return res, gidx, rec
+            return res, gidx, rec, zbuf
         return step
 
     def timed(step, K, warm):
-        """EXACTLY K steps between barrier + synchronize, CUDA events, max over ranks."""
+        """EXACTLY K steps between barrier + synchronize, CUDA events, max over ranks.  Also returns what
+        the last step returned."""
         for _ in range(warm):
             step()
         agg = dict(k2_ms=0.0, step_ms=0.0, rounds=0, bytes=0.0, evals=0.0, fused=0, grid=0, block=0)
@@ -340,7 +342,8 @@ def run_ours(args, wl, rank, local_rank, world):
         e0.record()
         for _ in range(K):
             t_dbg = time.perf_counter()
-            res, gidx, rec = step(timers)
+            last = step(timers)
+            res = last[0]
             if os.environ.get("BENCH_DEBUG"):
                 sys.stderr.write(f"step {1e3 * (time.perf_counter() - t_dbg):.1f} ms rounds {res['rounds']} evals {res['evals']}\n")
             total_evals += res["evals"]
@@ -359,7 +362,7 @@ def run_ours(args, wl, rank, local_rank, world):
             elapsed_ms, evals_all = tmax[0].item(), tsum[1].item()
         else:
             evals_all = float(total_evals)
-        return elapsed_ms, evals_all, agg, timers
+        return elapsed_ms, evals_all, agg, timers, last
 
     peak_ffma = ffma_peak_tflops(local_rank)
     peaks = {}
@@ -388,14 +391,23 @@ def run_ours(args, wl, rank, local_rank, world):
         if os.environ.get("BENCH_DEBUG"):
             torch.cuda.synchronize()
             sys.stderr.write(f"warm-up step {1e3 * (time.perf_counter() - t_w):.1f} ms\n")
-    elapsed_ms, evals_all, agg, timers = timed(step_weak, K, 0)
+    elapsed_ms, evals_all, agg, timers, last = timed(step_weak, K, 0)
     ms_per_step = elapsed_ms / K
     value = evals_all / (elapsed_ms * 1e-3)
+    outputs = None
+    if args.dump_outputs:
+        # the next step resets the parameters in place: copy them (and the loss buffer) now, on the device
+        res, gidx, rec, screen = last
+        outputs = dict(fit_params=params.clone(), fit_loss=loss_d.clone(), screen_pred=screen,
+                       **{"argmax_" + k: res[k] for k in ("x", "fun", "nit", "nfev", "status", "task")},
+                       winner_index=np.array([-1 if gidx is None else gidx]),
+                       winner_x_fun=np.full(D + 1, np.nan) if rec is None else rec)
+    del last
 
     # ---- strong scaling: the SAME 65,536 starts in total, split over the ranks ----
     # (right behind the headline steps: measured after the 0.3 s of host work and idle GPU that used to sit
     #  here, the same three steps took anything from 131 to 205 ms on one GPU, where they ARE the headline step)
-    s_ms, s_evals, s_agg, s_tim = timed(step_strong, Ks, 3)
+    s_ms, s_evals, s_agg, s_tim, _ = timed(step_strong, Ks, 3)
     clocks = sampler.stop()
 
     # ---- e2e: the public API with HOST buffers (H2D/D2H inside the timed region) ----
@@ -435,6 +447,8 @@ def run_ours(args, wl, rank, local_rank, world):
     cfg4 = None
     if not args.no_cfg4:
         cfg4 = cfg4_measure(rank, local_rank, world, steps=2, warm=1)
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs, f"_rank{rank}" if world > 1 else "")
 
     if rank != 0:
         return
@@ -521,6 +535,15 @@ def run_ours(args, wl, rank, local_rank, world):
         line["cpu_baseline"] = cpu_baseline(wl, X, z, perms, w0)
         line["lstm"] = lstm_measure()
     print(json.dumps(line), flush=True)
+
+
+def write_outputs(out_dir, arrays, suffix=""):
+    """--dump-outputs: one DIR/<name><suffix>.npy per array, float32 kept, everything else as float64 (the integer
+    outputs are far below 2**53, so exactly).  cfg 3, the largest workload, writes 29 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
 def cpu_baseline(wl, X, z, perms, w0):
@@ -721,7 +744,14 @@ def main():
     ap.add_argument("--workload", default="cfg3", choices=sorted(WORKLOADS) + ["cfg4"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cfg4", action="store_true", help="skip the short cfg 4 sub-record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (inputs are seeded, so two "
+                         "builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "cfg4"):
+        ap.error("--dump-outputs is for the GPU arm of cfg2 / cfg3 / cfg5")
     from bore_b200 import distributed as bd
     rank, local_rank, world = bd.env_world()
     if args.workload == "cfg4":

@@ -32,6 +32,7 @@ def test_library_is_sm100a_and_torch_free():
     out = subprocess.run(["cuobjdump", "--list-elf", path], capture_output=True, text=True).stdout
     assert "sm_100a" in out
     ldd = subprocess.run(["ldd", path], capture_output=True, text=True).stdout
+    ldd = re.sub(r"\(0x[0-9a-f]+\)", "", ldd)  # load addresses are random and may contain "c10"
     assert "torch" not in ldd and "c10" not in ldd  # plain C ABI: no torch types or libs
 
 
