@@ -45,14 +45,8 @@ int bore_mlp_create(int n_layers, const int *dims, const int *acts, int n_models
   for (int l = 0; l < n_layers; ++l)
     BORE_CHECK(acts[l] >= BORE_ACT_LINEAR && acts[l] <= BORE_ACT_TANH,
                "bore_mlp_create: unknown activation code %d", acts[l]);
-  BORE_CHECK(bore_device_count() > 0,
-             "bore_mlp_create: no CUDA device visible -- bore_b200 has no CPU fallback");
-  BORE_CUDA(cudaSetDevice(device));
-  bore_mlp *h = new bore_mlp();
-  memset(h, 0, sizeof(*h));
-  h->pack = new MlpPackCache();
-  memset(h->pack, 0, sizeof(*h->pack));
-  MlpDesc &d = h->desc;
+  MlpDesc d;
+  memset(&d, 0, sizeof(d));
   d.n_layers = n_layers;
   int off = 0;
   for (int l = 0; l <= n_layers; ++l) d.dims[l] = dims[l];
@@ -62,6 +56,17 @@ int bore_mlp_create(int n_layers, const int *dims, const int *acts, int n_models
     d.b_off[l] = off; off += dims[l + 1];
   }
   d.n_params = off;
+  // the limits above are necessary, not sufficient: a net inside them can still need more shared
+  // memory than an SM has.  Refuse it here rather than at its first predict / fit / argmax.
+  if (mlp_eval_check_envelope(d) != 0 || fit_check_envelope(d) != 0) return -1;
+  BORE_CHECK(bore_device_count() > 0,
+             "bore_mlp_create: no CUDA device visible -- bore_b200 has no CPU fallback");
+  BORE_CUDA(cudaSetDevice(device));
+  bore_mlp *h = new bore_mlp();
+  memset(h, 0, sizeof(*h));
+  h->pack = new MlpPackCache();
+  memset(h->pack, 0, sizeof(*h->pack));
+  h->desc = d;
   h->n_models = n_models;
   h->lr = 1e-3f; h->beta1 = 0.9f; h->beta2 = 0.999f; h->eps = 1e-7f;  // Keras "adam"
   h->device = device;

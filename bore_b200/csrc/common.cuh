@@ -90,6 +90,10 @@ int mlp_eval_prepare(const bore_mlp *h, int model0, int n_models, bool want_grad
 int launch_mlp_eval_multi(const bore_mlp *h, int model0, int n_models, int per_model, bool want_grad,
                           int transform, int negate, const float *X, float *f, float *g,
                           const int *flags, cudaStream_t stream, int prepacked = 0);
+// bore_mlp_create's check of a net against the kernels' shared-memory plans (mlp_eval.cu, fit.cu): 0 when
+// it runs, else -1 with the shared memory needed and the limit in the error text.  Host only, no device.
+int mlp_eval_check_envelope(const MlpDesc &d);
+int fit_check_envelope(const MlpDesc &d);
 // K1t (fit_mma.cu): 1 launched, 0 shape not taken (caller falls back to the FFMA kernels), < 0 error
 int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                    int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,

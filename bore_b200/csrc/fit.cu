@@ -1226,7 +1226,38 @@ evaluate_kernel(const MlpDesc d, const float *__restrict__ params, const float *
   }
 }
 
+constexpr size_t FIT_MAX_SMEM = 227 * 1024;
+
+// the sample-split cluster kernel's plan; false when it does not fit (shared memory, or weight images
+// too large for the 16-bit offsets of its index table)
+bool fitc_plan(const MlpDesc &d, int batch, FitCPlan &p, size_t &smem) {
+  make_fitc_plan(d, batch, p);
+  smem = (size_t)p.total * sizeof(float);
+  return smem <= 226 * 1024 && p.wend < 0xffff;
+}
+
+// the one-CTA kernel's plan for CTAs of `threads` threads; returns its shared memory in bytes
+size_t fit_onecta_plan(const MlpDesc &d, int batch, int threads, int narrow, FitPlan &p) {
+  make_fit_plan(d, batch, threads, 226 * 1024 / (int)sizeof(float), p, narrow);
+  return (size_t)p.total * sizeof(float);
+}
+
 }  // namespace
+
+// bore_mlp_create: automatic-mode training at batch 64 must have a kernel for one model and for many.
+// Many models run the one-CTA kernel (256 threads, 128 from 2 x SMs models on); it is also where one
+// model ends up when neither cluster kernel takes the net, so its plan decides both.
+int fit_check_envelope(const MlpDesc &d) {
+  const int B = 64;
+  for (int threads : {FIT_THREADS, 128}) {
+    FitPlan p;
+    const size_t need = fit_onecta_plan(d, B, threads, 1, p);
+    BORE_CHECK(need <= FIT_MAX_SMEM,
+               "bore_mlp_create: training at batch %d needs %zu B of shared memory per model (limit %zu B)", B,
+               need, FIT_MAX_SMEM);
+  }
+  return 0;
+}
 
 extern "C" {
 
@@ -1296,9 +1327,8 @@ int bore_mlp_fit(bore_mlp *h, int model0, int count, const float *X_dev, const f
   }
   {
     FitCPlan CP;
-    make_fitc_plan(a.d, B, CP);
-    const size_t csmem = (size_t)CP.total * sizeof(float);
-    const bool fits = csmem <= 226 * 1024 && CP.wend < 0xffff;
+    size_t csmem;
+    const bool fits = fitc_plan(a.d, B, CP, csmem);
     const bool want = h->fit_mode == 2 || (h->fit_mode == 0 && count * FIT_CLUSTER <= h->sm_count);
     BORE_CHECK(!(h->fit_mode == 2 && !fits), "bore_mlp_fit: cluster mode needs %zu B of shared memory", csmem);
     if (want && fits) {
@@ -1330,16 +1360,16 @@ int bore_mlp_fit(bore_mlp *h, int model0, int count, const float *X_dev, const f
     }
     if (forced == 32 || forced == 64 || forced == 128 || forced == 256) threads = forced;
   }
+  size_t smem;
   {
     static int narrow = -1;
     if (narrow < 0) {
       const char *e = getenv("BORE_FIT_NARROW");
       narrow = e ? atoi(e) : 1;
     }
-    make_fit_plan(a.d, B, threads, 226 * 1024 / (int)sizeof(float), a.P, narrow);
+    smem = fit_onecta_plan(a.d, B, threads, narrow, a.P);
   }
-  const size_t smem = (size_t)a.P.total * sizeof(float);
-  BORE_CHECK(smem <= 227 * 1024, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
+  BORE_CHECK(smem <= FIT_MAX_SMEM, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
   BORE_CUDA(cudaFuncSetAttribute(fit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   fit_kernel<<<count, threads, smem, (cudaStream_t)stream>>>(a);
   BORE_CUDA(cudaGetLastError());

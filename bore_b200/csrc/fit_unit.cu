@@ -862,6 +862,14 @@ static int fu_launch(const FuArgs &a, int count, size_t smem, cudaStream_t strea
 
 }  // namespace
 
+// The plan for a (padded) batch; false when the kernel does not take the net: no hidden layer, more
+// than 64 samples (the loss reduction assumes the samples sit in two warps), or shared memory
+static bool fu_plan(const MlpDesc &d, int batch, FuPlan &p, size_t &smem) {
+  if (!make_fu_plan(d, batch, p)) return false;
+  smem = (size_t)p.total * sizeof(float);
+  return p.SP <= 64 && smem <= 226 * 1024;
+}
+
 // 1 launched, 0 shape not taken (the caller falls back to the sample-split cluster kernel), < 0 error
 int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                     int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
@@ -878,10 +886,8 @@ int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev
   for (int i = 2; i <= nh; ++i) uniform = uniform && a.d.dims[i] == hw;
   const bool fixed_shape = !generic && uniform && B <= 64 &&
                            ((nh == 3 && (hw == 64 || hw == 32)) || (nh == 2 && (hw == 32 || hw == 16)));
-  if (!make_fu_plan(a.d, fixed_shape ? 64 : B, a.P)) return 0;
-  if (a.P.SP > 64) return 0;  // the loss reduction assumes the samples sit in two warps
-  const size_t smem = (size_t)a.P.total * sizeof(float);
-  if (smem > 226 * 1024) return 0;
+  size_t smem;
+  if (!fu_plan(a.d, fixed_shape ? 64 : B, a.P, smem)) return 0;
   a.params = h->params; a.adam_m = h->adam_m; a.adam_v = h->adam_v; a.adam_t = h->adam_t;
   a.model0 = model0;
   a.X = X_dev; a.z = z_dev; a.N = N; a.shared_data = shared_data; a.batch = batch_size;

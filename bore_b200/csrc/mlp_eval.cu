@@ -535,6 +535,15 @@ static int pack_variant(const bore_mlp *h, int model0, int n_models, cudaStream_
   return 0;
 }
 
+constexpr int EVAL_MAX_SMEM = 227 * 1024;  // per CTA (opt-in)
+constexpr int EVAL_STATIC_SMEM = 256;       // left for the kernel's static shared memory (mbarrier, counter, alignment)
+
+// dynamic shared memory of an mlp_eval_kernel launch: the weight image, one activation strip per
+// warp and, in batched mode with flags, the compacted start list
+static size_t eval_smem_bytes(const SmemPlan &P, int warps, size_t list_bytes) {
+  return (size_t)(P.weights_total + warps * P.warp_total) * sizeof(float) + list_bytes;
+}
+
 template <bool GRAD, int UGB>
 static int launch_variant(const bore_mlp *h, const MlpDesc &d, int model0, const float *X,
                           int S, float *f, float *g, const int *list, const int *n_dev,
@@ -543,19 +552,16 @@ static int launch_variant(const bore_mlp *h, const MlpDesc &d, int model0, const
   using M = Map<UGB>;
   SmemPlan P;
   make_plan(d, GRAD, M::CH, M::AST, P);
-  const int max_smem = 227 * 1024;
+  const int max_smem = EVAL_MAX_SMEM;
   const bool multi = per_model > 0;
   const size_t list_bytes = (multi && flags) ? (size_t)per_model * sizeof(int) : 0;
   // warps per CTA: as many as fit (<= 16) -- in batched mode no more than the model has tiles
   int warps = 16;
   if (multi) warps = std::min(16, std::max(1, (per_model + M::TP - 1) / M::TP));
-  // 256 B are left for the kernel's static shared memory (mbarrier, counter, alignment)
-  while (warps > 1 && (size_t)(P.weights_total + warps * P.warp_total) * sizeof(float) + list_bytes + 256 >
-                          (size_t)max_smem)
-    --warps;
-  const size_t smem = (size_t)(P.weights_total + warps * P.warp_total) * sizeof(float) + list_bytes;
-  BORE_CHECK(smem + 256 <= (size_t)max_smem, "mlp_eval: model needs %zu B of shared memory (> %d)",
-             smem, max_smem);
+  while (warps > 1 && eval_smem_bytes(P, warps, list_bytes) + EVAL_STATIC_SMEM > (size_t)max_smem) --warps;
+  const size_t smem = eval_smem_bytes(P, warps, list_bytes);
+  BORE_CHECK(smem + EVAL_STATIC_SMEM <= (size_t)max_smem, "mlp_eval: model needs %zu B of shared memory (> %d)",
+             smem + EVAL_STATIC_SMEM, max_smem);
   if (!prepacked && pack_variant<GRAD, UGB>(h, model0, n_models, stream)) return -1;
   const float *params = h->params + (size_t)model0 * d.n_params;
   const float *packed = h->pack->buf[variant_index(GRAD, UGB)] + (size_t)model0 * P.weights_total;
@@ -609,6 +615,22 @@ static int dispatch(const bore_mlp *h, int model0, bool want_grad, int transform
   if (want_grad) return wide ? BORE_EVAL(true, 4) : BORE_EVAL(true, 3);
   return wide ? BORE_EVAL(false, 4) : BORE_EVAL(false, 3);
 #undef BORE_EVAL
+}
+
+// bore_mlp_create: K0 and K2 must be able to stage the net with ONE warp (dispatch's variant, the
+// plan and shared-memory sum of launch_variant); otherwise its first predict / argmax would fail
+int mlp_eval_check_envelope(const MlpDesc &d) {
+  const bool wide = is_wide(d);
+  for (int grad = 0; grad < 2; ++grad) {
+    SmemPlan P;
+    if (wide) make_plan(d, grad != 0, Map<4>::CH, Map<4>::AST, P);
+    else make_plan(d, grad != 0, Map<3>::CH, Map<3>::AST, P);
+    const size_t need = eval_smem_bytes(P, 1, 0) + EVAL_STATIC_SMEM;
+    BORE_CHECK(need <= (size_t)EVAL_MAX_SMEM,
+               "bore_mlp_create: %s needs %zu B of shared memory for one warp (limit %d B)",
+               grad ? "value and gradient (K2)" : "predict (K0)", need, EVAL_MAX_SMEM);
+  }
+  return 0;
 }
 
 int mlp_eval_prepare(const bore_mlp *h, int model0, int n_models, bool want_grad, cudaStream_t stream) {

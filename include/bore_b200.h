@@ -38,6 +38,10 @@ enum { BORE_TRANSFORM_IDENTITY = 0, BORE_TRANSFORM_SIGMOID = 1, BORE_TRANSFORM_E
 /* per-start termination status, scipy.optimize.OptimizeResult.status for L-BFGS-B */
 enum { BORE_STATUS_CONVERGED = 0, BORE_STATUS_LIMIT = 1, BORE_STATUS_ABNORMAL = 2 };
 
+/* Necessary bounds of a net, not sufficient ones: the kernels keep a model's weights in one SM's
+ * shared memory, so wide and deep nets with a large input dimension can exceed it inside these
+ * limits.  bore_mlp_create refuses such a net and names the shared memory it would need (DESIGN.md,
+ * "The net-shape envelope"). */
 #define BORE_MAX_LAYERS 8     /* Dense layers per model, final layer included */
 #define BORE_MAX_WIDTH 128    /* widest hidden layer */
 #define BORE_MAX_DIM 512      /* input dimension */
