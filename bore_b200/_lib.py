@@ -39,6 +39,10 @@ SIGNATURES = {
     "bore_mlp_fit": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int,
                                vp, C.c_int, vp, vp]),
     "bore_mlp_evaluate": (C.c_int, [vp, C.c_int, vp, vp, C.c_int, vp, vp]),
+    "bore_mlp_fit_weighted": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, vp, C.c_int, C.c_int, C.c_float,
+                                        C.c_float, C.c_int, C.c_int, vp, C.c_int, vp, vp]),
+    "bore_mlp_evaluate_weighted": (C.c_int, [vp, C.c_int, vp, vp, vp, C.c_float, C.c_float, C.c_int,
+                                             vp, vp]),
     "bore_mlp_set_regularizers": (C.c_int, [vp, vp, vp]),
     "bore_lbfgsb_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "bore_lbfgsb_minimize_workspace_bytes": (C.c_size_t, [vp, C.c_int, C.c_int]),

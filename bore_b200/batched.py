@@ -16,6 +16,7 @@ from sklearn.utils import check_random_state
 from . import ops
 from .engine import NativeMLP, lbfgsb_message
 from .layers import Dense, BinaryCrossentropy, Adam
+from .models import check_class_weight, sample_weights
 from .optimizers.utils import from_bounds
 
 
@@ -151,11 +152,14 @@ class BatchedMaximizableSequential:
         return [self._net.get_weights(model=p) for p in range(self.n_problems)]
 
     def fit(self, x, y, batch_size=32, epochs=1, permutations=None, shuffle=True, verbose=0,
-            gamma=None):
+            gamma=None, sample_weight=None, class_weight=None):
         """x (M, N, D), y (M, N): every problem trains on its own N observations, all in one
         launch.  ``permutations``: (epochs, N) shared by all problems or (M, epochs, N).
         With ``gamma`` given, ``y`` holds the RAW targets and every problem is labelled
         ``z = y < quantile(y, gamma)`` on the device (bore/data.py:31-35) before training.
+        ``sample_weight`` (M, N), or (N,) shared by all problems, and ``class_weight``
+        {0: w0, 1: w1} weight each sample's loss as Keras' ``fit`` does; with ``gamma`` the
+        class weights are applied on the device to the labels made there.
         Returns the per-problem history loss, shape (M, epochs), as a ``LazyLoss`` (array-like;
         the launch is asynchronous and the values are fetched on first use)."""
         if not self._compiled:
@@ -164,6 +168,20 @@ class BatchedMaximizableSequential:
         z = np.asarray(y)
         M, N, D = X.shape
         assert M == self.n_problems and z.shape == (M, N) and D == self.dims[0]
+        w = cw = None
+        if sample_weight is not None:
+            sw = np.asarray(sample_weight, np.float32)
+            if sw.shape not in ((M, N), (N,)):
+                raise ValueError(f"sample_weight must have shape ({M}, {N}) or ({N},), got {sw.shape}")
+            w = np.broadcast_to(sw, (M, N)).reshape(-1)
+        if class_weight is not None:
+            if gamma is None:  # labels known here: Keras' rule, class int(y)
+                w = sample_weights(z.reshape(-1), w, class_weight)
+            else:  # labels 0 / 1 made on the device: both need a weight
+                cwd = check_class_weight(class_weight)
+                if not {0, 1} <= set(cwd):
+                    raise ValueError("class_weight needs weights for the classes 0 and 1 of the labels")
+                cw = (cwd[0], cwd[1])
         z_dev = None
         if gamma is not None:
             z_dev = self._net.quantile_labels_dev(
@@ -182,7 +200,8 @@ class BatchedMaximizableSequential:
                            z_dev if z_dev is not None else
                            net.to_device(z.reshape(-1), np.float32),
                            N, int(batch_size), int(epochs), net.to_device(perm, np.int32),
-                           model0=0, count=M, shared_data=False, shared_perm=shared_perm)
+                           model0=0, count=M, shared_data=False, shared_perm=shared_perm,
+                           w_dev=None if w is None else net.to_device(w, np.float32), class_weight=cw)
         out = LazyLoss(loss)
         if verbose:
             print(f"fit: {M} problems x {epochs} epochs, mean loss {out[:, 0].mean():.4f} -> "

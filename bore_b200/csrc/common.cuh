@@ -75,6 +75,22 @@ struct bore_mlp {
 
 static inline int round_up(int a, int b) { return (a + b - 1) / b * b; }
 
+// Per-sample loss weights of a weighted fit / evaluate (bore_mlp_fit_weighted): the weight of sample i is
+// w[i] (1 when w is NULL) times cw1 if its label is 1, else cw0.  w has the layout of the labels.  on == 0:
+// unweighted, the kernels run the arithmetic of bore_mlp_fit unchanged.
+struct FitWeights {
+  const float *w;
+  float cw0, cw1;
+  int on;
+};
+
+// the loss weight of one sample (device code; row >= 0)
+#ifdef __CUDACC__
+__device__ __forceinline__ float fit_sample_weight(const FitWeights &fw, const float *w, int row, float z) {
+  return (w ? w[row] : 1.f) * (z != 0.f ? fw.cw1 : fw.cw0);
+}
+#endif
+
 // ---------------------------------------------------------------- launchers (one per .cu)
 // K0 / K2.  `list` (may be NULL) is a device array of row indices: point i of the launch
 // is row list[i] of X / f / g (used by the L-BFGS-B driver's compacted active list);
@@ -97,9 +113,9 @@ int fit_check_envelope(const MlpDesc &d);
 // K1t (fit_mma.cu): 1 launched, 0 shape not taken (caller falls back to the FFMA kernels), < 0 error
 int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                    int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                   float *loss_out_dev, cudaStream_t stream);
+                   float *loss_out_dev, const FitWeights &fw, cudaStream_t stream);
 // K1u (fit_unit.cu): one cluster per model, hidden units split over the CTAs.  1 launched, 0 shape not
 // taken (caller falls back to the sample-split cluster kernel), < 0 error
 int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                     int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                    float *loss_out_dev, cudaStream_t stream);
+                    float *loss_out_dev, const FitWeights &fw, cudaStream_t stream);

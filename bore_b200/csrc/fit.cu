@@ -125,6 +125,7 @@ struct FitArgs {
   int any_l2;
   float *loss_out;
   float lr, beta1, beta2, eps;
+  FitWeights fw;
 };
 
 // acc[i][u] += sum_k A[k*lda + i] * B[k*ldb + u]: the 4 x 4 register tile of every GEMM below
@@ -188,6 +189,8 @@ __device__ __forceinline__ void narrow_tile(const float *__restrict__ Hin, const
 // use dot-product forms instead of 4x4 tiles padded with zeros.  (The first version gave every
 // 4x4 gradient tile to one thread: with Dense32 layers 64 / 16 / 8 of 128 threads worked while
 // the rest waited at the barrier -- 44 % of all stall samples, profiles/r01_notes.md.)
+// WEIGHTED: per-sample loss weights (FitArgs::fw); the unweighted build runs none of their code
+template <bool WEIGHTED>
 __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
   extern __shared__ __align__(16) float sm[];
   const MlpDesc &d = a.d;
@@ -201,9 +204,13 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
   const float *X = a.X + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N * d.dims[0]);
   const float *zg = a.z + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N);
   const int *perm = a.perm + (a.shared_perm ? 0 : (size_t)blockIdx.x * a.epochs * a.N);
+  const float *wg = WEIGHTED && a.fw.w ? a.fw.w + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N) : nullptr;
   int *idxb = reinterpret_cast<int *>(sm + P.idx);
   float *red = sm + P.red;
   float *gs = sm + P.gs;
+  // loss weights of the minibatch (weighted fits): delta buffer 1 is first written by the reverse pass,
+  // after the loss has read them, and last read before the barrier that ends the previous step
+  float *wsm = sm + P.dl[1];
   const int D = d.dims[0];
 
   // ---- stage the weights: W_l [in][JP], W_l^T [out][KP] (l>0), bias ----
@@ -238,7 +245,9 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
       for (int p = tid; p < BP; p += NT) {
         const int row = p < nb ? perm[(size_t)ep * a.N + s0 + p] : -1;
         idxb[p] = row;
-        sm[P.zb + p] = row >= 0 ? zg[row] : 0.f;
+        const float zz = row >= 0 ? zg[row] : 0.f;
+        sm[P.zb + p] = zz;
+        if (WEIGHTED) wsm[p] = row >= 0 ? fit_sample_weight(a.fw, wg, row, zz) : 0.f;
       }
       __syncthreads();
       for (int e = tid; e < BP * D; e += NT) {
@@ -309,7 +318,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
         __syncthreads();
       }
 
-      // ---- loss and dL/dlogit (mean over the batch) ----
+      // ---- loss and dL/dlogit (mean over the batch; weighted: sum of w_i l_i over the batch size) ----
       const float inv_nb = 1.f / (float)nb;
       float lsum = 0.f;
       {
@@ -319,8 +328,10 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
           float dl = 0.f;
           if (p < nb) {
             const float u = U[p], zz = sm[P.zb + p];
-            lsum += fmaxf(u, 0.f) - u * zz + log1pf(expf(-fabsf(u)));
-            dl = (stable_sigmoid(u) - zz) * inv_nb;
+            float l = fmaxf(u, 0.f) - u * zz + log1pf(expf(-fabsf(u))), g = stable_sigmoid(u) - zz;
+            if (WEIGHTED) { const float ws = wsm[p]; l *= ws; g *= ws; }
+            lsum += l;
+            dl = g * inv_nb;
           }
           dz[p] = dl;
         }
@@ -774,6 +785,7 @@ struct FitCArgs {
   int any_l2;
   float *loss_out;
   float lr, beta1, beta2, eps;
+  FitWeights fw;
 };
 
 __device__ __forceinline__ uint32_t cluster_rank() {
@@ -868,6 +880,7 @@ __device__ __forceinline__ float4 f_act_bwd4(int a, float4 acc, float4 h) {
                      acc.w * f_act_bwd(a, h.w));
 }
 
+template <bool WEIGHTED>
 __global__ void __cluster_dims__(FIT_CLUSTER, 1, 1) __launch_bounds__(FIT_CTHREADS)
 fit_cluster_kernel(const FitCArgs a) {
   extern __shared__ __align__(16) float sm[];
@@ -884,8 +897,12 @@ fit_cluster_kernel(const FitCArgs a) {
   const float *X = a.X + (a.shared_data ? 0 : (size_t)cl * a.N * d.dims[0]);
   const float *zg = a.z + (a.shared_data ? 0 : (size_t)cl * a.N);
   const int *perm = a.perm + (a.shared_perm ? 0 : (size_t)cl * a.epochs * a.N);
+  const float *wg = WEIGHTED && a.fw.w ? a.fw.w + (a.shared_data ? 0 : (size_t)cl * a.N) : nullptr;
   int *idxb = reinterpret_cast<int *>(sm + P.idx);
   float *red = sm + P.red;
+  // loss weights of this CTA's samples (weighted fits): delta buffer 1 is dead from the end of one reverse
+  // pass (where the next minibatch is gathered) to the reverse pass of the next step
+  float *wsm = sm + P.dl[1];
   const int D = d.dims[0];
   const int i0 = rank * P.chunk;                       // this CTA's parameter slice
   const int i1 = min(i0 + P.chunk, d.n_params);
@@ -901,7 +918,9 @@ fit_cluster_kernel(const FitCArgs a) {
     for (int p = tid; p < SP; p += NT) {
       const int row = p < mine ? perm[(size_t)ep * a.N + s0 + p0 + p] : -1;
       idxb[p] = row;
-      sm[P.zb + p] = row >= 0 ? zg[row] : 0.f;
+      const float zz = row >= 0 ? zg[row] : 0.f;
+      sm[P.zb + p] = zz;
+      if (WEIGHTED) wsm[p] = row >= 0 ? fit_sample_weight(a.fw, wg, row, zz) : 0.f;
     }
     __syncthreads();
     for (int e = tid; e < SP * D; e += NT) {
@@ -1002,8 +1021,10 @@ fit_cluster_kernel(const FitCArgs a) {
           float dl = 0.f;
           if (p < mine) {
             const float u = U[p], zz = sm[P.zb + p];
-            lsum += fmaxf(u, 0.f) - u * zz + log1pf(expf(-fabsf(u)));
-            dl = (stable_sigmoid(u) - zz) * inv_nb;
+            float l = fmaxf(u, 0.f) - u * zz + log1pf(expf(-fabsf(u))), g = stable_sigmoid(u) - zz;
+            if (WEIGHTED) { const float ws = wsm[p]; l *= ws; g *= ws; }
+            lsum += l;
+            dl = g * inv_nb;
           }
           dz[p] = dl;
         }
@@ -1200,16 +1221,23 @@ fit_cluster_kernel(const FitCArgs a) {
 // ---------------------------------------------------------------- evaluate (loss, accuracy)
 __global__ void __launch_bounds__(256)
 evaluate_kernel(const MlpDesc d, const float *__restrict__ params, const float *__restrict__ logits,
-                const float *__restrict__ z, int N, const float *__restrict__ l2vec, float *out2) {
+                const float *__restrict__ z, int N, const float *__restrict__ l2vec, const FitWeights fw,
+                float *out2) {
   // logits: final pre-activation computed by K0 on a copy of the model with a linear head
   __shared__ float red[32];
-  float ls = 0.f, acc = 0.f, reg = 0.f;
+  float ls = 0.f, acc = 0.f, reg = 0.f, wsum = 0.f;
   const int act_last = d.act[d.n_layers - 1];
   for (int i = threadIdx.x; i < N; i += blockDim.x) {
     const float u = logits[i], zz = z[i];
-    ls += fmaxf(u, 0.f) - u * zz + log1pf(expf(-fabsf(u)));
+    float l = fmaxf(u, 0.f) - u * zz + log1pf(expf(-fabsf(u)));
     const float outv = act_last == BORE_ACT_SIGMOID ? stable_sigmoid(u) : u;
-    acc += ((outv > 0.5f ? 1.f : 0.f) == zz) ? 1.f : 0.f;  // Keras quirk: thresholds the OUTPUT
+    float hit = ((outv > 0.5f ? 1.f : 0.f) == zz) ? 1.f : 0.f;  // Keras quirk: thresholds the OUTPUT
+    if (fw.on) {
+      const float ws = fit_sample_weight(fw, fw.w, i, zz);
+      l *= ws; hit *= ws; wsum += ws;
+    }
+    ls += l;
+    acc += hit;
   }
   if (l2vec)  // l2vec[2l] = kernel factor, l2vec[2l+1] = bias factor of layer l
     for (int l = 0; l < d.n_layers; ++l) {
@@ -1220,9 +1248,11 @@ evaluate_kernel(const MlpDesc d, const float *__restrict__ params, const float *
   ls = block_sum(ls, red);
   acc = block_sum(acc, red);
   reg = block_sum(reg, red);
+  if (fw.on) wsum = block_sum(wsum, red);
   if (threadIdx.x == 0) {
     out2[0] = ls / (float)N + reg;
-    out2[1] = acc / (float)N;
+    // weighted accuracy: Keras' Mean metric, sum(w hit) / sum(w), 0 when sum(w) = 0 (div_no_nan)
+    out2[1] = fw.on ? (wsum != 0.f ? acc / wsum : 0.f) : acc / (float)N;
   }
 }
 
@@ -1259,12 +1289,11 @@ int fit_check_envelope(const MlpDesc &d) {
   return 0;
 }
 
-extern "C" {
-
-int bore_mlp_fit(bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
-                 int shared_data, int batch_size, int epochs, const int32_t *perm_dev,
-                 int shared_perm, float *loss_out_dev, void *stream) {
-  BORE_NVTX("bore:fit (K1)");
+// bore_mlp_fit and bore_mlp_fit_weighted: the same checks and the same choice of kernel; fw.on == 0 runs
+// every kernel with its unweighted arithmetic
+static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
+                   int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
+                   float *loss_out_dev, const FitWeights &fw, void *stream) {
   BORE_CHECK(h != nullptr, "NULL handle");
   BORE_CHECK(model0 >= 0 && count >= 1 && model0 + count <= h->n_models,
              "bore_mlp_fit: models [%d,%d) outside [0,%d)", model0, model0 + count, h->n_models);
@@ -1291,6 +1320,7 @@ int bore_mlp_fit(bore_mlp *h, int model0, int count, const float *X_dev, const f
   }
   a.loss_out = loss_out_dev;
   a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
+  a.fw = fw;
   // Tensor-pipe kernel (fit_mma.cu: 3xTF32 mma.sync GEMMs, one CTA per model) on request only (fit mode 3 or
   // BORE_FIT_MMA=1): measured SLOWER than both FFMA mappings below on B200 -- the legacy HMMA path gives
   // 3xTF32 only 1.3x the FFMA peak and every HMMA needs ~14 more instructions for fragments and splits
@@ -1303,7 +1333,7 @@ int bore_mlp_fit(bore_mlp *h, int model0, int count, const float *X_dev, const f
     }
     if (h->fit_mode == 3 || (h->fit_mode == 0 && mma_env)) {
       const int rc = launch_fit_mma(h, model0, count, X_dev, z_dev, N, shared_data, batch_size, epochs, perm_dev,
-                                    shared_perm, loss_out_dev, (cudaStream_t)stream);
+                                    shared_perm, loss_out_dev, fw, (cudaStream_t)stream);
       if (rc != 0) return rc < 0 ? rc : 0;
       BORE_CHECK(h->fit_mode != 3, "bore_mlp_fit: the tensor-pipe kernel does not take this net / batch size");
     }
@@ -1320,7 +1350,7 @@ int bore_mlp_fit(bore_mlp *h, int model0, int count, const float *X_dev, const f
     }
     if (h->fit_mode == 4 || (h->fit_mode == 0 && unit_env && count * FIT_CLUSTER <= h->sm_count)) {
       const int rc = launch_fit_unit(h, model0, count, X_dev, z_dev, N, shared_data, batch_size, epochs, perm_dev,
-                                     shared_perm, loss_out_dev, (cudaStream_t)stream);
+                                     shared_perm, loss_out_dev, fw, (cudaStream_t)stream);
       if (rc != 0) return rc < 0 ? rc : 0;
       BORE_CHECK(h->fit_mode != 4, "bore_mlp_fit: the unit-split cluster kernel does not take this net / batch size");
     }
@@ -1340,9 +1370,10 @@ int bore_mlp_fit(bore_mlp *h, int model0, int count, const float *X_dev, const f
       for (int l = 0; l < BORE_MAX_LAYERS; ++l) { c.l2k[l] = a.l2k[l]; c.l2b[l] = a.l2b[l]; }
       c.any_l2 = a.any_l2; c.loss_out = a.loss_out;
       c.lr = a.lr; c.beta1 = a.beta1; c.beta2 = a.beta2; c.eps = a.eps;
-      BORE_CUDA(cudaFuncSetAttribute(fit_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     (int)csmem));
-      fit_cluster_kernel<<<count * FIT_CLUSTER, FIT_CTHREADS, csmem, (cudaStream_t)stream>>>(c);
+      c.fw = a.fw;
+      const auto kern = a.fw.on ? fit_cluster_kernel<true> : fit_cluster_kernel<false>;
+      BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csmem));
+      kern<<<count * FIT_CLUSTER, FIT_CTHREADS, csmem, (cudaStream_t)stream>>>(c);
       BORE_CUDA(cudaGetLastError());
       return 0;
     }
@@ -1370,21 +1401,23 @@ int bore_mlp_fit(bore_mlp *h, int model0, int count, const float *X_dev, const f
     smem = fit_onecta_plan(a.d, B, threads, narrow, a.P);
   }
   BORE_CHECK(smem <= FIT_MAX_SMEM, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
-  BORE_CUDA(cudaFuncSetAttribute(fit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  fit_kernel<<<count, threads, smem, (cudaStream_t)stream>>>(a);
+  const auto kern = a.fw.on ? fit_kernel<true> : fit_kernel<false>;
+  BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<count, threads, smem, (cudaStream_t)stream>>>(a);
   BORE_CUDA(cudaGetLastError());
   return 0;
 }
 
-int bore_mlp_set_fit_mode(bore_mlp *h, int mode) {
-  BORE_CHECK(h != nullptr, "NULL handle");
-  BORE_CHECK(mode >= 0 && mode <= 4, "bore_mlp_set_fit_mode: mode %d outside [0,4]", mode);
-  h->fit_mode = mode;
-  return 0;
+// sample weights w (may be NULL) and class weights (cw0, cw1) -> the kernels' FitWeights; all ones is unweighted
+static FitWeights fit_weights(const float *w, float cw0, float cw1) {
+  FitWeights fw;
+  fw.w = w; fw.cw0 = cw0; fw.cw1 = cw1;
+  fw.on = w != nullptr || cw0 != 1.f || cw1 != 1.f;
+  return fw;
 }
 
-int bore_mlp_evaluate(bore_mlp *h, int model, const float *X_dev, const float *z_dev, int N,
-                      float *out_host, void *stream_) {
+static int evaluate_run(bore_mlp *h, int model, const float *X_dev, const float *z_dev, int N,
+                        const FitWeights &fw, float *out_host, void *stream_) {
   BORE_CHECK(h != nullptr, "NULL handle");
   BORE_CHECK(model >= 0 && model < h->n_models, "model index %d outside [0,%d)", model, h->n_models);
   BORE_CHECK(N >= 1 && X_dev && z_dev && out_host, "bore_mlp_evaluate: bad arguments");
@@ -1409,7 +1442,7 @@ int bore_mlp_evaluate(bore_mlp *h, int model, const float *X_dev, const float *z
                            nullptr, nullptr, stream);
   if (!rc) {
     evaluate_kernel<<<1, 256, 0, stream>>>(h->desc, h->params + (size_t)model * h->desc.n_params,
-                                           logits, z_dev, N, any ? l2dev : nullptr, out2);
+                                           logits, z_dev, N, any ? l2dev : nullptr, fw, out2);
     cudaMemcpyAsync(out_host, out2, 2 * sizeof(float), cudaMemcpyDeviceToHost, stream);
     cudaError_t e = cudaStreamSynchronize(stream);
     if (e != cudaSuccess) { bore_set_error("bore_mlp_evaluate: %s", cudaGetErrorString(e)); rc = -2; }
@@ -1417,6 +1450,44 @@ int bore_mlp_evaluate(bore_mlp *h, int model, const float *X_dev, const float *z
   cudaFree(logits);
   cudaFree(out2);
   return rc;
+}
+
+extern "C" {
+
+int bore_mlp_fit(bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
+                 int shared_data, int batch_size, int epochs, const int32_t *perm_dev,
+                 int shared_perm, float *loss_out_dev, void *stream) {
+  BORE_NVTX("bore:fit (K1)");
+  return fit_run(h, model0, count, X_dev, z_dev, N, shared_data, batch_size, epochs, perm_dev, shared_perm,
+                 loss_out_dev, fit_weights(nullptr, 1.f, 1.f), stream);
+}
+
+int bore_mlp_fit_weighted(bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev,
+                          const float *w_dev, int N, int shared_data, float class_weight0,
+                          float class_weight1, int batch_size, int epochs, const int32_t *perm_dev,
+                          int shared_perm, float *loss_out_dev, void *stream) {
+  BORE_NVTX("bore:fit weighted (K1)");
+  return fit_run(h, model0, count, X_dev, z_dev, N, shared_data, batch_size, epochs, perm_dev, shared_perm,
+                 loss_out_dev, fit_weights(w_dev, class_weight0, class_weight1), stream);
+}
+
+int bore_mlp_set_fit_mode(bore_mlp *h, int mode) {
+  BORE_CHECK(h != nullptr, "NULL handle");
+  BORE_CHECK(mode >= 0 && mode <= 4, "bore_mlp_set_fit_mode: mode %d outside [0,4]", mode);
+  h->fit_mode = mode;
+  return 0;
+}
+
+int bore_mlp_evaluate(bore_mlp *h, int model, const float *X_dev, const float *z_dev, int N,
+                      float *out_host, void *stream) {
+  return evaluate_run(h, model, X_dev, z_dev, N, fit_weights(nullptr, 1.f, 1.f), out_host, stream);
+}
+
+int bore_mlp_evaluate_weighted(bore_mlp *h, int model, const float *X_dev, const float *z_dev,
+                               const float *w_dev, float class_weight0, float class_weight1, int N,
+                               float *out_host, void *stream) {
+  return evaluate_run(h, model, X_dev, z_dev, N, fit_weights(w_dev, class_weight0, class_weight1), out_host,
+                      stream);
 }
 
 }  // extern "C"

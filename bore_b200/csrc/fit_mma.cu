@@ -136,6 +136,7 @@ struct FitMArgs {
   int any_l2;
   float *loss_out;
   float lr, beta1, beta2, eps;
+  FitWeights fw;
 };
 
 // ------------------------------------------------------------------------------------ mma plumbing
@@ -300,6 +301,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
   const float *X = a.X + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N * d.dims[0]);
   const float *zg = a.z + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N);
   const int *perm = a.perm + (a.shared_perm ? 0 : (size_t)blockIdx.x * a.epochs * a.N);
+  const float *wg = a.fw.w ? a.fw.w + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N) : nullptr;
   const int D = d.dims[0], lda = P.lda, ldx = P.ldx;
   float *red = sm + P.red;
 
@@ -359,6 +361,12 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
       const int row = idx[tid];
       if (row >= 0) cp_async4(sm + P.zb[buf] + tid, zg + row);
       else sm[P.zb[buf] + tid] = 0.f;
+      // sample weights into dL/dlogit's slot: dead from the end of the output-layer phase (this is issued
+      // after it) to the next loss, which reads a sample's weight before it writes its dL/dlogit there
+      if (wg) {
+        if (row >= 0) cp_async4(sm + P.du + tid, wg + row);
+        else sm[P.du + tid] = 0.f;
+      }
     }
     cp_async_commit();
   };
@@ -441,6 +449,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
       const int in = P.kp[LH];
       float lsum = 0.f;
       for (int r = warp; r < BP; r += NW) {
+        const float wr = wg ? sm[P.du + r] : 1.f;  // (read before the shuffles, written after them)
         float u = 0.f;
         for (int k = lane; k < in; k += 32) u = fmaf(H[r * lda + k], w[k], u);
 #pragma unroll
@@ -449,8 +458,13 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         float dl = 0.f;
         if (r < nb) {
           const float zz = sm[P.zb[cur] + r];
-          lsum += fmaxf(u, 0.f) - u * zz + log1pf(expf(-fabsf(u)));
-          dl = (stable_sigmoid(u) - zz) * inv_nb;
+          float l = fmaxf(u, 0.f) - u * zz + log1pf(expf(-fabsf(u))), g = stable_sigmoid(u) - zz;
+          if (a.fw.on) {
+            const float ws = wr * (zz != 0.f ? a.fw.cw1 : a.fw.cw0);
+            l *= ws; g *= ws;
+          }
+          lsum += l;
+          dl = g * inv_nb;
         }
         if (lane == 0) sm[P.du + r] = dl;
       }
@@ -670,7 +684,7 @@ int launch_nw(const FitMArgs &a, int count, size_t smem, cudaStream_t stream) {
 // 1: launched; 0: shape not taken by the tensor kernel (caller falls back); < 0: error
 int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                    int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                   float *loss_out_dev, cudaStream_t stream) {
+                   float *loss_out_dev, const FitWeights &fw, cudaStream_t stream) {
   const int B = batch_size < N ? batch_size : N;
   // few models: one 16-warp CTA per model (latency); many: 4-warp CTAs, several per SM (throughput)
   int nw = count * 2 <= h->sm_count ? 16 : (count <= 2 * h->sm_count ? 8 : 4);
@@ -703,6 +717,7 @@ int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev,
   }
   a.loss_out = loss_out_dev;
   a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
+  a.fw = fw;
   int rc;
   if (nw == 16) rc = launch_nw<16>(a, count, smem, stream);
   else if (nw == 8) rc = launch_nw<8>(a, count, smem, stream);

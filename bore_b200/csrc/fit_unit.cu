@@ -94,6 +94,7 @@ struct FuPlan {
   int scratch, wstride;             // [FU_KS][wstride = umax * SP]
   int lg;                           // logit partials [FU_THREADS / SP][SP]
   int dz, zb, idx;                  // dL/dlogit [SP]; labels [2][SP]; row indices of the next step [SP] (ints)
+  int wb;                           // sample weights of a weighted fit [SP]
   int slots;                        // lsum[2][2], reg[2]
   int bars;                         // mbarriers (8 bytes each): h_i at 2 (i - 1) + buffer, delta_i at 2 L + i
   int total;
@@ -134,7 +135,9 @@ __host__ __device__ inline bool make_fu_plan(const MlpDesc &d, int batch, FuPlan
   p.lg = off; off += (FU_THREADS / p.SP) * p.SP;
   p.dz = off; off += p.SP;
   p.zb = off; off += 2 * p.SP;
-  p.idx = off; off += 2 * p.SP;
+  p.idx = off; off += p.SP;
+  // one buffer: the loss reads it before the barrier after which the next step's weights are requested
+  p.wb = off; off += p.SP;
   p.slots = off; off += 8;
   off = fu_r2(off);  // mbarriers are 8 bytes
   p.bars = off; off += 2 * FU_NBAR;
@@ -156,6 +159,7 @@ struct FuArgs {
   int any_l2;
   float *loss_out;
   float lr, beta1, beta2, eps;
+  FitWeights fw;
 };
 
 // ---------------------------------------------------------------- cluster / packed-FMA primitives
@@ -360,7 +364,8 @@ __device__ __forceinline__ float fu_row_sum(const float *__restrict__ a, int SP)
 
 // NH > 0: the net has NH hidden layers of HW units each (HW a multiple of 16) and the padded batch is SPT --
 // compile-time shape, D stays a run-time value; NH == 0: everything from the descriptor and the plan.
-template <int NH, int HW, int SPT>
+// WT: per-sample loss weights (FuArgs::fw); the unweighted build runs none of their code.
+template <int NH, int HW, int SPT, bool WT>
 __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_unit_kernel(const FuArgs a) {
   extern __shared__ __align__(16) float sm[];
   constexpr bool FIX = NH > 0;
@@ -383,6 +388,7 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
   const float *X = a.X + (a.shared_data ? 0 : (size_t)cl * a.N * D);
   const float *zg = a.z + (a.shared_data ? 0 : (size_t)cl * a.N);
   const int *perm = a.perm + (a.shared_perm ? 0 : (size_t)cl * a.epochs * a.N);
+  const float *wg = WT && a.fw.w ? a.fw.w + (a.shared_data ? 0 : (size_t)cl * a.N) : nullptr;
   const int steps_per_epoch = (a.N + a.batch - 1) / a.batch;
   float *W = sm + P.par0, *Mm = W + P.npar, *Vv = Mm + P.npar, *Gg = Vv + P.npar;
   const int wstride = FIX ? (HW / FU_C) * SPT : P.wstride;  // floats per warp of the scratch
@@ -469,7 +475,10 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
       const int row = idxs[p];
       const float *xr = X + (size_t)max(row, 0) * D;
       for (int k = lane; k < D; k += 32) cp4(H0 + k * SPP + p, xr + k, row >= 0);
-      if (lane == 0) cp4(sm + P.zb + buf * SP + p, zg + max(row, 0), row >= 0);
+      if (lane == 0) {
+        cp4(sm + P.zb + buf * SP + p, zg + max(row, 0), row >= 0);
+        if (wg) cp4(sm + P.wb + p, wg + max(row, 0), row >= 0);
+      }
     }
   };
   auto gather_wait = [&]() { asm volatile("cp.async.wait_all;" ::: "memory"); };
@@ -572,8 +581,13 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
           for (int kp = 0; kp < NLG; ++kp) u += sm[P.lg + kp * SP + tid];
           if (tid < nb) {
             const float zz = sm[P.zb + par * SP + tid];
+            float g = stable_sigmoid(u) - zz;
             lt = fmaxf(u, 0.f) - u * zz + log1pf(expf(-fabsf(u)));
-            dl = (stable_sigmoid(u) - zz) * inv_nb;
+            if (WT) {
+              const float ws = (wg ? sm[P.wb + tid] : 1.f) * (zz != 0.f ? a.fw.cw1 : a.fw.cw0);
+              lt *= ws; g *= ws;
+            }
+            dl = g * inv_nb;
           }
           sm[P.dz + tid] = dl;
         }
@@ -854,8 +868,9 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
 
 template <int NH, int HW, int SPT>
 static int fu_launch(const FuArgs &a, int count, size_t smem, cudaStream_t stream) {
-  BORE_CUDA(cudaFuncSetAttribute(fit_unit_kernel<NH, HW, SPT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  fit_unit_kernel<NH, HW, SPT><<<count * FU_C, FU_THREADS, smem, stream>>>(a);
+  const auto kern = a.fw.on ? fit_unit_kernel<NH, HW, SPT, true> : fit_unit_kernel<NH, HW, SPT, false>;
+  BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<count * FU_C, FU_THREADS, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());
   return 1;
 }
@@ -873,7 +888,7 @@ static bool fu_plan(const MlpDesc &d, int batch, FuPlan &p, size_t &smem) {
 // 1 launched, 0 shape not taken (the caller falls back to the sample-split cluster kernel), < 0 error
 int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                     int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                    float *loss_out_dev, cudaStream_t stream) {
+                    float *loss_out_dev, const FitWeights &fw, cudaStream_t stream) {
   FuArgs a;
   a.d = h->desc;
   const int B = batch_size < N ? batch_size : N;
@@ -900,6 +915,7 @@ int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev
   }
   a.loss_out = loss_out_dev;
   a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
+  a.fw = fw;
   if (fixed_shape) {
     if (nh == 3 && hw == 64) return fu_launch<3, 64, 64>(a, count, smem, stream);
     if (nh == 3 && hw == 32) return fu_launch<3, 32, 64>(a, count, smem, stream);

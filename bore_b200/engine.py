@@ -463,28 +463,42 @@ class NativeMLP:
 
     # ------------------------------------------------------------------ K1
     def fit_dev(self, X_dev, z_dev, N, batch_size, epochs, perm_dev, loss_dev=None,
-                model0=0, count=1, shared_data=True, shared_perm=True):
+                model0=0, count=1, shared_data=True, shared_perm=True, w_dev=None, class_weight=None):
+        """``w_dev`` (float32, the layout of ``z_dev``) and ``class_weight`` ((weight of label 0,
+        weight of label 1)) weight each sample's loss (bore_mlp_fit_weighted); without them this
+        is bore_mlp_fit."""
         torch = _torch()
         assert X_dev.dtype == torch.float32 and z_dev.dtype == torch.float32
         assert perm_dev.dtype == torch.int32 and perm_dev.is_contiguous()
         if loss_dev is None:
             loss_dev = torch.empty(count, epochs, dtype=torch.float32, device=self._tdev())
-        _lib.check(self.lib.bore_mlp_fit(self.h, model0, count, _ptr(X_dev), _ptr(z_dev), int(N),
-                                         1 if shared_data else 0, int(batch_size), int(epochs),
-                                         _ptr(perm_dev), 1 if shared_perm else 0,
-                                         _ptr(loss_dev), self._stream()))
+        if w_dev is None and class_weight is None:
+            _lib.check(self.lib.bore_mlp_fit(self.h, model0, count, _ptr(X_dev), _ptr(z_dev), int(N),
+                                             1 if shared_data else 0, int(batch_size), int(epochs),
+                                             _ptr(perm_dev), 1 if shared_perm else 0,
+                                             _ptr(loss_dev), self._stream()))
+            return loss_dev
+        assert w_dev is None or (w_dev.dtype == torch.float32 and w_dev.is_contiguous()
+                                 and w_dev.numel() == z_dev.numel())
+        cw0, cw1 = (1.0, 1.0) if class_weight is None else class_weight
+        _lib.check(self.lib.bore_mlp_fit_weighted(self.h, model0, count, _ptr(X_dev), _ptr(z_dev), _ptr(w_dev),
+                                                  int(N), 1 if shared_data else 0, float(cw0), float(cw1),
+                                                  int(batch_size), int(epochs), _ptr(perm_dev),
+                                                  1 if shared_perm else 0, _ptr(loss_dev), self._stream()))
         return loss_dev
 
-    def fit(self, X, z, epochs, batch_size, permutations, l2=None, model=0):
-        """Keras ``fit`` with explicit per-epoch permutations -> history loss (epochs,)."""
+    def fit(self, X, z, epochs, batch_size, permutations, l2=None, model=0, w=None, class_weight=None):
+        """Keras ``fit`` with explicit per-epoch permutations -> history loss (epochs,).
+        ``w`` (N,) sample weights and ``class_weight`` (cw0, cw1) as in ``fit_dev``."""
         if l2 is not None:
             self.set_regularizers(l2)
         X = np.asarray(X)
         N = X.shape[0]
         perm = np.ascontiguousarray(permutations, np.int32).reshape(epochs, N)
-        return self.fit_async(X, z, epochs, batch_size, perm, model=model).cpu().numpy()[0]
+        return self.fit_async(X, z, epochs, batch_size, perm, model=model, w=w,
+                              class_weight=class_weight).cpu().numpy()[0]
 
-    def fit_async(self, X, z, epochs, batch_size, permutations, l2=None, model=0):
+    def fit_async(self, X, z, epochs, batch_size, permutations, l2=None, model=0, w=None, class_weight=None):
         """Like ``fit`` but returns the (1, epochs) device tensor of epoch losses without waiting
         for the training kernel: the host is free (e.g. to draw the start points of the next
         argmax) while the GPU trains."""
@@ -493,20 +507,31 @@ class NativeMLP:
         X = np.asarray(X)
         N = X.shape[0]
         perm = np.ascontiguousarray(permutations, np.int32).reshape(epochs, N)
+        w_dev = None if w is None else self.to_device(np.asarray(w, np.float32).reshape(N), np.float32)
         return self.fit_dev(self.to_device(X, np.float32),
                             self.to_device(np.asarray(z).astype(np.float32), np.float32),
                             N, batch_size, epochs, self.to_device(perm, np.int32),
-                            model0=model, count=1)
+                            model0=model, count=1, w_dev=w_dev, class_weight=class_weight)
 
-    def evaluate(self, X, z, l2=None, model=0):
+    def evaluate(self, X, z, l2=None, model=0, w=None, class_weight=None):
+        """Keras ``evaluate`` -> [loss, accuracy]; ``w`` / ``class_weight`` weight the loss and the
+        accuracy (bore_mlp_evaluate_weighted)."""
         if l2 is not None:
             self.set_regularizers(l2)
         X = np.asarray(X)
+        N = X.shape[0]
         out = np.zeros(2, np.float32)
         Xd = self.to_device(X, np.float32)
         zd = self.to_device(np.asarray(z).astype(np.float32), np.float32)
-        _lib.check(self.lib.bore_mlp_evaluate(self.h, model, _ptr(Xd), _ptr(zd), X.shape[0],
-                                              _np_ptr(out), self._stream()))
+        if w is None and class_weight is None:
+            _lib.check(self.lib.bore_mlp_evaluate(self.h, model, _ptr(Xd), _ptr(zd), N,
+                                                  _np_ptr(out), self._stream()))
+        else:
+            wd = None if w is None else self.to_device(np.asarray(w, np.float32).reshape(N), np.float32)
+            cw0, cw1 = (1.0, 1.0) if class_weight is None else class_weight
+            _lib.check(self.lib.bore_mlp_evaluate_weighted(self.h, model, _ptr(Xd), _ptr(zd), _ptr(wd),
+                                                           float(cw0), float(cw1), N, _np_ptr(out),
+                                                           self._stream()))
         return [float(out[0]), float(out[1])]
 
 

@@ -16,6 +16,40 @@ from .layers import Dense, BinaryCrossentropy, Adam
 from .mixins import MaximizableMixin, BatchMaximizableMixin
 
 
+def check_class_weight(class_weight):
+    """Keras' check of ``class_weight`` (data_adapter._make_class_weight_map_fn): the keys must be
+    exactly the classes 0 .. K-1.  Returns {class: weight}."""
+    keys = sorted(class_weight)
+    if keys != list(range(len(keys))):
+        raise ValueError(f"Expected `class_weight` to be a dict with keys from 0 to one less than the "
+                         f"number of classes, found {class_weight}")
+    return {int(k): float(v) for k, v in class_weight.items()}
+
+
+def check_sample_weight(sample_weight, n):
+    """``sample_weight`` of n samples, shape (n,) or (n, 1) -> float32 (n,); values pass unchecked."""
+    w = np.asarray(sample_weight, np.float32)
+    if w.shape not in ((n,), (n, 1)):
+        raise ValueError(f"sample_weight must have shape ({n},) or ({n}, 1), got {w.shape}")
+    return np.ascontiguousarray(w.reshape(n))
+
+
+def sample_weights(z, sample_weight=None, class_weight=None):
+    """Keras' weight of every sample of labels ``z`` (N,): ``sample_weight`` times the class weight of
+    the sample's class int(z_i); None when neither is given.  A class without a key raises."""
+    n = len(z)
+    w = None if sample_weight is None else check_sample_weight(sample_weight, n)
+    if class_weight is not None:
+        cw = check_class_weight(class_weight)
+        cls = np.asarray(z).reshape(n).astype(np.int64)
+        missing = sorted(set(np.unique(cls).tolist()) - set(cw))
+        if missing:
+            raise ValueError(f"class_weight has no weight for the classes {missing} of the labels")
+        by_class = np.array([cw[c] for c in range(len(cw))], np.float32)[cls]
+        w = by_class if w is None else w * by_class
+    return w
+
+
 class History:
     """``history["loss"]`` like Keras' History.  ``loss`` may be a zero-argument callable: the
     training kernel is launched asynchronously and the epoch losses are fetched from the device
@@ -160,9 +194,12 @@ class Sequential:
 
     # ------------------------------------------------------------------ training / inference
     def fit(self, x, y, batch_size=None, epochs=1, verbose=1, callbacks=None, shuffle=True,
-            permutations=None, **kwargs):
+            permutations=None, sample_weight=None, class_weight=None, **kwargs):
         """Minibatch Adam on binary cross-entropy, the whole run in one kernel launch.
         Returns a ``History`` with ``history["loss"]`` (Keras' sample-weighted epoch means).
+
+        ``sample_weight`` (N,) or (N, 1) and ``class_weight`` {0: w0, 1: w1} weight each sample's
+        loss as Keras does: a minibatch's loss is sum(w_i bce_i) / batch size.
 
         ``permutations`` (epochs, N): explicit per-epoch shuffles (build extension for parity);
         otherwise drawn from the model's RandomState when ``shuffle`` else the identity."""
@@ -176,6 +213,7 @@ class Sequential:
         z = np.asarray(y).reshape(-1)
         N = X.shape[0]
         assert z.shape[0] == N, "x and y sizes do not match"
+        w = sample_weights(z, sample_weight, class_weight)
         batch_size = 32 if batch_size is None else int(batch_size)
         epochs = int(epochs)
         net = self._engine(X.shape[1])
@@ -186,7 +224,7 @@ class Sequential:
                 permutations = np.stack([self._rs.permutation(N) for _ in range(epochs)])
             else:
                 permutations = np.tile(np.arange(N), (epochs, 1))
-        loss_dev = net.fit_async(X, z, epochs, batch_size, permutations, l2=self._l2())
+        loss_dev = net.fit_async(X, z, epochs, batch_size, permutations, l2=self._l2(), w=w)
         hist = History(lambda: loss_dev.cpu().numpy()[0], epochs)
         if verbose:
             loss = hist.history["loss"]
@@ -198,11 +236,15 @@ class Sequential:
         X = np.asarray(x)
         return self._engine(X.shape[1]).predict(X)
 
-    def evaluate(self, x, y, verbose=0, **kwargs):
+    def evaluate(self, x, y, verbose=0, sample_weight=None, **kwargs):
+        """[loss, accuracy] (or the loss alone without metrics); ``sample_weight`` (N,) or (N, 1):
+        loss sum(w_i bce_i) / N, accuracy sum(w_i hit_i) / sum(w_i) (0 when the weights sum to 0)."""
         if self._compiled is None:
             raise RuntimeError("You must compile your model before training/testing.")
         X = np.asarray(x)
-        out = self._engine(X.shape[1]).evaluate(X, np.asarray(y).reshape(-1), l2=self._l2())
+        z = np.asarray(y).reshape(-1)
+        w = sample_weights(z, sample_weight)
+        out = self._engine(X.shape[1]).evaluate(X, z, l2=self._l2(), w=w)
         return out if self._compiled["metrics"] else out[0]
 
     def __call__(self, x):

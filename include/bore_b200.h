@@ -137,6 +137,29 @@ int bore_mlp_set_fit_mode(bore_mlp *h, int mode);
 int bore_mlp_evaluate(bore_mlp *h, int model, const float *X_dev, const float *z_dev,
                       int N, float *out_host, void *stream);
 
+/* ---- K1, weighted: Keras fit(..., sample_weight=w, class_weight={0: cw0, 1: cw1}) ------------
+ * bore_mlp_fit with a loss weight per sample: sample i of a minibatch of nb weighs
+ * w_i * cw[z_i] (w_i = 1 when w_dev is NULL; z_i is its 0/1 label, so the class weights also
+ * apply to labels made on the device), and the minibatch loss is sum_i w_i cw[z_i] bce_i / nb
+ * (+ the l2 terms): Keras' SUM_OVER_BATCH_SIZE, divided by the sample count, not by the weights.
+ * history["loss"] keeps its form (the epoch mean weighs each minibatch by its sample count).
+ *   w_dev: the layout of z_dev, [count][N] or one shared [N] when `shared_data != 0`; any
+ *     values (zeros and negatives pass through, as in Keras).
+ * Same kernels, fit modes, environment overrides and refusals as bore_mlp_fit.  With w_dev NULL
+ * and class weights (1, 1) it is bore_mlp_fit; an all-ones w_dev gives the same bits too.    */
+int bore_mlp_fit_weighted(bore_mlp *h, int model0, int count, const float *X_dev,
+                          const float *z_dev, const float *w_dev, int N, int shared_data,
+                          float class_weight0, float class_weight1, int batch_size, int epochs,
+                          const int32_t *perm_dev, int shared_perm, float *loss_out_dev,
+                          void *stream);
+
+/* Keras evaluate(..., sample_weight=w) with class weights as in bore_mlp_fit_weighted:
+ * out_host[0] = sum_i w_i cw[z_i] bce_i / N (+ l2), out_host[1] = sum_i w_i cw[z_i] [correct_i] /
+ * sum_i w_i cw[z_i], 0 when the weights sum to 0.  w_dev [N] may be NULL.  synchronous.     */
+int bore_mlp_evaluate_weighted(bore_mlp *h, int model, const float *X_dev, const float *z_dev,
+                               const float *w_dev, float class_weight0, float class_weight1,
+                               int N, float *out_host, void *stream);
+
 /* ---- K3: batched bound-constrained L-BFGS-B -------------------------------------------
  * Replaces the per-start scipy.optimize.minimize(fun, x0, method="L-BFGS-B", jac=True,
  * bounds=..., options=dict(maxiter, ftol)) loop of bore/mixins.py:57-61 (also
