@@ -43,6 +43,8 @@ SIGNATURES = {
                                         C.c_float, C.c_int, C.c_int, vp, C.c_int, vp, vp]),
     "bore_mlp_evaluate_weighted": (C.c_int, [vp, C.c_int, vp, vp, vp, C.c_float, C.c_float, C.c_int,
                                              vp, vp]),
+    "bore_mlp_fit_ragged": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, vp, vp, vp, C.c_float, C.c_float, C.c_int,
+                                      vp, vp, vp]),
     "bore_mlp_set_regularizers": (C.c_int, [vp, vp, vp]),
     "bore_lbfgsb_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "bore_lbfgsb_minimize_workspace_bytes": (C.c_size_t, [vp, C.c_int, C.c_int]),
@@ -72,6 +74,9 @@ SIGNATURES = {
     "bore_quantile_labels": (C.c_int, [vp, C.c_int, C.c_int, C.c_double, vp, vp, vp, C.c_int, vp]),
     "bore_is_duplicate": (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.c_double, C.c_double,
                                     vp, vp, C.c_int, vp]),
+    "bore_quantile_labels_ragged": (C.c_int, [vp, C.c_int, vp, C.c_double, vp, vp, vp, C.c_int, vp]),
+    "bore_is_duplicate_ragged": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, C.c_int, C.c_double, C.c_double,
+                                           vp, vp, C.c_int, vp]),
     "bore_truncnorm_distort": (C.c_int, [vp, C.c_int, C.c_int, C.c_double, vp, vp, vp, vp, C.c_int, vp]),
     "bore_svgd_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "bore_svgd_maximize": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, vp, C.c_double, C.c_int,

@@ -18,6 +18,7 @@ from .engine import NativeMLP, lbfgsb_message
 from .layers import Dense, BinaryCrossentropy, Adam
 from .models import check_class_weight, sample_weights
 from .optimizers.utils import from_bounds
+from .ragged import ragged_inputs, ragged_rows
 
 
 def problem_shard(n_problems, rank, world):
@@ -32,15 +33,31 @@ class LazyLoss:
     stage the next ``argmax``'s screening samples while the GPU trains (the single-model
     ``History`` of ``models.py`` does the same).  Behaves like the ndarray it wraps."""
 
-    def __init__(self, loss_dev):
-        self._dev, self._host = loss_dev, None
-        self.shape = tuple(loss_dev.shape)
+    def __init__(self, loss_dev, layout=None):
+        self._dev, self._host, self._layout = loss_dev, None, layout
+        if layout is None:
+            self.shape = tuple(loss_dev.shape)
+        else:  # ragged problems: the losses come concatenated, problem p has layout.epochs[p] of them
+            self.shape = (len(layout), int(layout.epochs.max()))
+            self.epochs = layout.epochs.copy()
 
     def numpy(self):
         if self._host is None:
             self._host = self._dev.cpu().numpy()
+            if self._layout is not None:
+                self._host = self._layout.pad_loss(self._host)
             self._dev = None
         return self._host
+
+    def first_last(self):
+        """Every problem's first and last epoch loss (NaN for a problem that did not train)."""
+        a = self.numpy()
+        if a.shape[1] == 0:
+            return np.full(a.shape[0], np.nan), np.full(a.shape[0], np.nan)
+        if self._layout is None:
+            return a[:, 0], a[:, -1]
+        last = np.maximum(self._layout.epochs - 1, 0)
+        return a[:, 0], a[np.arange(a.shape[0]), last]
 
     def __array__(self, dtype=None, copy=None):
         a = self.numpy()
@@ -155,6 +172,11 @@ class BatchedMaximizableSequential:
             gamma=None, sample_weight=None, class_weight=None):
         """x (M, N, D), y (M, N): every problem trains on its own N observations, all in one
         launch.  ``permutations``: (epochs, N) shared by all problems or (M, epochs, N).
+        Ragged problems: ``x`` a list of M arrays (N_p, D) and ``y`` of M arrays (N_p,); then
+        ``epochs`` is an int or M ints (0 leaves a problem untouched), ``sample_weight`` and
+        ``permutations`` are lists of M arrays (N_p,) and (epochs_p, N_p), and the loss has shape
+        (M, max epochs_p), NaN beyond each problem's epochs (``LazyLoss.epochs``).  Per problem the
+        result is that of a fit of the problem alone.
         With ``gamma`` given, ``y`` holds the RAW targets and every problem is labelled
         ``z = y < quantile(y, gamma)`` on the device (bore/data.py:31-35) before training.
         ``sample_weight`` (M, N), or (N,) shared by all problems, and ``class_weight``
@@ -164,24 +186,20 @@ class BatchedMaximizableSequential:
         the launch is asynchronous and the values are fetched on first use)."""
         if not self._compiled:
             raise RuntimeError("You must compile your model before training/testing.")
+        if isinstance(x, (list, tuple)):
+            return self._fit_ragged(x, y, batch_size, epochs, permutations, shuffle, verbose, gamma,
+                                    sample_weight, class_weight)
         X = np.asarray(x)
         z = np.asarray(y)
         M, N, D = X.shape
         assert M == self.n_problems and z.shape == (M, N) and D == self.dims[0]
-        w = cw = None
+        w = None
         if sample_weight is not None:
             sw = np.asarray(sample_weight, np.float32)
             if sw.shape not in ((M, N), (N,)):
                 raise ValueError(f"sample_weight must have shape ({M}, {N}) or ({N},), got {sw.shape}")
             w = np.broadcast_to(sw, (M, N)).reshape(-1)
-        if class_weight is not None:
-            if gamma is None:  # labels known here: Keras' rule, class int(y)
-                w = sample_weights(z.reshape(-1), w, class_weight)
-            else:  # labels 0 / 1 made on the device: both need a weight
-                cwd = check_class_weight(class_weight)
-                if not {0, 1} <= set(cwd):
-                    raise ValueError("class_weight needs weights for the classes 0 and 1 of the labels")
-                cw = (cwd[0], cwd[1])
+        w, cw = self._class_weights(class_weight, gamma, z.reshape(-1), w)
         z_dev = None
         if gamma is not None:
             z_dev = self._net.quantile_labels_dev(
@@ -208,6 +226,41 @@ class BatchedMaximizableSequential:
                   f"{out[:, -1].mean():.4f}")
         return out
 
+    def _class_weights(self, class_weight, gamma, z, w):
+        """(sample weights with Keras' class weights folded in, class weights for labels made on the
+        device): the rule of ``fit`` for host labels ``z`` or, with ``gamma``, device labels."""
+        if class_weight is None:
+            return w, None
+        if gamma is None:  # labels known here: Keras' rule, class int(y)
+            return sample_weights(z, w, class_weight), None
+        cwd = check_class_weight(class_weight)  # labels 0 / 1 made on the device: both need a weight
+        if not {0, 1} <= set(cwd):
+            raise ValueError("class_weight needs weights for the classes 0 and 1 of the labels")
+        return w, (cwd[0], cwd[1])
+
+    def _fit_ragged(self, x, y, batch_size, epochs, permutations, shuffle, verbose, gamma, sample_weight,
+                    class_weight):
+        """``fit`` for lists of per-problem arrays (bore_mlp_fit_ragged): see ``fit``."""
+        M, net = self.n_problems, self._net
+        layout, X, z, w, perm = ragged_inputs(x, y, M, self.dims[0], epochs, sample_weight, permutations,
+                                              self._rs, shuffle)
+        w, cw = self._class_weights(class_weight, gamma, z, w)
+        if gamma is not None:
+            z_dev = net.quantile_labels_ragged_dev(net.to_device(z, np.float64), layout.n, gamma)
+        else:
+            z_dev = net.to_device(z, np.float32)
+        loss = net.fit_ragged_dev(net.to_device(X, np.float32), z_dev, layout, int(batch_size),
+                                  net.to_device(perm, np.int32), model0=0,
+                                  w_dev=None if w is None else net.to_device(w, np.float32), class_weight=cw)
+        out = LazyLoss(loss, layout)
+        if verbose:
+            first, last = out.first_last()
+            trained = layout.epochs > 0
+            msg = (f"mean loss {first[trained].mean():.4f} -> {last[trained].mean():.4f}" if trained.any()
+                   else "nothing trained")
+            print(f"fit: {M} problems x {layout.epochs.min()}..{layout.epochs.max()} epochs, {msg}")
+        return out
+
     def predict(self, x):
         X = np.asarray(x)
         M, P, D = X.shape
@@ -223,7 +276,8 @@ class BatchedMaximizableSequential:
         bore/mixins.py:22-89 for each of them.
         ``random_state`` draws the (M, num_samples, D) screening samples problem after problem
         (what M sequential ``argmax`` calls sharing one RandomState would consume); ``X_init``
-        overrides the draw.  ``exclude`` (M, N, D): each problem's stored observations -- results
+        overrides the draw.  ``exclude`` (M, N, D), or a list of M arrays (n_p, D) with n_p >= 0: each
+        problem's stored observations -- results
         ``np.allclose`` to one of them are dropped before the selection, which is the plugin's
         ``filter_fn=_is_unique`` (bore/plugins/hpbandster/base.py:227-231, bore/data.py:42-48).
         ``distortion``: the plugin's truncated-normal resample of the suggestion
@@ -232,6 +286,8 @@ class BatchedMaximizableSequential:
         screening samples, one row per problem (problems without a winner consume theirs too)."""
         import torch
         assert num_samples >= num_starts > 0
+        if isinstance(exclude, (list, tuple)):  # ragged: checked before anything is drawn or enqueued
+            n_prev, prev = ragged_rows(exclude, self.n_problems, self.dims[0])
         if method != "L-BFGS-B":
             raise NotImplementedError("only L-BFGS-B has a device path")
         (low, high), dim = from_bounds(bounds)
@@ -261,7 +317,10 @@ class BatchedMaximizableSequential:
                                    gtol=opts.get("gtol", 1e-5), maxiter=opts.get("maxiter", 15000),
                                    maxfun=opts.get("maxfun", 15000), maxls=opts.get("maxls", 20))
         keep = None
-        if exclude is not None:
+        if isinstance(exclude, (list, tuple)):  # ragged: problem p stores its own n_p rows
+            keep = net.keep_unique_ragged_dev(res["x"], n_prev, net.to_device(prev, np.float64), rtol=rtol,
+                                              atol=atol)
+        elif exclude is not None:
             prev = np.ascontiguousarray(exclude, np.float64)
             assert prev.ndim == 3 and prev.shape[0] == M and prev.shape[2] == dim
             if prev.shape[1] > 0:

@@ -97,6 +97,11 @@ int bore_mlp_destroy(bore_mlp *h) {
     for (int v = 0; v < 4; ++v) cudaFree(h->pack->buf[v]);
     delete h->pack;
   }
+  if (h->tab_done) {
+    cudaEventSynchronize(h->tab_done);
+    cudaEventDestroy(h->tab_done);
+  }
+  if (h->tab_pinned) cudaFreeHost(h->tab_pinned);
   delete h;
   return 0;
 }

@@ -29,6 +29,13 @@ void bore_set_error(const char *fmt, ...);
     }                                                                            \
   } while (0)
 
+// a call returning 0 or < 0 (error text already set): pass the error on
+#define BORE_CHECK_RC(call)   \
+  do {                        \
+    const int rc__ = (call);  \
+    if (rc__ != 0) return rc__; \
+  } while (0)
+
 // ---------------------------------------------------------------- NVTX ranges (SURVEY.md section 5)
 // Header-only NVTX 3: a no-op unless a tool (nsys, ncu --nvtx) injects itself; no link dependency.
 #include <nvtx3/nvToolsExt.h>
@@ -71,6 +78,9 @@ struct bore_mlp {
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];  // l2 regularisers per layer
   int fit_mode;  // 0 auto, 1 one CTA per model (FFMA), 2 one cluster per model, samples split (FFMA), 3 tensor
                  // pipe, 4 one cluster per model, units split (FFMA2)  (bore_mlp_set_fit_mode)
+  void *tab_pinned;      // pinned staging buffer of the ragged fit's problem table (FitTable), tab_cap bytes
+  size_t tab_cap;
+  cudaEvent_t tab_done;  // recorded behind the last copy out of tab_pinned
 };
 
 static inline int round_up(int a, int b) { return (a + b - 1) / b * b; }
@@ -84,12 +94,70 @@ struct FitWeights {
   int on;
 };
 
-// the loss weight of one sample (device code; row >= 0)
+// One problem of a fit launch, read by its CTA (or cluster) at entry: the model it trains, the first of its
+// rows of X / z / w, of its permutation entries ([epochs][N] from there) and of its epoch losses, and its
+// observation count and epochs.  bore_mlp_fit_ragged passes a device table of them in launch order; the
+// uniform entry points pass none and every problem is derived from the launch's scalars (fit_problem).
+struct FitProblem {
+  long long row0, perm0, loss0;
+  int model, N, epochs, pad_;
+};
+
 #ifdef __CUDACC__
+// the loss weight of one sample (device code; row >= 0)
 __device__ __forceinline__ float fit_sample_weight(const FitWeights &fw, const float *w, int row, float z) {
   return (w ? w[row] : 1.f) * (z != 0.f ? fw.cw1 : fw.cw0);
 }
+
+// problem `b` of a uniform launch whose arguments `a` carry model0 / N / epochs / shared_data / shared_perm
+template <class A>
+__device__ __forceinline__ FitProblem fit_problem_uniform(const A &a, int b) {
+  FitProblem p;
+  p.model = a.model0 + b;
+  p.N = a.N;
+  p.epochs = a.epochs;
+  p.row0 = a.shared_data ? 0 : (long long)b * a.N;
+  p.perm0 = a.shared_perm ? 0 : (long long)b * a.epochs * a.N;
+  p.loss0 = (long long)b * a.epochs;
+  p.pad_ = 0;
+  return p;
+}
+// problem `b` of any launch: from the table a.probs when there is one
+template <class A>
+__device__ __forceinline__ FitProblem fit_problem(const A &a, int b) {
+  return a.probs ? a.probs[b] : fit_problem_uniform(a, b);
+}
 #endif
+
+// A small host table for one launch, copied to the device on the launch's stream (cudaMallocAsync, plain
+// cudaMemcpyAsync) and freed on that stream when the object goes out of scope, i.e. after every launch
+// enqueued before: a later call never overwrites a table an earlier launch may still read.
+struct StreamTable {
+  void *dev = nullptr;
+  cudaStream_t stream = nullptr;
+  cudaError_t upload(const void *host, size_t bytes, cudaStream_t s) {
+    stream = s;
+    cudaError_t e = cudaMallocAsync(&dev, bytes, s);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(dev, host, bytes, cudaMemcpyHostToDevice, s);
+    return e;
+  }
+  ~StreamTable() {
+    if (dev) cudaFreeAsync(dev, stream);
+  }
+};
+
+// The problem table of a ragged fit (FitProblem, launch order) on its way to the device.  get() stages it through
+// the handle's pinned buffer (so that the copy is asynchronous) into a StreamTable on the launch's stream; the
+// launchers call it after their last refusal, right before the launch, so that a refused call enqueues nothing.
+// A uniform fit has no table: host == NULL, get() gives NULL.
+struct FitTable {
+  bore_mlp *h;
+  const FitProblem *host;
+  int n;
+  cudaStream_t stream;
+  StreamTable dev;
+  int get(const FitProblem **out);  // 0, or < 0 with the error text set
+};
 
 // ---------------------------------------------------------------- launchers (one per .cu)
 // K0 / K2.  `list` (may be NULL) is a device array of row indices: point i of the launch
@@ -110,12 +178,13 @@ int launch_mlp_eval_multi(const bore_mlp *h, int model0, int n_models, int per_m
 // it runs, else -1 with the shared memory needed and the limit in the error text.  Host only, no device.
 int mlp_eval_check_envelope(const MlpDesc &d);
 int fit_check_envelope(const MlpDesc &d);
-// K1t (fit_mma.cu): 1 launched, 0 shape not taken (caller falls back to the FFMA kernels), < 0 error
+// K1t (fit_mma.cu): 1 launched, 0 shape not taken (caller falls back to the FFMA kernels), < 0 error.
+// `tab`: the launch's problems (a ragged fit; N is then the largest N_p) or no table (uniform).
 int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                    int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                   float *loss_out_dev, const FitWeights &fw, cudaStream_t stream);
+                   float *loss_out_dev, const FitWeights &fw, FitTable &tab, cudaStream_t stream);
 // K1u (fit_unit.cu): one cluster per model, hidden units split over the CTAs.  1 launched, 0 shape not
 // taken (caller falls back to the sample-split cluster kernel), < 0 error
 int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                     int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                    float *loss_out_dev, const FitWeights &fw, cudaStream_t stream);
+                    float *loss_out_dev, const FitWeights &fw, FitTable &tab, cudaStream_t stream);

@@ -30,17 +30,27 @@ __device__ __forceinline__ double from_orderable64(unsigned long long k) {
   return __longlong_as_double((long long)u);
 }
 
+__host__ __device__ int pow2_at_least(int v) { int p = 1; while (p < v) p <<= 1; return p; }
+
 // one CTA per problem: keys of the N targets sorted in shared memory (bitonic, padded to a power
 // of two), the two order statistics around the virtual index (N-1)*q read off, numpy's _lerp
-// applied, labels written as fp32 0/1 (what fit consumes) and/or bytes.
+// applied, labels written as fp32 0/1 (what fit consumes) and/or bytes.  `off` (ragged problems;
+// NULL: every problem holds N targets): problem b is y[off[b], off[b+1]); its CTA sorts its own
+// power of two inside shared memory sized for the largest.
 __global__ void __launch_bounds__(1024)
-quantile_labels_kernel(const double *__restrict__ y, int N, int n_pow2, double q,
-                       float *__restrict__ z_f32, uint8_t *__restrict__ z_u8,
+quantile_labels_kernel(const double *__restrict__ y, const long long *__restrict__ off, int N, int n_pow2,
+                       double q, float *__restrict__ z_f32, uint8_t *__restrict__ z_u8,
                        double *__restrict__ tau_out) {
   extern __shared__ unsigned long long sk[];
   __shared__ double s_tau;
   __shared__ int s_nan;
-  const double *yp = y + (size_t)blockIdx.x * N;
+  long long o0 = (long long)blockIdx.x * N;
+  if (off) {
+    o0 = off[blockIdx.x];
+    N = (int)(off[blockIdx.x + 1] - o0);
+    n_pow2 = max(2, pow2_at_least(N));
+  }
+  const double *yp = y + o0;
   if (threadIdx.x == 0) s_nan = 0;
   __syncthreads();
   bool has_nan = false;
@@ -93,23 +103,29 @@ quantile_labels_kernel(const double *__restrict__ y, int N, int n_pow2, double q
   const double tau = s_tau;
   for (int i = threadIdx.x; i < N; i += blockDim.x) {
     const bool z = yp[i] < tau;  // STRICT (np.less); false against a NaN threshold
-    if (z_f32) z_f32[(size_t)blockIdx.x * N + i] = z ? 1.f : 0.f;
-    if (z_u8) z_u8[(size_t)blockIdx.x * N + i] = z ? 1 : 0;
+    if (z_f32) z_f32[o0 + i] = z ? 1.f : 0.f;
+    if (z_u8) z_u8[o0 + i] = z ? 1 : 0;
   }
 }
 
 // one warp per candidate: lanes walk the stored rows of the candidate's group; a row matches
 // when every coordinate satisfies numpy.isclose(a = x_prev, b = x):
 //   |a - b| <= atol + rtol * |b|  and b finite,  or  a == b
+// `off` (ragged groups; NULL: every group stores n_prev rows): group g's rows are [off[g], off[g+1])
 __global__ void __launch_bounds__(256)
 duplicate_kernel(const double *__restrict__ x, int n_groups, int per_group,
-                 const double *__restrict__ x_prev, int n_prev, int D, double rtol, double atol,
-                 uint8_t *__restrict__ dup_out, uint8_t *__restrict__ keep_out) {
+                 const double *__restrict__ x_prev, const long long *__restrict__ off, int n_prev, int D,
+                 double rtol, double atol, uint8_t *__restrict__ dup_out, uint8_t *__restrict__ keep_out) {
   const int cand = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (cand >= n_groups * per_group) return;
   const int g = cand / per_group;
   const double *xc = x + (size_t)cand * D;
-  const double *xp = x_prev + (size_t)g * n_prev * D;
+  long long r0 = (long long)g * n_prev;
+  if (off) {
+    r0 = off[g];
+    n_prev = (int)(off[g + 1] - r0);
+  }
+  const double *xp = x_prev + r0 * D;
   bool found = false;
   for (int r0 = 0; r0 < n_prev && !found; r0 += 32) {
     const int r = r0 + lane;
@@ -126,8 +142,6 @@ duplicate_kernel(const double *__restrict__ x, int n_groups, int per_group,
     if (keep_out) keep_out[cand] = found ? 0 : 1;
   }
 }
-
-int pow2_at_least(int v) { int p = 1; while (p < v) p <<= 1; return p; }
 
 // maybe_distort (bore/base.py:45-64): x = truncnorm(a, b, loc, scale).rvs(random_state) with
 // a = (lower - loc) / scale, b = (upper - loc) / scale.  scipy draws ONE uniform variate per
@@ -162,12 +176,10 @@ truncnorm_distort_kernel(const double *__restrict__ loc, long n_total, int D, do
 
 }  // namespace
 
-extern "C" {
-
-int bore_quantile_labels(const double *y_dev, int n_problems, int N, double q, float *z_f32_dev,
-                         uint8_t *z_u8_dev, double *tau_dev, int device, void *stream_) {
-  BORE_CHECK(bore_device_count() > 0, "no CUDA device visible -- bore_b200 has no CPU fallback");
-  BORE_CHECK(n_problems >= 1 && N >= 1, "bore_quantile_labels: n_problems=%d, N=%d", n_problems, N);
+// bore_quantile_labels and its ragged form: N the (largest) number of targets, off_host (ragged; may be NULL)
+// the n_problems + 1 offsets of the problems in y
+static int quantile_run(const double *y_dev, int n_problems, const long long *off_host, int N, double q,
+                        float *z_f32_dev, uint8_t *z_u8_dev, double *tau_dev, int device, void *stream_) {
   BORE_CHECK(q >= 0.0 && q <= 1.0, "Quantiles must be in the range [0, 1]");  // numpy's message
   BORE_CHECK(y_dev && (z_f32_dev || z_u8_dev || tau_dev), "bore_quantile_labels: NULL buffer");
   const int n = std::max(2, pow2_at_least(N));
@@ -180,11 +192,58 @@ int bore_quantile_labels(const double *y_dev, int n_problems, int N, double q, f
                                    224 * 1024));
     if (device < 64) attr_done[device] = true;
   }
+  const cudaStream_t stream = (cudaStream_t)stream_;
+  StreamTable table;  // freed on the stream after the launch
+  if (off_host) BORE_CUDA(table.upload(off_host, (size_t)(n_problems + 1) * sizeof(long long), stream));
   const int threads = std::min(1024, std::max(32, n / 2));
-  quantile_labels_kernel<<<n_problems, threads, smem, (cudaStream_t)stream_>>>(y_dev, N, n, q, z_f32_dev,
-                                                                             z_u8_dev, tau_dev);
+  quantile_labels_kernel<<<n_problems, threads, smem, stream>>>(y_dev, static_cast<const long long *>(table.dev),
+                                                                N, n, q, z_f32_dev, z_u8_dev, tau_dev);
   BORE_CUDA(cudaGetLastError());
   return 0;
+}
+
+// bore_is_duplicate and its ragged form: off_host (ragged; may be NULL) the n_groups + 1 offsets of the groups'
+// stored rows in x_prev, any_prev whether there is a stored row at all
+static int duplicate_run(const double *x_dev, int n_groups, int per_group, const double *x_prev_dev,
+                         const long long *off_host, int n_prev, bool any_prev, int D, double rtol, double atol,
+                         uint8_t *dup_dev, uint8_t *keep_dev, int device, void *stream_) {
+  BORE_CHECK(x_dev && (!any_prev || x_prev_dev) && (dup_dev || keep_dev), "bore_is_duplicate: NULL buffer");
+  BORE_CUDA(cudaSetDevice(device));
+  const cudaStream_t stream = (cudaStream_t)stream_;
+  StreamTable table;  // freed on the stream after the launch
+  if (off_host) BORE_CUDA(table.upload(off_host, (size_t)(n_groups + 1) * sizeof(long long), stream));
+  const long warps = (long)n_groups * per_group;
+  const int blocks = (int)((warps * 32 + 255) / 256);
+  duplicate_kernel<<<blocks, 256, 0, stream>>>(x_dev, n_groups, per_group, x_prev_dev,
+                                               static_cast<const long long *>(table.dev), n_prev, D, rtol, atol,
+                                               dup_dev, keep_dev);
+  BORE_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" {
+
+int bore_quantile_labels(const double *y_dev, int n_problems, int N, double q, float *z_f32_dev,
+                         uint8_t *z_u8_dev, double *tau_dev, int device, void *stream_) {
+  BORE_CHECK(bore_device_count() > 0, "no CUDA device visible -- bore_b200 has no CPU fallback");
+  BORE_CHECK(n_problems >= 1 && N >= 1, "bore_quantile_labels: n_problems=%d, N=%d", n_problems, N);
+  return quantile_run(y_dev, n_problems, nullptr, N, q, z_f32_dev, z_u8_dev, tau_dev, device, stream_);
+}
+
+int bore_quantile_labels_ragged(const double *y_dev, int n_problems, const int32_t *n_host, double q,
+                                float *z_f32_dev, uint8_t *z_u8_dev, double *tau_dev, int device, void *stream_) {
+  BORE_CHECK(bore_device_count() > 0, "no CUDA device visible -- bore_b200 has no CPU fallback");
+  BORE_CHECK(n_problems >= 1 && n_host, "bore_quantile_labels_ragged: n_problems=%d, n_host=%p", n_problems,
+             (const void *)n_host);
+  std::vector<long long> off(n_problems + 1, 0);
+  int maxN = 1;
+  for (int p = 0; p < n_problems; ++p) {
+    // N_p <= 16384 is checked below (through the largest), so the sum cannot overflow
+    BORE_CHECK(n_host[p] >= 1, "bore_quantile_labels_ragged: problem %d has N=%d", p, n_host[p]);
+    off[p + 1] = off[p] + n_host[p];
+    maxN = std::max(maxN, (int)n_host[p]);
+  }
+  return quantile_run(y_dev, n_problems, off.data(), maxN, q, z_f32_dev, z_u8_dev, tau_dev, device, stream_);
 }
 
 int bore_is_duplicate(const double *x_dev, int n_groups, int per_group, const double *x_prev_dev,
@@ -194,14 +253,27 @@ int bore_is_duplicate(const double *x_dev, int n_groups, int per_group, const do
   BORE_CHECK(n_groups >= 1 && per_group >= 1 && n_prev >= 0 && D >= 1,
              "bore_is_duplicate: n_groups=%d, per_group=%d, n_prev=%d, D=%d", n_groups, per_group,
              n_prev, D);
-  BORE_CHECK(x_dev && (n_prev == 0 || x_prev_dev) && (dup_dev || keep_dev), "bore_is_duplicate: NULL buffer");
-  BORE_CUDA(cudaSetDevice(device));
-  const long warps = (long)n_groups * per_group;
-  const int blocks = (int)((warps * 32 + 255) / 256);
-  duplicate_kernel<<<blocks, 256, 0, (cudaStream_t)stream_>>>(x_dev, n_groups, per_group, x_prev_dev,
-                                                             n_prev, D, rtol, atol, dup_dev, keep_dev);
-  BORE_CUDA(cudaGetLastError());
-  return 0;
+  return duplicate_run(x_dev, n_groups, per_group, x_prev_dev, nullptr, n_prev, n_prev > 0, D, rtol, atol,
+                       dup_dev, keep_dev, device, stream_);
+}
+
+int bore_is_duplicate_ragged(const double *x_dev, int n_groups, int per_group, const double *x_prev_dev,
+                             const int32_t *n_prev_host, int D, double rtol, double atol, uint8_t *dup_dev,
+                             uint8_t *keep_dev, int device, void *stream_) {
+  BORE_CHECK(bore_device_count() > 0, "no CUDA device visible -- bore_b200 has no CPU fallback");
+  BORE_CHECK(n_groups >= 1 && per_group >= 1 && D >= 1 && n_prev_host,
+             "bore_is_duplicate_ragged: n_groups=%d, per_group=%d, D=%d, n_prev_host=%p", n_groups, per_group, D,
+             (const void *)n_prev_host);
+  BORE_CHECK((long long)n_groups * per_group <= 0x7fffffffLL / 32,
+             "bore_is_duplicate_ragged: %d x %d candidates", n_groups, per_group);
+  std::vector<long long> off(n_groups + 1, 0);
+  for (int g = 0; g < n_groups; ++g) {
+    BORE_CHECK(n_prev_host[g] >= 0, "bore_is_duplicate_ragged: group %d has n_prev=%d", g, n_prev_host[g]);
+    off[g + 1] = off[g] + n_prev_host[g];  // < 2^31 * 2^31: no overflow
+  }
+  BORE_CHECK(off[n_groups] <= 0x7fffffffffffffffLL / D, "bore_is_duplicate_ragged: the stored rows overflow 64 bits");
+  return duplicate_run(x_dev, n_groups, per_group, x_prev_dev, off.data(), 0, off[n_groups] > 0, D, rtol, atol,
+                       dup_dev, keep_dev, device, stream_);
 }
 
 int bore_truncnorm_distort(const double *loc_dev, int n_points, int D, double scale,

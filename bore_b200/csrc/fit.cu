@@ -18,6 +18,9 @@
 // Weights never leave shared memory during the run; HBM traffic is the minibatch gather
 // (B*(D+1)*4 bytes per step) plus the per-epoch loss.
 #include <stdlib.h>
+#include <string.h>
+
+#include <algorithm>
 
 #include "common.cuh"
 #include "fit_common.cuh"
@@ -126,6 +129,7 @@ struct FitArgs {
   float *loss_out;
   float lr, beta1, beta2, eps;
   FitWeights fw;
+  const FitProblem *probs;  // NULL: uniform launch
 };
 
 // acc[i][u] += sum_k A[k*lda + i] * B[k*ldb + u]: the 4 x 4 register tile of every GEMM below
@@ -189,22 +193,29 @@ __device__ __forceinline__ void narrow_tile(const float *__restrict__ Hin, const
 // use dot-product forms instead of 4x4 tiles padded with zeros.  (The first version gave every
 // 4x4 gradient tile to one thread: with Dense32 layers 64 / 16 / 8 of 128 threads worked while
 // the rest waited at the barrier -- 44 % of all stall samples, profiles/r01_notes.md.)
-// WEIGHTED: per-sample loss weights (FitArgs::fw); the unweighted build runs none of their code
-template <bool WEIGHTED>
+// WEIGHTED: per-sample loss weights (FitArgs::fw); the unweighted build runs none of their code.
+// RAGGED: the problems come from the table FitArgs::probs (bore_mlp_fit_ragged); the uniform build keeps the
+// expressions of before: deriving its problem through fit_problem() cost cfg 4 0.4 % (132.0 -> 132.5 ms)
+template <bool WEIGHTED, bool RAGGED>
 __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
   extern __shared__ __align__(16) float sm[];
   const MlpDesc &d = a.d;
   const FitPlan &P = a.P;
   const int L = d.n_layers, BS = P.BS;
   const int tid = threadIdx.x, NT = blockDim.x;
-  const int model = a.model0 + blockIdx.x;
+  // this CTA's problem: from the table (ragged), else the expressions of the uniform launch
+  const FitProblem pb = RAGGED ? a.probs[blockIdx.x] : FitProblem{};
+  const int model = RAGGED ? pb.model : a.model0 + blockIdx.x;
+  const int N = RAGGED ? pb.N : a.N, epochs = RAGGED ? pb.epochs : a.epochs;
+  const size_t row0 = RAGGED ? (size_t)pb.row0 : (a.shared_data ? 0 : (size_t)blockIdx.x * a.N);
   float *gp = a.params + (size_t)model * d.n_params;
   float *gm = a.adam_m + (size_t)model * d.n_params;
   float *gv = a.adam_v + (size_t)model * d.n_params;
-  const float *X = a.X + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N * d.dims[0]);
-  const float *zg = a.z + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N);
-  const int *perm = a.perm + (a.shared_perm ? 0 : (size_t)blockIdx.x * a.epochs * a.N);
-  const float *wg = WEIGHTED && a.fw.w ? a.fw.w + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N) : nullptr;
+  const float *X = a.X + (RAGGED ? (size_t)pb.row0 * d.dims[0]
+                                 : (a.shared_data ? 0 : (size_t)blockIdx.x * a.N * d.dims[0]));
+  const float *zg = a.z + row0;
+  const int *perm = a.perm + (RAGGED ? (size_t)pb.perm0 : (a.shared_perm ? 0 : (size_t)blockIdx.x * a.epochs * a.N));
+  const float *wg = WEIGHTED && a.fw.w ? a.fw.w + row0 : nullptr;
   int *idxb = reinterpret_cast<int *>(sm + P.idx);
   float *red = sm + P.red;
   float *gs = sm + P.gs;
@@ -233,17 +244,17 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
   const float inv_D = 1.f / (float)D;
   __syncthreads();
 
-  const int steps_per_epoch = (a.N + a.batch - 1) / a.batch;
-  for (int ep = 0; ep < a.epochs; ++ep) {
+  const int steps_per_epoch = (N + a.batch - 1) / a.batch;
+  for (int ep = 0; ep < epochs; ++ep) {
     float epoch_tot = 0.f;
     for (int st = 0; st < steps_per_epoch; ++st) {
       const int s0 = st * a.batch;
-      const int nb = min(a.batch, a.N - s0);
+      const int nb = min(a.batch, N - s0);
       const int BP = r4(nb), nchunk = BP >> 2;
       const float inv_nchunk = 1.f / (float)nchunk;
       // ---- gather the minibatch (transposed) ----
       for (int p = tid; p < BP; p += NT) {
-        const int row = p < nb ? perm[(size_t)ep * a.N + s0 + p] : -1;
+        const int row = p < nb ? perm[(size_t)ep * N + s0 + p] : -1;
         idxb[p] = row;
         const float zz = row >= 0 ? zg[row] : 0.f;
         sm[P.zb + p] = zz;
@@ -685,7 +696,8 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
       if (a.any_l2) loss += block_sum(reg, red);
       epoch_tot += loss * (float)nb;
     }
-    if (tid == 0 && a.loss_out) a.loss_out[(size_t)blockIdx.x * a.epochs + ep] = epoch_tot / (float)a.N;
+    if (tid == 0 && a.loss_out)
+      a.loss_out[(RAGGED ? (size_t)pb.loss0 : (size_t)blockIdx.x * epochs) + ep] = epoch_tot / (float)N;
   }
 
   // ---- write the trained weights back ----
@@ -781,6 +793,7 @@ struct FitCArgs {
   int N, shared_data, batch, epochs;
   const int *perm;
   int shared_perm;
+  const FitProblem *probs;  // NULL: uniform launch (fit_problem)
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
   int any_l2;
   float *loss_out;
@@ -889,15 +902,15 @@ fit_cluster_kernel(const FitCArgs a) {
   const int L = d.n_layers, SP = P.SP;
   const int tid = threadIdx.x, NT = blockDim.x;
   const int rank = (int)cluster_rank();
-  const int cl = blockIdx.x / FIT_CLUSTER;  // which model of the launch
-  const int model = a.model0 + cl;
+  const FitProblem pb = fit_problem(a, blockIdx.x / FIT_CLUSTER);  // which problem of the launch
+  const int model = pb.model, N = pb.N, epochs = pb.epochs;
   float *gp = a.params + (size_t)model * d.n_params;
   float *gm = a.adam_m + (size_t)model * d.n_params;
   float *gv = a.adam_v + (size_t)model * d.n_params;
-  const float *X = a.X + (a.shared_data ? 0 : (size_t)cl * a.N * d.dims[0]);
-  const float *zg = a.z + (a.shared_data ? 0 : (size_t)cl * a.N);
-  const int *perm = a.perm + (a.shared_perm ? 0 : (size_t)cl * a.epochs * a.N);
-  const float *wg = WEIGHTED && a.fw.w ? a.fw.w + (a.shared_data ? 0 : (size_t)cl * a.N) : nullptr;
+  const float *X = a.X + pb.row0 * d.dims[0];
+  const float *zg = a.z + pb.row0;
+  const int *perm = a.perm + pb.perm0;
+  const float *wg = WEIGHTED && a.fw.w ? a.fw.w + pb.row0 : nullptr;
   int *idxb = reinterpret_cast<int *>(sm + P.idx);
   float *red = sm + P.red;
   // loss weights of this CTA's samples (weighted fits): delta buffer 1 is dead from the end of one reverse
@@ -906,17 +919,17 @@ fit_cluster_kernel(const FitCArgs a) {
   const int D = d.dims[0];
   const int i0 = rank * P.chunk;                       // this CTA's parameter slice
   const int i1 = min(i0 + P.chunk, d.n_params);
-  const int steps_per_epoch = (a.N + a.batch - 1) / a.batch;
+  const int steps_per_epoch = (N + a.batch - 1) / a.batch;
 
   // gathers this CTA's slice of minibatch (ep, st), transposed and zero padded; ends published
   auto gather = [&](int ep, int st) {
     const int s0 = st * a.batch;
-    const int nb = min(a.batch, a.N - s0);
+    const int nb = min(a.batch, N - s0);
     const int spc = (nb + FIT_CLUSTER - 1) / FIT_CLUSTER;
     const int p0 = rank * spc;
     const int mine = max(0, min(spc, nb - p0));
     for (int p = tid; p < SP; p += NT) {
-      const int row = p < mine ? perm[(size_t)ep * a.N + s0 + p0 + p] : -1;
+      const int row = p < mine ? perm[(size_t)ep * N + s0 + p0 + p] : -1;
       idxb[p] = row;
       const float zz = row >= 0 ? zg[row] : 0.f;
       sm[P.zb + p] = zz;
@@ -989,11 +1002,11 @@ fit_cluster_kernel(const FitCArgs a) {
 
   const float inv_chunk = 1.f / (float)P.chunk;
   int par = 0;  // slot parity of the current step
-  for (int ep = 0; ep < a.epochs; ++ep) {
+  for (int ep = 0; ep < epochs; ++ep) {
     float epoch_tot = 0.f;
     for (int st = 0; st < steps_per_epoch; ++st, par ^= 1) {
       const int s0 = st * a.batch;
-      const int nb = min(a.batch, a.N - s0);
+      const int nb = min(a.batch, N - s0);
       const int spc = (nb + FIT_CLUSTER - 1) / FIT_CLUSTER;  // samples per CTA
       const int mine = max(0, min(spc, nb - rank * spc));     // this CTA's samples
 
@@ -1164,7 +1177,7 @@ fit_cluster_kernel(const FitCArgs a) {
       {
         int nst = st + 1, nep = ep;
         if (nst == steps_per_epoch) { nst = 0; ++nep; }
-        if (nep < a.epochs) gather(nep, nst);
+        if (nep < epochs) gather(nep, nst);
       }
       cluster_wait();  // updated slices (and this step's loss / reg slots) are published
 
@@ -1195,7 +1208,7 @@ fit_cluster_kernel(const FitCArgs a) {
       __syncthreads();  // images rewritten before the next forward
     }
     if (rank == 0 && tid == 0 && a.loss_out)
-      a.loss_out[(size_t)cl * a.epochs + ep] = epoch_tot / (float)a.N;
+      a.loss_out[pb.loss0 + ep] = epoch_tot / (float)N;
   }
 
   // ---- write back: rank 0 the weights, every CTA its Adam slice ----
@@ -1289,11 +1302,13 @@ int fit_check_envelope(const MlpDesc &d) {
   return 0;
 }
 
-// bore_mlp_fit and bore_mlp_fit_weighted: the same checks and the same choice of kernel; fw.on == 0 runs
-// every kernel with its unweighted arithmetic
+// bore_mlp_fit, bore_mlp_fit_weighted and bore_mlp_fit_ragged: the same checks and the same choice of kernel;
+// fw.on == 0 runs every kernel with its unweighted arithmetic.  probs_host (ragged fits; NULL otherwise): the
+// `count` problems of the launch in launch order, N the largest N_p and epochs the largest epochs_p.
 static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                    int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                   float *loss_out_dev, const FitWeights &fw, void *stream) {
+                   float *loss_out_dev, const FitWeights &fw, void *stream,
+                   const FitProblem *probs_host = nullptr) {
   BORE_CHECK(h != nullptr, "NULL handle");
   BORE_CHECK(model0 >= 0 && count >= 1 && model0 + count <= h->n_models,
              "bore_mlp_fit: models [%d,%d) outside [0,%d)", model0, model0 + count, h->n_models);
@@ -1321,6 +1336,10 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
   a.loss_out = loss_out_dev;
   a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
   a.fw = fw;
+  // ragged fits: uploaded by the launch path that takes the net, after its refusals; freed on the stream after
+  // the launch
+  FitTable table{h, probs_host, count, (cudaStream_t)stream, {}};
+  a.probs = nullptr;
   // Tensor-pipe kernel (fit_mma.cu: 3xTF32 mma.sync GEMMs, one CTA per model) on request only (fit mode 3 or
   // BORE_FIT_MMA=1): measured SLOWER than both FFMA mappings below on B200 -- the legacy HMMA path gives
   // 3xTF32 only 1.3x the FFMA peak and every HMMA needs ~14 more instructions for fragments and splits
@@ -1333,7 +1352,7 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
     }
     if (h->fit_mode == 3 || (h->fit_mode == 0 && mma_env)) {
       const int rc = launch_fit_mma(h, model0, count, X_dev, z_dev, N, shared_data, batch_size, epochs, perm_dev,
-                                    shared_perm, loss_out_dev, fw, (cudaStream_t)stream);
+                                    shared_perm, loss_out_dev, fw, table, (cudaStream_t)stream);
       if (rc != 0) return rc < 0 ? rc : 0;
       BORE_CHECK(h->fit_mode != 3, "bore_mlp_fit: the tensor-pipe kernel does not take this net / batch size");
     }
@@ -1350,7 +1369,7 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
     }
     if (h->fit_mode == 4 || (h->fit_mode == 0 && unit_env && count * FIT_CLUSTER <= h->sm_count)) {
       const int rc = launch_fit_unit(h, model0, count, X_dev, z_dev, N, shared_data, batch_size, epochs, perm_dev,
-                                     shared_perm, loss_out_dev, fw, (cudaStream_t)stream);
+                                     shared_perm, loss_out_dev, fw, table, (cudaStream_t)stream);
       if (rc != 0) return rc < 0 ? rc : 0;
       BORE_CHECK(h->fit_mode != 4, "bore_mlp_fit: the unit-split cluster kernel does not take this net / batch size");
     }
@@ -1363,10 +1382,12 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
     BORE_CHECK(!(h->fit_mode == 2 && !fits), "bore_mlp_fit: cluster mode needs %zu B of shared memory", csmem);
     if (want && fits) {
       FitCArgs c;
+      BORE_CHECK_RC(table.get(&a.probs));
       c.d = a.d; c.P = CP;
       c.params = a.params; c.adam_m = a.adam_m; c.adam_v = a.adam_v; c.adam_t = a.adam_t;
       c.model0 = a.model0; c.X = a.X; c.z = a.z; c.N = a.N; c.shared_data = a.shared_data;
       c.batch = a.batch; c.epochs = a.epochs; c.perm = a.perm; c.shared_perm = a.shared_perm;
+      c.probs = a.probs;
       for (int l = 0; l < BORE_MAX_LAYERS; ++l) { c.l2k[l] = a.l2k[l]; c.l2b[l] = a.l2b[l]; }
       c.any_l2 = a.any_l2; c.loss_out = a.loss_out;
       c.lr = a.lr; c.beta1 = a.beta1; c.beta2 = a.beta2; c.eps = a.eps;
@@ -1401,10 +1422,34 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
     smem = fit_onecta_plan(a.d, B, threads, narrow, a.P);
   }
   BORE_CHECK(smem <= FIT_MAX_SMEM, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
-  const auto kern = a.fw.on ? fit_kernel<true> : fit_kernel<false>;
+  BORE_CHECK_RC(table.get(&a.probs));
+  const auto kern = a.probs ? (a.fw.on ? fit_kernel<true, true> : fit_kernel<false, true>)
+                            : (a.fw.on ? fit_kernel<true, false> : fit_kernel<false, false>);
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count, threads, smem, (cudaStream_t)stream>>>(a);
   BORE_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int FitTable::get(const FitProblem **out) {
+  *out = static_cast<const FitProblem *>(dev.dev);
+  if (!host || dev.dev) return 0;
+  const size_t bytes = (size_t)n * sizeof(FitProblem);
+  if (!h->tab_done) BORE_CUDA(cudaEventCreateWithFlags(&h->tab_done, cudaEventDisableTiming));
+  BORE_CUDA(cudaEventSynchronize(h->tab_done));  // the previous table has left the staging buffer
+  if (h->tab_cap < bytes) {
+    if (h->tab_pinned) cudaFreeHost(h->tab_pinned);
+    h->tab_pinned = nullptr;
+    h->tab_cap = 0;
+    size_t cap = 4096;
+    while (cap < bytes) cap *= 2;
+    BORE_CUDA(cudaMallocHost(&h->tab_pinned, cap));
+    h->tab_cap = cap;
+  }
+  memcpy(h->tab_pinned, host, bytes);
+  BORE_CUDA(dev.upload(h->tab_pinned, bytes, stream));
+  BORE_CUDA(cudaEventRecord(h->tab_done, stream));
+  *out = static_cast<const FitProblem *>(dev.dev);
   return 0;
 }
 
@@ -1469,6 +1514,57 @@ int bore_mlp_fit_weighted(bore_mlp *h, int model0, int count, const float *X_dev
   BORE_NVTX("bore:fit weighted (K1)");
   return fit_run(h, model0, count, X_dev, z_dev, N, shared_data, batch_size, epochs, perm_dev, shared_perm,
                  loss_out_dev, fit_weights(w_dev, class_weight0, class_weight1), stream);
+}
+
+int bore_mlp_fit_ragged(bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev,
+                        const float *w_dev, const int32_t *n_host, const int32_t *epochs_host, float class_weight0,
+                        float class_weight1, int batch_size, const int32_t *perm_dev, float *loss_out_dev,
+                        void *stream) {
+  BORE_NVTX("bore:fit ragged (K1)");
+  BORE_CHECK(h != nullptr, "NULL handle");
+  BORE_CHECK(model0 >= 0 && count >= 1 && count <= h->n_models - model0,
+             "bore_mlp_fit_ragged: models [%d,%d) outside [0,%d)", model0, model0 + count, h->n_models);
+  BORE_CHECK(n_host && epochs_host, "bore_mlp_fit_ragged: NULL count array");
+  BORE_CHECK(X_dev && z_dev && perm_dev, "bore_mlp_fit_ragged: NULL buffer");
+  BORE_CHECK(batch_size >= 1, "bore_mlp_fit_ragged: batch=%d", batch_size);
+  const long long D = h->desc.dims[0];
+  // every problem gets its descriptor; the ones with epochs_p = 0 are not launched (their state is untouched)
+  std::vector<FitProblem> probs;
+  std::vector<long long> work;
+  long long R = 0, Q = 0, E = 0;
+  int maxN = 0, maxE = 0;
+  for (int p = 0; p < count; ++p) {
+    const int n = n_host[p], e = epochs_host[p];
+    BORE_CHECK(n >= 1 && e >= 0, "bore_mlp_fit_ragged: problem %d has N=%d, epochs=%d", p, n, e);
+    FitProblem f;
+    f.row0 = R; f.perm0 = Q; f.loss0 = E;
+    f.model = model0 + p; f.N = n; f.epochs = e; f.pad_ = 0;
+    long long rows_x, ne;
+    BORE_CHECK(!__builtin_add_overflow(R, (long long)n, &R) && !__builtin_mul_overflow(R, D, &rows_x) &&
+                   !__builtin_mul_overflow((long long)n, (long long)e, &ne) &&
+                   !__builtin_add_overflow(Q, ne, &Q) && !__builtin_add_overflow(E, (long long)e, &E),
+               "bore_mlp_fit_ragged: the sizes overflow 64 bits at problem %d", p);
+    if (e == 0) continue;
+    probs.push_back(f);
+    work.push_back((long long)e * (((long long)n + batch_size - 1) / batch_size));
+    maxN = n > maxN ? n : maxN;
+    maxE = e > maxE ? e : maxE;
+  }
+  // launch order: longest problem first (Adam steps), ties in problem order, so that a long problem does not
+  // start in the last wave of CTAs (DESIGN.md, "Ragged batched problems").  BORE_FIT_RAGGED_ORDER=0 launches
+  // in problem order (read on every call: lets one process time both orders).  Results do not depend on it.
+  const char *order_env = getenv("BORE_FIT_RAGGED_ORDER");
+  if (!(order_env && order_env[0] == '0')) {
+    std::vector<int> idx(probs.size());
+    for (size_t i = 0; i < idx.size(); ++i) idx[i] = (int)i;
+    std::stable_sort(idx.begin(), idx.end(), [&](int x, int y) { return work[x] > work[y]; });
+    std::vector<FitProblem> sorted(probs.size());
+    for (size_t i = 0; i < idx.size(); ++i) sorted[i] = probs[idx[i]];
+    probs.swap(sorted);
+  }
+  return fit_run(h, model0, probs.empty() ? count : (int)probs.size(), X_dev, z_dev, probs.empty() ? 1 : maxN,
+                 0, batch_size, maxE, perm_dev, 0, loss_out_dev, fit_weights(w_dev, class_weight0, class_weight1),
+                 stream, probs.empty() ? nullptr : probs.data());
 }
 
 int bore_mlp_set_fit_mode(bore_mlp *h, int mode) {

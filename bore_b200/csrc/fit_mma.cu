@@ -132,6 +132,7 @@ struct FitMArgs {
   int N, shared_data, batch, epochs;
   const int *perm;
   int shared_perm;
+  const FitProblem *probs;  // NULL: uniform launch (fit_problem)
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
   int any_l2;
   float *loss_out;
@@ -294,14 +295,15 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
   constexpr int NT = NW * 32;
   const int L = P.L, LH = P.L - 1;  // LH hidden layers; layer LH is the 1-unit output layer
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-  const int model = a.model0 + blockIdx.x;
+  const FitProblem pb = fit_problem(a, blockIdx.x);
+  const int model = pb.model, N = pb.N, epochs = pb.epochs;
   float *gp = a.params + (size_t)model * d.n_params;
   float *gm = a.adam_m + (size_t)model * d.n_params;
   float *gv = a.adam_v + (size_t)model * d.n_params;
-  const float *X = a.X + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N * d.dims[0]);
-  const float *zg = a.z + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N);
-  const int *perm = a.perm + (a.shared_perm ? 0 : (size_t)blockIdx.x * a.epochs * a.N);
-  const float *wg = a.fw.w ? a.fw.w + (a.shared_data ? 0 : (size_t)blockIdx.x * a.N) : nullptr;
+  const float *X = a.X + pb.row0 * d.dims[0];
+  const float *zg = a.z + pb.row0;
+  const int *perm = a.perm + pb.perm0;
+  const float *wg = a.fw.w ? a.fw.w + pb.row0 : nullptr;
   const int D = d.dims[0], lda = P.lda, ldx = P.ldx;
   float *red = sm + P.red;
 
@@ -333,8 +335,8 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
   long long t_step = a.adam_t[model];
   double b1p_d = pow((double)a.beta1, (double)t_step), b2p_d = pow((double)a.beta2, (double)t_step);
   const float om1 = 1.f - a.beta1, om2 = 1.f - a.beta2;
-  const int spe = (a.N + a.batch - 1) / a.batch;
-  const int total_steps = a.epochs * spe;
+  const int spe = (N + a.batch - 1) / a.batch;
+  const int total_steps = epochs * spe;
 
   // row index of sample `tid` of global step `gs` (threads < 64; -1 beyond the batch): requested a step
   // ahead so that its latency hides behind the forward pass; rows and labels follow by cp.async
@@ -342,8 +344,8 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
     int row = -1;
     if (tid < MT_MAXB && gs < total_steps) {
       const int ep = gs / spe, st = gs - ep * spe;
-      const int s0 = st * a.batch, nb = min(a.batch, a.N - s0);
-      if (tid < nb) row = __ldg(perm + (size_t)ep * a.N + s0 + tid);
+      const int s0 = st * a.batch, nb = min(a.batch, N - s0);
+      if (tid < nb) row = __ldg(perm + (size_t)ep * N + s0 + tid);
     }
     return row;
   };
@@ -410,7 +412,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
   for (int gs = 0; gs < total_steps; ++gs) {
     const int cur = gs & 1;
     const int ep = gs / spe, st = gs - ep * spe;
-    const int nb = min(a.batch, a.N - st * a.batch);
+    const int nb = min(a.batch, N - st * a.batch);
     const int nmb = (nb + 15) >> 4, BP = nmb << 4;
     const float inv_nb = 1.f / (float)nb;
     reg = 0.f;
@@ -629,7 +631,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
       if (tid == 0) epoch_tot += r * (float)nb;
     }
     if (st == spe - 1) {
-      if (tid == 0 && a.loss_out) a.loss_out[(size_t)blockIdx.x * a.epochs + ep] = epoch_tot / (float)a.N;
+      if (tid == 0 && a.loss_out) a.loss_out[pb.loss0 + ep] = epoch_tot / (float)N;
       epoch_tot = 0.f;
     }
   }
@@ -684,7 +686,7 @@ int launch_nw(const FitMArgs &a, int count, size_t smem, cudaStream_t stream) {
 // 1: launched; 0: shape not taken by the tensor kernel (caller falls back); < 0: error
 int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                    int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                   float *loss_out_dev, const FitWeights &fw, cudaStream_t stream) {
+                   float *loss_out_dev, const FitWeights &fw, FitTable &tab, cudaStream_t stream) {
   const int B = batch_size < N ? batch_size : N;
   // few models: one 16-warp CTA per model (latency); many: 4-warp CTAs, several per SM (throughput)
   int nw = count * 2 <= h->sm_count ? 16 : (count <= 2 * h->sm_count ? 8 : 4);
@@ -718,6 +720,10 @@ int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev,
   a.loss_out = loss_out_dev;
   a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
   a.fw = fw;
+  {
+    const int rc = tab.get(&a.probs);  // taken: the table goes up now
+    if (rc) return rc;
+  }
   int rc;
   if (nw == 16) rc = launch_nw<16>(a, count, smem, stream);
   else if (nw == 8) rc = launch_nw<8>(a, count, smem, stream);

@@ -155,6 +155,7 @@ struct FuArgs {
   int N, shared_data, batch, epochs;
   const int *perm;
   int shared_perm;
+  const FitProblem *probs;  // NULL: uniform launch (fit_problem)
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
   int any_l2;
   float *loss_out;
@@ -380,16 +381,16 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
 #define FU_U(i) (FIX ? HW / FU_C : P.U[i])
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int rank = (int)fu_rank();
-  const int cl = blockIdx.x / FU_C;  // which model of the launch
-  const int model = a.model0 + cl;
+  const FitProblem pb = fit_problem(a, blockIdx.x / FU_C);  // which problem of the launch
+  const int model = pb.model, N = pb.N, epochs = pb.epochs;
   float *gp = a.params + (size_t)model * d.n_params;
   float *gm = a.adam_m + (size_t)model * d.n_params;
   float *gv = a.adam_v + (size_t)model * d.n_params;
-  const float *X = a.X + (a.shared_data ? 0 : (size_t)cl * a.N * D);
-  const float *zg = a.z + (a.shared_data ? 0 : (size_t)cl * a.N);
-  const int *perm = a.perm + (a.shared_perm ? 0 : (size_t)cl * a.epochs * a.N);
-  const float *wg = WT && a.fw.w ? a.fw.w + (a.shared_data ? 0 : (size_t)cl * a.N) : nullptr;
-  const int steps_per_epoch = (a.N + a.batch - 1) / a.batch;
+  const float *X = a.X + pb.row0 * D;
+  const float *zg = a.z + pb.row0;
+  const int *perm = a.perm + pb.perm0;
+  const float *wg = WT && a.fw.w ? a.fw.w + pb.row0 : nullptr;
+  const int steps_per_epoch = (N + a.batch - 1) / a.batch;
   float *W = sm + P.par0, *Mm = W + P.npar, *Vv = Mm + P.npar, *Gg = Vv + P.npar;
   const int wstride = FIX ? (HW / FU_C) * SPT : P.wstride;  // floats per warp of the scratch
   const float inv_sp = 1.f / (float)SP, inv_nso = 1.f / (float)(SP >> 3), inv_nq = 1.f / (float)(SP >> 2);
@@ -456,8 +457,8 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
   int *idxs = reinterpret_cast<int *>(sm + P.idx);
   auto row_of = [&](int ep, int st, int p) -> int {
     const int s0 = st * a.batch;
-    const int nb = min(a.batch, a.N - s0);
-    return p < nb ? perm[(size_t)ep * a.N + s0 + p] : -1;
+    const int nb = min(a.batch, N - s0);
+    return p < nb ? perm[(size_t)ep * N + s0 + p] : -1;
   };
   const int gt = tid - 32 * FU_KS;  // thread index among the warps that idle during the GEMM passes
   auto index_stage = [&](int ep, int st) {  // visible after the next __syncthreads
@@ -512,13 +513,13 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
   int par = 0;           // parity of the current step: minibatch buffer, h_1 buffer, loss slots
   uint32_t step_no = 0;  // steps done: phase parity of the mbarriers
   float epoch_tot = 0.f;
-  for (int ep = 0; ep < a.epochs; ++ep) {
+  for (int ep = 0; ep < epochs; ++ep) {
     for (int st = 0; st < steps_per_epoch; ++st, par ^= 1, ++step_no) {
       const int s0 = st * a.batch;
-      const int nb = min(a.batch, a.N - s0);
+      const int nb = min(a.batch, N - s0);
       int nst = st + 1, nep = ep;
       if (nst == steps_per_epoch) { nst = 0; ++nep; }
-      const bool more = nep < a.epochs;
+      const bool more = nep < epochs;
       if (more) index_stage(nep, nst);  // read by gather_async in the gradient phase
 #ifdef FU_TRACE
       ntr = 0;
@@ -831,7 +832,7 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
       }
 #endif
     }
-    if (rank == 0 && tid == 0 && a.loss_out) a.loss_out[(size_t)cl * a.epochs + ep] = epoch_tot / (float)a.N;
+    if (rank == 0 && tid == 0 && a.loss_out) a.loss_out[pb.loss0 + ep] = epoch_tot / (float)N;
     epoch_tot = 0.f;
   }
 
@@ -888,7 +889,7 @@ static bool fu_plan(const MlpDesc &d, int batch, FuPlan &p, size_t &smem) {
 // 1 launched, 0 shape not taken (the caller falls back to the sample-split cluster kernel), < 0 error
 int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                     int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                    float *loss_out_dev, const FitWeights &fw, cudaStream_t stream) {
+                    float *loss_out_dev, const FitWeights &fw, FitTable &tab, cudaStream_t stream) {
   FuArgs a;
   a.d = h->desc;
   const int B = batch_size < N ? batch_size : N;
@@ -916,6 +917,10 @@ int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev
   a.loss_out = loss_out_dev;
   a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
   a.fw = fw;
+  {
+    const int rc = tab.get(&a.probs);  // taken: the table goes up now
+    if (rc) return rc;
+  }
   if (fixed_shape) {
     if (nh == 3 && hw == 64) return fu_launch<3, 64, 64>(a, count, smem, stream);
     if (nh == 3 && hw == 32) return fu_launch<3, 32, 64>(a, count, smem, stream);

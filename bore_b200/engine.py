@@ -420,6 +420,37 @@ class NativeMLP:
                                               None, _ptr(keep), self.device, self._stream()))
         return keep
 
+    def quantile_labels_ragged_dev(self, y_dev, n, gamma, want_tau=False):
+        """y_dev (sum n_p,) float64, the targets of M problems one after the other, n (M,) their
+        counts -> z (sum n_p,) float32 of 0/1 (and tau (M,)): every problem labelled over its own
+        targets (bore_quantile_labels_ragged)."""
+        torch = _torch()
+        n = np.ascontiguousarray(n, np.int32)
+        assert y_dev.dtype == torch.float64 and y_dev.dim() == 1 and y_dev.is_contiguous()
+        assert y_dev.shape[0] == int(n.astype(np.int64).sum())
+        z = torch.empty(y_dev.shape[0], dtype=torch.float32, device=self._tdev())
+        tau = torch.empty(len(n), dtype=torch.float64, device=self._tdev()) if want_tau else None
+        _lib.check(self.lib.bore_quantile_labels_ragged(_ptr(y_dev), len(n), _np_ptr(n), float(gamma), _ptr(z),
+                                                        None, _ptr(tau), self.device, self._stream()))
+        return (z, tau) if want_tau else z
+
+    def keep_unique_ragged_dev(self, x_dev, n_prev, x_prev_dev, rtol=1e-5, atol=1e-8):
+        """x_dev (G, K, D) float64, n_prev (G,) stored rows per group (0 allowed), x_prev_dev
+        (sum n_prev, D) float64 the groups' rows one group after the other -> keep (G, K) uint8
+        (bore_is_duplicate_ragged)."""
+        torch = _torch()
+        G, K, D = x_dev.shape
+        n_prev = np.ascontiguousarray(n_prev, np.int32)
+        assert x_dev.dtype == torch.float64 and x_dev.is_contiguous() and len(n_prev) == G
+        assert x_prev_dev.dtype == torch.float64 and x_prev_dev.is_contiguous()
+        assert tuple(x_prev_dev.shape) == (int(n_prev.astype(np.int64).sum()), D)
+        keep = torch.empty(G, K, dtype=torch.uint8, device=self._tdev())
+        _lib.check(self.lib.bore_is_duplicate_ragged(_ptr(x_dev), int(G), int(K),
+                                                     _ptr(x_prev_dev) if x_prev_dev.numel() else None,
+                                                     _np_ptr(n_prev), int(D), float(rtol), float(atol), None,
+                                                     _ptr(keep), self.device, self._stream()))
+        return keep
+
     def distort_dev(self, loc_dev, distortion, low, high, u_dev):
         """loc_dev (P, D) float64 suggestions -> truncated-normal resamples around them
         (bore/base.py:45-64) from the uniform variates u_dev (P, D) drawn on the host."""
@@ -486,6 +517,29 @@ class NativeMLP:
                                                   int(batch_size), int(epochs), _ptr(perm_dev),
                                                   1 if shared_perm else 0, _ptr(loss_dev), self._stream()))
         return loss_dev
+
+    def fit_ragged_dev(self, X_dev, z_dev, layout, batch_size, perm_dev, model0=0, w_dev=None,
+                       class_weight=None):
+        """Problems model0 .. model0 + M - 1 with their own observation counts and epochs
+        (``layout``: a ``ragged.RaggedLayout``) in one launch (bore_mlp_fit_ragged).  X_dev
+        (sum N_p, D), z_dev / w_dev (sum N_p,) float32 and perm_dev (sum epochs_p * N_p,) int32 hold
+        the problems one after the other.  Returns the concatenated epoch losses (sum epochs_p,)."""
+        torch = _torch()
+        assert X_dev.dtype == torch.float32 and z_dev.dtype == torch.float32
+        assert perm_dev.dtype == torch.int32 and perm_dev.is_contiguous()
+        n = np.ascontiguousarray(layout.n, np.int32)
+        e = np.ascontiguousarray(layout.epochs, np.int32)
+        R, Q, E = int(layout.rows[-1]), int(layout.perms[-1]), int(layout.losses[-1])
+        assert X_dev.shape == (R, self.D) and z_dev.numel() == R and perm_dev.numel() == Q
+        assert w_dev is None or (w_dev.dtype == torch.float32 and w_dev.is_contiguous() and w_dev.numel() == R)
+        if Q == 0:  # nothing trains; the call still checks its arguments
+            perm_dev = torch.zeros(1, dtype=torch.int32, device=self._tdev())
+        loss_dev = torch.empty(max(E, 1), dtype=torch.float32, device=self._tdev())
+        cw0, cw1 = (1.0, 1.0) if class_weight is None else class_weight
+        _lib.check(self.lib.bore_mlp_fit_ragged(self.h, int(model0), len(n), _ptr(X_dev), _ptr(z_dev), _ptr(w_dev),
+                                                _np_ptr(n), _np_ptr(e), float(cw0), float(cw1), int(batch_size),
+                                                _ptr(perm_dev), _ptr(loss_dev), self._stream()))
+        return loss_dev[:E]
 
     def fit(self, X, z, epochs, batch_size, permutations, l2=None, model=0, w=None, class_weight=None):
         """Keras ``fit`` with explicit per-epoch permutations -> history loss (epochs,).

@@ -160,6 +160,29 @@ int bore_mlp_evaluate_weighted(bore_mlp *h, int model, const float *X_dev, const
                                const float *w_dev, float class_weight0, float class_weight1,
                                int N, float *out_host, void *stream);
 
+/* ---- K1, ragged: problems with their own observation counts and epochs -----------------------
+ * bore_mlp_fit_weighted for `count` problems that each hold N_p >= 1 observations and train for
+ * epochs_p >= 0 epochs (n_host[p], epochs_host[p]; host arrays).  Problem p is model model0 + p and
+ * computes what a fit of that model alone on its own data computes: minibatches of min(batch, N_p),
+ * ceil(N_p / batch) steps per epoch (the last one short), Adam's `iterations` advanced by
+ * epochs_p * ceil(N_p / batch), history["loss"] over its N_p samples.  epochs_p = 0 leaves the model
+ * untouched (weights, Adam m / v and iterations).  With R, Q, E the prefix sums over the problems in
+ * their order (64-bit: R_p = sum_{q<p} N_q, Q_p = sum_{q<p} epochs_q * N_q, E_p = sum_{q<p} epochs_q):
+ *   X_dev [R_count][D], z_dev / w_dev [R_count]: problem p's rows are [R_p, R_p + N_p); w_dev may be NULL
+ *   perm_dev: problem p's shuffles are the [epochs_p][N_p] int32 block at Q_p (indices in [0, N_p))
+ *   loss_out_dev (may be NULL): problem p's epoch losses are the epochs_p floats at E_p
+ * The batch size, the net and the class weights are shared.  Same kernels, fit modes, environment
+ * overrides and refusals as bore_mlp_fit; the plans are made for the batch min(batch, max N_p) over the
+ * problems that train, and the kernel is chosen for their number.  w_dev NULL with class weights (1, 1)
+ * runs the unweighted arithmetic.  With every N_p = N and epochs_p = E this is bore_mlp_fit(_weighted)
+ * with shared_data = shared_perm = 0, bit for bit.  The problems are launched longest first
+ * (epochs_p * ceil(N_p / batch)); the results do not depend on the order.  Every argument is checked
+ * before anything is enqueued.                                                                     */
+int bore_mlp_fit_ragged(bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev,
+                        const float *w_dev, const int32_t *n_host, const int32_t *epochs_host,
+                        float class_weight0, float class_weight1, int batch_size, const int32_t *perm_dev,
+                        float *loss_out_dev, void *stream);
+
 /* ---- K3: batched bound-constrained L-BFGS-B -------------------------------------------
  * Replaces the per-start scipy.optimize.minimize(fun, x0, method="L-BFGS-B", jac=True,
  * bounds=..., options=dict(maxiter, ftol)) loop of bore/mixins.py:57-61 (also
@@ -307,6 +330,17 @@ int bore_quantile_labels(const double *y_dev, int n_problems, int N, double q, f
 int bore_is_duplicate(const double *x_dev, int n_groups, int per_group, const double *x_prev_dev,
                       int n_prev, int D, double rtol, double atol, uint8_t *dup_dev,
                       uint8_t *keep_dev, int device, void *stream);
+/* Ragged forms of the two above.  bore_quantile_labels_ragged: problem p holds n_host[p] >= 1 targets
+ * (<= 16384), y_dev / z_f32_dev / z_u8_dev are the problems' vectors one after the other (problem p
+ * at the sum of the counts before it), tau_dev [n_problems]; each problem is labelled over its own
+ * targets, bit-identical to numpy.  bore_is_duplicate_ragged: group g stores n_prev_host[g] >= 0 rows
+ * (0 allowed: nothing is a duplicate), x_prev_dev holds the groups' rows one group after the other;
+ * x_dev, dup_dev and keep_dev keep the layout of bore_is_duplicate.                                */
+int bore_quantile_labels_ragged(const double *y_dev, int n_problems, const int32_t *n_host, double q,
+                                float *z_f32_dev, uint8_t *z_u8_dev, double *tau_dev, int device, void *stream);
+int bore_is_duplicate_ragged(const double *x_dev, int n_groups, int per_group, const double *x_prev_dev,
+                             const int32_t *n_prev_host, int D, double rtol, double atol, uint8_t *dup_dev,
+                             uint8_t *keep_dev, int device, void *stream);
 
 /* ---- batch argmax by SVGD (SURVEY.md section 8f, row 3) ---------------------------------
  * Replaces BatchMaximizableMixin.argmax_batch (bore/mixins.py:100-116), i.e.
