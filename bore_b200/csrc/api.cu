@@ -43,7 +43,7 @@ int bore_mlp_create(int n_layers, const int *dims, const int *acts, int n_models
     BORE_CHECK(dims[l] >= 1 && dims[l] <= BORE_MAX_WIDTH,
                "bore_mlp_create: hidden width %d outside [1,%d]", dims[l], BORE_MAX_WIDTH);
   for (int l = 0; l < n_layers; ++l)
-    BORE_CHECK(acts[l] >= BORE_ACT_LINEAR && acts[l] <= BORE_ACT_TANH,
+    BORE_CHECK(acts[l] >= BORE_ACT_LINEAR && acts[l] <= BORE_ACT_EXPONENTIAL,
                "bore_mlp_create: unknown activation code %d", acts[l]);
   MlpDesc d;
   memset(&d, 0, sizeof(d));

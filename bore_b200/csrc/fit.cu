@@ -196,7 +196,8 @@ __device__ __forceinline__ void narrow_tile(const float *__restrict__ Hin, const
 // WEIGHTED: per-sample loss weights (FitArgs::fw); the unweighted build runs none of their code.
 // RAGGED: the problems come from the table FitArgs::probs (bore_mlp_fit_ragged); the uniform build keeps the
 // expressions of before: deriving its problem through fit_problem() cost cfg 4 0.4 % (132.0 -> 132.5 ms)
-template <bool WEIGHTED, bool RAGGED>
+// EXT: the activation codes above BORE_ACT_TANH (act.cuh).
+template <bool WEIGHTED, bool RAGGED, bool EXT>
 __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
   extern __shared__ __align__(16) float sm[];
   const MlpDesc &d = a.d;
@@ -301,8 +302,8 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
             }
             if (valid && s == 0) {
               const float b = bs[0];
-              *reinterpret_cast<float4 *>(H + 4 * c) = make_float4(f_act(act, acc.x + b), f_act(act, acc.y + b),
-                                                                   f_act(act, acc.z + b), f_act(act, acc.w + b));
+              *reinterpret_cast<float4 *>(H + 4 * c) = make_float4(act_fwd<EXT>(act, acc.x + b), act_fwd<EXT>(act, acc.y + b),
+                                                                   act_fwd<EXT>(act, acc.z + b), act_fwd<EXT>(act, acc.w + b));
             }
           }
         } else {
@@ -317,10 +318,10 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
               if (j < out) {
                 const float b = bs[j];
                 float4 o;
-                o.x = f_act(act, acc[0][u] + b);
-                o.y = f_act(act, acc[1][u] + b);
-                o.z = f_act(act, acc[2][u] + b);
-                o.w = f_act(act, acc[3][u] + b);
+                o.x = act_fwd<EXT>(act, acc[0][u] + b);
+                o.y = act_fwd<EXT>(act, acc[1][u] + b);
+                o.z = act_fwd<EXT>(act, acc[2][u] + b);
+                o.w = act_fwd<EXT>(act, acc[3][u] + b);
                 *reinterpret_cast<float4 *>(H + j * BS + tp * 4) = o;
               }
             }
@@ -379,8 +380,8 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
               const float4 hv = *reinterpret_cast<const float4 *>(Hin + k * BS + 4 * c);
               const float w = WT[k];
               *reinterpret_cast<float4 *>(DN + k * BS + 4 * c) =
-                  make_float4(dv.x * w * f_act_bwd(actp, hv.x), dv.y * w * f_act_bwd(actp, hv.y),
-                              dv.z * w * f_act_bwd(actp, hv.z), dv.w * w * f_act_bwd(actp, hv.w));
+                  make_float4(dv.x * w * act_bwd<EXT>(actp, hv.x), dv.y * w * act_bwd<EXT>(actp, hv.y),
+                              dv.z * w * act_bwd<EXT>(actp, hv.z), dv.w * w * act_bwd<EXT>(actp, hv.w));
             }
           } else {
             const int ntile = nchunk * (r4(in) / 4);
@@ -394,10 +395,10 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
                 if (k < in) {
                   const float4 hv = *reinterpret_cast<const float4 *>(Hin + k * BS + tp * 4);
                   float4 o;
-                  o.x = acc[0][u] * f_act_bwd(actp, hv.x);
-                  o.y = acc[1][u] * f_act_bwd(actp, hv.y);
-                  o.z = acc[2][u] * f_act_bwd(actp, hv.z);
-                  o.w = acc[3][u] * f_act_bwd(actp, hv.w);
+                  o.x = acc[0][u] * act_bwd<EXT>(actp, hv.x);
+                  o.y = acc[1][u] * act_bwd<EXT>(actp, hv.y);
+                  o.z = acc[2][u] * act_bwd<EXT>(actp, hv.z);
+                  o.w = acc[3][u] * act_bwd<EXT>(actp, hv.w);
                   *reinterpret_cast<float4 *>(DN + k * BS + tp * 4) = o;
                 }
               }
@@ -876,24 +877,26 @@ __device__ __forceinline__ void dense_pass(const float *A, const float *Wm, int 
   }
 }
 
-// activation of four values with ONE dispatch (the switch of f_act per element showed up with
+// activation of four values with ONE dispatch (the switch of act_fwd per element showed up with
 // 4.6 % of the cluster kernel's instructions)
+template <bool EXT>
 __device__ __forceinline__ float4 f_act4(int a, float4 v) {
   if (a == BORE_ACT_RELU) return make_float4(fmaxf(v.x, 0.f), fmaxf(v.y, 0.f), fmaxf(v.z, 0.f), fmaxf(v.w, 0.f));
   if (a == BORE_ACT_LINEAR) return v;
-  return make_float4(f_act(a, v.x), f_act(a, v.y), f_act(a, v.z), f_act(a, v.w));
+  return make_float4(act_fwd<EXT>(a, v.x), act_fwd<EXT>(a, v.y), act_fwd<EXT>(a, v.z), act_fwd<EXT>(a, v.w));
 }
 // acc * act'(h), four values
+template <bool EXT>
 __device__ __forceinline__ float4 f_act_bwd4(int a, float4 acc, float4 h) {
   if (a == BORE_ACT_RELU)
     return make_float4(h.x > 0.f ? acc.x : 0.f, h.y > 0.f ? acc.y : 0.f, h.z > 0.f ? acc.z : 0.f,
                        h.w > 0.f ? acc.w : 0.f);
   if (a == BORE_ACT_LINEAR) return acc;
-  return make_float4(acc.x * f_act_bwd(a, h.x), acc.y * f_act_bwd(a, h.y), acc.z * f_act_bwd(a, h.z),
-                     acc.w * f_act_bwd(a, h.w));
+  return make_float4(acc.x * act_bwd<EXT>(a, h.x), acc.y * act_bwd<EXT>(a, h.y), acc.z * act_bwd<EXT>(a, h.z),
+                     acc.w * act_bwd<EXT>(a, h.w));
 }
 
-template <bool WEIGHTED>
+template <bool WEIGHTED, bool EXT>
 __global__ void __cluster_dims__(FIT_CLUSTER, 1, 1) __launch_bounds__(FIT_CTHREADS)
 fit_cluster_kernel(const FitCArgs a) {
   extern __shared__ __align__(16) float sm[];
@@ -1019,7 +1022,7 @@ fit_cluster_kernel(const FitCArgs a) {
         dense_pass(sm + P.h[l], sm + P.w[l], in, ldo(out), out, SP, [&](int j, int q, float4 acc) {
           const float b = bs[j];
           *reinterpret_cast<float4 *>(H + j * SP + 4 * q) =
-              f_act4(act, make_float4(acc.x + b, acc.y + b, acc.z + b, acc.w + b));
+              f_act4<EXT>(act, make_float4(acc.x + b, acc.y + b, acc.z + b, acc.w + b));
         });
         __syncthreads();
       }
@@ -1064,7 +1067,7 @@ fit_cluster_kernel(const FitCArgs a) {
           const int actp = d.act[l - 1];
           dense_pass(DL, sm + P.wt[l], out, ldo(in), in, SP, [&](int k, int q, float4 acc) {
             const float4 hv = *reinterpret_cast<const float4 *>(Hin + k * SP + 4 * q);
-            *reinterpret_cast<float4 *>(DN + k * SP + 4 * q) = f_act_bwd4(actp, acc, hv);
+            *reinterpret_cast<float4 *>(DN + k * SP + 4 * q) = f_act_bwd4<EXT>(actp, acc, hv);
           });
         }
         {
@@ -1340,6 +1343,7 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
   // the launch
   FitTable table{h, probs_host, count, (cudaStream_t)stream, {}};
   a.probs = nullptr;
+  const bool ext = acts_ext(a.d.act, a.d.n_layers);
   // Tensor-pipe kernel (fit_mma.cu: 3xTF32 mma.sync GEMMs, one CTA per model) on request only (fit mode 3 or
   // BORE_FIT_MMA=1): measured SLOWER than both FFMA mappings below on B200 -- the legacy HMMA path gives
   // 3xTF32 only 1.3x the FFMA peak and every HMMA needs ~14 more instructions for fragments and splits
@@ -1392,7 +1396,8 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
       c.any_l2 = a.any_l2; c.loss_out = a.loss_out;
       c.lr = a.lr; c.beta1 = a.beta1; c.beta2 = a.beta2; c.eps = a.eps;
       c.fw = a.fw;
-      const auto kern = a.fw.on ? fit_cluster_kernel<true> : fit_cluster_kernel<false>;
+      const auto kern = ext ? (a.fw.on ? fit_cluster_kernel<true, true> : fit_cluster_kernel<false, true>)
+                            : (a.fw.on ? fit_cluster_kernel<true, false> : fit_cluster_kernel<false, false>);
       BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csmem));
       kern<<<count * FIT_CLUSTER, FIT_CTHREADS, csmem, (cudaStream_t)stream>>>(c);
       BORE_CUDA(cudaGetLastError());
@@ -1423,8 +1428,10 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
   }
   BORE_CHECK(smem <= FIT_MAX_SMEM, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
   BORE_CHECK_RC(table.get(&a.probs));
-  const auto kern = a.probs ? (a.fw.on ? fit_kernel<true, true> : fit_kernel<false, true>)
-                            : (a.fw.on ? fit_kernel<true, false> : fit_kernel<false, false>);
+  const auto kern = ext ? (a.probs ? (a.fw.on ? fit_kernel<true, true, true> : fit_kernel<false, true, true>)
+                                   : (a.fw.on ? fit_kernel<true, false, true> : fit_kernel<false, false, true>))
+                        : (a.probs ? (a.fw.on ? fit_kernel<true, true, false> : fit_kernel<false, true, false>)
+                                   : (a.fw.on ? fit_kernel<true, false, false> : fit_kernel<false, false, false>));
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count, threads, smem, (cudaStream_t)stream>>>(a);
   BORE_CUDA(cudaGetLastError());

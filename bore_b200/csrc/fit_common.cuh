@@ -1,27 +1,10 @@
 // Device helpers shared by the training kernels (fit.cu: FP32 FFMA; fit_mma.cu: 3xTF32 tensor pipe).
 #pragma once
 #include "common.cuh"
+#include "act.cuh"
 
 namespace {
 
-__device__ __forceinline__ float f_act(int a, float v) {
-  switch (a) {
-    case BORE_ACT_RELU: return fmaxf(v, 0.f);
-    case BORE_ACT_ELU: return v > 0.f ? v : expm1f(v);
-    case BORE_ACT_SIGMOID: return 1.f / (1.f + expf(-v));
-    case BORE_ACT_TANH: return tanhf(v);
-    default: return v;
-  }
-}
-__device__ __forceinline__ float f_act_bwd(int a, float h) {
-  switch (a) {
-    case BORE_ACT_RELU: return h > 0.f ? 1.f : 0.f;
-    case BORE_ACT_ELU: return h > 0.f ? 1.f : h + 1.f;
-    case BORE_ACT_SIGMOID: return h * (1.f - h);
-    case BORE_ACT_TANH: return 1.f - h * h;
-    default: return 1.f;
-  }
-}
 __device__ __forceinline__ float stable_sigmoid(float u) {
   if (u >= 0.f) return 1.f / (1.f + expf(-u));
   const float e = expf(u);

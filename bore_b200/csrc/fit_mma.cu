@@ -235,7 +235,7 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
 // forward unit: NG tiles of H_l = act(A W_l + b_l), rows mb*16.., columns n0..
-template <int NG>
+template <int NG, bool EXT>
 __device__ __forceinline__ void fwd_unit(const float *A, int a_rs, const float2 *Wp, int ldw, const float *bs, float *H,
                                          int lda, int mb, int n0, int K, int act, int lane) {
   const int g = lane >> 2, t = lane & 3;
@@ -248,13 +248,13 @@ __device__ __forceinline__ void fwd_unit(const float *A, int a_rs, const float2 
     const int n = n0 + q * 8 + 2 * t;
     const float2 b = *reinterpret_cast<const float2 *>(bs + n);
     float *h0 = H + (mb * 16 + g) * lda + n;
-    *reinterpret_cast<float2 *>(h0) = make_float2(f_act(act, acc[q][0] + b.x), f_act(act, acc[q][1] + b.y));
-    *reinterpret_cast<float2 *>(h0 + 8 * lda) = make_float2(f_act(act, acc[q][2] + b.x), f_act(act, acc[q][3] + b.y));
+    *reinterpret_cast<float2 *>(h0) = make_float2(act_fwd<EXT>(act, acc[q][0] + b.x), act_fwd<EXT>(act, acc[q][1] + b.y));
+    *reinterpret_cast<float2 *>(h0 + 8 * lda) = make_float2(act_fwd<EXT>(act, acc[q][2] + b.x), act_fwd<EXT>(act, acc[q][3] + b.y));
   }
 }
 
 // reverse unit: NG tiles of D_{l-1} = (D_l W_l') . act'(H_{l-1}) and their column sums (bias gradient partials)
-template <int NG>
+template <int NG, bool EXT>
 __device__ __forceinline__ void bwd_unit(const float *Dl, int lda, const float2 *Wp, int ldw, const float *Hin, int h_rs,
                                          float *DN, float *cs, int mb, bool live, int n0, int K, int actp, int lane) {
   const int g = lane >> 2, t = lane & 3;
@@ -270,8 +270,8 @@ __device__ __forceinline__ void bwd_unit(const float *Dl, int lda, const float2 
       const float *h0 = Hin + (mb * 16 + g) * h_rs + n;
       const float2 hv0 = *reinterpret_cast<const float2 *>(h0);
       const float2 hv1 = *reinterpret_cast<const float2 *>(h0 + 8 * h_rs);
-      d0 = make_float2(acc[q][0] * f_act_bwd(actp, hv0.x), acc[q][1] * f_act_bwd(actp, hv0.y));
-      d1 = make_float2(acc[q][2] * f_act_bwd(actp, hv1.x), acc[q][3] * f_act_bwd(actp, hv1.y));
+      d0 = make_float2(acc[q][0] * act_bwd<EXT>(actp, hv0.x), acc[q][1] * act_bwd<EXT>(actp, hv0.y));
+      d1 = make_float2(acc[q][2] * act_bwd<EXT>(actp, hv1.x), acc[q][3] * act_bwd<EXT>(actp, hv1.y));
       float *o0 = DN + (mb * 16 + g) * lda + n;
       *reinterpret_cast<float2 *>(o0) = d0;
       *reinterpret_cast<float2 *>(o0 + 8 * lda) = d1;
@@ -287,7 +287,7 @@ __device__ __forceinline__ void bwd_unit(const float *Dl, int lda, const float2 
 }
 
 // ------------------------------------------------------------------------------------ the kernel
-template <int NW, int TPW>
+template <int NW, int TPW, bool EXT>
 __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit_mma_kernel(const FitMArgs a) {
   extern __shared__ __align__(16) float sm[];
   const MlpDesc &d = a.d;
@@ -436,9 +436,9 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
       const int groups = ntn / ng;
       for (int u = warp; u < nmb * groups; u += NW) {
         const int mb = u / groups, n0 = (u - mb * groups) * ng * 8;
-        if (ng == 4) fwd_unit<4>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane);
-        else if (ng == 2) fwd_unit<2>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane);
-        else fwd_unit<1>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane);
+        if (ng == 4) fwd_unit<4, EXT>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane);
+        else if (ng == 2) fwd_unit<2, EXT>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane);
+        else fwd_unit<1, EXT>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane);
       }
       __syncthreads();
     }
@@ -492,7 +492,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         float csum = 0.f;
         for (int r = rg; r < BP; r += RG) {
           const float hv = H[r * lda + j];
-          const float dv = du[r] * wj * f_act_bwd(actp, hv);
+          const float dv = du[r] * wj * act_bwd<EXT>(actp, hv);
           DN[r * lda + j] = dv;
           csum += dv;
         }
@@ -589,9 +589,9 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         for (int u = warp; u < 4 * groups; u += NW) {  // all four row blocks: dead ones publish zero column sums
           const int mb = u / groups, n0 = (u - mb * groups) * ng * 8;
           const bool live = mb < nmb;
-          if (ng == 4) bwd_unit<4>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane);
-          else if (ng == 2) bwd_unit<2>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane);
-          else bwd_unit<1>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane);
+          if (ng == 4) bwd_unit<4, EXT>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane);
+          else if (ng == 2) bwd_unit<2, EXT>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane);
+          else bwd_unit<1, EXT>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane);
         }
       }
       // (4) dW_l = H_{l-1}' delta_l on the tiles this warp owns
@@ -667,8 +667,9 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
 
 template <int NW, int TPW>
 int launch_cfg(const FitMArgs &a, int count, size_t smem, cudaStream_t stream) {
-  BORE_CUDA(cudaFuncSetAttribute(fit_mma_kernel<NW, TPW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  fit_mma_kernel<NW, TPW><<<count, NW * 32, smem, stream>>>(a);
+  const auto kern = acts_ext(a.d.act, a.d.n_layers) ? fit_mma_kernel<NW, TPW, true> : fit_mma_kernel<NW, TPW, false>;
+  BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<count, NW * 32, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());
   return 0;
 }

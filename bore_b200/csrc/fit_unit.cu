@@ -366,7 +366,8 @@ __device__ __forceinline__ float fu_row_sum(const float *__restrict__ a, int SP)
 // NH > 0: the net has NH hidden layers of HW units each (HW a multiple of 16) and the padded batch is SPT --
 // compile-time shape, D stays a run-time value; NH == 0: everything from the descriptor and the plan.
 // WT: per-sample loss weights (FuArgs::fw); the unweighted build runs none of their code.
-template <int NH, int HW, int SPT, bool WT>
+// EXT: the activation codes above BORE_ACT_TANH (act.cuh).
+template <int NH, int HW, int SPT, bool WT, bool EXT>
 __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_unit_kernel(const FuArgs a) {
   extern __shared__ __align__(16) float sm[];
   constexpr bool FIX = NH > 0;
@@ -548,7 +549,7 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
           if (rank * U + u < outd) {
             const float b = bs[u];
             *reinterpret_cast<float4 *>(Hn + u * SPP + s) =
-                make_float4(f_act(act, sum.x + b), f_act(act, sum.y + b), f_act(act, sum.z + b), f_act(act, sum.w + b));
+                make_float4(act_fwd<EXT>(act, sum.x + b), act_fwd<EXT>(act, sum.y + b), act_fwd<EXT>(act, sum.z + b), act_fwd<EXT>(act, sum.w + b));
           }
         });
         if (warp < FU_KS || U * (SP >> 2) > 32 * FU_KS) fu_fence_async();  // the slice's writers: generic-proxy stores -> visible to the bulk-copy engine
@@ -619,10 +620,10 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
           const float4 dz = *reinterpret_cast<const float4 *>(sm + P.dz + 4 * q);
           const float w = W[P.wl + k];
           float4 o;
-          o.x = dz.x * w * f_act_bwd(actp, hv.x);
-          o.y = dz.y * w * f_act_bwd(actp, hv.y);
-          o.z = dz.z * w * f_act_bwd(actp, hv.z);
-          o.w = dz.w * w * f_act_bwd(actp, hv.w);
+          o.x = dz.x * w * act_bwd<EXT>(actp, hv.x);
+          o.y = dz.y * w * act_bwd<EXT>(actp, hv.y);
+          o.z = dz.z * w * act_bwd<EXT>(actp, hv.z);
+          o.w = dz.w * w * act_bwd<EXT>(actp, hv.w);
           *reinterpret_cast<float4 *>(DF + k * SPP + 4 * q) = o;
         }
       }
@@ -652,8 +653,8 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
           if (rank * U + u < width) {
             const float4 hv = *reinterpret_cast<const float4 *>(Hi + u * SPP + s);
             *reinterpret_cast<float4 *>(Dn + u * SPP + s) =
-                make_float4(sum.x * f_act_bwd(actp, hv.x), sum.y * f_act_bwd(actp, hv.y), sum.z * f_act_bwd(actp, hv.z),
-                            sum.w * f_act_bwd(actp, hv.w));
+                make_float4(sum.x * act_bwd<EXT>(actp, hv.x), sum.y * act_bwd<EXT>(actp, hv.y), sum.z * act_bwd<EXT>(actp, hv.z),
+                            sum.w * act_bwd<EXT>(actp, hv.w));
           }
         });
         if (i >= 2) {
@@ -869,7 +870,9 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
 
 template <int NH, int HW, int SPT>
 static int fu_launch(const FuArgs &a, int count, size_t smem, cudaStream_t stream) {
-  const auto kern = a.fw.on ? fit_unit_kernel<NH, HW, SPT, true> : fit_unit_kernel<NH, HW, SPT, false>;
+  const auto kern = acts_ext(a.d.act, a.d.n_layers)
+                        ? (a.fw.on ? fit_unit_kernel<NH, HW, SPT, true, true> : fit_unit_kernel<NH, HW, SPT, false, true>)
+                        : (a.fw.on ? fit_unit_kernel<NH, HW, SPT, true, false> : fit_unit_kernel<NH, HW, SPT, false, false>);
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count * FU_C, FU_THREADS, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());

@@ -41,6 +41,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "act.cuh"
 #include "lbfgsb_fused.h"
 #include "lbfgsb_types.h"
 
@@ -159,26 +160,6 @@ struct FusedArgs {
   FusedPlan plan;
 };
 
-__device__ __forceinline__ float f_act_fwd(int a, float v) {
-  switch (a) {
-    case BORE_ACT_RELU: return fmaxf(v, 0.f);
-    case BORE_ACT_ELU: return v > 0.f ? v : expm1f(v);
-    case BORE_ACT_SIGMOID: return 1.f / (1.f + expf(-v));
-    case BORE_ACT_TANH: return tanhf(v);
-    default: return v;
-  }
-}
-// derivative wrt the pre-activation, through the layer OUTPUT h (as TF's *Grad kernels)
-__device__ __forceinline__ float f_act_bwd(int a, float h) {
-  switch (a) {
-    case BORE_ACT_RELU: return h > 0.f ? 1.f : 0.f;
-    case BORE_ACT_ELU: return h > 0.f ? 1.f : h + 1.f;
-    case BORE_ACT_SIGMOID: return h * (1.f - h);
-    case BORE_ACT_TANH: return 1.f - h * h;
-    default: return 1.f;
-  }
-}
-
 // CTA header in dynamic shared memory
 struct FusedHeader {
   FusedPlan plan;
@@ -209,7 +190,7 @@ template <> struct FVec<4> { float v[4]; __device__ __forceinline__ void load(co
 // -- the dtype flow of bore/decorators.py:54-56).  `strip` is the warp's activation scratch.
 // WIDTH = the net's width class; a lane owns T = WIDTH / 32 (>= 1) adjacent output units on the
 // way forward and input units lane, lane + 32, ... on the way back.
-template <int WIDTH>
+template <int WIDTH, bool EXT>
 __device__ __noinline__ float fused_eval(const FusedHeader *H, const float *__restrict__ wsm,
                                          float *__restrict__ strip, const double *__restrict__ x,
                                          double *__restrict__ g) {
@@ -261,7 +242,7 @@ __device__ __noinline__ float fused_eval(const FusedHeader *H, const float *__re
       FVec<T> bv, hv;
       bv.load(wsm + pl.b[l] + j0);
 #pragma unroll
-      for (int t = 0; t < T; ++t) hv.v[t] = f_act_fwd(a, acc[t] + bv.v[t]);
+      for (int t = 0; t < T; ++t) hv.v[t] = act_fwd<EXT>(a, acc[t] + bv.v[t]);
       hv.store(Hn + j0);  // pad units: zero weights and bias -> act(0), multiplied by zero rows later
     }
     __syncwarp();
@@ -280,7 +261,7 @@ __device__ __noinline__ float fused_eval(const FusedHeader *H, const float *__re
     for (int o = 1; o < UG; o <<= 1) up += __shfl_xor_sync(0xffffffffu, up, o);
   }
   const int act_last = pl.act[G];
-  const float u = f_act_fwd(act_last, up + H->b_last);
+  const float u = act_fwd<EXT>(act_last, up + H->b_last);
   const float v = -u;  // the mixin minimises transform(-u) (bore/mixins.py:20)
   float fval, dT;
   if (H->transform == BORE_TRANSFORM_SIGMOID) {
@@ -293,7 +274,7 @@ __device__ __noinline__ float fused_eval(const FusedHeader *H, const float *__re
     fval = v;
     dT = 1.f;
   }
-  const float dpre = -dT * f_act_bwd(act_last, u);
+  const float dpre = -dT * act_bwd<EXT>(act_last, u);
   // ---- reverse through the input ----
   if (G == 0) {
 #pragma unroll 1
@@ -304,7 +285,7 @@ __device__ __noinline__ float fused_eval(const FusedHeader *H, const float *__re
   {
     const int a = pl.act[G - 1];
 #pragma unroll 1
-    for (int k = lane; k < WIDTH; k += 32) HL[k] = dpre * wl[k] * f_act_bwd(a, HL[k]);  // (wl pad is zero)
+    for (int k = lane; k < WIDTH; k += 32) HL[k] = dpre * wl[k] * act_bwd<EXT>(a, HL[k]);  // (wl pad is zero)
   }
   __syncwarp();
 #pragma unroll 1
@@ -345,8 +326,8 @@ __device__ __noinline__ float fused_eval(const FusedHeader *H, const float *__re
       }
       if (l > 0) {
         // in place: every lane reads and writes only its own units, the j loop reads the strip above
-        if (va) Hin[ia] = a0 * f_act_bwd(a, Hin[ia]);
-        if (vb) Hin[ib] = b0 * f_act_bwd(a, Hin[ib]);
+        if (va) Hin[ia] = a0 * act_bwd<EXT>(a, Hin[ia]);
+        if (vb) Hin[ib] = b0 * act_bwd<EXT>(a, Hin[ib]);
       } else {
         if (va) g[ia] = (double)a0;
         if (vb) g[ib] = (double)b0;
@@ -357,13 +338,14 @@ __device__ __noinline__ float fused_eval(const FusedHeader *H, const float *__re
   return fval;
 }
 
+template <bool EXT>
 __device__ __forceinline__ float fused_eval_any(const FusedHeader *H, const float *wsm, float *strip,
                                                 const double *x, double *g) {
   switch (H->plan.width) {  // warp-uniform
-    case 16: return fused_eval<16>(H, wsm, strip, x, g);
-    case 32: return fused_eval<32>(H, wsm, strip, x, g);
-    case 64: return fused_eval<64>(H, wsm, strip, x, g);
-    default: return fused_eval<128>(H, wsm, strip, x, g);
+    case 16: return fused_eval<16, EXT>(H, wsm, strip, x, g);
+    case 32: return fused_eval<32, EXT>(H, wsm, strip, x, g);
+    case 64: return fused_eval<64, EXT>(H, wsm, strip, x, g);
+    default: return fused_eval<128, EXT>(H, wsm, strip, x, g);
   }
 }
 
@@ -407,7 +389,7 @@ __device__ __forceinline__ float *fused_carve(Work &w, unsigned char *base, int 
 
 constexpr int FUSED_MAX_WARPS = 12;
 
-template <int MC>
+template <int MC, bool EXT>
 __global__ void __launch_bounds__(FUSED_MAX_WARPS * 32, 1) lbfgsb_fused_kernel(const FusedArgs A) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int n = A.P.n, m = MC ? MC : A.P.m;
@@ -558,7 +540,7 @@ __global__ void __launch_bounds__(FUSED_MAX_WARPS * 32, 1) lbfgsb_fused_kernel(c
         } else {
           if (stage == 2) stage = 1;
           if (r == 1) {
-            s.f = (double)fused_eval_any(H, wsm, strip, w.x, w.g);
+            s.f = (double)fused_eval_any<EXT>(H, wsm, strip, w.x, w.g);
             if (!resumed_first) my_evals += 1;
             resumed_first = false;
           } else {
@@ -605,17 +587,17 @@ __global__ void __launch_bounds__(FUSED_MAX_WARPS * 32, 1) lbfgsb_fused_kernel(c
   if (lane == 0 && my_evals) atomicAdd(A.evals, my_evals);
 }
 
-template <int MC>
+template <int MC, bool EXT>
 int launch_fused_mc(const FusedArgs &A, int grid, int block, size_t smem, cudaStream_t stream) {
   static bool attr_done[64] = {};
   int dev = 0;
   BORE_CUDA(cudaGetDevice(&dev));
   if (dev >= 64 || !attr_done[dev]) {
-    BORE_CUDA(cudaFuncSetAttribute(lbfgsb_fused_kernel<MC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    BORE_CUDA(cudaFuncSetAttribute(lbfgsb_fused_kernel<MC, EXT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    227 * 1024));
     if (dev < 64) attr_done[dev] = true;
   }
-  lbfgsb_fused_kernel<MC><<<grid, block, smem, stream>>>(A);
+  lbfgsb_fused_kernel<MC, EXT><<<grid, block, smem, stream>>>(A);
   BORE_CUDA(cudaGetLastError());
   return 0;
 }
@@ -703,8 +685,11 @@ int launch_lbfgsb_fused(const bore_mlp *h, int model0, int n_models, int per_mod
   const size_t smem = fixed + wpb * A.warp_bytes;
   if (resume) BORE_CUDA(cudaMemsetAsync(resume->qhead, 0, sizeof(int), stream));
   else BORE_CUDA(cudaMemsetAsync(work_dev, 0, 16, stream));
-  const int rc = m == 10 ? launch_fused_mc<10>(A, grid, wpb * 32, smem, stream)
-                         : launch_fused_mc<0>(A, grid, wpb * 32, smem, stream);
+  const bool ext = acts_ext(h->desc.act, h->desc.n_layers);
+  const int rc = m == 10 ? (ext ? launch_fused_mc<10, true>(A, grid, wpb * 32, smem, stream)
+                                : launch_fused_mc<10, false>(A, grid, wpb * 32, smem, stream))
+                         : (ext ? launch_fused_mc<0, true>(A, grid, wpb * 32, smem, stream)
+                                : launch_fused_mc<0, false>(A, grid, wpb * 32, smem, stream));
   if (rc) return rc;
   if (info) { info->grid = grid; info->block = wpb * 32; info->smem = smem; }
   if (evals_out) {

@@ -25,6 +25,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "act.cuh"
 
 #define LSTM_MAX_LAYERS 4
 #define LSTM_MAX_UNITS 32
@@ -53,24 +54,6 @@ struct bore_lstm {
 
 namespace {
 
-__device__ __forceinline__ float l_act(int a, float v) {
-  switch (a) {
-    case BORE_ACT_RELU: return fmaxf(v, 0.f);
-    case BORE_ACT_ELU: return v > 0.f ? v : expm1f(v);
-    case BORE_ACT_SIGMOID: return 1.f / (1.f + expf(-v));
-    case BORE_ACT_TANH: return tanhf(v);
-    default: return v;
-  }
-}
-__device__ __forceinline__ float l_act_bwd(int a, float h) {  // through the OUTPUT, as TF's *Grad kernels
-  switch (a) {
-    case BORE_ACT_RELU: return h > 0.f ? 1.f : 0.f;
-    case BORE_ACT_ELU: return h > 0.f ? 1.f : h + 1.f;
-    case BORE_ACT_SIGMOID: return h * (1.f - h);
-    case BORE_ACT_TANH: return 1.f - h * h;
-    default: return 1.f;
-  }
-}
 __device__ __forceinline__ float l_sigmoid(float v) { return 1.f / (1.f + expf(-v)); }
 
 __host__ __device__ inline int in_dim(const LstmDesc &d, int l) { return l == 0 ? d.D : d.U; }
@@ -115,6 +98,7 @@ __device__ __forceinline__ Strip carve_strip(const LstmDesc &d, float *base) {
 // strip, c in the caller's registers: c[l] is the state of unit `lane`).  With `keep` the gate
 // values are stored for the way back.  `live` = the step is not masked.  Returns nothing; the top
 // cell's output is s.h + (L-1)*U.
+template <bool EXT>
 __device__ __forceinline__ void stack_forward(const LstmDesc &d, const float *__restrict__ ws, const Strip &s,
                                               float (&c)[LSTM_MAX_LAYERS], int t, bool live, bool keep,
                                               int lane) {
@@ -142,10 +126,10 @@ __device__ __forceinline__ void stack_forward(const LstmDesc &d, const float *__
       const float *w = W + (in + k) * LD;
       z0 = fmaf(hv, w[0], z0); z1 = fmaf(hv, w[U], z1); z2 = fmaf(hv, w[2 * U], z2); z3 = fmaf(hv, w[3 * U], z3);
     }
-    const float gi = l_sigmoid(z0), gf = l_sigmoid(z1), gg = l_act(act, z2), go = l_sigmoid(z3);
+    const float gi = l_sigmoid(z0), gf = l_sigmoid(z1), gg = act_fwd<EXT>(act, z2), go = l_sigmoid(z3);
     const float cp = c[l];
     const float cn = gf * cp + gi * gg;
-    const float ac = l_act(act, cn);
+    const float ac = act_fwd<EXT>(act, cn);
     __syncwarp();  // every lane has read the old h of this cell
     if (on) {
       hl[lane] = go * ac;
@@ -164,6 +148,7 @@ __device__ __forceinline__ void stack_forward(const LstmDesc &d, const float *__
 // c_t from step t+1.  Leaves the gate gradient dz (4U) in s.dz and  din = dz W'  (gradient wrt the
 // cell's input, rows [0, in), and wrt h_{t-1}, rows [in, in+U)) in s.din; returns the gradient wrt
 // c_{t-1} of unit `lane`.
+template <bool EXT>
 __device__ __forceinline__ float cell_backward(const LstmDesc &d, const float *__restrict__ ws, const Strip &s,
                                                int t, int l, float dht, float dc_in, int lane) {
   const int U = d.U, LD = ldw(d), act = d.act, G4 = 4 * U;
@@ -172,10 +157,10 @@ __device__ __forceinline__ float cell_backward(const LstmDesc &d, const float *_
   const float *a = s.acts + ((size_t)(t * d.L + l) * 6) * U + (on ? lane : 0);
   const float gi = a[0], gf = a[U], gg = a[2 * U], go = a[3 * U], ac = a[4 * U], cp = a[5 * U];
   const float d_o = dht * ac * go * (1.f - go);
-  const float dct = dht * go * l_act_bwd(act, ac) + dc_in;
+  const float dct = dht * go * act_bwd<EXT>(act, ac) + dc_in;
   const float d_i = dct * gg * gi * (1.f - gi);
   const float d_f = dct * cp * gf * (1.f - gf);
-  const float d_g = dct * gi * l_act_bwd(act, gg);
+  const float d_g = dct * gi * act_bwd<EXT>(act, gg);
   __syncwarp();
   if (on) { s.dz[lane] = d_i; s.dz[U + lane] = d_f; s.dz[2 * U + lane] = d_g; s.dz[3 * U + lane] = d_o; }
   __syncwarp();
@@ -200,6 +185,7 @@ __device__ __forceinline__ float cell_backward(const LstmDesc &d, const float *_
 // forward of many sequences (predict / evaluate of the many-to-many network, and the one-to-one
 // network when x_repeat != 0): warp per sample.  X [S][T][D] (or [S][D] repeated T times), out [S][T]
 // logits (or [S] = the last step's logit when last_only).
+template <bool EXT>
 __global__ void __launch_bounds__(256)
 lstm_forward_kernel(const LstmDesc d, const float *__restrict__ params, const float *__restrict__ X, int S,
                     int T, int x_repeat, float mask_value, int use_mask, int last_only, float *__restrict__ out) {
@@ -223,7 +209,7 @@ lstm_forward_kernel(const LstmDesc d, const float *__restrict__ params, const fl
       for (int k = lane; k < d.D; k += 32) { const float v = xt[k]; s.xin[k] = v; differs |= (v != mask_value); }
       const bool live = !use_mask || __any_sync(0xffffffffu, differs);
       __syncwarp();
-      stack_forward(d, ws, s, c, t, live, false, lane);
+      stack_forward<EXT>(d, ws, s, c, t, live, false, lane);
       if (!last_only || t == T - 1) {
         float u = lane < U ? s.h[(d.L - 1) * U + lane] * ws[d.s_wd + lane] : 0.f;
 #pragma unroll
@@ -236,6 +222,7 @@ lstm_forward_kernel(const LstmDesc d, const float *__restrict__ params, const fl
 }
 
 // value f = T(sign * u(x)) and df/dx of the one-to-one network with T steps (x repeated): warp per point
+template <bool EXT>
 __global__ void __launch_bounds__(128)
 lstm_value_grad_kernel(const LstmDesc d, const float *__restrict__ params, const void *__restrict__ Xv, int x_is_f64,
                        int S, int T, int transform, float sign, const int *__restrict__ flags,
@@ -264,7 +251,7 @@ lstm_value_grad_kernel(const LstmDesc d, const float *__restrict__ params, const
       for (int k = lane; k < d.D; k += 32) s.xin[k] = x[k];
     }
     __syncwarp();
-    for (int t = 0; t < T; ++t) stack_forward(d, ws, s, c, t, true, true, lane);
+    for (int t = 0; t < T; ++t) stack_forward<EXT>(d, ws, s, c, t, true, true, lane);
     float u = lane < U ? s.h[(L - 1) * U + lane] * ws[d.s_wd + lane] : 0.f;
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) u += __shfl_xor_sync(0xffffffffu, u, o);
@@ -283,7 +270,7 @@ lstm_value_grad_kernel(const LstmDesc d, const float *__restrict__ params, const
       float dabove = (t == T - 1 && lane < U) ? du * ws[d.s_wd + lane] : 0.f;  // the Dense layer sees the last step
       for (int l = L - 1; l >= 0; --l) {
         const int in = in_dim(d, l);
-        const float dcp = cell_backward(d, ws, s, t, l, dh[l] + dabove, dc[l], lane);
+        const float dcp = cell_backward<EXT>(d, ws, s, t, l, dh[l] + dabove, dc[l], lane);
         dh[l] = lane < U ? s.din[in + lane] : 0.f;
         dc[l] = dcp;
         dabove = (l > 0 && lane < U) ? s.din[lane] : 0.f;
@@ -313,6 +300,7 @@ struct LstmFitArgs {
   float *scratch;       // A [L][T][B][AW] | Z [L][T][B][4U] | HT [T][B][U] | DU [T][B]
 };
 
+template <bool EXT>
 __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
   extern __shared__ __align__(16) float sm[];
   const LstmDesc &d = a.d;
@@ -362,7 +350,7 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
           const bool live = __any_sync(0xffffffffu, differs);
           if (live) live_mask |= 1u << t;
           __syncwarp();
-          stack_forward(d, ws, s, c, t, live, true, lane);
+          stack_forward<EXT>(d, ws, s, c, t, live, true, lane);
           float u = lane < U ? s.h[(L - 1) * U + lane] * ws[d.s_wd + lane] : 0.f;
 #pragma unroll
           for (int o = 16; o > 0; o >>= 1) u += __shfl_xor_sync(0xffffffffu, u, o);
@@ -409,7 +397,7 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
           float dabove = lane < U ? du_t[t] * ws[d.s_wd + lane] : 0.f;  // TimeDistributed(Dense) at this step
           for (int l = L - 1; l >= 0; --l) {
             const int in = in_dim(d, l);
-            const float dcp = cell_backward(d, ws, s, t, l, dh[l] + dabove, dc[l], lane);
+            const float dcp = cell_backward<EXT>(d, ws, s, t, l, dh[l] + dabove, dc[l], lane);
             // rows for the weight GEMMs: [input of the cell at step t ; h_{t-1}] and dz
             float *Zr = gZ + (((size_t)l * T + t) * B + b) * G4;
             float *Ar = gA + (((size_t)l * T + t) * B + b) * AW;
@@ -614,7 +602,7 @@ int bore_lstm_create(int input_dim, int units, int num_layers, int activation, i
              LSTM_MAX_UNITS);
   BORE_CHECK(num_layers >= 1 && num_layers <= LSTM_MAX_LAYERS, "bore_lstm_create: num_layers=%d outside [1,%d]",
              num_layers, LSTM_MAX_LAYERS);
-  BORE_CHECK(activation >= BORE_ACT_LINEAR && activation <= BORE_ACT_TANH, "bore_lstm_create: unknown activation %d",
+  BORE_CHECK(activation >= BORE_ACT_LINEAR && activation <= BORE_ACT_EXPONENTIAL, "bore_lstm_create: unknown activation %d",
              activation);
   BORE_CHECK(bore_device_count() > 0, "bore_lstm_create: no CUDA device visible -- bore_b200 has no CPU fallback");
   BORE_CUDA(cudaSetDevice(device));
@@ -707,10 +695,11 @@ int bore_lstm_predict_sequences(bore_lstm *h, const float *X_dev, int S, int T, 
   BORE_CUDA(cudaSetDevice(h->device));
   const int warps = 8;
   const size_t smem = ((size_t)((h->desc.s_total + 3) & ~3) + (size_t)warps * strip_floats(h->desc, T, false)) * sizeof(float);
-  BORE_CUDA(cudaFuncSetAttribute(lstm_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const auto kernel = acts_ext(&h->desc.act, 1) ? lstm_forward_kernel<true> : lstm_forward_kernel<false>;
+  BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int grid = std::min((S + warps - 1) / warps, h->sm_count * 2);
-  lstm_forward_kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(h->desc, h->params, X_dev, S, T, 0, mask_value,
-                                                                       use_mask, 0, out_dev);
+  kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(h->desc, h->params, X_dev, S, T, 0, mask_value, use_mask, 0,
+                                                          out_dev);
   BORE_CUDA(cudaGetLastError());
   return 0;
 }
@@ -725,10 +714,11 @@ int bore_lstm_predict(bore_lstm *h, const float *X_dev, int S, int num_steps, fl
   BORE_CUDA(cudaSetDevice(h->device));
   const int warps = 8;
   const size_t smem = ((size_t)((h->desc.s_total + 3) & ~3) + (size_t)warps * strip_floats(h->desc, num_steps, false)) * sizeof(float);
-  BORE_CUDA(cudaFuncSetAttribute(lstm_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const auto kernel = acts_ext(&h->desc.act, 1) ? lstm_forward_kernel<true> : lstm_forward_kernel<false>;
+  BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int grid = std::min((S + warps - 1) / warps, h->sm_count * 2);
-  lstm_forward_kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(h->desc, h->params, X_dev, S, num_steps, 1, 0.f,
-                                                                       0, 1, out_dev);
+  kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(h->desc, h->params, X_dev, S, num_steps, 1, 0.f, 0, 1,
+                                                          out_dev);
   BORE_CUDA(cudaGetLastError());
   return 0;
 }
@@ -748,9 +738,10 @@ int bore_lstm_value_and_grad(bore_lstm *h, int num_steps, int transform, int neg
   const int warps = 4;
   const size_t smem = ((size_t)((h->desc.s_total + 3) & ~3) + (size_t)warps * strip_floats(h->desc, num_steps, true)) * sizeof(float);
   BORE_CHECK(smem <= 227 * 1024, "bore_lstm_value_and_grad: needs %zu B of shared memory", smem);
-  BORE_CUDA(cudaFuncSetAttribute(lstm_value_grad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const auto kernel = acts_ext(&h->desc.act, 1) ? lstm_value_grad_kernel<true> : lstm_value_grad_kernel<false>;
+  BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int grid = std::min((S + warps - 1) / warps, h->sm_count * 2);
-  lstm_value_grad_kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(
+  kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(
       h->desc, h->params, X_dev, x_is_f64, S, num_steps, transform, negate ? -1.f : 1.f, flags_dev, f_dev, g_dev);
   BORE_CUDA(cudaGetLastError());
   return 0;
@@ -791,8 +782,9 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   const size_t tiles = (size_t)LSTM_MAX_BATCH * (AW + 4 * h->desc.U);
   const size_t smem = ((size_t)((h->desc.s_total + 3) & ~3) + std::max(strips, tiles)) * sizeof(float);
   BORE_CHECK(smem <= 227 * 1024, "bore_lstm_fit: needs %zu B of shared memory", smem);
-  BORE_CUDA(cudaFuncSetAttribute(lstm_fit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  lstm_fit_kernel<<<1, warps * 32, smem, (cudaStream_t)stream>>>(a);
+  const auto kernel = acts_ext(&h->desc.act, 1) ? lstm_fit_kernel<true> : lstm_fit_kernel<false>;
+  BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kernel<<<1, warps * 32, smem, (cudaStream_t)stream>>>(a);
   BORE_CUDA(cudaGetLastError());
   h->adam_t += (long long)epochs * ((N + batch_size - 1) / batch_size);
   return 0;

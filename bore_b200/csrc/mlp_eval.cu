@@ -30,6 +30,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "act.cuh"
 
 namespace {
 
@@ -41,26 +42,6 @@ struct Map {
   static constexpr int CH = 4 * UG;          // units per chunk
   static constexpr int AST = TP + 4;         // activation strip row stride (floats)
 };
-
-__device__ __forceinline__ float act_fwd(int a, float v) {
-  switch (a) {
-    case BORE_ACT_RELU: return fmaxf(v, 0.f);
-    case BORE_ACT_ELU: return v > 0.f ? v : expm1f(v);
-    case BORE_ACT_SIGMOID: return 1.f / (1.f + expf(-v));
-    case BORE_ACT_TANH: return tanhf(v);
-    default: return v;
-  }
-}
-// derivative wrt the pre-activation, through the layer OUTPUT h
-__device__ __forceinline__ float act_bwd(int a, float h) {
-  switch (a) {
-    case BORE_ACT_RELU: return h > 0.f ? 1.f : 0.f;
-    case BORE_ACT_ELU: return h > 0.f ? 1.f : h + 1.f;
-    case BORE_ACT_SIGMOID: return h * (1.f - h);
-    case BORE_ACT_TANH: return 1.f - h * h;
-    default: return 1.f;
-  }
-}
 
 struct SmemPlan {
   int wf[BORE_MAX_LAYERS];   // weights [inP][outP + 4] (rows >= in and columns >= out are zero)
@@ -253,7 +234,7 @@ mlp_pack_kernel(const MlpDesc d, const SmemPlan P, int CH, int grad, const float
 
 __device__ __forceinline__ uint32_t smem_addr(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
-template <bool GRAD, int UGB, bool F2>
+template <bool GRAD, int UGB, bool F2, bool EXT>
 __global__ void __launch_bounds__(512)
 mlp_eval_kernel(const MlpDesc d, const SmemPlan P, const float *__restrict__ params,
                 const float *__restrict__ packed, const float *__restrict__ X,
@@ -381,10 +362,10 @@ mlp_eval_kernel(const MlpDesc d, const SmemPlan P, const float *__restrict__ par
           const int unit = c + ug * 4 + u;
           const float b = bs[unit];
           float4 o;
-          o.x = act_fwd(a, acc[0][u] + b);
-          o.y = act_fwd(a, acc[1][u] + b);
-          o.z = act_fwd(a, acc[2][u] + b);
-          o.w = act_fwd(a, acc[3][u] + b);
+          o.x = act_fwd<EXT>(a, acc[0][u] + b);
+          o.y = act_fwd<EXT>(a, acc[1][u] + b);
+          o.z = act_fwd<EXT>(a, acc[2][u] + b);
+          o.w = act_fwd<EXT>(a, acc[3][u] + b);
           *reinterpret_cast<float4 *>(H + unit * AST + pg * 4) = o;
         }
       }
@@ -410,7 +391,7 @@ mlp_eval_kernel(const MlpDesc d, const SmemPlan P, const float *__restrict__ par
     float dpre[4];
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-      const float u = act_fwd(act_last, up[i] + b_last);
+      const float u = act_fwd<EXT>(act_last, up[i] + b_last);
       float fval, dT;
       if (GRAD) {
         const float v = sign * u;
@@ -424,7 +405,7 @@ mlp_eval_kernel(const MlpDesc d, const SmemPlan P, const float *__restrict__ par
           fval = v;
           dT = 1.f;
         }
-        dpre[i] = dT * sign * act_bwd(act_last, u);
+        dpre[i] = dT * sign * act_bwd<EXT>(act_last, u);
       } else {
         fval = u;
       }
@@ -452,10 +433,10 @@ mlp_eval_kernel(const MlpDesc d, const SmemPlan P, const float *__restrict__ par
       for (int k = ug; k < P.wl_len; k += UG) {
         float4 hv = *reinterpret_cast<const float4 *>(HL + k * AST + pg * 4);
         const float w = wl[k];
-        hv.x = dpre[0] * w * act_bwd(a, hv.x);
-        hv.y = dpre[1] * w * act_bwd(a, hv.y);
-        hv.z = dpre[2] * w * act_bwd(a, hv.z);
-        hv.w = dpre[3] * w * act_bwd(a, hv.w);
+        hv.x = dpre[0] * w * act_bwd<EXT>(a, hv.x);
+        hv.y = dpre[1] * w * act_bwd<EXT>(a, hv.y);
+        hv.z = dpre[2] * w * act_bwd<EXT>(a, hv.z);
+        hv.w = dpre[3] * w * act_bwd<EXT>(a, hv.w);
         *reinterpret_cast<float4 *>(HL + k * AST + pg * 4) = hv;
       }
     }
@@ -475,10 +456,10 @@ mlp_eval_kernel(const MlpDesc d, const SmemPlan P, const float *__restrict__ par
           for (int u = 0; u < 4; ++u) {
             float *hp = Hin + (c + ug + UG * u) * AST + pg * 4;
             float4 hv = *reinterpret_cast<const float4 *>(hp);
-            hv.x = acc[0][u] * act_bwd(a, hv.x);
-            hv.y = acc[1][u] * act_bwd(a, hv.y);
-            hv.z = acc[2][u] * act_bwd(a, hv.z);
-            hv.w = acc[3][u] * act_bwd(a, hv.w);
+            hv.x = acc[0][u] * act_bwd<EXT>(a, hv.x);
+            hv.y = acc[1][u] * act_bwd<EXT>(a, hv.y);
+            hv.z = acc[2][u] * act_bwd<EXT>(a, hv.z);
+            hv.w = acc[3][u] * act_bwd<EXT>(a, hv.w);
             *reinterpret_cast<float4 *>(hp) = hv;
           }
         }
@@ -581,18 +562,16 @@ static int launch_variant(const bore_mlp *h, const MlpDesc &d, int model0, const
   // packed FFMA2 inner loops unless BORE_K2_FFMA2=0 (the scalar-FFMA build stays for A/B timing; the
   // two give bit-identical results)
   static const bool f2 = [] { const char *e = getenv("BORE_K2_FFMA2"); return !(e && e[0] == '0'); }();
-  static bool attr_done[2][64] = {};  // per device: the attribute belongs to the device's context
-  if (h->device >= 64 || !attr_done[f2][h->device]) {
-    BORE_CUDA(cudaFuncSetAttribute(f2 ? mlp_eval_kernel<GRAD, UGB, true> : mlp_eval_kernel<GRAD, UGB, false>,
-                                   cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 256));
-    if (h->device < 64) attr_done[f2][h->device] = true;
+  const bool ext = acts_ext(d.act, d.n_layers);
+  const auto kernel = f2 ? (ext ? mlp_eval_kernel<GRAD, UGB, true, true> : mlp_eval_kernel<GRAD, UGB, true, false>)
+                         : (ext ? mlp_eval_kernel<GRAD, UGB, false, true> : mlp_eval_kernel<GRAD, UGB, false, false>);
+  static bool attr_done[2][2][64] = {};  // per device: the attribute belongs to the device's context
+  if (h->device >= 64 || !attr_done[f2][ext][h->device]) {
+    BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 256));
+    if (h->device < 64) attr_done[f2][ext][h->device] = true;
   }
-  if (f2)
-    mlp_eval_kernel<GRAD, UGB, true><<<grid, warps * 32, smem, stream>>>(d, P, params, packed, X, S, n_dev, list,
-                                                                       f, g, transform, sign, per_model, flags);
-  else
-    mlp_eval_kernel<GRAD, UGB, false><<<grid, warps * 32, smem, stream>>>(d, P, params, packed, X, S, n_dev, list,
-                                                                        f, g, transform, sign, per_model, flags);
+  kernel<<<grid, warps * 32, smem, stream>>>(d, P, params, packed, X, S, n_dev, list, f, g, transform, sign, per_model,
+                                             flags);
   BORE_CUDA(cudaGetLastError());
   return 0;
 }

@@ -12,7 +12,9 @@ import numpy as np
 
 from . import _lib
 
-ACT_CODES = {"linear": 0, None: 0, "relu": 1, "elu": 2, "sigmoid": 3, "tanh": 4}
+# BORE_ACT_* of include/bore_b200.h
+ACT_CODES = {"linear": 0, None: 0, "relu": 1, "elu": 2, "sigmoid": 3, "tanh": 4, "selu": 5, "softplus": 6,
+             "softsign": 7, "hard_sigmoid": 8, "exponential": 9}
 TRANSFORM_CODES = {"identity": 0, "sigmoid": 1, "exp": 2}
 
 # scipy.optimize L-BFGS-B task codes -> message (scipy/optimize/_lbfgsb_py.py:49-90)

@@ -4,7 +4,22 @@ Keras itself is absent (and not wanted on the path); these are plain spec object
 ``bore_b200.models.Sequential`` lowers onto the native handle.  Names and arguments follow
 the call sites README.rst:60-66 and bore/plugins/hpbandster/base.py:113-116,147-158."""
 
-_ACTIVATIONS = ("linear", "relu", "elu", "sigmoid", "tanh")
+# Keras 2.5 element-wise activations whose derivative is a function of the layer output, the one value the
+# kernels keep (swish and gelu are not: DESIGN.md, "Activations")
+_ACTIVATIONS = ("linear", "relu", "elu", "sigmoid", "tanh", "selu", "softplus", "softsign", "hard_sigmoid",
+                "exponential")
+
+
+def activation_name(activation, owner):
+    """The Keras name of ``activation`` (a name, a Keras-named callable or None, which is linear);
+    ValueError naming the accepted ones for any other."""
+    if callable(activation):
+        activation = getattr(activation, "__name__", activation)
+    if activation is None:
+        activation = "linear"
+    if activation not in _ACTIVATIONS:
+        raise ValueError(f"{owner}: activation must be one of {_ACTIVATIONS}, got {activation!r}")
+    return activation
 
 
 class L2:
@@ -28,12 +43,7 @@ class Dense:
             raise TypeError(f"Dense: unsupported arguments {sorted(kwargs)}")
         if not use_bias:
             raise NotImplementedError("Dense(use_bias=False) is not on the BORE-MLP path")
-        if callable(activation):
-            activation = getattr(activation, "__name__", activation)
-        if activation is None:
-            activation = "linear"
-        if activation not in _ACTIVATIONS:
-            raise ValueError(f"Dense: activation must be one of {_ACTIVATIONS}, got {activation!r}")
+        activation = activation_name(activation, "Dense")
         if input_shape is not None and input_dim is None:
             (input_dim,) = input_shape
         self.units = int(units)

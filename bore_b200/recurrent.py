@@ -22,7 +22,7 @@ import numpy as np
 
 from . import _lib, ops
 from .engine import ACT_CODES, TRANSFORM_CODES, NativeMLP, _np_ptr, _ptr, _torch
-from .layers import Adam, BinaryCrossentropy, Dense
+from .layers import Adam, BinaryCrossentropy, Dense, activation_name
 from .mixins import MaximizableMixin
 from .models import History
 
@@ -38,10 +38,7 @@ class LSTMCell:
                  bias_regularizer=None, **kwargs):
         if kwargs:
             raise TypeError(f"LSTMCell: unsupported arguments {sorted(kwargs)}")
-        if activation is None:
-            activation = "linear"
-        if activation not in ACT_CODES:
-            raise ValueError(f"LSTMCell: unknown activation {activation!r}")
+        activation = activation_name(activation, "LSTMCell")
         self.units = int(units)
         self.activation = activation
         self.kernel_regularizer = kernel_regularizer

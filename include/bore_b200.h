@@ -30,9 +30,11 @@ extern "C" {
 
 #define BORE_ABI_VERSION 1
 
-/* activations of a Dense layer (Keras names: linear, relu, elu, sigmoid, tanh) */
+/* activations of a Dense layer or an LSTM cell (Keras names: linear, relu, elu, sigmoid, tanh, selu,
+ * softplus, softsign, hard_sigmoid, exponential) */
 enum { BORE_ACT_LINEAR = 0, BORE_ACT_RELU = 1, BORE_ACT_ELU = 2, BORE_ACT_SIGMOID = 3,
-       BORE_ACT_TANH = 4 };
+       BORE_ACT_TANH = 4, BORE_ACT_SELU = 5, BORE_ACT_SOFTPLUS = 6, BORE_ACT_SOFTSIGN = 7,
+       BORE_ACT_HARD_SIGMOID = 8, BORE_ACT_EXPONENTIAL = 9 };
 /* output transforms, TRANSFORMS of bore/plugins/hpbandster/base.py:18 */
 enum { BORE_TRANSFORM_IDENTITY = 0, BORE_TRANSFORM_SIGMOID = 1, BORE_TRANSFORM_EXP = 2 };
 /* per-start termination status, scipy.optimize.OptimizeResult.status for L-BFGS-B */
