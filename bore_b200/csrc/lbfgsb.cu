@@ -230,6 +230,18 @@ __device__ __forceinline__ void bulk_prefetch_l2(const void *src, uint32_t bytes
 __device__ __forceinline__ void fence_async_smem() {  // generic-proxy smem writes -> async proxy
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 }
+// per-lane asynchronous copies (4 or 8 bytes: rows of any length and alignment), and the arrive on an
+// mbarrier that fires once all of this lane's earlier copies have landed (.noinc: the barrier's
+// expected count includes these arrivals)
+template <int BYTES>
+__device__ __forceinline__ void cp_async_g2s(void *dst_smem, const void *src) {
+  static_assert(BYTES == 4 || BYTES == 8, "cp.async.ca copies 4, 8 or 16 bytes");
+  asm volatile("cp.async.ca.shared.global [%0], [%1], %2;" ::"r"(smem_u32(dst_smem)), "l"(src), "n"(BYTES)
+               : "memory");
+}
+__device__ __forceinline__ void cp_async_arrive(uint64_t *bar) {
+  asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
 
 // Extra barriers per new iteration at which the warps of a CTA re-align (lb_advance's
 // mem.phase()): at most 4 (before the Cauchy point, the K factorisation, the subspace
@@ -240,7 +252,8 @@ __device__ __forceinline__ void fence_async_smem() {  // generic-proxy smem writ
 constexpr int LB_NPHASE_MAX = 4;
 
 // A start's block is staged in two pieces: the prefix (scalars | t r d z) when the item is
-// claimed, the limited-memory part (W and the m x m matrices, 87 % of the bytes) only when the
+// claimed -- together with the request x, the gradient row and f that its light stage reads, all on
+// one mbarrier -- the limited-memory part (W and the m x m matrices, 87 % of the bytes) only when the
 // light stage finds that a new iteration begins -- about half of all steps just continue a line
 // search and never touch it.  The kernel requests the second piece right before the rendezvous
 // (whose wait hides the latency); load() -- the hook lb_advance calls where the matrices are first
@@ -315,26 +328,25 @@ __global__ void __maxnreg__(168) lbfgsb_warp_kernel(LbDev D, int round, size_t w
   int &kn_wait = reinterpret_cast<int *>(bars + 2 * wpb)[0];
   int &kn_done = reinterpret_cast<int *>(bars + 2 * wpb)[1];
   if (threadIdx.x == 0) { kn_wait = 0; kn_done = 0; }
-  // claim a position of the active list (>= n_active: the list is exhausted)
-  auto claim = [&]() {
-    int v = 0;
-    if (lane == 0) v = atomicAdd(qhead, 1);
-    return __shfl_sync(0xffffffffu, v, 0);
-  };
-  // cur_i: the item whose block is staged (or on its way) in this warp's workspace;
-  // nxt_i: the one after it, already claimed and prefetched into L2
-  int cur_i = claim();
-  int nxt_sid = -1;  // start id of the item claimed ahead (loaded with the claim)
+  // cur_i: the item whose block is staged (or on its way) in this warp's workspace, cur_sid its
+  // start; nxt_i / nxt_sid: the one after it, claimed while cur_i runs and prefetched into L2
+  // (a position >= n_active: the list is exhausted)
+  int cur_i = 0;
+  if (lane == 0) cur_i = atomicAdd(qhead, 1);
+  cur_i = __shfl_sync(0xffffffffu, cur_i, 0);
+  int cur_sid = cur_i < n_active ? list_cur[cur_i] : -1;
   if (lane == 0) {
-    mbar_init(bar, 1);
+    // the first piece's barrier completes on the bulk copy (one arrival with its byte count) and
+    // on one cp.async arrival per lane (the light stage's x, g and f rows)
+    mbar_init(bar, 1 + 32);
     mbar_init(bar2, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    if (cur_i < n_active) {
+    if (cur_sid >= 0) {
       mbar_expect_tx(bar, p1_bytes);
-      bulk_g2s(base, D.blocks + D.block_stride * list_cur[cur_i], p1_bytes, bar);
+      bulk_g2s(base, D.blocks + D.block_stride * cur_sid, p1_bytes, bar);
     }
   }
-  int nxt_i = n_active;
+  int nxt_i = n_active, nxt_sid = -1;
 #pragma unroll 1
   for (int o = threadIdx.x; o < LB_FORMK_ACC * 32; o += blockDim.x) ftab[o] = lbw::lb_formk_code(o, m);
 #pragma unroll 1
@@ -357,6 +369,26 @@ __global__ void __maxnreg__(168) lbfgsb_warp_kernel(LbDev D, int round, size_t w
   uint32_t parity = 0, parity2 = 0;
   unsigned long long my_bytes = 0, my_evals = 0;
 
+  // The light stage's inputs of item `st`, copied asynchronously into the workspace: the request
+  // x straight into w.x, the g row into w.g -- an fp32 row into its upper half, widened in place
+  // once it has landed -- and f into w.q (scratch that nothing reads before the heavy stage).
+  // Per-lane copies, so that a row of any length and alignment lands; each lane's arrival on `bar`
+  // fires when its copies are done.  Callers order the workspace's earlier generic accesses first.
+  const int g_off = sizeof(FG) == 4 ? LB_NV(n) : 0;  // in FG elements
+  auto stage_light = [&](int st) {
+    const double *xr = D.xreq + (size_t)st * n;
+    const FG *gr = G + (size_t)st * n;
+    FG *gs = reinterpret_cast<FG *>(w.g) + g_off;
+#pragma unroll 1
+    for (int i = lane; i < n; i += 32) {
+      cp_async_g2s<8>(w.x + i, xr + i);
+      cp_async_g2s<sizeof(FG)>(gs + i, gr + i);
+    }
+    if (lane == 31) cp_async_g2s<sizeof(FG)>(w.q, F + st);
+    cp_async_arrive(bar);
+  };
+  if (cur_sid >= 0) stage_light(cur_sid);
+
   LbScal s;
   BlockMem mem;
   int sid = 0, col_in = 0;
@@ -364,6 +396,9 @@ __global__ void __maxnreg__(168) lbfgsb_warp_kernel(LbDev D, int round, size_t w
 
   // write an item back and put the next one on its way
   auto finish = [&](int pend) {
+    // the slot in the next round's list: the atomic's result is used only after the stores below
+    int pos = 0;
+    if (pend && lane == 0) pos = atomicAdd(&D.cnt[nxt], 1);
     char *gblock = D.blocks + D.block_stride * sid;
     double *xr = D.xreq + (size_t)sid * n;
     if (mem.requested) {  // the second piece must have landed before its workspace is reused
@@ -373,16 +408,16 @@ __global__ void __maxnreg__(168) lbfgsb_warp_kernel(LbDev D, int round, size_t w
     __syncwarp();
     my_bytes += step_bytes(n, (int)sizeof(FG), was_ls, mem.loaded, col_in, s.col, pend != 0, mem.is_dirty);
     if (pend) {
-      int changed = 0;
       float *xf = D.xf ? D.xf + (size_t)sid * n : nullptr;
 #pragma unroll 1
       for (int i = lane; i < n; i += 32) {
         const double xi = w.x[i];
-        changed |= (xr[i] != xi);
         xr[i] = xi;
         if (xf) xf[i] = (float)xi;
       }
-      if (__any_sync(0xffffffffu, changed)) s.nfev += 1;
+      // a request equal to the point evaluated last is no new evaluation (SciPy memoises on x);
+      // lb_advance has compared the two as it posted the request
+      if (w.changed) s.nfev += 1;
     } else {
 #pragma unroll 1
       for (int i = lane; i < n; i += 32) xr[i] = w.x[i];  // final iterate
@@ -392,6 +427,9 @@ __global__ void __maxnreg__(168) lbfgsb_warp_kernel(LbDev D, int round, size_t w
     fence_async_smem();
     __syncwarp();
     cur_i = nxt_i;
+    cur_sid = nxt_sid;
+    // x, g and f of the next item lie outside the block, so they need not wait for the store below
+    if (cur_sid >= 0) stage_light(cur_sid);
     if (lane == 0) {
       uint32_t bytes = SCAL_BYTES;
       if (pend && mem.vec_dirty) bytes += 4 * LB_NV(n) * sizeof(double);
@@ -399,16 +437,15 @@ __global__ void __maxnreg__(168) lbfgsb_warp_kernel(LbDev D, int round, size_t w
       bulk_s2g(gblock, base, bytes);
       bulk_commit();
       if (pend) {
-        const int pos = atomicAdd(&D.cnt[nxt], 1);
         list_nxt[pos] = sid;
         my_evals += 1;
       }
       if (D.pend) D.pend[sid] = pend;
       // the workspace may be overwritten once the store has read it
       bulk_wait_read();
-      if (cur_i < n_active) {
+      if (cur_sid >= 0) {
         mbar_expect_tx(bar, p1_bytes);
-        bulk_g2s(base, D.blocks + D.block_stride * list_cur[cur_i], p1_bytes, bar);
+        bulk_g2s(base, D.blocks + D.block_stride * cur_sid, p1_bytes, bar);
       }
     }
     __syncwarp();
@@ -420,12 +457,46 @@ __global__ void __maxnreg__(168) lbfgsb_warp_kernel(LbDev D, int round, size_t w
     bool holding = false;
 #pragma unroll 1
     while (cur_i < n_active) {
-      // (the id of this item came with the claim of the previous iteration, see below)
-      sid = nxt_sid >= 0 ? nxt_sid : list_cur[cur_i];
-      // claim the item after this one and pull what its light stage reads into L2 meanwhile: the
-      // head of its block, its request x, and the g / f rows K2 wrote -- 0.9 GB of blocks stream
-      // through the 126 MB L2 every round, so none of them would still be there
-      nxt_i = claim();
+      sid = cur_sid;
+      // claim the item after this one; the claim's result is first needed once the light stage is done
+      int claimed = 0;
+      if (lane == 0) claimed = atomicAdd(qhead, 1);
+#pragma unroll 1
+      for (int i = lane; i < n; i += 32) {
+        const int nb = s_nbd[i];
+        w.iwhere[i] = nb == 0 ? -1 : ((nb == 2 && s_hi[i] - s_lo[i] <= 0.0) ? 3 : 0);
+      }
+      // the block's prefix, x, g and f (staged by the previous item's finish, or above)
+      mbar_wait(bar, parity);
+      parity ^= 1;
+      __syncwarp();
+      if (sizeof(FG) == 4) {
+        // widen the fp32 row in place, 32 values at a time: a chunk's doubles overwrite only floats
+        // of this chunk and of earlier ones, and every lane reads before any lane writes
+        const float *gs = reinterpret_cast<const float *>(w.g) + g_off;
+#pragma unroll 1
+        for (int i0 = 0; i0 < n; i0 += 32) {
+          const int i = i0 + lane;
+          const float gi = i < n ? gs[i] : 0.f;
+          __syncwarp();
+          if (i < n) w.g[i] = (double)gi;
+        }
+        __syncwarp();
+      }
+      s = *s_smem;
+      s.f = (double)*reinterpret_cast<const FG *>(w.q);
+      __syncwarp();
+      mem = BlockMem();
+      mem.cap = nphase < 0 ? 0 : nphase;
+      mem.bar = bar2;
+      mem.parity = parity2;
+      col_in = s.col;
+      was_ls = s.phase == LB_PH_LNSRCH;
+      const int r = LbCore<MC>::advance(P, w, s, mem, 1);
+      // the item claimed above, and what its light stage reads pulled into L2 (the head of its
+      // block, its request x, the g / f rows K2 wrote -- 0.9 GB of blocks stream through the 126 MB
+      // L2 every round, so none of them would still be there): it is staged when this item finishes
+      nxt_i = __shfl_sync(0xffffffffu, claimed, 0);
       nxt_sid = nxt_i < n_active ? list_cur[nxt_i] : -1;
       if (nxt_sid >= 0 && lane == 0) bulk_prefetch_l2(D.blocks + D.block_stride * nxt_sid, p1_bytes);
       if (nxt_sid >= 0 && pf) {
@@ -438,28 +509,6 @@ __global__ void __maxnreg__(168) lbfgsb_warp_kernel(LbDev D, int round, size_t w
         else p = reinterpret_cast<const char *>(F + nxt_sid);
         if (p) asm volatile("prefetch.global.L2 [%0];" ::"l"(p));
       }
-      const double *xr = D.xreq + (size_t)sid * n;
-      const FG *gr = G + (size_t)sid * n;
-      const double fval = (double)F[sid];
-#pragma unroll 1
-      for (int i = lane; i < n; i += 32) {
-        w.x[i] = xr[i];
-        w.g[i] = (double)gr[i];
-        const int nb = s_nbd[i];
-        w.iwhere[i] = nb == 0 ? -1 : ((nb == 2 && s_hi[i] - s_lo[i] <= 0.0) ? 3 : 0);
-      }
-      mbar_wait(bar, parity);
-      parity ^= 1;
-      __syncwarp();
-      s = *s_smem;
-      s.f = fval;
-      mem = BlockMem();
-      mem.cap = nphase < 0 ? 0 : nphase;
-      mem.bar = bar2;
-      mem.parity = parity2;
-      col_in = s.col;
-      was_ls = s.phase == LB_PH_LNSRCH;
-      const int r = LbCore<MC>::advance(P, w, s, mem, 1);
       if (r == 2) {
         // a new iteration begins: request W and the matrices now, wait in mem.load()
         if (lane == 0) {
