@@ -5,7 +5,7 @@ Same Python surface as the reference for that path; hand-written CUDA kernels be
 """
 __version__ = "0.1.0"
 
-from .layers import Dense, BinaryCrossentropy, Adam, l2  # noqa: F401
+from .layers import Dense, BinaryCrossentropy, Adam, RMSprop, Adagrad, Adadelta, Adamax, Nadam, l2  # noqa: F401
 from .ops import identity, sigmoid, exp, TRANSFORMS  # noqa: F401
 from .base import convert, maybe_distort, maybe_distort_batch, truncated_normal  # noqa: F401
 from .models import (Sequential, DenseSequential, MaximizableModel,  # noqa: F401

@@ -32,6 +32,9 @@ SIGNATURES = {
     "bore_mlp_get_adam_state": (C.c_int, [vp, C.c_int, vp, vp, C.POINTER(C.c_int64)]),
     "bore_mlp_reset_optimizer": (C.c_int, [vp, C.c_int, C.c_int, vp]),
     "bore_mlp_set_optimizer": (C.c_int, [vp, C.c_float, C.c_float, C.c_float, C.c_float]),
+    "bore_mlp_set_optimizer_kind": (C.c_int, [vp, C.c_int, vp]),
+    "bore_mlp_get_nadam_cache": (C.c_int, [vp, C.c_int, C.POINTER(C.c_float)]),
+    "bore_mlp_set_nadam_cache": (C.c_int, [vp, C.c_int, C.c_float]),
     "bore_mlp_set_fit_mode": (C.c_int, [vp, C.c_int]),
     "bore_mlp_params_dev": (C.c_int, [vp, C.POINTER(vp)]),
     "bore_mlp_predict": (C.c_int, [vp, C.c_int, vp, C.c_int, vp, vp]),
@@ -93,6 +96,9 @@ SIGNATURES = {
     "bore_lstm_get_weights": (C.c_int, [vp, vp]),
     "bore_lstm_set_adam_state": (C.c_int, [vp, vp, vp, C.c_int64]),
     "bore_lstm_get_adam_state": (C.c_int, [vp, vp, vp, C.POINTER(C.c_int64)]),
+    "bore_lstm_set_optimizer_kind": (C.c_int, [vp, C.c_int, vp]),
+    "bore_lstm_get_nadam_cache": (C.c_int, [vp, C.POINTER(C.c_float)]),
+    "bore_lstm_set_nadam_cache": (C.c_int, [vp, C.c_float]),
     "bore_lstm_set_regularizers": (C.c_int, [vp, vp]),
     "bore_lstm_predict_sequences": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_float, C.c_int, vp, vp]),
     "bore_lstm_predict": (C.c_int, [vp, vp, C.c_int, C.c_int, vp, vp]),

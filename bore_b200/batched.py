@@ -15,7 +15,7 @@ from sklearn.utils import check_random_state
 
 from . import ops
 from .engine import NativeMLP, lbfgsb_message
-from .layers import Dense, BinaryCrossentropy, Adam
+from .layers import Dense, BinaryCrossentropy, optimizer_spec
 from .models import check_class_weight, sample_weights
 from .optimizers.utils import from_bounds
 from .ragged import ragged_inputs, ragged_rows
@@ -140,10 +140,7 @@ class BatchedMaximizableSequential:
 
     # ------------------------------------------------------------------ keras-shaped surface
     def compile(self, optimizer="adam", loss="binary_crossentropy", metrics=None):
-        if isinstance(optimizer, str):
-            if optimizer.lower() != "adam":
-                raise NotImplementedError("only the Adam optimizer has a fused training kernel")
-            optimizer = Adam()
+        optimizer = optimizer_spec(optimizer)
         final = self.acts[-1]
         from_logits = isinstance(loss, BinaryCrossentropy) and loss.from_logits
         if not (isinstance(loss, BinaryCrossentropy) or loss == "binary_crossentropy"):
@@ -151,8 +148,7 @@ class BatchedMaximizableSequential:
         if from_logits != (final == "linear"):
             raise NotImplementedError("sigmoid output + 'binary_crossentropy', or linear output + "
                                       "BinaryCrossentropy(from_logits=True)")
-        self._net.set_optimizer(optimizer.learning_rate, optimizer.beta_1, optimizer.beta_2,
-                                optimizer.epsilon)
+        self._net.set_optimizer_kind(optimizer)
         l2 = []
         for lyr in self.layers:
             for r in (lyr.kernel_regularizer, lyr.bias_regularizer):

@@ -14,6 +14,60 @@ void bore_set_error(const char *fmt, ...) {
   va_end(ap);
 }
 
+// ---------------------------------------------------------------- optimizer state
+__global__ void fill_kernel(float *p, size_t n, float v) {
+  for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) p[i] = v;
+}
+
+// v = 0 is a memset (the only path Adam takes); other values (Adagrad's initial accumulator, Nadam's cache
+// of 1) are no byte pattern and need the fill kernel
+static int fill_async(float *p, size_t n, float v, cudaStream_t st) {
+  if (v == 0.f) {
+    BORE_CUDA(cudaMemsetAsync(p, 0, n * sizeof(float), st));
+  } else {
+    const size_t blocks = (n + 255) / 256;
+    fill_kernel<<<(unsigned)(blocks < 1024 ? blocks : 1024), 256, 0, st>>>(p, n, v);
+    BORE_CUDA(cudaGetLastError());
+  }
+  return 0;
+}
+
+int opt_reset_state(const OptHyper &opt, float *s0, float *s1, size_t n_params, long long *t_dev, float *cache,
+                    int count, cudaStream_t st) {
+  const size_t n = (size_t)count * n_params;
+  BORE_CHECK_RC(fill_async(s0, n, opt.kind == BORE_OPT_ADAGRAD ? opt.init_acc : 0.f, st));
+  BORE_CUDA(cudaMemsetAsync(s1, 0, n * sizeof(float), st));
+  if (t_dev) BORE_CUDA(cudaMemsetAsync(t_dev, 0, count * sizeof(long long), st));
+  if (opt.kind != BORE_OPT_ADAM) BORE_CHECK_RC(fill_async(cache, count, 1.f, st));
+  return 0;
+}
+
+int opt_from_array(int kind, const float *hp, OptHyper &o, const char *who) {
+  BORE_CHECK(kind >= BORE_OPT_ADAM && kind <= BORE_OPT_NADAM,
+             "%s: unknown optimizer kind %d (BORE_OPT_ADAM .. BORE_OPT_NADAM; SGD and Ftrl have no kernel)", who, kind);
+  BORE_CHECK(hp != nullptr, "%s: hyper-parameter array is NULL", who);
+  o = OptHyper{hp[0], hp[1], hp[2], hp[3], hp[4], hp[5], kind, hp[6] != 0.f};
+  const bool rho = kind == BORE_OPT_RMSPROP || kind == BORE_OPT_ADADELTA;
+  const bool betas = kind == BORE_OPT_ADAM || kind == BORE_OPT_ADAMAX || kind == BORE_OPT_NADAM;
+  BORE_CHECK(o.lr > 0.f, "%s: learning_rate must be > 0, got %g", who, o.lr);
+  BORE_CHECK(!(rho || betas) || (o.b1 >= 0.f && o.b1 < 1.f), "%s: %s must be in [0, 1), got %g", who,
+             rho ? "rho" : "beta_1", o.b1);
+  BORE_CHECK(!betas || (o.b2 >= 0.f && o.b2 < 1.f), "%s: beta_2 must be in [0, 1), got %g", who, o.b2);
+  // eps > 0 keeps the zero-gradient, zero-slot padding parameters of the kernels at exactly zero (0/0 else)
+  BORE_CHECK(kind == BORE_OPT_ADAM ? o.eps >= 0.f : o.eps > 0.f, "%s: epsilon must be %s 0, got %g", who,
+             kind == BORE_OPT_ADAM ? ">=" : ">", o.eps);
+  BORE_CHECK(o.momentum >= 0.f && o.momentum < 1.f, "%s: momentum must be in [0, 1), got %g", who, o.momentum);
+  BORE_CHECK(o.init_acc >= 0.f, "%s: initial_accumulator_value must be >= 0, got %g", who, o.init_acc);
+  BORE_CHECK(hp[6] == 0.f || hp[6] == 1.f, "%s: centered must be 0 or 1, got %g", who, hp[6]);
+  BORE_CHECK(!(kind == BORE_OPT_RMSPROP && o.centered && o.momentum > 0.f),
+             "%s: RMSprop(centered=True, momentum>0) needs a third slot per parameter, which no kernel keeps", who);
+  if (kind != BORE_OPT_RMSPROP) { o.momentum = 0.f; o.centered = 0; }
+  if (kind != BORE_OPT_ADAGRAD) o.init_acc = 0.f;
+  if (!rho && !betas) o.b1 = 0.f;
+  if (!betas) o.b2 = 0.f;
+  return 0;
+}
+
 extern "C" {
 
 int bore_abi_version(void) { return BORE_ABI_VERSION; }
@@ -68,7 +122,7 @@ int bore_mlp_create(int n_layers, const int *dims, const int *acts, int n_models
   memset(h->pack, 0, sizeof(*h->pack));
   h->desc = d;
   h->n_models = n_models;
-  h->lr = 1e-3f; h->beta1 = 0.9f; h->beta2 = 0.999f; h->eps = 1e-7f;  // Keras "adam"
+  h->opt = OptHyper{1e-3f, 0.9f, 0.999f, 1e-7f, 0.f, 0.f, BORE_OPT_ADAM, 0};  // Keras "adam"
   h->device = device;
   cudaDeviceProp prop;
   BORE_CUDA(cudaGetDeviceProperties(&prop, device));
@@ -78,10 +132,10 @@ int bore_mlp_create(int n_layers, const int *dims, const int *acts, int n_models
   BORE_CUDA(cudaMalloc(&h->adam_m, nb));
   BORE_CUDA(cudaMalloc(&h->adam_v, nb));
   BORE_CUDA(cudaMalloc(&h->adam_t, n_models * sizeof(long long)));
+  BORE_CUDA(cudaMalloc(&h->opt_cache, n_models * sizeof(float)));
   BORE_CUDA(cudaMemset(h->params, 0, nb));
-  BORE_CUDA(cudaMemset(h->adam_m, 0, nb));
-  BORE_CUDA(cudaMemset(h->adam_v, 0, nb));
-  BORE_CUDA(cudaMemset(h->adam_t, 0, n_models * sizeof(long long)));
+  BORE_CHECK_RC(opt_reset_state(h->opt, h->adam_m, h->adam_v, off, h->adam_t, h->opt_cache, n_models, 0));
+  BORE_CUDA(cudaDeviceSynchronize());
   *out = h;
   return 0;
 }
@@ -93,6 +147,7 @@ int bore_mlp_destroy(bore_mlp *h) {
   cudaFree(h->adam_m);
   cudaFree(h->adam_v);
   cudaFree(h->adam_t);
+  cudaFree(h->opt_cache);
   if (h->pack) {
     for (int v = 0; v < 4; ++v) cudaFree(h->pack->buf[v]);
     delete h->pack;
@@ -167,10 +222,20 @@ int bore_mlp_reset_optimizer(bore_mlp *h, int model0, int count, void *stream) {
              h->n_models);
   BORE_CUDA(cudaSetDevice(h->device));
   const size_t np = h->desc.n_params;
-  cudaStream_t st = (cudaStream_t)stream;
-  BORE_CUDA(cudaMemsetAsync(h->adam_m + model0 * np, 0, count * np * sizeof(float), st));
-  BORE_CUDA(cudaMemsetAsync(h->adam_v + model0 * np, 0, count * np * sizeof(float), st));
-  BORE_CUDA(cudaMemsetAsync(h->adam_t + model0, 0, count * sizeof(long long), st));
+  return opt_reset_state(h->opt, h->adam_m + model0 * np, h->adam_v + model0 * np, np, h->adam_t + model0,
+                         h->opt_cache + model0, count, (cudaStream_t)stream);
+}
+
+// a change of kind: every model starts from the new kind's initial state (Keras builds fresh slots)
+static int mlp_change_optimizer(bore_mlp *h, const OptHyper &o) {
+  if (o.kind != h->opt.kind) {
+    BORE_CUDA(cudaSetDevice(h->device));
+    BORE_CUDA(cudaDeviceSynchronize());
+    BORE_CHECK_RC(opt_reset_state(o, h->adam_m, h->adam_v, h->desc.n_params, h->adam_t, h->opt_cache,
+                                  h->n_models, 0));
+    BORE_CUDA(cudaDeviceSynchronize());
+  }
+  h->opt = o;
   return 0;
 }
 
@@ -178,7 +243,28 @@ int bore_mlp_set_optimizer(bore_mlp *h, float lr, float beta1, float beta2, floa
   BORE_CHECK(h != nullptr, "NULL handle");
   BORE_CHECK(lr > 0.f && beta1 >= 0.f && beta1 < 1.f && beta2 >= 0.f && beta2 < 1.f && eps >= 0.f,
              "bore_mlp_set_optimizer: invalid Adam hyper-parameters");
-  h->lr = lr; h->beta1 = beta1; h->beta2 = beta2; h->eps = eps;
+  return mlp_change_optimizer(h, OptHyper{lr, beta1, beta2, eps, 0.f, 0.f, BORE_OPT_ADAM, 0});
+}
+
+int bore_mlp_set_optimizer_kind(bore_mlp *h, int kind, const float *hp) {
+  OptHyper o;
+  BORE_CHECK_RC(opt_from_array(kind, hp, o, "bore_mlp_set_optimizer_kind"));
+  BORE_CHECK(h != nullptr, "NULL handle");
+  return mlp_change_optimizer(h, o);
+}
+
+int bore_mlp_get_nadam_cache(bore_mlp *h, int model, float *cache_host) {
+  CHECK_MODEL(h, model);
+  BORE_CHECK(cache_host != nullptr, "NULL argument");
+  BORE_CUDA(cudaDeviceSynchronize());
+  BORE_CUDA(cudaMemcpy(cache_host, h->opt_cache + model, sizeof(float), cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+int bore_mlp_set_nadam_cache(bore_mlp *h, int model, float cache) {
+  CHECK_MODEL(h, model);
+  BORE_CUDA(cudaDeviceSynchronize());
+  BORE_CUDA(cudaMemcpy(h->opt_cache + model, &cache, sizeof(float), cudaMemcpyHostToDevice));
   return 0;
 }
 

@@ -59,6 +59,19 @@ struct MlpDesc {
 // K0/K2 stage their weights from a pre-packed, zero-padded image (one per kernel variant:
 // grad / no grad x narrow / wide lane mapping) with a single bulk copy; the cache is shared by
 // shallow copies of the handle.
+// Optimizer of a handle (bore_mlp_set_optimizer_kind / bore_lstm_set_optimizer_kind), passed by value to the fit
+// kernels.  lr .. eps keep the places of Adam's former fields.
+struct OptHyper {
+  float lr;
+  float b1;  // beta_1 (Adam, Adamax, Nadam) or rho (RMSprop, Adadelta)
+  float b2;  // beta_2 (Adam, Adamax, Nadam)
+  float eps;
+  float momentum;  // RMSprop
+  float init_acc;  // Adagrad's initial_accumulator_value
+  int kind;        // BORE_OPT_*
+  int centered;    // RMSprop
+};
+
 struct MlpPackCache {
   float *buf[4];
   size_t cap[4];  // floats allocated
@@ -74,7 +87,8 @@ struct bore_mlp {
   float *adam_m;       // [n_models][n_params]
   float *adam_v;       // [n_models][n_params]
   long long *adam_t;   // [n_models]   Keras `iterations`
-  float lr, beta1, beta2, eps;  // Adam hyper-parameters
+  float *opt_cache;    // [n_models]   Nadam's momentum cache
+  OptHyper opt;
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];  // l2 regularisers per layer
   int fit_mode;  // 0 auto, 1 one CTA per model (FFMA), 2 one cluster per model, samples split (FFMA), 3 tensor
                  // pipe, 4 one cluster per model, units split (FFMA2)  (bore_mlp_set_fit_mode)
@@ -158,6 +172,14 @@ struct FitTable {
   StreamTable dev;
   int get(const FitProblem **out);  // 0, or < 0 with the error text set
 };
+
+// ---------------------------------------------------------------- optimizer state
+// Slot 0, slot 1, `iterations` and the Nadam cache of `count` consecutive models, set to the initial values of
+// the kind (opt.init_acc for Adagrad's accumulator, 1 for the cache, zeros else) on `stream`.
+int opt_reset_state(const OptHyper &opt, float *s0, float *s1, size_t n_params, long long *t_dev, float *cache,
+                    int count, cudaStream_t stream);
+// bore_*_set_optimizer_kind's check of (kind, hp); 0, or -1 with the error text set
+int opt_from_array(int kind, const float *hp, OptHyper &out, const char *who);
 
 // ---------------------------------------------------------------- launchers (one per .cu)
 // K0 / K2.  `list` (may be NULL) is a device array of row indices: point i of the launch

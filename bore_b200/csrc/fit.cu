@@ -127,9 +127,10 @@ struct FitArgs {
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
   int any_l2;
   float *loss_out;
-  float lr, beta1, beta2, eps;
+  OptHyper opt;
   FitWeights fw;
   const FitProblem *probs;  // NULL: uniform launch
+  float *opt_cache;         // [n_models] Nadam's momentum cache
 };
 
 // acc[i][u] += sum_k A[k*lda + i] * B[k*ldb + u]: the 4 x 4 register tile of every GEMM below
@@ -196,8 +197,8 @@ __device__ __forceinline__ void narrow_tile(const float *__restrict__ Hin, const
 // WEIGHTED: per-sample loss weights (FitArgs::fw); the unweighted build runs none of their code.
 // RAGGED: the problems come from the table FitArgs::probs (bore_mlp_fit_ragged); the uniform build keeps the
 // expressions of before: deriving its problem through fit_problem() cost cfg 4 0.4 % (132.0 -> 132.5 ms)
-// EXT: the activation codes above BORE_ACT_TANH (act.cuh).
-template <bool WEIGHTED, bool RAGGED, bool EXT>
+// EXT: the activation codes above BORE_ACT_TANH (act.cuh).  OPT: the optimizers other than Adam (opt.cuh).
+template <bool WEIGHTED, bool RAGGED, bool EXT, bool OPT>
 __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
   extern __shared__ __align__(16) float sm[];
   const MlpDesc &d = a.d;
@@ -239,9 +240,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
         sm[P.wt[l] + e] = k < in ? gp[d.w_off[l] + k * out + j] : 0.f;
       }
   }
-  long long t_step = a.adam_t[model];
-  // beta^t as running products in fp64 (one multiplication per step instead of two powf calls)
-  double b1p_d = pow((double)a.beta1, (double)t_step), b2p_d = pow((double)a.beta2, (double)t_step);
+  OptRun<OPT> run(a.opt, a.adam_t[model], a.opt_cache + model);
   const float inv_D = 1.f / (float)D;
   __syncthreads();
 
@@ -350,13 +349,8 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
       }
       float loss = block_sum(lsum, red) * inv_nb;  // (also the barrier publishing dz)
 
-      // ---- Adam scalars for this step (Keras: t starts at 1) ----
-      t_step += 1;
-      b1p_d *= (double)a.beta1;
-      b2p_d *= (double)a.beta2;
-      const float b1p = (float)b1p_d, b2p = (float)b2p_d;
-      const float alpha = a.lr * sqrtf(1.f - b2p) / (1.f - b1p);
-      const float om1 = 1.f - a.beta1, om2 = 1.f - a.beta2;
+      // ---- optimizer scalars for this step ----
+      const OptStep os = run.step(a.opt);
       float reg = 0.f;
 
       // ---- reverse + update, top layer first ----
@@ -459,7 +453,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
                   float g = acc[q];
                   if (l2k != 0.f) { reg += l2k * wv * wv; g += 2.f * l2k * wv; }
                   float m = am[q], v = av[q];
-                  wv = adam_update(wv, g, m, v, om1, om2, alpha, a.eps);
+                  wv = opt_update<OPT>(a.opt, os, wv, g, m, v);
                   gm[gi] = m; gv[gi] = v;
                   W[k * JP + j] = wv;
                   if (l > 0) WT[j * KP + k] = wv;
@@ -470,7 +464,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
               const int gi = d.b_off[l] + jb;
               float bv = sm[P.b[l] + jb];
               if (l2b != 0.f) { reg += l2b * bv * bv; gb += 2.f * l2b * bv; }
-              bv = adam_update(bv, gb, bm, bvv, om1, om2, alpha, a.eps);
+              bv = opt_update<OPT>(a.opt, os, bv, gb, bm, bvv);
               gm[gi] = bm; gv[gi] = bvv;
               sm[P.b[l] + jb] = bv;
             }
@@ -597,7 +591,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
                 const int k = fdiv(e, inv_out), j = e - k * out;
                 float wv = W[k * JP + j];
                 if (l2k != 0.f) { reg += l2k * wv * wv; g += 2.f * l2k * wv; }
-                wv = adam_update(wv, g, mq[q], vq[q], om1, om2, alpha, a.eps);
+                wv = opt_update<OPT>(a.opt, os, wv, g, mq[q], vq[q]);
                 W[k * JP + j] = wv;
                 if (l > 0) WT[j * KP + k] = wv;
                 gm[g0 + e] = mq[q];
@@ -610,7 +604,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
               float bv = bsm[j];
               if (l2b != 0.f) { reg += l2b * bv * bv; g += 2.f * l2b * bv; }
               float m = __ldcg(gm + g0 + e), v = __ldcg(gv + g0 + e);
-              bsm[j] = adam_update(bv, g, m, v, om1, om2, alpha, a.eps);
+              bsm[j] = opt_update<OPT>(a.opt, os, bv, g, m, v);
               gm[g0 + e] = m;
               gv[g0 + e] = v;
             }
@@ -671,7 +665,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
                 float g = acc[i][u];
                 if (l2k != 0.f) { reg += l2k * wv * wv; g += 2.f * l2k * wv; }
                 float m = am[i][u], v = av[i][u];
-                wv = adam_update(wv, g, m, v, om1, om2, alpha, a.eps);
+                wv = opt_update<OPT>(a.opt, os, wv, g, m, v);
                 gm[gi] = m; gv[gi] = v;
                 W[k * JP + j] = wv;
                 if (l > 0) WT[j * KP + k] = wv;
@@ -686,7 +680,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
             float bv = sm[P.b[l] + j];
             if (l2b != 0.f) { reg += l2b * bv * bv; g += 2.f * l2b * bv; }
             float m = gm[gi], v = gv[gi];
-            bv = adam_update(bv, g, m, v, om1, om2, alpha, a.eps);
+            bv = opt_update<OPT>(a.opt, os, bv, g, m, v);
             gm[gi] = m; gv[gi] = v;
             sm[P.b[l] + j] = bv;
           }
@@ -711,7 +705,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
     }
     for (int e = tid; e < out; e += NT) gp[d.b_off[l] + e] = sm[P.b[l] + e];
   }
-  if (tid == 0) a.adam_t[model] = t_step;
+  if (tid == 0) run.store(a.adam_t + model, a.opt_cache + model);
 }
 
 // ---------------------------------------------------------------- K1c: one model = one CLUSTER
@@ -798,8 +792,9 @@ struct FitCArgs {
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
   int any_l2;
   float *loss_out;
-  float lr, beta1, beta2, eps;
+  OptHyper opt;
   FitWeights fw;
+  float *opt_cache;  // [n_models] Nadam's momentum cache
 };
 
 __device__ __forceinline__ uint32_t cluster_rank() {
@@ -896,7 +891,7 @@ __device__ __forceinline__ float4 f_act_bwd4(int a, float4 acc, float4 h) {
                      acc.w * act_bwd<EXT>(a, h.w));
 }
 
-template <bool WEIGHTED, bool EXT>
+template <bool WEIGHTED, bool EXT, bool OPT>
 __global__ void __cluster_dims__(FIT_CLUSTER, 1, 1) __launch_bounds__(FIT_CTHREADS)
 fit_cluster_kernel(const FitCArgs a) {
   extern __shared__ __align__(16) float sm[];
@@ -994,8 +989,7 @@ fit_cluster_kernel(const FitCArgs a) {
     tab[i] = code;
   }
   if (tid < 4) sm[P.slots + tid] = 0.f;
-  long long t_step = a.adam_t[model];
-  double b1p_d = pow((double)a.beta1, (double)t_step), b2p_d = pow((double)a.beta2, (double)t_step);
+  OptRun<OPT> run(a.opt, a.adam_t[model], a.opt_cache + model);
   uint32_t peer[FIT_CLUSTER];  // base of every CTA's dynamic shared memory
 #pragma unroll
   for (int c = 0; c < FIT_CLUSTER; ++c) peer[c] = dsmem_addr(sm, c);
@@ -1048,13 +1042,8 @@ fit_cluster_kernel(const FitCArgs a) {
       lsum = block_sum(lsum, red);  // (also the barrier publishing dz)
       if (tid == 0) sm[P.slots + par] = lsum;
 
-      // ---- Adam scalars for this step (Keras: t starts at 1) ----
-      t_step += 1;
-      b1p_d *= (double)a.beta1;
-      b2p_d *= (double)a.beta2;
-      const float b1p = (float)b1p_d, b2p = (float)b2p_d;
-      const float alpha = a.lr * sqrtf(1.f - b2p) / (1.f - b1p);
-      const float om1 = 1.f - a.beta1, om2 = 1.f - a.beta2;
+      // ---- optimizer scalars for this step ----
+      const OptStep os = run.step(a.opt);
 
       // ---- reverse: per layer, delta_{l-1} and this CTA's partial dW_l / db_l ----
       int cur = 0;
@@ -1160,7 +1149,7 @@ fit_cluster_kernel(const FitCArgs a) {
               if (l2 != 0.f) { reg += l2 * wv * wv; g += 2.f * l2 * wv; }
             }
             float m = sm[P.am + i4 + e], v = sm[P.av + i4 + e];
-            wv = adam_update(wv, g, m, v, om1, om2, alpha, a.eps);
+            wv = opt_update<OPT>(a.opt, os, wv, g, m, v);
             sm[P.am + i4 + e] = m;
             sm[P.av + i4 + e] = v;
             outv[e] = wv;
@@ -1224,7 +1213,7 @@ fit_cluster_kernel(const FitCArgs a) {
       }
       for (int e = tid; e < out; e += NT) gp[d.b_off[l] + e] = sm[P.b[l] + e];
     }
-    if (tid == 0) a.adam_t[model] = t_step;
+    if (tid == 0) run.store(a.adam_t + model, a.opt_cache + model);
   }
   for (int i = i0 + tid; i < i1; i += NT) {
     gm[i] = sm[P.am + i - i0];
@@ -1233,6 +1222,12 @@ fit_cluster_kernel(const FitCArgs a) {
   cluster_arrive();
   cluster_wait();  // nobody exits while a peer may still read its shared memory
 }
+
+// the build of a kernel for an optimizer kind: OPT for every kind but Adam
+template <bool W, bool R, bool E>
+static auto fit_onecta_for(bool opt) { return opt ? fit_kernel<W, R, E, true> : fit_kernel<W, R, E, false>; }
+template <bool W, bool E>
+static auto fit_cluster_for(bool opt) { return opt ? fit_cluster_kernel<W, E, true> : fit_cluster_kernel<W, E, false>; }
 
 // ---------------------------------------------------------------- evaluate (loss, accuracy)
 __global__ void __launch_bounds__(256)
@@ -1337,13 +1332,13 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
     if (a.l2k[l] != 0.f || a.l2b[l] != 0.f) a.any_l2 = 1;
   }
   a.loss_out = loss_out_dev;
-  a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
+  a.opt = h->opt; a.opt_cache = h->opt_cache;
   a.fw = fw;
   // ragged fits: uploaded by the launch path that takes the net, after its refusals; freed on the stream after
   // the launch
   FitTable table{h, probs_host, count, (cudaStream_t)stream, {}};
   a.probs = nullptr;
-  const bool ext = acts_ext(a.d.act, a.d.n_layers);
+  const bool ext = acts_ext(a.d.act, a.d.n_layers), opt = h->opt.kind != BORE_OPT_ADAM;
   // Tensor-pipe kernel (fit_mma.cu: 3xTF32 mma.sync GEMMs, one CTA per model) on request only (fit mode 3 or
   // BORE_FIT_MMA=1): measured SLOWER than both FFMA mappings below on B200 -- the legacy HMMA path gives
   // 3xTF32 only 1.3x the FFMA peak and every HMMA needs ~14 more instructions for fragments and splits
@@ -1394,10 +1389,10 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
       c.probs = a.probs;
       for (int l = 0; l < BORE_MAX_LAYERS; ++l) { c.l2k[l] = a.l2k[l]; c.l2b[l] = a.l2b[l]; }
       c.any_l2 = a.any_l2; c.loss_out = a.loss_out;
-      c.lr = a.lr; c.beta1 = a.beta1; c.beta2 = a.beta2; c.eps = a.eps;
+      c.opt = a.opt; c.opt_cache = a.opt_cache;
       c.fw = a.fw;
-      const auto kern = ext ? (a.fw.on ? fit_cluster_kernel<true, true> : fit_cluster_kernel<false, true>)
-                            : (a.fw.on ? fit_cluster_kernel<true, false> : fit_cluster_kernel<false, false>);
+      const auto kern = ext ? (a.fw.on ? fit_cluster_for<true, true>(opt) : fit_cluster_for<false, true>(opt))
+                            : (a.fw.on ? fit_cluster_for<true, false>(opt) : fit_cluster_for<false, false>(opt));
       BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csmem));
       kern<<<count * FIT_CLUSTER, FIT_CTHREADS, csmem, (cudaStream_t)stream>>>(c);
       BORE_CUDA(cudaGetLastError());
@@ -1428,10 +1423,10 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
   }
   BORE_CHECK(smem <= FIT_MAX_SMEM, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
   BORE_CHECK_RC(table.get(&a.probs));
-  const auto kern = ext ? (a.probs ? (a.fw.on ? fit_kernel<true, true, true> : fit_kernel<false, true, true>)
-                                   : (a.fw.on ? fit_kernel<true, false, true> : fit_kernel<false, false, true>))
-                        : (a.probs ? (a.fw.on ? fit_kernel<true, true, false> : fit_kernel<false, true, false>)
-                                   : (a.fw.on ? fit_kernel<true, false, false> : fit_kernel<false, false, false>));
+  const auto kern = ext ? (a.probs ? (a.fw.on ? fit_onecta_for<true, true, true>(opt) : fit_onecta_for<false, true, true>(opt))
+                                   : (a.fw.on ? fit_onecta_for<true, false, true>(opt) : fit_onecta_for<false, false, true>(opt)))
+                        : (a.probs ? (a.fw.on ? fit_onecta_for<true, true, false>(opt) : fit_onecta_for<false, true, false>(opt))
+                                   : (a.fw.on ? fit_onecta_for<true, false, false>(opt) : fit_onecta_for<false, false, false>(opt)));
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count, threads, smem, (cudaStream_t)stream>>>(a);
   BORE_CUDA(cudaGetLastError());

@@ -2,6 +2,7 @@
 #pragma once
 #include "common.cuh"
 #include "act.cuh"
+#include "opt.cuh"
 
 namespace {
 
@@ -21,18 +22,6 @@ __device__ __forceinline__ float block_sum(float v, float *red) {
   const int nw = blockDim.x >> 5;
   for (int i = 0; i < nw; ++i) t += red[i];
   return t;
-}
-
-// Keras-form Adam on one parameter (eps outside the bias correction); returns the new value.
-// sqrt.approx / div.approx (<= 2 ulp each): the IEEE forms cost ~25 instructions per parameter,
-// a fifth of the whole kernel at Dense32 sizes, for digits far below fp32 re-association noise.
-__device__ __forceinline__ float adam_update(float wv, float g, float &m, float &v, float om1, float om2,
-                                             float alpha, float eps) {
-  m += (g - m) * om1;
-  v += (g * g - v) * om2;
-  float r;
-  asm("sqrt.approx.f32 %0, %1;" : "=f"(r) : "f"(v));
-  return wv - __fdividef(m * alpha, r + eps);
 }
 
 // e / n for 0 <= e < 2^20 through a precomputed reciprocal (inv = 1.f / n): exact, the offset .5

@@ -136,8 +136,9 @@ struct FitMArgs {
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
   int any_l2;
   float *loss_out;
-  float lr, beta1, beta2, eps;
+  OptHyper opt;
   FitWeights fw;
+  float *opt_cache;  // [n_models] Nadam's momentum cache
 };
 
 // ------------------------------------------------------------------------------------ mma plumbing
@@ -287,7 +288,7 @@ __device__ __forceinline__ void bwd_unit(const float *Dl, int lda, const float2 
 }
 
 // ------------------------------------------------------------------------------------ the kernel
-template <int NW, int TPW, bool EXT>
+template <int NW, int TPW, bool EXT, bool OPT>
 __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit_mma_kernel(const FitMArgs a) {
   extern __shared__ __align__(16) float sm[];
   const MlpDesc &d = a.d;
@@ -332,9 +333,8 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
       sm[P.bv[l] + e] = gv[d.b_off[l] + e];
     }
   }
-  long long t_step = a.adam_t[model];
-  double b1p_d = pow((double)a.beta1, (double)t_step), b2p_d = pow((double)a.beta2, (double)t_step);
-  const float om1 = 1.f - a.beta1, om2 = 1.f - a.beta2;
+  OptRun<OPT> run(a.opt, a.adam_t[model], a.opt_cache + model);
+  OptStep os = OptRun<OPT>::consts(a.opt);
   const int spe = (N + a.batch - 1) / a.batch;
   const int total_steps = epochs * spe;
 
@@ -378,7 +378,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
   if (total_steps > 0) issue_rows(0);
 
   // Adam on the update tiles this warp owns of layer `l` (gradients in acc, slots in mm / vv)
-  float reg = 0.f, alpha = 0.f;
+  float reg = 0.f;
   auto adam_tiles = [&](int l, float (&acc)[TPW][4], float (&mm)[TPW][4], float (&vv)[TPW][4]) {
     const int in = d.dims[l], out = d.dims[l + 1], ldw = P.ldw[l], ntn = P.np[l] >> 3, tpw = P.tpw[l];
     const int T0 = warp * tpw;
@@ -398,7 +398,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
             float gr = acc[q][c];
             if (l2 != 0.f) { reg += l2 * wv * wv; gr += 2.f * l2 * wv; }
             float m = mm[q][c], v = vv[q][c];
-            wv = adam_update(wv, gr, m, v, om1, om2, alpha, a.eps);
+            wv = opt_update<OPT>(a.opt, os, wv, gr, m, v);
             const int gi = d.w_off[l] + i * out + j;
             gm[gi] = m; gv[gi] = v;
             Wp[i * ldw + j] = split_pair(wv);
@@ -416,10 +416,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
     const int nmb = (nb + 15) >> 4, BP = nmb << 4;
     const float inv_nb = 1.f / (float)nb;
     reg = 0.f;
-    t_step += 1;
-    b1p_d *= (double)a.beta1;
-    b2p_d *= (double)a.beta2;
-    alpha = a.lr * sqrtf(1.f - (float)b2p_d) / (1.f - (float)b1p_d);
+    run.advance(a.opt, os);
 
     const int row_next = row_of(gs + 1);  // (consumed after the forward pass)
     cp_async_wait_all();
@@ -509,7 +506,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         const float l2 = a.l2k[LH];
         if (l2 != 0.f) { reg += l2 * wv * wv; gk += 2.f * l2 * wv; }
         float m = sm[P.wm + tb], v = sm[P.wv + tb];
-        wl_new = adam_update(wv, gk, m, v, om1, om2, alpha, a.eps);
+        wl_new = opt_update<OPT>(a.opt, os, wv, gk, m, v);
         sm[P.wm + tb] = m; sm[P.wv + tb] = v;
       } else if (tb == in) {
         float gb = 0.f;
@@ -518,7 +515,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         const float l2 = a.l2b[LH];
         if (l2 != 0.f) { reg += l2 * bv * bv; gb += 2.f * l2 * bv; }
         float m = sm[P.bm[LH]], v = sm[P.bv[LH]];
-        bl_new = adam_update(bv, gb, m, v, om1, om2, alpha, a.eps);
+        bl_new = opt_update<OPT>(a.opt, os, bv, gb, m, v);
         sm[P.bm[LH]] = m; sm[P.bv[LH]] = v;
       }
       if (tid == 0) {  // the step's data loss (fixed order)
@@ -557,7 +554,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         const float l2 = a.l2b[l];
         if (l2 != 0.f) { reg += l2 * bv * bv; gb += 2.f * l2 * bv; }
         float m = sm[P.bm[l] + tid], v = sm[P.bv[l] + tid];
-        bv = adam_update(bv, gb, m, v, om1, om2, alpha, a.eps);
+        bv = opt_update<OPT>(a.opt, os, bv, gb, m, v);
         sm[P.bm[l] + tid] = m; sm[P.bv[l] + tid] = v;
         sm[P.b[l] + tid] = bv;
       }
@@ -662,12 +659,14 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
       gv[d.b_off[l] + e] = sm[P.bv[l] + e];
     }
   }
-  if (tid == 0) a.adam_t[model] = t_step;
+  if (tid == 0) run.store(a.adam_t + model, a.opt_cache + model);
 }
 
 template <int NW, int TPW>
 int launch_cfg(const FitMArgs &a, int count, size_t smem, cudaStream_t stream) {
-  const auto kern = acts_ext(a.d.act, a.d.n_layers) ? fit_mma_kernel<NW, TPW, true> : fit_mma_kernel<NW, TPW, false>;
+  const bool ext = acts_ext(a.d.act, a.d.n_layers), opt = a.opt.kind != BORE_OPT_ADAM;
+  const auto kern = ext ? (opt ? fit_mma_kernel<NW, TPW, true, true> : fit_mma_kernel<NW, TPW, true, false>)
+                        : (opt ? fit_mma_kernel<NW, TPW, false, true> : fit_mma_kernel<NW, TPW, false, false>);
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count, NW * 32, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());
@@ -719,7 +718,7 @@ int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev,
     if (a.l2k[l] != 0.f || a.l2b[l] != 0.f) a.any_l2 = 1;
   }
   a.loss_out = loss_out_dev;
-  a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
+  a.opt = h->opt; a.opt_cache = h->opt_cache;
   a.fw = fw;
   {
     const int rc = tab.get(&a.probs);  // taken: the table goes up now

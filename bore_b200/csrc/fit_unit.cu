@@ -159,8 +159,9 @@ struct FuArgs {
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
   int any_l2;
   float *loss_out;
-  float lr, beta1, beta2, eps;
+  OptHyper opt;
   FitWeights fw;
+  float *opt_cache;  // [n_models] Nadam's momentum cache
 };
 
 // ---------------------------------------------------------------- cluster / packed-FMA primitives
@@ -366,8 +367,8 @@ __device__ __forceinline__ float fu_row_sum(const float *__restrict__ a, int SP)
 // NH > 0: the net has NH hidden layers of HW units each (HW a multiple of 16) and the padded batch is SPT --
 // compile-time shape, D stays a run-time value; NH == 0: everything from the descriptor and the plan.
 // WT: per-sample loss weights (FuArgs::fw); the unweighted build runs none of their code.
-// EXT: the activation codes above BORE_ACT_TANH (act.cuh).
-template <int NH, int HW, int SPT, bool WT, bool EXT>
+// EXT: the activation codes above BORE_ACT_TANH (act.cuh).  OPT: the optimizers other than Adam (opt.cuh).
+template <int NH, int HW, int SPT, bool WT, bool EXT, bool OPT>
 __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_unit_kernel(const FuArgs a) {
   extern __shared__ __align__(16) float sm[];
   constexpr bool FIX = NH > 0;
@@ -435,8 +436,7 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
     const int gi = k < d.dims[L - 1] ? d.w_off[L - 1] + k : d.b_off[L - 1];
     W[P.wl + k] = gp[gi]; Mm[P.wl + k] = gm[gi]; Vv[P.wl + k] = gv[gi];
   }
-  long long t_step = a.adam_t[model];
-  double b1p_d = pow((double)a.beta1, (double)t_step), b2p_d = pow((double)a.beta2, (double)t_step);
+  OptRun<OPT> run(a.opt, a.adam_t[model], a.opt_cache + model);
   uint32_t peer[FU_C];  // base of every CTA's dynamic shared memory
 #pragma unroll
   for (int c = 0; c < FU_C; ++c) peer[c] = fu_peer(sm, c);
@@ -597,15 +597,10 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
         if (lane == 0) sm[P.slots + 2 * par + warp] = lt;
       }
 
-      // ---- Adam scalars of this step (Keras: t starts at 1) ----
+      // ---- optimizer scalars of this step ----
       FU_T();
       FU_T();
-      t_step += 1;
-      b1p_d *= (double)a.beta1;
-      b2p_d *= (double)a.beta2;
-      const float b1p = (float)b1p_d, b2p = (float)b2p_d;
-      const float alpha = a.lr * sqrtf(1.f - b2p) / (1.f - b1p);
-      const float om1 = 1.f - a.beta1, om2 = 1.f - a.beta2;
+      const OptStep os = run.step(a.opt);
       FU_T();
       __syncthreads();  // dz and the loss slots are in place
       FU_T();
@@ -783,7 +778,7 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
       }
       __syncthreads();  // gradients complete
 
-      // ---- Adam, in place, all parameters of this CTA (padding: zero gradient, stays zero) ----
+      // ---- optimizer, in place, all parameters of this CTA (padding: zero gradient and slots, stays zero) ----
       float reg = 0.f;
       for (int pi = tid; pi < P.npar; pi += FU_THREADS) {
         float wv = W[pi], gg = Gg[pi] + Gg[P.npar + pi], m = Mm[pi], v = Vv[pi];
@@ -804,7 +799,7 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
           }
           if (l2 != 0.f) { if (cnt) reg += l2 * wv * wv; gg += 2.f * l2 * wv; }
         }
-        wv = adam_update(wv, gg, m, v, om1, om2, alpha, a.eps);
+        wv = opt_update<OPT>(a.opt, os, wv, gg, m, v);
         W[pi] = wv; Mm[pi] = m; Vv[pi] = v;
       }
       FU_T();
@@ -861,22 +856,27 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
       const int gi = k < hl ? d.w_off[L - 1] + k : d.b_off[L - 1];
       gp[gi] = W[P.wl + k]; gm[gi] = Mm[P.wl + k]; gv[gi] = Vv[P.wl + k];
     }
-    if (tid == 0) a.adam_t[model] = t_step;
+    if (tid == 0) run.store(a.adam_t + model, a.opt_cache + model);
   }
   fu_cluster_sync();  // nobody exits while a peer may still address its shared memory
 #undef FU_DIM
 #undef FU_U
 }
 
-template <int NH, int HW, int SPT>
+template <int NH, int HW, int SPT, bool OPT>
 static int fu_launch(const FuArgs &a, int count, size_t smem, cudaStream_t stream) {
   const auto kern = acts_ext(a.d.act, a.d.n_layers)
-                        ? (a.fw.on ? fit_unit_kernel<NH, HW, SPT, true, true> : fit_unit_kernel<NH, HW, SPT, false, true>)
-                        : (a.fw.on ? fit_unit_kernel<NH, HW, SPT, true, false> : fit_unit_kernel<NH, HW, SPT, false, false>);
+                        ? (a.fw.on ? fit_unit_kernel<NH, HW, SPT, true, true, OPT> : fit_unit_kernel<NH, HW, SPT, false, true, OPT>)
+                        : (a.fw.on ? fit_unit_kernel<NH, HW, SPT, true, false, OPT> : fit_unit_kernel<NH, HW, SPT, false, false, OPT>);
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count * FU_C, FU_THREADS, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());
   return 1;
+}
+template <int NH, int HW, int SPT>
+static int fu_launch(const FuArgs &a, int count, size_t smem, cudaStream_t stream) {
+  return a.opt.kind != BORE_OPT_ADAM ? fu_launch<NH, HW, SPT, true>(a, count, smem, stream)
+                                     : fu_launch<NH, HW, SPT, false>(a, count, smem, stream);
 }
 
 }  // namespace
@@ -918,7 +918,7 @@ int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev
     if (a.l2k[l] != 0.f || a.l2b[l] != 0.f) a.any_l2 = 1;
   }
   a.loss_out = loss_out_dev;
-  a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
+  a.opt = h->opt; a.opt_cache = h->opt_cache;
   a.fw = fw;
   {
     const int rc = tab.get(&a.probs);  // taken: the table goes up now

@@ -26,6 +26,7 @@
 
 #include "common.cuh"
 #include "act.cuh"
+#include "opt.cuh"
 
 #define LSTM_MAX_LAYERS 4
 #define LSTM_MAX_UNITS 32
@@ -46,7 +47,8 @@ struct bore_lstm {
   int device, sm_count;
   float *params, *adam_m, *adam_v;
   long long adam_t;
-  float lr, beta1, beta2, eps;
+  float *opt_cache;  // (device, 1 float) Nadam's momentum cache
+  OptHyper opt;
   float l2[3 * LSTM_MAX_LAYERS + 2];  // per array, Keras order
   float *scratch;
   size_t scratch_bytes;
@@ -294,13 +296,15 @@ struct LstmFitArgs {
   int N, T, batch, epochs;
   const int *perm;      // [epochs][N]
   float mask_value;
-  float lr, beta1, beta2, eps;
+  OptHyper opt;
   float l2[3 * LSTM_MAX_LAYERS + 2];
   float *loss_out;      // [epochs]
   float *scratch;       // A [L][T][B][AW] | Z [L][T][B][4U] | HT [T][B][U] | DU [T][B]
+  float *opt_cache;     // Nadam's momentum cache (1 float)
 };
 
-template <bool EXT>
+// OPT: the optimizers other than Adam (opt.cuh); the Adam build keeps its own IEEE arithmetic
+template <bool EXT, bool OPT>
 __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
   extern __shared__ __align__(16) float sm[];
   const LstmDesc &d = a.d;
@@ -322,8 +326,7 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
   float *gH = gZ + (size_t)L * T * B * G4;
   float *gU = gH + (size_t)T * B * U;
   const int spe = (a.N + B - 1) / B;
-  long long tstep = a.t0;
-  double b1p = pow((double)a.beta1, (double)tstep), b2p = pow((double)a.beta2, (double)tstep);
+  OptRun<OPT> run(a.opt, a.t0, a.opt_cache);
   __syncthreads();
 
   for (int ep = 0; ep < a.epochs; ++ep) {
@@ -427,19 +430,31 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
         s_loss = ls * inv_n;
       }
       // ---- phase 2: weight gradients as small GEMMs + Adam ----
-      tstep += 1;
-      b1p *= (double)a.beta1; b2p *= (double)a.beta2;
-      const float alpha = (float)((double)a.lr * sqrt(1.0 - b2p) / (1.0 - b1p));
-      const float omb1 = 1.f - a.beta1, omb2 = 1.f - a.beta2;
+      OptStep os;
+      float alpha = 0.f;
+      if (OPT) {
+        os = run.step(a.opt);
+      } else {
+        run.t += 1;
+        run.p1 *= (double)a.opt.b1; run.p2 *= (double)a.opt.b2;
+        alpha = (float)((double)a.opt.lr * sqrt(1.0 - run.p2) / (1.0 - run.p1));
+      }
+      const float omb1 = 1.f - a.opt.b1, omb2 = 1.f - a.opt.b2;
       float reg = 0.f;  // this thread's share of the l2 penalty (value, for the reported loss)
       auto adam = [&](int pi, float g, float l2f) {
         const float wv = a.params[pi];
         if (l2f != 0.f) { reg += l2f * wv * wv; g += 2.f * l2f * wv; }
         float mm = a.adam_m[pi], vv = a.adam_v[pi];
+        if (OPT) {
+          const float wn = opt_update<true>(a.opt, os, wv, g, mm, vv);
+          a.adam_m[pi] = mm; a.adam_v[pi] = vv;
+          a.params[pi] = wn;
+          return wn;
+        }
         mm += (g - mm) * omb1;
         vv += (g * g - vv) * omb2;
         a.adam_m[pi] = mm; a.adam_v[pi] = vv;
-        const float wn = wv - (mm * alpha) / (sqrtf(vv) + a.eps);
+        const float wn = wv - (mm * alpha) / (sqrtf(vv) + a.opt.eps);
         a.params[pi] = wn;
         return wn;
       };
@@ -512,6 +527,7 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
     }
     if (tid == 0) a.loss_out[ep] = tot / (float)a.N;
   }
+  if (OPT && tid == 0) *a.opt_cache = run.cache;
 }
 
 // evaluate(): masked BCE-with-logits of precomputed logits [N][T] divided by N x T (+ the l2 penalty),
@@ -613,14 +629,15 @@ int bore_lstm_create(int input_dim, int units, int num_layers, int activation, i
   cudaDeviceProp prop;
   BORE_CUDA(cudaGetDeviceProperties(&prop, device));
   h->sm_count = prop.multiProcessorCount;
-  h->lr = 1e-3f; h->beta1 = 0.9f; h->beta2 = 0.999f; h->eps = 1e-7f;
+  h->opt = OptHyper{1e-3f, 0.9f, 0.999f, 1e-7f, 0.f, 0.f, BORE_OPT_ADAM, 0};  // Keras "adam"
   const size_t nb = (size_t)h->desc.n_params * sizeof(float);
   BORE_CUDA(cudaMalloc(&h->params, nb));
   BORE_CUDA(cudaMalloc(&h->adam_m, nb));
   BORE_CUDA(cudaMalloc(&h->adam_v, nb));
+  BORE_CUDA(cudaMalloc(&h->opt_cache, sizeof(float)));
   BORE_CUDA(cudaMemset(h->params, 0, nb));
-  BORE_CUDA(cudaMemset(h->adam_m, 0, nb));
-  BORE_CUDA(cudaMemset(h->adam_v, 0, nb));
+  BORE_CHECK_RC(opt_reset_state(h->opt, h->adam_m, h->adam_v, h->desc.n_params, nullptr, h->opt_cache, 1, 0));
+  BORE_CUDA(cudaDeviceSynchronize());
   *out = h;
   return 0;
 }
@@ -628,7 +645,7 @@ int bore_lstm_create(int input_dim, int units, int num_layers, int activation, i
 int bore_lstm_destroy(bore_lstm *h) {
   if (!h) return 0;
   cudaSetDevice(h->device);
-  cudaFree(h->params); cudaFree(h->adam_m); cudaFree(h->adam_v);
+  cudaFree(h->params); cudaFree(h->adam_m); cudaFree(h->adam_v); cudaFree(h->opt_cache);
   if (h->scratch) cudaFree(h->scratch);
   delete h;
   return 0;
@@ -671,6 +688,37 @@ int bore_lstm_get_adam_state(bore_lstm *h, float *m_host, float *v_host, int64_t
   BORE_CUDA(cudaMemcpy(m_host, h->adam_m, nb, cudaMemcpyDeviceToHost));
   BORE_CUDA(cudaMemcpy(v_host, h->adam_v, nb, cudaMemcpyDeviceToHost));
   *iterations = h->adam_t;
+  return 0;
+}
+
+int bore_lstm_set_optimizer_kind(bore_lstm *h, int kind, const float *hp) {
+  OptHyper o;
+  BORE_CHECK_RC(opt_from_array(kind, hp, o, "bore_lstm_set_optimizer_kind"));
+  BORE_CHECK(h != nullptr, "NULL handle");
+  BORE_CUDA(cudaSetDevice(h->device));
+  if (o.kind != h->opt.kind) {  // a new optimizer starts from fresh slots, as Keras builds them
+    BORE_CUDA(cudaDeviceSynchronize());
+    BORE_CHECK_RC(opt_reset_state(o, h->adam_m, h->adam_v, h->desc.n_params, nullptr, h->opt_cache, 1, 0));
+    BORE_CUDA(cudaDeviceSynchronize());
+    h->adam_t = 0;
+  }
+  h->opt = o;
+  return 0;
+}
+
+int bore_lstm_get_nadam_cache(bore_lstm *h, float *cache_host) {
+  BORE_CHECK(h && cache_host, "NULL argument");
+  BORE_CUDA(cudaSetDevice(h->device));
+  BORE_CUDA(cudaDeviceSynchronize());
+  BORE_CUDA(cudaMemcpy(cache_host, h->opt_cache, sizeof(float), cudaMemcpyDeviceToHost));
+  return 0;
+}
+
+int bore_lstm_set_nadam_cache(bore_lstm *h, float cache) {
+  BORE_CHECK(h != nullptr, "NULL handle");
+  BORE_CUDA(cudaSetDevice(h->device));
+  BORE_CUDA(cudaDeviceSynchronize());
+  BORE_CUDA(cudaMemcpy(h->opt_cache, &cache, sizeof(float), cudaMemcpyHostToDevice));
   return 0;
 }
 
@@ -772,7 +820,7 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   a.t0 = h->adam_t;
   a.X = X_dev; a.Y = Y_dev; a.N = N; a.T = T; a.batch = batch_size; a.epochs = epochs;
   a.perm = perm_dev; a.mask_value = mask_value;
-  a.lr = h->lr; a.beta1 = h->beta1; a.beta2 = h->beta2; a.eps = h->eps;
+  a.opt = h->opt; a.opt_cache = h->opt_cache;
   for (int i = 0; i < 3 * LSTM_MAX_LAYERS + 2; ++i) a.l2[i] = h->l2[i];
   a.loss_out = loss_dev;
   a.scratch = h->scratch;
@@ -782,7 +830,9 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   const size_t tiles = (size_t)LSTM_MAX_BATCH * (AW + 4 * h->desc.U);
   const size_t smem = ((size_t)((h->desc.s_total + 3) & ~3) + std::max(strips, tiles)) * sizeof(float);
   BORE_CHECK(smem <= 227 * 1024, "bore_lstm_fit: needs %zu B of shared memory", smem);
-  const auto kernel = acts_ext(&h->desc.act, 1) ? lstm_fit_kernel<true> : lstm_fit_kernel<false>;
+  const bool ext = acts_ext(&h->desc.act, 1), opt = h->opt.kind != BORE_OPT_ADAM;
+  const auto kernel = ext ? (opt ? lstm_fit_kernel<true, true> : lstm_fit_kernel<true, false>)
+                          : (opt ? lstm_fit_kernel<false, true> : lstm_fit_kernel<false, false>);
   BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kernel<<<1, warps * 32, smem, (cudaStream_t)stream>>>(a);
   BORE_CUDA(cudaGetLastError());

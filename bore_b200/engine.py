@@ -16,6 +16,7 @@ from . import _lib
 ACT_CODES = {"linear": 0, None: 0, "relu": 1, "elu": 2, "sigmoid": 3, "tanh": 4, "selu": 5, "softplus": 6,
              "softsign": 7, "hard_sigmoid": 8, "exponential": 9}
 TRANSFORM_CODES = {"identity": 0, "sigmoid": 1, "exp": 2}
+OPT_NADAM = 5  # BORE_OPT_NADAM (layers.OPT_CODES): the kind with a momentum cache
 
 # scipy.optimize L-BFGS-B task codes -> message (scipy/optimize/_lbfgsb_py.py:49-90)
 _STATUS_MSG = {0: "CONVERGENCE", 1: "STOP", 2: "ABNORMAL"}
@@ -202,12 +203,36 @@ class NativeMLP:
         return self._unflatten(mf), self._unflatten(vf), it.value
 
     def reset_optimizer(self, model0=0, count=None):
-        """Zero Adam's m, v, iterations on the current stream (asynchronous)."""
+        """The optimizer state of models [model0, model0 + count) back to its initial values (zeros; Adagrad's
+        accumulator at initial_accumulator_value, Nadam's cache at 1) on the current stream (asynchronous)."""
         count = self.n_models - model0 if count is None else count
         _lib.check(self.lib.bore_mlp_reset_optimizer(self.h, model0, count, self._stream()))
 
+    opt_kind = 0  # BORE_OPT_* of the handle (Adam when created)
+
     def set_optimizer(self, lr=1e-3, beta1=0.9, beta2=0.999, eps=1e-7):
         _lib.check(self.lib.bore_mlp_set_optimizer(self.h, lr, beta1, beta2, eps))
+        self.opt_kind = 0
+
+    def set_optimizer_kind(self, optimizer):
+        """Every model's optimizer: a ``bore_b200.layers`` optimizer.  A new kind resets every model's state."""
+        kind, hp = optimizer.hyper()
+        _lib.check(self.lib.bore_mlp_set_optimizer_kind(self.h, kind, _np_ptr(np.asarray(hp, np.float32))))
+        self.opt_kind = kind
+
+    def get_optimizer_state(self, model=0):
+        """(slot 0, slot 1, iterations), and Nadam's momentum cache as a fourth entry under Nadam."""
+        state = self.get_adam_state(model)
+        if self.opt_kind != OPT_NADAM:
+            return state
+        c = C.c_float()
+        _lib.check(self.lib.bore_mlp_get_nadam_cache(self.h, model, C.byref(c)))
+        return state + (c.value,)
+
+    def set_optimizer_state(self, m, v, iterations, cache=None, model=0):
+        self.set_adam_state(m, v, iterations, model)
+        if cache is not None:
+            _lib.check(self.lib.bore_mlp_set_nadam_cache(self.h, model, float(cache)))
 
     def set_fit_mode(self, mode):
         """0 automatic, 1 one CTA per model, 2 one thread-block cluster per model."""

@@ -12,7 +12,7 @@ parity testing: ``fit(..., permutations=...)`` and ``get/set_optimizer_state``.
 import numpy as np
 
 from . import ops
-from .layers import Dense, BinaryCrossentropy, Adam
+from .layers import Dense, BinaryCrossentropy, optimizer_spec
 from .mixins import MaximizableMixin, BatchMaximizableMixin
 
 
@@ -130,18 +130,12 @@ class Sequential:
                 ws.append(np.zeros(fo, np.float32))
             net.set_weights(ws)
         if self._compiled is not None:
-            o = self._compiled["optimizer"]
-            net.set_optimizer(o.learning_rate, o.beta_1, o.beta_2, o.epsilon)
+            net.set_optimizer_kind(self._compiled["optimizer"])
         self._net = net
         return net
 
     def compile(self, optimizer="adam", loss=None, metrics=None, **kwargs):
-        if isinstance(optimizer, str):
-            if optimizer.lower() != "adam":
-                raise NotImplementedError("only the Adam optimizer has a fused training kernel")
-            optimizer = Adam()
-        elif not isinstance(optimizer, Adam):
-            raise NotImplementedError("optimizer must be 'adam' or bore_b200.layers.Adam")
+        optimizer = optimizer_spec(optimizer)
         final = self.layers[-1].activation if self.layers else None
         if isinstance(loss, str):
             if loss != "binary_crossentropy":
@@ -156,8 +150,7 @@ class Sequential:
                                       "(Keras then takes the loss on its logits)")
         self._compiled = dict(optimizer=optimizer, loss=loss, metrics=list(metrics or []))
         if self._net is not None:
-            self._net.set_optimizer(optimizer.learning_rate, optimizer.beta_1, optimizer.beta_2,
-                                    optimizer.epsilon)
+            self._net.set_optimizer_kind(optimizer)
 
     # ------------------------------------------------------------------ weights
     def get_weights(self):
@@ -172,11 +165,13 @@ class Sequential:
         self._engine().set_weights(weights)
 
     def get_optimizer_state(self):
-        """(m list, v list, iterations) of Adam -- persists across fit() calls like in Keras."""
-        return self._engine().get_adam_state()
+        """(slot 0 list, slot 1 list, iterations) -- Adam's m and v, or the slots of the compiled optimizer
+        (DESIGN.md, "Optimizers"), and under Nadam its momentum cache as a fourth entry.  Persists across
+        fit() calls like in Keras."""
+        return self._engine().get_optimizer_state()
 
-    def set_optimizer_state(self, m, v, iterations):
-        self._engine().set_adam_state(m, v, iterations)
+    def set_optimizer_state(self, m, v, iterations, cache=None):
+        self._engine().set_optimizer_state(m, v, iterations, cache)
 
     def count_params(self):
         dims = [self.input_dim] + [lyr.units for lyr in self.layers]

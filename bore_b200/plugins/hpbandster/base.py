@@ -25,7 +25,7 @@ from .types import DenseConfigurationSpace, array_from_dict, dict_from_array
 from ... import ops
 from ...base import maybe_distort
 from ...data import Record, UniqueFilter
-from ...layers import BinaryCrossentropy, activation_name, l2
+from ...layers import BinaryCrossentropy, activation_name, l2, optimizer_spec
 from ...math import steps_per_epoch
 from ...models import MaximizableDenseSequential
 
@@ -91,6 +91,7 @@ class ClassifierConfigGenerator(base_config_generator):
         self.num_units = classifier_kws.get("num_units", 32)
         self.activation = activation_name(classifier_kws.get("activation", "elu"), "BORE")
         self.optimizer = classifier_kws.get("optimizer", "adam")
+        optimizer_spec(self.optimizer, "BORE")  # refused here, not at the first fit
         l2_factor = classifier_kws.get("l2_factor")
         self.kernel_regularizer = None if l2_factor is None else l2(l2_factor)
         self.bias_regularizer = None if l2_factor is None else l2(l2_factor)

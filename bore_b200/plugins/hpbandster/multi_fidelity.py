@@ -21,7 +21,7 @@ from .base import TRANSFORMS
 from .types import DenseConfigurationSpace, array_from_dict, dict_from_array
 from ...base import maybe_distort
 from ...data import MultiFidelityRecord, UniqueFilter
-from ...layers import BinaryCrossentropy, l2
+from ...layers import BinaryCrossentropy, l2, optimizer_spec
 from ...math import steps_per_epoch
 from ...models import StackedRecurrentFactory
 
@@ -80,6 +80,7 @@ class SequenceClassifierConfigGenerator(base_config_generator):
 
         # classifier
         self.optimizer = classifier_kws.get("optimizer", "adam")
+        optimizer_spec(self.optimizer, "BOREHyperband")  # refused here, not at the first fit
         self.mask_value = classifier_kws.get("mask_value", -1.)
         factor = classifier_kws.get("l2_factor")
         penalty = None if factor is None else l2(factor)

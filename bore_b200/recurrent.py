@@ -21,8 +21,8 @@ import os
 import numpy as np
 
 from . import _lib, ops
-from .engine import ACT_CODES, TRANSFORM_CODES, NativeMLP, _np_ptr, _ptr, _torch
-from .layers import Adam, BinaryCrossentropy, Dense, activation_name
+from .engine import ACT_CODES, OPT_NADAM, TRANSFORM_CODES, NativeMLP, _np_ptr, _ptr, _torch
+from .layers import BinaryCrossentropy, Dense, activation_name, optimizer_spec
 from .mixins import MaximizableMixin
 from .models import History
 
@@ -112,6 +112,28 @@ class NativeLSTM:
         it = C.c_int64()
         _lib.check(self.lib.bore_lstm_get_adam_state(self.h, _np_ptr(mf), _np_ptr(vf), C.byref(it)))
         return self._unflatten(mf), self._unflatten(vf), it.value
+
+    opt_kind = 0  # BORE_OPT_* of the handle (Adam when created)
+
+    def set_optimizer_kind(self, optimizer):
+        """The optimizer: a ``bore_b200.layers`` optimizer.  A new kind resets the state."""
+        kind, hp = optimizer.hyper()
+        _lib.check(self.lib.bore_lstm_set_optimizer_kind(self.h, kind, _np_ptr(np.asarray(hp, np.float32))))
+        self.opt_kind = kind
+
+    def get_optimizer_state(self):
+        """(slot 0, slot 1, iterations), and Nadam's momentum cache as a fourth entry under Nadam."""
+        state = self.get_adam_state()
+        if self.opt_kind != OPT_NADAM:
+            return state
+        c = C.c_float()
+        _lib.check(self.lib.bore_lstm_get_nadam_cache(self.h, C.byref(c)))
+        return state + (c.value,)
+
+    def set_optimizer_state(self, m, v, iterations, cache=None):
+        self.set_adam_state(m, v, iterations)
+        if cache is not None:
+            _lib.check(self.lib.bore_lstm_set_nadam_cache(self.h, float(cache)))
 
     def set_regularizers(self, l2):
         """Per-array l2 factors in Keras weight order (3 per cell + 2)."""
@@ -307,16 +329,12 @@ class RecurrentSequential:
         self._rs = factory._rs
 
     def compile(self, optimizer="adam", loss=None, metrics=None, **kwargs):
-        if isinstance(optimizer, str):
-            if optimizer.lower() != "adam":
-                raise NotImplementedError("only the Adam optimizer has a fused training kernel")
-            optimizer = Adam()
+        optimizer = optimizer_spec(optimizer)
         if not isinstance(loss, BinaryCrossentropy) or not loss.from_logits:
             raise NotImplementedError("the recurrent classifier trains on BinaryCrossentropy(from_logits=True)")
-        o = optimizer
-        if (o.learning_rate, o.beta_1, o.beta_2, o.epsilon) != (1e-3, 0.9, 0.999, 1e-7):
-            raise NotImplementedError("the recurrent training kernel uses Keras' default Adam")
         self._compiled = dict(optimizer=optimizer, loss=loss, metrics=list(metrics or []))
+        if self.factory._net is not None:
+            self.factory._net.set_optimizer_kind(optimizer)
 
     def get_weights(self):
         return self.factory._engine().get_weights()
@@ -325,10 +343,18 @@ class RecurrentSequential:
         self.factory._engine().set_weights(weights)
 
     def get_optimizer_state(self):
-        return self.factory._engine().get_adam_state()
+        """(slot 0, slot 1, iterations) -- and Nadam's momentum cache under Nadam."""
+        return self._optimized_engine().get_optimizer_state()
 
-    def set_optimizer_state(self, m, v, iterations):
-        self.factory._engine().set_adam_state(m, v, iterations)
+    def set_optimizer_state(self, m, v, iterations, cache=None):
+        self._optimized_engine().set_optimizer_state(m, v, iterations, cache)
+
+    # the handle, running the compiled optimizer
+    def _optimized_engine(self):
+        net = self.factory._engine()
+        if self._compiled is not None:
+            net.set_optimizer_kind(self._compiled["optimizer"])
+        return net
 
     def count_params(self):
         return sum(int(np.prod(s)) for s in self.factory._engine().shapes())
@@ -346,7 +372,7 @@ class RecurrentSequential:
 
     def fit(self, x, y, batch_size=None, epochs=1, verbose=1, callbacks=None, shuffle=True,
             permutations=None, **kwargs):
-        """Adam on the masked BCE-with-logits of padded sequences x (N, T, D), y (N, T, 1); one
+        """The compiled optimizer on the masked BCE-with-logits of padded sequences x (N, T, D), y (N, T, 1); one
         kernel launch.  ``permutations`` (epochs, N) as in ``Sequential.fit``."""
         if kwargs:
             raise TypeError(f"fit: unsupported arguments {sorted(kwargs)}")
@@ -364,7 +390,7 @@ class RecurrentSequential:
         epochs = int(epochs)
         if epochs <= 0 or N == 0:
             return History([])
-        net = self.factory._engine()
+        net = self._optimized_engine()
         net.set_regularizers(self.factory._l2())
         if permutations is None:
             permutations = (np.stack([self._rs.permutation(N) for _ in range(epochs)]) if shuffle

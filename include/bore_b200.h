@@ -37,6 +37,11 @@ enum { BORE_ACT_LINEAR = 0, BORE_ACT_RELU = 1, BORE_ACT_ELU = 2, BORE_ACT_SIGMOI
        BORE_ACT_HARD_SIGMOID = 8, BORE_ACT_EXPONENTIAL = 9 };
 /* output transforms, TRANSFORMS of bore/plugins/hpbandster/base.py:18 */
 enum { BORE_TRANSFORM_IDENTITY = 0, BORE_TRANSFORM_SIGMOID = 1, BORE_TRANSFORM_EXP = 2 };
+/* optimizers of the training kernels (Keras names: adam, rmsprop, adagrad, adadelta, adamax, nadam);
+ * bore_mlp_set_optimizer_kind / bore_lstm_set_optimizer_kind take BORE_OPT_NHP hyper-parameters */
+enum { BORE_OPT_ADAM = 0, BORE_OPT_RMSPROP = 1, BORE_OPT_ADAGRAD = 2, BORE_OPT_ADADELTA = 3,
+       BORE_OPT_ADAMAX = 4, BORE_OPT_NADAM = 5 };
+#define BORE_OPT_NHP 7
 /* per-start termination status, scipy.optimize.OptimizeResult.status for L-BFGS-B */
 enum { BORE_STATUS_CONVERGED = 0, BORE_STATUS_LIMIT = 1, BORE_STATUS_ABNORMAL = 2 };
 
@@ -70,18 +75,38 @@ int bore_mlp_num_models(const bore_mlp *h);
 /* keras Model.set_weights / get_weights (host buffers, n_params floats); synchronous */
 int bore_mlp_set_weights(bore_mlp *h, int model, const float *params_host);
 int bore_mlp_get_weights(bore_mlp *h, int model, float *params_host);
-/* Adam slots m, v (n_params floats each) and the step counter `iterations`; Keras keeps
- * them alive across fit() calls on one model (README.rst:93 loop).  synchronous        */
+/* Adam slots m, v (n_params floats each) -- slot 0 and slot 1 of the other kinds -- and the step
+ * counter `iterations`; Keras keeps them alive across fit() calls on one model (README.rst:93
+ * loop).  synchronous                                                                   */
 int bore_mlp_set_adam_state(bore_mlp *h, int model, const float *m_host,
                             const float *v_host, int64_t iterations);
 int bore_mlp_get_adam_state(bore_mlp *h, int model, float *m_host, float *v_host,
                             int64_t *iterations);
-/* zero Adam's m, v and `iterations` of models [model0, model0+count) on `stream` (what
- * re-compiling a Keras model does to its optimizer); asynchronous                         */
+/* reset the optimizer state of models [model0, model0+count) on `stream` (what re-compiling a
+ * Keras model does to its optimizer): zero slots and `iterations` -- Adagrad's accumulator at
+ * initial_accumulator_value, Nadam's momentum cache at 1; asynchronous                     */
 int bore_mlp_reset_optimizer(bore_mlp *h, int model0, int count, void *stream);
 /* Adam hyper-parameters (keras.optimizers.Adam(learning_rate, beta_1, beta_2, epsilon));
- * defaults are Keras' "adam": 1e-3, 0.9, 0.999, 1e-7.                                   */
+ * defaults are Keras' "adam": 1e-3, 0.9, 0.999, 1e-7.  Makes Adam the handle's optimizer; coming
+ * from another kind, every model's state is reset as bore_mlp_set_optimizer_kind does.     */
 int bore_mlp_set_optimizer(bore_mlp *h, float lr, float beta1, float beta2, float eps);
+/* The handle's optimizer: kind = BORE_OPT_*, hp[BORE_OPT_NHP] =
+ *   {learning_rate, beta_1 or rho, beta_2, epsilon, momentum, initial_accumulator_value, centered}
+ * with the Keras 2.5 meaning of each (entries a kind does not have are ignored):
+ *   Adam, Adamax, Nadam  learning_rate, beta_1, beta_2 in [0,1), epsilon
+ *   RMSprop              learning_rate, rho in [0,1), epsilon, momentum in [0,1), centered (0 / 1);
+ *                        centered with momentum > 0 is refused (a third slot per parameter)
+ *   Adagrad              learning_rate, epsilon, initial_accumulator_value >= 0
+ *   Adadelta             learning_rate, rho in [0,1), epsilon
+ * learning_rate > 0; epsilon > 0 (Adam: >= 0).  Unknown kinds are refused.  A new kind resets every
+ * model's state to that kind's initial values: zero slots and `iterations`, Adagrad's accumulator
+ * (slot 0) at initial_accumulator_value, Nadam's momentum cache at 1.  The same kind only changes the
+ * hyper-parameters.  bore_mlp_{get,set}_adam_state read and write slot 0 and slot 1 of any kind
+ * (DESIGN.md, "Optimizers", has the slot of each kind).  Synchronous.                         */
+int bore_mlp_set_optimizer_kind(bore_mlp *h, int kind, const float *hp);
+/* Nadam's momentum cache (Keras' m_cache, one fp32 scalar per model; 1 after a reset).  synchronous */
+int bore_mlp_get_nadam_cache(bore_mlp *h, int model, float *cache_host);
+int bore_mlp_set_nadam_cache(bore_mlp *h, int model, float cache);
 /* l2 regularisers (keras.regularizers.l2) per Dense layer: l2_kernel[l] * sum(W_l^2) +
  * l2_bias[l] * sum(b_l^2) is added to the training loss (n_layers floats each; zeros = none).
  * The plugin regularises its hidden layers only (plugins/hpbandster/base.py:113-116,152-155). */
@@ -105,7 +130,8 @@ int bore_mlp_value_and_grad(bore_mlp *h, int model, int transform, int negate,
                             void *stream);
 
 /* ---- K1: fused training ----------------------------------------------------------------
- * Replaces keras Model.fit(X, z, epochs, batch_size, shuffle=True) compiled with adam +
+ * Replaces keras Model.fit(X, z, epochs, batch_size, shuffle=True) compiled with the handle's optimizer
+ * (Adam unless bore_mlp_set_optimizer_kind chose another) +
  * binary cross-entropy (README.rst:66,93; bore/plugins/hpbandster/base.py:156-157,184):
  * the whole run is one launch, one CTA group per model.  Models [model0, model0+count)
  * train concurrently, model j on rows [j*N, (j+1)*N) of X_dev/z_dev when
@@ -387,7 +413,8 @@ int bore_svgd_kernel_value_and_grad(const double *x_dev, int n, int D, double le
  *       selects the rows to evaluate (the stepper's pending flags); X_dev is fp32, or fp64 when
  *       x_is_f64 (the stepper's xreq_dev; rounded to fp32 as Keras casts its input).
  *   bore_lstm_fit                Model.fit on padded sequences (multi_fidelity.py:198-225): X_dev
- *       [N][T][D], Y_dev [N][T], adam + BinaryCrossentropy(from_logits=True) with the mask as sample
+ *       [N][T][D], Y_dev [N][T], the handle's optimizer (Adam unless bore_lstm_set_optimizer_kind chose
+ *       another) + BinaryCrossentropy(from_logits=True) with the mask as sample
  *       weight, divided by batch x steps; perm_dev [epochs][N] int32; loss_dev [epochs].  One launch,
  *       asynchronous on `stream`.
  *   bore_lstm_evaluate           Model.evaluate (multi_fidelity.py:226): out_host[0] = masked loss
@@ -401,6 +428,10 @@ int bore_lstm_set_weights(bore_lstm *h, const float *params_host);
 int bore_lstm_get_weights(bore_lstm *h, float *params_host);
 int bore_lstm_set_adam_state(bore_lstm *h, const float *m_host, const float *v_host, int64_t iterations);
 int bore_lstm_get_adam_state(bore_lstm *h, float *m_host, float *v_host, int64_t *iterations);
+/* the optimizer and Nadam's momentum cache, as bore_mlp_set_optimizer_kind / bore_mlp_{get,set}_nadam_cache */
+int bore_lstm_set_optimizer_kind(bore_lstm *h, int kind, const float *hp);
+int bore_lstm_get_nadam_cache(bore_lstm *h, float *cache_host);
+int bore_lstm_set_nadam_cache(bore_lstm *h, float cache);
 int bore_lstm_set_regularizers(bore_lstm *h, const float *l2_per_array_host);
 int bore_lstm_predict_sequences(bore_lstm *h, const float *X_dev, int S, int T, float mask_value,
                                 int use_mask, float *out_dev, void *stream);
