@@ -49,6 +49,7 @@ SIGNATURES = {
     "bore_mlp_fit_ragged": (C.c_int, [vp, C.c_int, C.c_int, vp, vp, vp, vp, vp, C.c_float, C.c_float, C.c_int,
                                       vp, vp, vp]),
     "bore_mlp_set_regularizers": (C.c_int, [vp, vp, vp]),
+    "bore_mlp_set_l1_regularizers": (C.c_int, [vp, vp, vp]),
     "bore_lbfgsb_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "bore_lbfgsb_minimize_workspace_bytes": (C.c_size_t, [vp, C.c_int, C.c_int]),
     "bore_lbfgsb_set_mode": (C.c_int, [C.c_int]),
@@ -100,6 +101,7 @@ SIGNATURES = {
     "bore_lstm_get_nadam_cache": (C.c_int, [vp, C.POINTER(C.c_float)]),
     "bore_lstm_set_nadam_cache": (C.c_int, [vp, C.c_float]),
     "bore_lstm_set_regularizers": (C.c_int, [vp, vp]),
+    "bore_lstm_set_l1_regularizers": (C.c_int, [vp, vp]),
     "bore_lstm_predict_sequences": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_float, C.c_int, vp, vp]),
     "bore_lstm_predict": (C.c_int, [vp, vp, C.c_int, C.c_int, vp, vp]),
     "bore_lstm_value_and_grad": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, C.c_int, vp, vp, vp, vp]),

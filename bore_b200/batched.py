@@ -15,7 +15,7 @@ from sklearn.utils import check_random_state
 
 from . import ops
 from .engine import NativeMLP, lbfgsb_message
-from .layers import Dense, BinaryCrossentropy, optimizer_spec
+from .layers import Dense, BinaryCrossentropy, optimizer_spec, regularizer_factors
 from .models import check_class_weight, sample_weights
 from .optimizers.utils import from_bounds
 from .ragged import ragged_inputs, ragged_rows
@@ -149,11 +149,8 @@ class BatchedMaximizableSequential:
             raise NotImplementedError("sigmoid output + 'binary_crossentropy', or linear output + "
                                       "BinaryCrossentropy(from_logits=True)")
         self._net.set_optimizer_kind(optimizer)
-        l2 = []
-        for lyr in self.layers:
-            for r in (lyr.kernel_regularizer, lyr.bias_regularizer):
-                l2.append(0.0 if r is None else float(r.l2))
-        self._net.set_regularizers(l2)
+        self._net.set_regularizers(*regularizer_factors(
+            r for lyr in self.layers for r in (lyr.kernel_regularizer, lyr.bias_regularizer)))
         self._compiled = True
 
     def set_weights(self, weights_per_problem):

@@ -278,6 +278,18 @@ int bore_mlp_set_regularizers(bore_mlp *h, const float *l2_kernel_host, const fl
   return 0;
 }
 
+int bore_mlp_set_l1_regularizers(bore_mlp *h, const float *l1_kernel_host, const float *l1_bias_host) {
+  BORE_CHECK(h != nullptr && l1_kernel_host && l1_bias_host, "NULL argument");
+  for (int l = 0; l < h->desc.n_layers; ++l)
+    for (const float f : {l1_kernel_host[l], l1_bias_host[l]})
+      BORE_CHECK(isfinite(f) && f >= 0.f, "l1 factor of layer %d is %g: it must be finite and >= 0", l, (double)f);
+  for (int l = 0; l < h->desc.n_layers; ++l) {
+    h->l1k[l] = l1_kernel_host[l];
+    h->l1b[l] = l1_bias_host[l];
+  }
+  return 0;
+}
+
 int bore_mlp_params_dev(bore_mlp *h, float **params_dev) {
   BORE_CHECK(h != nullptr && params_dev != nullptr, "NULL argument");
   *params_dev = h->params;

@@ -90,6 +90,7 @@ struct bore_mlp {
   float *opt_cache;    // [n_models]   Nadam's momentum cache
   OptHyper opt;
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];  // l2 regularisers per layer
+  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];  // l1 regularisers per layer
   int fit_mode;  // 0 auto, 1 one CTA per model (FFMA), 2 one cluster per model, samples split (FFMA), 3 tensor
                  // pipe, 4 one cluster per model, units split (FFMA2)  (bore_mlp_set_fit_mode)
   void *tab_pinned;      // pinned staging buffer of the ragged fit's problem table (FitTable), tab_cap bytes

@@ -125,7 +125,8 @@ struct FitArgs {
   const int *perm;
   int shared_perm;
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
-  int any_l2;
+  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];
+  int any_reg;  // some l1 or l2 factor is non-zero
   float *loss_out;
   OptHyper opt;
   FitWeights fw;
@@ -197,7 +198,8 @@ __device__ __forceinline__ void narrow_tile(const float *__restrict__ Hin, const
 // WEIGHTED: per-sample loss weights (FitArgs::fw); the unweighted build runs none of their code.
 // RAGGED: the problems come from the table FitArgs::probs (bore_mlp_fit_ragged); the uniform build keeps the
 // expressions of before: deriving its problem through fit_problem() cost cfg 4 0.4 % (132.0 -> 132.5 ms)
-// EXT: the activation codes above BORE_ACT_TANH (act.cuh).  OPT: the optimizers other than Adam (opt.cuh).
+// EXT: the activation codes above BORE_ACT_TANH (act.cuh).  OPT: the optimizers other than Adam (opt.cuh) and the l1
+// regulariser terms, which cost the default build 1.8 % of the cfg-4 fit when they were in it (DESIGN.md, "Regularizers").
 template <bool WEIGHTED, bool RAGGED, bool EXT, bool OPT>
 __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
   extern __shared__ __align__(16) float sm[];
@@ -441,7 +443,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
           {
             float *W = sm + P.w[l];
             float *WT = sm + P.wt[l];
-            const float l2k = a.l2k[l], l2b = a.l2b[l];
+            const float l2k = a.l2k[l], l2b = a.l2b[l], l1k = OPT ? a.l1k[l] : 0.f, l1b = OPT ? a.l1b[l] : 0.f;
             if (has) {
 #pragma unroll
               for (int q = 0; q < 8; ++q) {
@@ -451,7 +453,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
                   const int gi = d.w_off[l] + k * out + j;
                   float wv = W[k * JP + j];
                   float g = acc[q];
-                  if (l2k != 0.f) { reg += l2k * wv * wv; g += 2.f * l2k * wv; }
+                  regularize(l1k, l2k, wv, reg, g);
                   float m = am[q], v = av[q];
                   wv = opt_update<OPT>(a.opt, os, wv, g, m, v);
                   gm[gi] = m; gv[gi] = v;
@@ -463,7 +465,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
             if (jb < out) {
               const int gi = d.b_off[l] + jb;
               float bv = sm[P.b[l] + jb];
-              if (l2b != 0.f) { reg += l2b * bv * bv; gb += 2.f * l2b * bv; }
+              regularize(l1b, l2b, bv, reg, gb);
               bv = opt_update<OPT>(a.opt, os, bv, gb, bm, bvv);
               gm[gi] = bm; gv[gi] = bvv;
               sm[P.b[l] + jb] = bv;
@@ -567,7 +569,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
             float *W = sm + P.w[l];
             float *WT = sm + P.wt[l];
             float *bsm = sm + P.b[l];
-            const float l2k = a.l2k[l], l2b = a.l2b[l];
+            const float l2k = a.l2k[l], l2b = a.l2b[l], l1k = OPT ? a.l1k[l] : 0.f, l1b = OPT ? a.l1b[l] : 0.f;
             const int nw = in * out, g0 = d.w_off[l];
             auto grad_sum = [&](int e) {
               float g = gs[e];
@@ -590,7 +592,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
                 float g = grad_sum(e);
                 const int k = fdiv(e, inv_out), j = e - k * out;
                 float wv = W[k * JP + j];
-                if (l2k != 0.f) { reg += l2k * wv * wv; g += 2.f * l2k * wv; }
+                regularize(l1k, l2k, wv, reg, g);
                 wv = opt_update<OPT>(a.opt, os, wv, g, mq[q], vq[q]);
                 W[k * JP + j] = wv;
                 if (l > 0) WT[j * KP + k] = wv;
@@ -602,7 +604,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
               const int e = nw + j;
               float g = grad_sum(e);
               float bv = bsm[j];
-              if (l2b != 0.f) { reg += l2b * bv * bv; g += 2.f * l2b * bv; }
+              regularize(l1b, l2b, bv, reg, g);
               float m = __ldcg(gm + g0 + e), v = __ldcg(gv + g0 + e);
               bsm[j] = opt_update<OPT>(a.opt, os, bv, g, m, v);
               gm[g0 + e] = m;
@@ -611,12 +613,12 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
           }
         } else {
           __syncthreads();  // delta_{l-1} done with W_l before W_l changes
-          // (2') enough tiles for every thread: dW_l = h_{l-1}^T delta_l (+2*l2*w) and Adam by the
+          // (2') enough tiles for every thread: dW_l = h_{l-1}^T delta_l (+ regulariser) and Adam by the
           //      tile's owner; thread tile 4(k) x 4(j), k strided so that consecutive lanes read
           //      consecutive activation rows
           float *W = sm + P.w[l];
           float *WT = sm + P.wt[l];
-          const float l2k = a.l2k[l], l2b = a.l2b[l];
+          const float l2k = a.l2k[l], l2b = a.l2b[l], l1k = OPT ? a.l1k[l] : 0.f, l1b = OPT ? a.l1b[l] : 0.f;
           const int tkn = (in + 3) / 4, tjn = JP / 4;
           const int ntile = tkn * tjn;
           for (int tt = tid; tt < ntile; tt += NT) {
@@ -663,7 +665,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
                 const int gi = d.w_off[l] + k * out + j;
                 float wv = W[k * JP + j];
                 float g = acc[i][u];
-                if (l2k != 0.f) { reg += l2k * wv * wv; g += 2.f * l2k * wv; }
+                regularize(l1k, l2k, wv, reg, g);
                 float m = am[i][u], v = av[i][u];
                 wv = opt_update<OPT>(a.opt, os, wv, g, m, v);
                 gm[gi] = m; gv[gi] = v;
@@ -678,7 +680,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
             for (int p = 0; p < BP; ++p) g += DL[j * BS + p];
             const int gi = d.b_off[l] + j;
             float bv = sm[P.b[l] + j];
-            if (l2b != 0.f) { reg += l2b * bv * bv; g += 2.f * l2b * bv; }
+            regularize(l1b, l2b, bv, reg, g);
             float m = gm[gi], v = gv[gi];
             bv = opt_update<OPT>(a.opt, os, bv, g, m, v);
             gm[gi] = m; gv[gi] = v;
@@ -688,7 +690,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
         __syncthreads();
         cur ^= 1;
       }
-      if (a.any_l2) loss += block_sum(reg, red);
+      if (a.any_reg) loss += block_sum(reg, red);
       epoch_tot += loss * (float)nb;
     }
     if (tid == 0 && a.loss_out)
@@ -790,7 +792,8 @@ struct FitCArgs {
   int shared_perm;
   const FitProblem *probs;  // NULL: uniform launch (fit_problem)
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
-  int any_l2;
+  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];
+  int any_reg;  // some l1 or l2 factor is non-zero
   float *loss_out;
   OptHyper opt;
   FitWeights fw;
@@ -941,19 +944,21 @@ fit_cluster_kernel(const FitCArgs a) {
     }
     __syncthreads();
   };
-  // flat parameter index -> offsets of that parameter in the W (or bias) and W^T images
-  auto locate = [&](int i, int &off_w, int &off_wt, float &l2) {
+  // flat parameter index -> offsets of that parameter in the W (or bias) and W^T images, its l1 / l2 factors
+  auto locate = [&](int i, int &off_w, int &off_wt, float &l1, float &l2) {
     int l = 0;
     while (l + 1 < L && i >= d.w_off[l + 1]) ++l;
     const int in = d.dims[l], out = d.dims[l + 1];
     off_wt = -1;
     if (i >= d.b_off[l]) {
       off_w = P.b[l] + (i - d.b_off[l]);
+      l1 = a.l1b[l];
       l2 = a.l2b[l];
     } else {
       const int e = i - d.w_off[l], k = e / out, j = e - k * out;
       off_w = P.w[l] + k * ldo(out) + j;
       if (l > 0) off_wt = P.wt[l] + j * ldo(in) + k;
+      l1 = a.l1k[l];
       l2 = a.l2k[l];
     }
   };
@@ -982,8 +987,8 @@ fit_cluster_kernel(const FitCArgs a) {
     int code = 0xffff;  // padding: no such parameter
     if (i < d.n_params) {
       int off_w, off_wt;
-      float l2;
-      locate(i, off_w, off_wt, l2);
+      float l1, l2;
+      locate(i, off_w, off_wt, l1, l2);
       code = off_w | (off_wt + 1) << 16;
     }
     tab[i] = code;
@@ -1142,11 +1147,11 @@ fit_cluster_kernel(const FitCArgs a) {
           if (i < i1) {
             const int off_w = tab[i] & 0xffff;
             float wv = sm[off_w], g = gs[e];
-            if (a.any_l2) {
+            if (a.any_reg) {
               int off_w2, off_wt2;
-              float l2;
-              locate(i, off_w2, off_wt2, l2);
-              if (l2 != 0.f) { reg += l2 * wv * wv; g += 2.f * l2 * wv; }
+              float l1, l2;
+              locate(i, off_w2, off_wt2, l1, l2);
+              regularize(l1, l2, wv, reg, g);
             }
             float m = sm[P.am + i4 + e], v = sm[P.av + i4 + e];
             wv = opt_update<OPT>(a.opt, os, wv, g, m, v);
@@ -1159,7 +1164,7 @@ fit_cluster_kernel(const FitCArgs a) {
         // follows their next backward pass, i.e. after they have all pulled it
         *reinterpret_cast<float4 *>(sm + P.wn + i4) = make_float4(outv[0], outv[1], outv[2], outv[3]);
       }
-      if (a.any_l2) {
+      if (a.any_reg) {
         reg = block_sum(reg, red);
         if (tid == 0) sm[P.slots + 2 + par] = reg;
       }
@@ -1193,7 +1198,7 @@ fit_cluster_kernel(const FitCArgs a) {
         float ls = 0.f, rg = 0.f;
         for (int c = 0; c < FIT_CLUSTER; ++c) {
           ls += dsmem_ld(peer[c] + (uint32_t)(P.slots + par) * 4u);
-          if (a.any_l2) rg += dsmem_ld(peer[c] + (uint32_t)(P.slots + 2 + par) * 4u);
+          if (a.any_reg) rg += dsmem_ld(peer[c] + (uint32_t)(P.slots + 2 + par) * 4u);
         }
         epoch_tot += (ls * inv_nb + rg) * (float)nb;
       }
@@ -1232,7 +1237,7 @@ static auto fit_cluster_for(bool opt) { return opt ? fit_cluster_kernel<W, E, tr
 // ---------------------------------------------------------------- evaluate (loss, accuracy)
 __global__ void __launch_bounds__(256)
 evaluate_kernel(const MlpDesc d, const float *__restrict__ params, const float *__restrict__ logits,
-                const float *__restrict__ z, int N, const float *__restrict__ l2vec, const FitWeights fw,
+                const float *__restrict__ z, int N, const float *__restrict__ regvec, const FitWeights fw,
                 float *out2) {
   // logits: final pre-activation computed by K0 on a copy of the model with a linear head
   __shared__ float red[32];
@@ -1250,11 +1255,20 @@ evaluate_kernel(const MlpDesc d, const float *__restrict__ params, const float *
     ls += l;
     acc += hit;
   }
-  if (l2vec)  // l2vec[2l] = kernel factor, l2vec[2l+1] = bias factor of layer l
+  if (regvec)  // regvec[4l .. 4l+3] = l2 kernel, l2 bias, l1 kernel, l1 bias factor of layer l
     for (int l = 0; l < d.n_layers; ++l) {
       const int nk = d.dims[l] * d.dims[l + 1], nbias = d.dims[l + 1];
-      for (int i = threadIdx.x; i < nk; i += blockDim.x) { const float w = params[d.w_off[l] + i]; reg += l2vec[2 * l] * w * w; }
-      for (int i = threadIdx.x; i < nbias; i += blockDim.x) { const float w = params[d.b_off[l] + i]; reg += l2vec[2 * l + 1] * w * w; }
+      const float l1k = regvec[4 * l + 2], l1b = regvec[4 * l + 3];
+      for (int i = threadIdx.x; i < nk; i += blockDim.x) {
+        const float w = params[d.w_off[l] + i];
+        reg += regvec[4 * l] * w * w;
+        if (l1k != 0.f) reg += l1k * fabsf(w);
+      }
+      for (int i = threadIdx.x; i < nbias; i += blockDim.x) {
+        const float w = params[d.b_off[l] + i];
+        reg += regvec[4 * l + 1] * w * w;
+        if (l1b != 0.f) reg += l1b * fabsf(w);
+      }
     }
   ls = block_sum(ls, red);
   acc = block_sum(acc, red);
@@ -1325,12 +1339,7 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
   a.model0 = model0;
   a.X = X_dev; a.z = z_dev; a.N = N; a.shared_data = shared_data; a.batch = batch_size;
   a.epochs = epochs; a.perm = perm_dev; a.shared_perm = shared_perm;
-  a.any_l2 = 0;
-  for (int l = 0; l < BORE_MAX_LAYERS; ++l) {
-    a.l2k[l] = l < a.d.n_layers ? h->l2k[l] : 0.f;
-    a.l2b[l] = l < a.d.n_layers ? h->l2b[l] : 0.f;
-    if (a.l2k[l] != 0.f || a.l2b[l] != 0.f) a.any_l2 = 1;
-  }
+  fit_regularizers(h, a);
   a.loss_out = loss_out_dev;
   a.opt = h->opt; a.opt_cache = h->opt_cache;
   a.fw = fw;
@@ -1338,7 +1347,8 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
   // the launch
   FitTable table{h, probs_host, count, (cudaStream_t)stream, {}};
   a.probs = nullptr;
-  const bool ext = acts_ext(a.d.act, a.d.n_layers), opt = h->opt.kind != BORE_OPT_ADAM;
+  const bool ext = acts_ext(a.d.act, a.d.n_layers);
+  bool opt = h->opt.kind != BORE_OPT_ADAM;
   // Tensor-pipe kernel (fit_mma.cu: 3xTF32 mma.sync GEMMs, one CTA per model) on request only (fit mode 3 or
   // BORE_FIT_MMA=1): measured SLOWER than both FFMA mappings below on B200 -- the legacy HMMA path gives
   // 3xTF32 only 1.3x the FFMA peak and every HMMA needs ~14 more instructions for fragments and splits
@@ -1387,8 +1397,8 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
       c.model0 = a.model0; c.X = a.X; c.z = a.z; c.N = a.N; c.shared_data = a.shared_data;
       c.batch = a.batch; c.epochs = a.epochs; c.perm = a.perm; c.shared_perm = a.shared_perm;
       c.probs = a.probs;
-      for (int l = 0; l < BORE_MAX_LAYERS; ++l) { c.l2k[l] = a.l2k[l]; c.l2b[l] = a.l2b[l]; }
-      c.any_l2 = a.any_l2; c.loss_out = a.loss_out;
+      fit_regularizers(h, c);
+      c.loss_out = a.loss_out;
       c.opt = a.opt; c.opt_cache = a.opt_cache;
       c.fw = a.fw;
       const auto kern = ext ? (a.fw.on ? fit_cluster_for<true, true>(opt) : fit_cluster_for<false, true>(opt))
@@ -1423,6 +1433,10 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
   }
   BORE_CHECK(smem <= FIT_MAX_SMEM, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
   BORE_CHECK_RC(table.get(&a.probs));
+  // the l1 terms are in the OPT build only; with Adam its arithmetic is the default build's
+  bool any_l1 = false;
+  for (int l = 0; l < BORE_MAX_LAYERS; ++l) any_l1 = any_l1 || a.l1k[l] != 0.f || a.l1b[l] != 0.f;
+  opt = opt || any_l1;
   const auto kern = ext ? (a.probs ? (a.fw.on ? fit_onecta_for<true, true, true>(opt) : fit_onecta_for<false, true, true>(opt))
                                    : (a.fw.on ? fit_onecta_for<true, false, true>(opt) : fit_onecta_for<false, false, true>(opt)))
                         : (a.probs ? (a.fw.on ? fit_onecta_for<true, true, false>(opt) : fit_onecta_for<false, true, false>(opt))
@@ -1472,16 +1486,19 @@ static int evaluate_run(bore_mlp *h, int model, const float *X_dev, const float 
   cudaStream_t stream = (cudaStream_t)stream_;
   float *logits = nullptr, *out2 = nullptr;
   BORE_CUDA(cudaMalloc(&logits, (size_t)N * sizeof(float)));
-  BORE_CUDA(cudaMalloc(&out2, (2 + 2 * BORE_MAX_LAYERS) * sizeof(float)));
-  float l2host[2 * BORE_MAX_LAYERS];
+  BORE_CUDA(cudaMalloc(&out2, (2 + 4 * BORE_MAX_LAYERS) * sizeof(float)));
+  float reghost[4 * BORE_MAX_LAYERS];
   bool any = false;
   for (int l = 0; l < BORE_MAX_LAYERS; ++l) {
-    l2host[2 * l] = l < h->desc.n_layers ? h->l2k[l] : 0.f;
-    l2host[2 * l + 1] = l < h->desc.n_layers ? h->l2b[l] : 0.f;
-    any = any || l2host[2 * l] != 0.f || l2host[2 * l + 1] != 0.f;
+    const bool in = l < h->desc.n_layers;
+    reghost[4 * l] = in ? h->l2k[l] : 0.f;
+    reghost[4 * l + 1] = in ? h->l2b[l] : 0.f;
+    reghost[4 * l + 2] = in ? h->l1k[l] : 0.f;
+    reghost[4 * l + 3] = in ? h->l1b[l] : 0.f;
+    for (int q = 0; q < 4; ++q) any = any || reghost[4 * l + q] != 0.f;
   }
-  float *l2dev = out2 + 2;
-  cudaMemcpyAsync(l2dev, l2host, sizeof(l2host), cudaMemcpyHostToDevice, stream);
+  float *regdev = out2 + 2;
+  cudaMemcpyAsync(regdev, reghost, sizeof(reghost), cudaMemcpyHostToDevice, stream);
   // forward with a linear head = the logits the loss is defined on
   bore_mlp tmp = *h;
   tmp.desc.act[tmp.desc.n_layers - 1] = BORE_ACT_LINEAR;
@@ -1489,7 +1506,7 @@ static int evaluate_run(bore_mlp *h, int model, const float *X_dev, const float 
                            nullptr, nullptr, stream);
   if (!rc) {
     evaluate_kernel<<<1, 256, 0, stream>>>(h->desc, h->params + (size_t)model * h->desc.n_params,
-                                           logits, z_dev, N, any ? l2dev : nullptr, fw, out2);
+                                           logits, z_dev, N, any ? regdev : nullptr, fw, out2);
     cudaMemcpyAsync(out_host, out2, 2 * sizeof(float), cudaMemcpyDeviceToHost, stream);
     cudaError_t e = cudaStreamSynchronize(stream);
     if (e != cudaSuccess) { bore_set_error("bore_mlp_evaluate: %s", cudaGetErrorString(e)); rc = -2; }

@@ -28,4 +28,19 @@ __device__ __forceinline__ float block_sum(float v, float *red) {
 // keeps the product away from integer boundaries
 __device__ __forceinline__ int fdiv(int e, float inv) { return __float2int_rz(((float)e + 0.5f) * inv); }
 
+// The handle's l1 / l2 factors into a fit kernel's arguments (zero past the net's last layer) and the gate
+// any_reg that adds the penalty to the reported loss.
+template <class Args>
+static void fit_regularizers(const bore_mlp *h, Args &a) {
+  a.any_reg = 0;
+  for (int l = 0; l < BORE_MAX_LAYERS; ++l) {
+    const bool in = l < h->desc.n_layers;
+    a.l2k[l] = in ? h->l2k[l] : 0.f;
+    a.l2b[l] = in ? h->l2b[l] : 0.f;
+    a.l1k[l] = in ? h->l1k[l] : 0.f;
+    a.l1b[l] = in ? h->l1b[l] : 0.f;
+    if (a.l2k[l] != 0.f || a.l2b[l] != 0.f || a.l1k[l] != 0.f || a.l1b[l] != 0.f) a.any_reg = 1;
+  }
+}
+
 }  // namespace

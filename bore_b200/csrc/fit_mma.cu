@@ -134,7 +134,8 @@ struct FitMArgs {
   int shared_perm;
   const FitProblem *probs;  // NULL: uniform launch (fit_problem)
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
-  int any_l2;
+  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];
+  int any_reg;  // some l1 or l2 factor is non-zero
   float *loss_out;
   OptHyper opt;
   FitWeights fw;
@@ -396,7 +397,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
             const float2 wp = Wp[i * ldw + j];
             float wv = wp.x + wp.y;  // the fp32 master value, exactly
             float gr = acc[q][c];
-            if (l2 != 0.f) { reg += l2 * wv * wv; gr += 2.f * l2 * wv; }
+            regularize(a.l1k[l], l2, wv, reg, gr);
             float m = mm[q][c], v = vv[q][c];
             wv = opt_update<OPT>(a.opt, os, wv, gr, m, v);
             const int gi = d.w_off[l] + i * out + j;
@@ -503,8 +504,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         float gk = 0.f;
         for (int r = 0; r < BP; ++r) gk = fmaf(H[r * lda + tb], du[r], gk);
         float wv = w[tb];
-        const float l2 = a.l2k[LH];
-        if (l2 != 0.f) { reg += l2 * wv * wv; gk += 2.f * l2 * wv; }
+        regularize(a.l1k[LH], a.l2k[LH], wv, reg, gk);
         float m = sm[P.wm + tb], v = sm[P.wv + tb];
         wl_new = opt_update<OPT>(a.opt, os, wv, gk, m, v);
         sm[P.wm + tb] = m; sm[P.wv + tb] = v;
@@ -512,8 +512,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         float gb = 0.f;
         for (int r = 0; r < BP; ++r) gb += du[r];
         float bv = sm[P.b[LH]];
-        const float l2 = a.l2b[LH];
-        if (l2 != 0.f) { reg += l2 * bv * bv; gb += 2.f * l2 * bv; }
+        regularize(a.l1b[LH], a.l2b[LH], bv, reg, gb);
         float m = sm[P.bm[LH]], v = sm[P.bv[LH]];
         bl_new = opt_update<OPT>(a.opt, os, bv, gb, m, v);
         sm[P.bm[LH]] = m; sm[P.bv[LH]] = v;
@@ -551,8 +550,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         const float *cs = sm + P.cs[csi];
         float gb = (cs[tid] + cs[lda + tid]) + (cs[2 * lda + tid] + cs[3 * lda + tid]);
         float bv = sm[P.b[l] + tid];
-        const float l2 = a.l2b[l];
-        if (l2 != 0.f) { reg += l2 * bv * bv; gb += 2.f * l2 * bv; }
+        regularize(a.l1b[l], a.l2b[l], bv, reg, gb);
         float m = sm[P.bm[l] + tid], v = sm[P.bv[l] + tid];
         bv = opt_update<OPT>(a.opt, os, bv, gb, m, v);
         sm[P.bm[l] + tid] = m; sm[P.bv[l] + tid] = v;
@@ -623,7 +621,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
       }
       lp = l;
     }
-    if (a.any_l2) {
+    if (a.any_reg) {
       const float r = block_sum(reg, red);
       if (tid == 0) epoch_tot += r * (float)nb;
     }
@@ -711,12 +709,7 @@ int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev,
   a.model0 = model0;
   a.X = X_dev; a.z = z_dev; a.N = N; a.shared_data = shared_data; a.batch = batch_size;
   a.epochs = epochs; a.perm = perm_dev; a.shared_perm = shared_perm;
-  a.any_l2 = 0;
-  for (int l = 0; l < BORE_MAX_LAYERS; ++l) {
-    a.l2k[l] = l < a.d.n_layers ? h->l2k[l] : 0.f;
-    a.l2b[l] = l < a.d.n_layers ? h->l2b[l] : 0.f;
-    if (a.l2k[l] != 0.f || a.l2b[l] != 0.f) a.any_l2 = 1;
-  }
+  fit_regularizers(h, a);
   a.loss_out = loss_out_dev;
   a.opt = h->opt; a.opt_cache = h->opt_cache;
   a.fw = fw;

@@ -157,7 +157,8 @@ struct FuArgs {
   int shared_perm;
   const FitProblem *probs;  // NULL: uniform launch (fit_problem)
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
-  int any_l2;
+  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];
+  int any_reg;  // some l1 or l2 factor is non-zero
   float *loss_out;
   OptHyper opt;
   FitWeights fw;
@@ -782,29 +783,33 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
       float reg = 0.f;
       for (int pi = tid; pi < P.npar; pi += FU_THREADS) {
         float wv = W[pi], gg = Gg[pi] + Gg[P.npar + pi], m = Mm[pi], v = Vv[pi];
-        if (a.any_l2) {
-          // which block does pi belong to: l2 coefficient, and whether its term counts in the loss (every
-          // parameter once: column copies and bias slices here, the output layer on rank 0)
-          float l2 = 0.f;
+        if (a.any_reg) {
+          // which block does pi belong to: l1 / l2 factors, and whether its term counts in the loss (every
+          // parameter once: column copies and bias slices here, the output layer on rank 0).  The gradient
+          // term goes on every copy and slice; padding (w = 0, g = 0) gets none, as sign(0) = 0.
+          float l1 = 0.f, l2 = 0.f;
           bool cnt = false;
-          if (pi >= P.wl) { l2 = pi < P.bl ? a.l2k[L - 1] : (pi == P.bl ? a.l2b[L - 1] : 0.f); cnt = rank == 0; }
-          else if (pi >= P.bs[0]) {
-            for (int l = 0; l <= L - 2; ++l) if (pi >= P.bs[l]) l2 = a.l2b[l];
+          if (pi >= P.wl) {
+            if (pi < P.bl) { l1 = a.l1k[L - 1]; l2 = a.l2k[L - 1]; }
+            else if (pi == P.bl) { l1 = a.l1b[L - 1]; l2 = a.l2b[L - 1]; }
+            cnt = rank == 0;
+          } else if (pi >= P.bs[0]) {
+            for (int l = 0; l <= L - 2; ++l) if (pi >= P.bs[l]) { l1 = a.l1b[l]; l2 = a.l2b[l]; }
             cnt = true;
           } else if (L > 2 && pi >= P.wr[1]) {
-            for (int l = 1; l <= L - 2; ++l) if (pi >= P.wr[l]) l2 = a.l2k[l];
+            for (int l = 1; l <= L - 2; ++l) if (pi >= P.wr[l]) { l1 = a.l1k[l]; l2 = a.l2k[l]; }
           } else {
-            for (int l = 0; l <= L - 2; ++l) if (pi >= P.wc[l]) l2 = a.l2k[l];
+            for (int l = 0; l <= L - 2; ++l) if (pi >= P.wc[l]) { l1 = a.l1k[l]; l2 = a.l2k[l]; }
             cnt = true;
           }
-          if (l2 != 0.f) { if (cnt) reg += l2 * wv * wv; gg += 2.f * l2 * wv; }
+          regularize(l1, l2, wv, reg, gg, cnt);
         }
         wv = opt_update<OPT>(a.opt, os, wv, gg, m, v);
         W[pi] = wv; Mm[pi] = m; Vv[pi] = v;
       }
       FU_T();
       if (rank == 0 && tid == 0) epoch_tot += (sm[P.slots + 2 * par] + sm[P.slots + 2 * par + 1]) * inv_nb * (float)nb;
-      if (a.any_l2) {
+      if (a.any_reg) {
         // regulariser terms: every CTA sums those of the parameters it owns (column copies, bias slices; rank 0
         // the output layer), rank 0 collects them after one cluster barrier (parity slots: the value is
         // overwritten two steps later, which no CTA reaches before rank 0 has passed the next barrier)
@@ -911,12 +916,7 @@ int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev
   a.model0 = model0;
   a.X = X_dev; a.z = z_dev; a.N = N; a.shared_data = shared_data; a.batch = batch_size;
   a.epochs = epochs; a.perm = perm_dev; a.shared_perm = shared_perm;
-  a.any_l2 = 0;
-  for (int l = 0; l < BORE_MAX_LAYERS; ++l) {
-    a.l2k[l] = l < a.d.n_layers ? h->l2k[l] : 0.f;
-    a.l2b[l] = l < a.d.n_layers ? h->l2b[l] : 0.f;
-    if (a.l2k[l] != 0.f || a.l2b[l] != 0.f) a.any_l2 = 1;
-  }
+  fit_regularizers(h, a);
   a.loss_out = loss_out_dev;
   a.opt = h->opt; a.opt_cache = h->opt_cache;
   a.fw = fw;

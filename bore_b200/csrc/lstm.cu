@@ -50,6 +50,7 @@ struct bore_lstm {
   float *opt_cache;  // (device, 1 float) Nadam's momentum cache
   OptHyper opt;
   float l2[3 * LSTM_MAX_LAYERS + 2];  // per array, Keras order
+  float l1[3 * LSTM_MAX_LAYERS + 2];
   float *scratch;
   size_t scratch_bytes;
 };
@@ -297,13 +298,14 @@ struct LstmFitArgs {
   const int *perm;      // [epochs][N]
   float mask_value;
   OptHyper opt;
-  float l2[3 * LSTM_MAX_LAYERS + 2];
+  float l2[3 * LSTM_MAX_LAYERS + 2], l1[3 * LSTM_MAX_LAYERS + 2];
   float *loss_out;      // [epochs]
   float *scratch;       // A [L][T][B][AW] | Z [L][T][B][4U] | HT [T][B][U] | DU [T][B]
   float *opt_cache;     // Nadam's momentum cache (1 float)
 };
 
-// OPT: the optimizers other than Adam (opt.cuh); the Adam build keeps its own IEEE arithmetic
+// OPT: the optimizers other than Adam (opt.cuh) and the l1 regulariser terms; the Adam build keeps its own IEEE
+// arithmetic
 template <bool EXT, bool OPT>
 __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
   extern __shared__ __align__(16) float sm[];
@@ -440,10 +442,10 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
         alpha = (float)((double)a.opt.lr * sqrt(1.0 - run.p2) / (1.0 - run.p1));
       }
       const float omb1 = 1.f - a.opt.b1, omb2 = 1.f - a.opt.b2;
-      float reg = 0.f;  // this thread's share of the l2 penalty (value, for the reported loss)
-      auto adam = [&](int pi, float g, float l2f) {
+      float reg = 0.f;  // this thread's share of the l1 / l2 penalty (value, for the reported loss)
+      auto adam = [&](int pi, float g, int ra) {  // ra: the parameter's array, Keras order
         const float wv = a.params[pi];
-        if (l2f != 0.f) { reg += l2f * wv * wv; g += 2.f * l2f * wv; }
+        regularize(OPT ? a.l1[ra] : 0.f, a.l2[ra], wv, reg, g);
         float mm = a.adam_m[pi], vv = a.adam_v[pi];
         if (OPT) {
           const float wn = opt_update<true>(a.opt, os, wv, g, mm, vv);
@@ -493,11 +495,11 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
             if (q < KH && k < nr) {
               const bool isK = k < in;
               const int pi = isK ? d.k_off[l] + k * G4 + j : d.r_off[l] + (k - in) * G4 + j;
-              const float wn = adam(pi, acc[q], a.l2[3 * l + (isK ? 0 : 1)]);
+              const float wn = adam(pi, acc[q], 3 * l + (isK ? 0 : 1));
               Wimg[k * LD + j] = wn;
             }
           }
-          if (half == 0) ws[d.s_b[l] + j] = adam(d.b_off[l] + j, accb, a.l2[3 * l + 2]);
+          if (half == 0) ws[d.s_b[l] + j] = adam(d.b_off[l] + j, accb, 3 * l + 2);
         }
       }
       // Dense layer: dWd[k] = sum_{t,b} h_top[t][b][k] du[t][b]; dbd = sum du  (warp 0, lane = k)
@@ -509,10 +511,10 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
             gb += du;
             if (lane < U) gk = fmaf(gH[((size_t)t * B + b) * U + lane], du, gk);
           }
-        if (lane < U) ws[d.s_wd + lane] = adam(d.wd_off + lane, gk, a.l2[3 * L]);
-        if (lane == 0) ws[d.s_bd] = adam(d.bd_off, gb, a.l2[3 * L + 1]);
+        if (lane < U) ws[d.s_wd + lane] = adam(d.wd_off + lane, gk, 3 * L);
+        if (lane == 0) ws[d.s_bd] = adam(d.bd_off, gb, 3 * L + 1);
       }
-      // l2 penalty into the reported loss (values BEFORE this step's update)
+      // regulariser penalty into the reported loss (values BEFORE this step's update)
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) reg += __shfl_xor_sync(0xffffffffu, reg, o);
       __syncthreads();
@@ -530,11 +532,12 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
   if (OPT && tid == 0) *a.opt_cache = run.cache;
 }
 
-// evaluate(): masked BCE-with-logits of precomputed logits [N][T] divided by N x T (+ the l2 penalty),
+// evaluate(): masked BCE-with-logits of precomputed logits [N][T] divided by N x T (+ the l1 / l2 penalty),
 // and Keras' binary_accuracy on the LOGIT (threshold 0.5, the from_logits quirk -- logging only)
 // averaged over the unmasked steps.  One CTA, fixed summation order.  out[0] = loss, out[1] = accuracy.
 __global__ void __launch_bounds__(256)
 lstm_evaluate_kernel(const LstmDesc d, const float *__restrict__ params, const float *__restrict__ l2,
+                     const float *__restrict__ l1,
                      const float *__restrict__ X, const float *__restrict__ Y, const float *__restrict__ logits,
                      int N, int T, float mask_value, float *__restrict__ out) {
   __shared__ float red[3][8];
@@ -551,8 +554,8 @@ lstm_evaluate_kernel(const LstmDesc d, const float *__restrict__ params, const f
   }
   float reg = 0.f;
   for (int a = 0; a < 3 * d.L + 2; ++a) {
-    const float f = l2[a];
-    if (f == 0.f) continue;
+    const float f = l2[a], f1 = l1[a];
+    if (f == 0.f && f1 == 0.f) continue;
     const int l = a / 3, r = a - 3 * l;
     int off, n;
     if (a == 3 * d.L) { off = d.wd_off; n = d.U; }
@@ -560,7 +563,11 @@ lstm_evaluate_kernel(const LstmDesc d, const float *__restrict__ params, const f
     else if (r == 0) { off = d.k_off[l]; n = in_dim(d, l) * 4 * d.U; }
     else if (r == 1) { off = d.r_off[l]; n = d.U * 4 * d.U; }
     else { off = d.b_off[l]; n = 4 * d.U; }
-    for (int e = threadIdx.x; e < n; e += blockDim.x) { const float w = params[off + e]; reg += f * w * w; }
+    for (int e = threadIdx.x; e < n; e += blockDim.x) {
+      const float w = params[off + e];
+      if (f != 0.f) reg += f * w * w;
+      if (f1 != 0.f) reg += f1 * fabsf(w);
+    }
   }
   ls = ls / (float)(N * T) + reg;
 #pragma unroll
@@ -731,6 +738,16 @@ int bore_lstm_set_regularizers(bore_lstm *h, const float *l2_host) {
   return 0;
 }
 
+int bore_lstm_set_l1_regularizers(bore_lstm *h, const float *l1_host) {
+  BORE_CHECK(h && l1_host, "NULL argument");
+  const int n = 3 * h->desc.L + 2;
+  for (int i = 0; i < n; ++i)
+    BORE_CHECK(isfinite(l1_host[i]) && l1_host[i] >= 0.f, "l1 factor %d is %g: it must be finite and >= 0", i,
+               (double)l1_host[i]);
+  for (int i = 0; i < n; ++i) h->l1[i] = l1_host[i];
+  return 0;
+}
+
 // logits of the many-to-many network: X_dev [S][T][D] -> out_dev [S][T]; with use_mask the steps
 // whose features all equal mask_value are masked (Masking layer).
 int bore_lstm_predict_sequences(bore_lstm *h, const float *X_dev, int S, int T, float mask_value, int use_mask,
@@ -821,7 +838,7 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   a.X = X_dev; a.Y = Y_dev; a.N = N; a.T = T; a.batch = batch_size; a.epochs = epochs;
   a.perm = perm_dev; a.mask_value = mask_value;
   a.opt = h->opt; a.opt_cache = h->opt_cache;
-  for (int i = 0; i < 3 * LSTM_MAX_LAYERS + 2; ++i) a.l2[i] = h->l2[i];
+  for (int i = 0; i < 3 * LSTM_MAX_LAYERS + 2; ++i) { a.l2[i] = h->l2[i]; a.l1[i] = h->l1[i]; }
   a.loss_out = loss_dev;
   a.scratch = h->scratch;
   const int warps = 8;
@@ -830,7 +847,9 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   const size_t tiles = (size_t)LSTM_MAX_BATCH * (AW + 4 * h->desc.U);
   const size_t smem = ((size_t)((h->desc.s_total + 3) & ~3) + std::max(strips, tiles)) * sizeof(float);
   BORE_CHECK(smem <= 227 * 1024, "bore_lstm_fit: needs %zu B of shared memory", smem);
-  const bool ext = acts_ext(&h->desc.act, 1), opt = h->opt.kind != BORE_OPT_ADAM;
+  bool any_l1 = false;
+  for (int i = 0; i < 3 * LSTM_MAX_LAYERS + 2; ++i) any_l1 = any_l1 || h->l1[i] != 0.f;
+  const bool ext = acts_ext(&h->desc.act, 1), opt = h->opt.kind != BORE_OPT_ADAM || any_l1;
   const auto kernel = ext ? (opt ? lstm_fit_kernel<true, true> : lstm_fit_kernel<true, false>)
                           : (opt ? lstm_fit_kernel<false, true> : lstm_fit_kernel<false, false>);
   BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -840,7 +859,7 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   return 0;
 }
 
-// Model.evaluate on padded sequences -> out_host[0] = loss (masked BCE / (N x T) + l2 terms),
+// Model.evaluate on padded sequences -> out_host[0] = loss (masked BCE / (N x T) + l1 / l2 terms),
 // out_host[1] = accuracy over the unmasked steps (multi_fidelity.py:226).  Synchronises `stream`.
 int bore_lstm_evaluate(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, int T, float mask_value,
                        float *out_host, void *stream) {
@@ -851,13 +870,14 @@ int bore_lstm_evaluate(bore_lstm *h, const float *X_dev, const float *Y_dev, int
   BORE_CUDA(cudaSetDevice(h->device));
   cudaStream_t st = (cudaStream_t)stream;
   const int nl2 = 3 * LSTM_MAX_LAYERS + 2;
-  float *buf = nullptr;  // logits [N][T] | l2 [nl2] | out [2]
-  BORE_CUDA(cudaMallocAsync(&buf, ((size_t)N * T + nl2 + 2) * sizeof(float), st));
-  float *l2d = buf + (size_t)N * T, *outd = l2d + nl2;
+  float *buf = nullptr;  // logits [N][T] | l2 [nl2] | l1 [nl2] | out [2]
+  BORE_CUDA(cudaMallocAsync(&buf, ((size_t)N * T + 2 * nl2 + 2) * sizeof(float), st));
+  float *l2d = buf + (size_t)N * T, *l1d = l2d + nl2, *outd = l1d + nl2;
   BORE_CUDA(cudaMemcpyAsync(l2d, h->l2, nl2 * sizeof(float), cudaMemcpyHostToDevice, st));
+  BORE_CUDA(cudaMemcpyAsync(l1d, h->l1, nl2 * sizeof(float), cudaMemcpyHostToDevice, st));
   int rc = bore_lstm_predict_sequences(h, X_dev, N, T, mask_value, 1, buf, stream);
   if (rc == 0) {
-    lstm_evaluate_kernel<<<1, 256, 0, st>>>(h->desc, h->params, l2d, X_dev, Y_dev, buf, N, T, mask_value, outd);
+    lstm_evaluate_kernel<<<1, 256, 0, st>>>(h->desc, h->params, l2d, l1d, X_dev, Y_dev, buf, N, T, mask_value, outd);
     BORE_CUDA(cudaGetLastError());
     BORE_CUDA(cudaMemcpyAsync(out_host, outd, 2 * sizeof(float), cudaMemcpyDeviceToHost, st));
     BORE_CUDA(cudaStreamSynchronize(st));

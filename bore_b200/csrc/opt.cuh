@@ -100,7 +100,17 @@ __device__ __forceinline__ float sqrt_approx(float v) {
   return r;
 }
 
-// One parameter: gradient g (l2 term included), slots s0 / s1 updated in place; returns the new value.
+// Keras L1L2 on one parameter w (DESIGN.md, "Regularizers"): adds the penalty l1 |w| + l2 w^2 to reg when
+// `count`, and its gradient l1 sign(w) + 2 l2 w to g.  sign(0) = 0, as TF's Abs gradient: a parameter at exactly 0
+// gets no l1 gradient.  That covers every bias on the first step, and it keeps the padding parameters of the
+// unit-split and tensor-pipe kernels (w = 0, g = 0) exactly zero.  A term whose factor is 0 is skipped, so with
+// l1 = 0 the arithmetic is the l2-only arithmetic it always was.
+__device__ __forceinline__ void regularize(float l1, float l2, float w, float &reg, float &g, bool count = true) {
+  if (l2 != 0.f) { if (count) reg += l2 * w * w; g += 2.f * l2 * w; }
+  if (l1 != 0.f) { if (count) reg += l1 * fabsf(w); g += l1 * (float)((w > 0.f) - (w < 0.f)); }
+}
+
+// One parameter: gradient g (regulariser terms included), slots s0 / s1 updated in place; returns the new value.
 // Adam is the Keras form (eps outside the bias correction).  sqrt.approx / div.approx (<= 2 ulp each): the IEEE
 // forms cost ~25 instructions per parameter, a fifth of the whole kernel at Dense32 sizes, for digits far below
 // fp32 re-association noise.  The other kinds restate the training_ops.cc functors (RMSprop without momentum:

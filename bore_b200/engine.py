@@ -238,15 +238,17 @@ class NativeMLP:
         """0 automatic, 1 one CTA per model, 2 one thread-block cluster per model."""
         _lib.check(self.lib.bore_mlp_set_fit_mode(self.h, int(mode)))
 
-    def set_regularizers(self, l2):
-        """``l2``: one factor for every kernel and bias, or a per-array sequence in Keras weight
-        order [k0, b0, k1, b1, ...]."""
+    def set_regularizers(self, l2, l1=None):
+        """``l2`` and ``l1``: one factor for every kernel and bias, or a per-array sequence in Keras weight
+        order [k0, b0, k1, b1, ...]; ``l1=None`` is no l1 penalty."""
         L = len(self.acts)
-        v = [float(l2)] * (2 * L) if np.isscalar(l2) else [float(t) for t in l2]
-        assert len(v) == 2 * L
-        lk = np.ascontiguousarray(v[0::2], np.float32)
-        lb = np.ascontiguousarray(v[1::2], np.float32)
-        _lib.check(self.lib.bore_mlp_set_regularizers(self.h, _np_ptr(lk), _np_ptr(lb)))
+        for fn, f in ((self.lib.bore_mlp_set_regularizers, l2), (self.lib.bore_mlp_set_l1_regularizers,
+                                                                    0.0 if l1 is None else l1)):
+            v = [float(f)] * (2 * L) if np.isscalar(f) else [float(t) for t in f]
+            assert len(v) == 2 * L
+            lk = np.ascontiguousarray(v[0::2], np.float32)
+            lb = np.ascontiguousarray(v[1::2], np.float32)
+            _lib.check(fn(self.h, _np_ptr(lk), _np_ptr(lb)))
 
     def params_tensor(self):
         """The flat [n_models, n_params] parameter block as a torch view (for NCCL broadcast)."""
@@ -568,23 +570,25 @@ class NativeMLP:
                                                 _ptr(perm_dev), _ptr(loss_dev), self._stream()))
         return loss_dev[:E]
 
-    def fit(self, X, z, epochs, batch_size, permutations, l2=None, model=0, w=None, class_weight=None):
+    def fit(self, X, z, epochs, batch_size, permutations, l2=None, model=0, w=None, class_weight=None, l1=None):
         """Keras ``fit`` with explicit per-epoch permutations -> history loss (epochs,).
-        ``w`` (N,) sample weights and ``class_weight`` (cw0, cw1) as in ``fit_dev``."""
+        ``w`` (N,) sample weights and ``class_weight`` (cw0, cw1) as in ``fit_dev``.  ``l2`` / ``l1``: when
+        ``l2`` is given, both factor sets are set first (``set_regularizers``)."""
         if l2 is not None:
-            self.set_regularizers(l2)
+            self.set_regularizers(l2, l1)
         X = np.asarray(X)
         N = X.shape[0]
         perm = np.ascontiguousarray(permutations, np.int32).reshape(epochs, N)
         return self.fit_async(X, z, epochs, batch_size, perm, model=model, w=w,
                               class_weight=class_weight).cpu().numpy()[0]
 
-    def fit_async(self, X, z, epochs, batch_size, permutations, l2=None, model=0, w=None, class_weight=None):
+    def fit_async(self, X, z, epochs, batch_size, permutations, l2=None, model=0, w=None, class_weight=None,
+                  l1=None):
         """Like ``fit`` but returns the (1, epochs) device tensor of epoch losses without waiting
         for the training kernel: the host is free (e.g. to draw the start points of the next
         argmax) while the GPU trains."""
         if l2 is not None:
-            self.set_regularizers(l2)
+            self.set_regularizers(l2, l1)
         X = np.asarray(X)
         N = X.shape[0]
         perm = np.ascontiguousarray(permutations, np.int32).reshape(epochs, N)
@@ -594,11 +598,11 @@ class NativeMLP:
                             N, batch_size, epochs, self.to_device(perm, np.int32),
                             model0=model, count=1, w_dev=w_dev, class_weight=class_weight)
 
-    def evaluate(self, X, z, l2=None, model=0, w=None, class_weight=None):
+    def evaluate(self, X, z, l2=None, model=0, w=None, class_weight=None, l1=None):
         """Keras ``evaluate`` -> [loss, accuracy]; ``w`` / ``class_weight`` weight the loss and the
-        accuracy (bore_mlp_evaluate_weighted)."""
+        accuracy (bore_mlp_evaluate_weighted); ``l2`` / ``l1`` as in ``fit``."""
         if l2 is not None:
-            self.set_regularizers(l2)
+            self.set_regularizers(l2, l1)
         X = np.asarray(X)
         N = X.shape[0]
         out = np.zeros(2, np.float32)

@@ -1,8 +1,10 @@
-"""Keras-shaped declarations the hot path needs: Dense, l2, BinaryCrossentropy and the optimizers.
+"""Keras-shaped declarations the hot path needs: Dense, the regularizers, BinaryCrossentropy and the optimizers.
 
 Keras itself is absent (and not wanted on the path); these are plain spec objects that
 ``bore_b200.models.Sequential`` lowers onto the native handle.  Names and arguments follow
 the call sites README.rst:60-66 and bore/plugins/hpbandster/base.py:113-116,147-158."""
+
+import numpy as np
 
 # Keras 2.5 element-wise activations whose derivative is a function of the layer output, the one value the
 # kernels keep (swish and gelu are not: DESIGN.md, "Activations")
@@ -22,6 +24,22 @@ def activation_name(activation, owner):
     return activation
 
 
+def _penalty(value, owner):
+    """A regularisation factor the kernels take: a finite number >= 0."""
+    v = float(value)
+    if not np.isfinite(v) or v < 0:
+        raise ValueError(f"{owner}: the regularisation factor must be finite and >= 0, got {value!r}")
+    return v
+
+
+class L1:
+    """``keras.regularizers.L1(l1=0.01)``: adds ``l1 * sum(abs(w))`` to the loss; its gradient is
+    ``l1 * sign(w)`` with sign(0) = 0 (TF's Abs gradient)."""
+
+    def __init__(self, l1=0.01):
+        self.l1 = _penalty(0.01 if l1 is None else l1, "L1")
+
+
 class L2:
     """``keras.regularizers.l2(l2)``: adds ``l2 * sum(w**2)`` to the loss."""
 
@@ -29,8 +47,51 @@ class L2:
         self.l2 = float(l2)
 
 
+class L1L2:
+    """``keras.regularizers.L1L2(l1=0., l2=0.)``: adds ``l1 * sum(abs(w)) + l2 * sum(w**2)``, each term only
+    when its factor is non-zero.  Its defaults are zeros; ``l1_l2()`` and the string ``"l1_l2"`` give 0.01 each."""
+
+    def __init__(self, l1=0.0, l2=0.0):
+        self.l1 = _penalty(0.0 if l1 is None else l1, "L1L2")
+        self.l2 = _penalty(0.0 if l2 is None else l2, "L1L2")
+
+
+l1 = L1
+
+
 def l2(l2=0.01):
     return L2(l2)
+
+
+def l1_l2(l1=0.01, l2=0.01):
+    """``keras.regularizers.l1_l2``: ``L1L2`` with 0.01 for each factor by default."""
+    return L1L2(l1=l1, l2=l2)
+
+
+# keras.regularizers.get / deserialize: the strings it takes and what they give ("l1_l2" is deserialize's special
+# case, L1L2(0.01, 0.01), not the class's zeros)
+_REGULARIZER_NAMES = {"l1": L1, "L1": L1, "l2": L2, "L2": L2, "L1L2": L1L2, "l1_l2": l1_l2}
+
+
+def regularizer_get(identifier, owner):
+    """``keras.regularizers.get``: None, an ``L1`` / ``L2`` / ``L1L2`` instance, or one of the names
+    ``"l1"``, ``"l2"``, ``"L1"``, ``"L2"``, ``"L1L2"`` (class defaults) and ``"l1_l2"`` (0.01 each).
+    ValueError naming what is accepted for anything else: the kernels apply no other penalty."""
+    if identifier is None or isinstance(identifier, (L1, L2, L1L2)):
+        return identifier
+    if isinstance(identifier, str) and identifier in _REGULARIZER_NAMES:
+        return _REGULARIZER_NAMES[identifier]()
+    raise ValueError(f"{owner}: a regularizer must be None, an instance of bore_b200.layers.{{L1, L2, L1L2}} "
+                     f"or one of the names {tuple(_REGULARIZER_NAMES)}, got {identifier!r}")
+
+
+def regularizer_factors(regularizers):
+    """The per-array (l2, l1) factor lists of a sequence of regularizers, as the native setters take them
+    (None: no penalty)."""
+    regularizers = list(regularizers)
+    l2s = [0.0 if r is None else float(getattr(r, "l2", 0.0)) for r in regularizers]
+    l1s = [0.0 if r is None else float(getattr(r, "l1", 0.0)) for r in regularizers]
+    return l2s, l1s
 
 
 class Dense:
@@ -49,8 +110,8 @@ class Dense:
         self.units = int(units)
         self.activation = activation
         self.input_dim = None if input_dim is None else int(input_dim)
-        self.kernel_regularizer = kernel_regularizer
-        self.bias_regularizer = bias_regularizer
+        self.kernel_regularizer = regularizer_get(kernel_regularizer, "Dense")
+        self.bias_regularizer = regularizer_get(bias_regularizer, "Dense")
 
 
 class BinaryCrossentropy:

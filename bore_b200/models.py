@@ -12,7 +12,7 @@ parity testing: ``fit(..., permutations=...)`` and ``get/set_optimizer_state``.
 import numpy as np
 
 from . import ops
-from .layers import Dense, BinaryCrossentropy, optimizer_spec
+from .layers import Dense, BinaryCrossentropy, optimizer_spec, regularizer_factors
 from .mixins import MaximizableMixin, BatchMaximizableMixin
 
 
@@ -94,14 +94,13 @@ class Sequential:
     def input_dim(self):
         return self.layers[0].input_dim if self.layers else None
 
-    def _l2(self):
-        """Per-array l2 factors in Keras weight order [k0, b0, k1, b1, ...] (the plugin
+    def _factors(self):
+        """Per-array (l2, l1) factors in Keras weight order [k0, b0, k1, b1, ...] (the plugin
         regularises its hidden layers only: plugins/hpbandster/base.py:113-116,152-155)."""
-        out = []
-        for lyr in self.layers:
-            for r in (lyr.kernel_regularizer, lyr.bias_regularizer):
-                out.append(0.0 if r is None else float(r.l2))
-        return out
+        return regularizer_factors(r for lyr in self.layers for r in (lyr.kernel_regularizer, lyr.bias_regularizer))
+
+    def _l2(self):
+        return self._factors()[0]
 
     def _engine(self, input_dim=None):
         """Build (once) the native handle; Keras builds lazily at the first call too."""
@@ -219,7 +218,8 @@ class Sequential:
                 permutations = np.stack([self._rs.permutation(N) for _ in range(epochs)])
             else:
                 permutations = np.tile(np.arange(N), (epochs, 1))
-        loss_dev = net.fit_async(X, z, epochs, batch_size, permutations, l2=self._l2(), w=w)
+        l2, l1 = self._factors()
+        loss_dev = net.fit_async(X, z, epochs, batch_size, permutations, l2=l2, w=w, l1=l1)
         hist = History(lambda: loss_dev.cpu().numpy()[0], epochs)
         if verbose:
             loss = hist.history["loss"]
@@ -239,7 +239,8 @@ class Sequential:
         X = np.asarray(x)
         z = np.asarray(y).reshape(-1)
         w = sample_weights(z, sample_weight)
-        out = self._engine(X.shape[1]).evaluate(X, z, l2=self._l2(), w=w)
+        l2, l1 = self._factors()
+        out = self._engine(X.shape[1]).evaluate(X, z, l2=l2, w=w, l1=l1)
         return out if self._compiled["metrics"] else out[0]
 
     def __call__(self, x):

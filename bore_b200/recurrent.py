@@ -22,7 +22,7 @@ import numpy as np
 
 from . import _lib, ops
 from .engine import ACT_CODES, OPT_NADAM, TRANSFORM_CODES, NativeMLP, _np_ptr, _ptr, _torch
-from .layers import BinaryCrossentropy, Dense, activation_name, optimizer_spec
+from .layers import BinaryCrossentropy, Dense, activation_name, optimizer_spec, regularizer_factors, regularizer_get
 from .mixins import MaximizableMixin
 from .models import History
 
@@ -41,9 +41,9 @@ class LSTMCell:
         activation = activation_name(activation, "LSTMCell")
         self.units = int(units)
         self.activation = activation
-        self.kernel_regularizer = kernel_regularizer
-        self.recurrent_regularizer = recurrent_regularizer
-        self.bias_regularizer = bias_regularizer
+        self.kernel_regularizer = regularizer_get(kernel_regularizer, "LSTMCell")
+        self.recurrent_regularizer = regularizer_get(recurrent_regularizer, "LSTMCell")
+        self.bias_regularizer = regularizer_get(bias_regularizer, "LSTMCell")
 
 
 class NativeLSTM:
@@ -135,11 +135,14 @@ class NativeLSTM:
         if cache is not None:
             _lib.check(self.lib.bore_lstm_set_nadam_cache(self.h, float(cache)))
 
-    def set_regularizers(self, l2):
-        """Per-array l2 factors in Keras weight order (3 per cell + 2)."""
+    def set_regularizers(self, l2, l1=None):
+        """Per-array l2 and l1 factors in Keras weight order (3 per cell + 2); ``l1=None`` is no l1 penalty."""
+        n = 3 * self.L + 2
         v = np.ascontiguousarray([float(t) for t in l2], np.float32)
-        assert v.shape == (3 * self.L + 2,)
+        v1 = np.zeros(n, np.float32) if l1 is None else np.ascontiguousarray([float(t) for t in l1], np.float32)
+        assert v.shape == (n,) and v1.shape == (n,)
         _lib.check(self.lib.bore_lstm_set_regularizers(self.h, _np_ptr(v)))
+        _lib.check(self.lib.bore_lstm_set_l1_regularizers(self.h, _np_ptr(v1)))
 
     # ------------------------------------------------------------------ inference
     def predict_sequences_dev(self, X_dev, mask_value=None):
@@ -295,18 +298,18 @@ class StackedRecurrentFactory:
             ws.append(self._rs.uniform(-lim, lim, size=(U, 1)).astype(np.float32))
             ws.append(np.zeros(1, np.float32))
             net.set_weights(ws)
-            net.set_regularizers(self._l2())
+            net.set_regularizers(*self._factors())
             self._net = net
         return self._net
 
+    def _factors(self):
+        """Per-array (l2, l1) factors in Keras weight order: kernel, recurrent kernel, bias of every cell, then
+        the final Dense layer's kernel and bias."""
+        regs = [r for c in self.cells for r in (c.kernel_regularizer, c.recurrent_regularizer, c.bias_regularizer)]
+        return regularizer_factors(regs + [self.final_layer.kernel_regularizer, self.final_layer.bias_regularizer])
+
     def _l2(self):
-        out = []
-        for c in self.cells:
-            for r in (c.kernel_regularizer, c.recurrent_regularizer, c.bias_regularizer):
-                out.append(0.0 if r is None else float(r.l2))
-        for r in (self.final_layer.kernel_regularizer, self.final_layer.bias_regularizer):
-            out.append(0.0 if r is None else float(r.l2))
-        return out
+        return self._factors()[0]
 
     def build_many_to_many(self, mask_value=1e+9):
         """Training network: masked many-to-many logits (bore/models.py:69-83)."""
@@ -391,7 +394,7 @@ class RecurrentSequential:
         if epochs <= 0 or N == 0:
             return History([])
         net = self._optimized_engine()
-        net.set_regularizers(self.factory._l2())
+        net.set_regularizers(*self.factory._factors())
         if permutations is None:
             permutations = (np.stack([self._rs.permutation(N) for _ in range(epochs)]) if shuffle
                             else np.tile(np.arange(N), (epochs, 1)))
@@ -406,7 +409,7 @@ class RecurrentSequential:
         if self._compiled is None:
             raise RuntimeError("You must compile your model before training/testing.")
         net = self.factory._engine()
-        net.set_regularizers(self.factory._l2())
+        net.set_regularizers(*self.factory._factors())
         out = net.evaluate(x, y, self.mask_value)
         return out if self._compiled["metrics"] else out[0]
 

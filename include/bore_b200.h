@@ -111,6 +111,11 @@ int bore_mlp_set_nadam_cache(bore_mlp *h, int model, float cache);
  * l2_bias[l] * sum(b_l^2) is added to the training loss (n_layers floats each; zeros = none).
  * The plugin regularises its hidden layers only (plugins/hpbandster/base.py:113-116,152-155). */
 int bore_mlp_set_regularizers(bore_mlp *h, const float *l2_kernel_host, const float *l2_bias_host);
+/* l1 regularisers (keras.regularizers.l1, the l1 half of l1_l2) per Dense layer: l1_kernel[l] * sum|W_l| +
+ * l1_bias[l] * sum|b_l| is added to the training loss and to evaluate's, next to the l2 terms; the gradient
+ * term is l1 * sign(w) with sign(0) = 0, as TF's Abs gradient.  n_layers floats each, finite and >= 0
+ * (anything else is refused); zeros = none, the state at create.                                      */
+int bore_mlp_set_l1_regularizers(bore_mlp *h, const float *l1_kernel_host, const float *l1_bias_host);
 /* device pointer of the flat parameter block [n_models][n_params] (for NCCL broadcast) */
 int bore_mlp_params_dev(bore_mlp *h, float **params_dev);
 
@@ -418,7 +423,7 @@ int bore_svgd_kernel_value_and_grad(const double *x_dev, int n, int D, double le
  *       weight, divided by batch x steps; perm_dev [epochs][N] int32; loss_dev [epochs].  One launch,
  *       asynchronous on `stream`.
  *   bore_lstm_evaluate           Model.evaluate (multi_fidelity.py:226): out_host[0] = masked loss
- *       (+ l2 terms), out_host[1] = binary accuracy of the LOGIT at 0.5 over the unmasked steps
+ *       (+ l1 / l2 terms), out_host[1] = binary accuracy of the LOGIT at 0.5 over the unmasked steps
  *       (the from_logits quirk; logging only).  Synchronises `stream`.                          */
 typedef struct bore_lstm bore_lstm;
 int bore_lstm_create(int input_dim, int units, int num_layers, int activation, int device, bore_lstm **out);
@@ -432,7 +437,11 @@ int bore_lstm_get_adam_state(bore_lstm *h, float *m_host, float *v_host, int64_t
 int bore_lstm_set_optimizer_kind(bore_lstm *h, int kind, const float *hp);
 int bore_lstm_get_nadam_cache(bore_lstm *h, float *cache_host);
 int bore_lstm_set_nadam_cache(bore_lstm *h, float cache);
+/* l2 and l1 factors per weight array in Keras order (kernel, recurrent kernel, bias of every cell, then
+ * the Dense kernel and bias: 3 * num_layers + 2 floats), as bore_mlp_set_regularizers /
+ * bore_mlp_set_l1_regularizers; the l1 factors must be finite and >= 0, and are 0 at create.      */
 int bore_lstm_set_regularizers(bore_lstm *h, const float *l2_per_array_host);
+int bore_lstm_set_l1_regularizers(bore_lstm *h, const float *l1_per_array_host);
 int bore_lstm_predict_sequences(bore_lstm *h, const float *X_dev, int S, int T, float mask_value,
                                 int use_mask, float *out_dev, void *stream);
 int bore_lstm_predict(bore_lstm *h, const float *X_dev, int S, int num_steps, float *out_dev, void *stream);
