@@ -295,6 +295,7 @@ struct LstmFitArgs {
   const float *X;       // [N][T][D]
   const float *Y;       // [N][T]
   int N, T, batch, epochs;
+  int sample_warps;     // warps that carve a BPTT strip and run phase 1 (<= 8, as many as shared memory holds)
   const int *perm;      // [epochs][N]
   float mask_value;
   OptHyper opt;
@@ -337,8 +338,8 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
       const int s0 = st * B, nb = min(B, a.N - s0);
       const float inv_n = 1.f / (float)(nb * T);
       float lsum = 0.f;
-      // ---- phase 1: forward + BPTT, warp per sample ----
-      for (int b = warp; b < nb; b += nw) {
+      // ---- phase 1: forward + BPTT, warp per sample (the warps without a strip add 0 to the loss) ----
+      for (int b = warp; warp < a.sample_warps && b < nb; b += a.sample_warps) {
         const int row = a.perm[(size_t)ep * a.N + s0 + b];
         const float *xs = a.X + (size_t)row * T * D;
         const float *ys = a.Y + (size_t)row * T;
@@ -613,6 +614,15 @@ size_t fit_scratch_floats(const LstmDesc &d, int T, int B) {
   return (size_t)d.L * T * B * AW + (size_t)d.L * T * B * 4 * d.U + (size_t)T * B * d.U + (size_t)T * B;
 }
 
+// Warps of a launch in which every warp keeps a strip of `strip` floats beside the weight image: as many
+// as 227 KB of shared memory holds, at most `max_warps`.  A net whose strips grow with steps and cells
+// (four cells of 32 units at 8 steps) runs on fewer warps instead of being refused; at least one, so
+// that a net not even one strip fits is refused by the launch's shared-memory check.
+int warps_that_fit(const LstmDesc &d, int strip, int max_warps) {
+  const int room = 227 * 1024 / (int)sizeof(float) - ((d.s_total + 3) & ~3);
+  return std::max(1, std::min(max_warps, room / strip));
+}
+
 }  // namespace
 
 extern "C" {
@@ -800,8 +810,9 @@ int bore_lstm_value_and_grad(bore_lstm *h, int num_steps, int transform, int neg
   BORE_CHECK(transform >= 0 && transform <= BORE_TRANSFORM_EXP, "unknown transform code %d", transform);
   if (S == 0) return 0;
   BORE_CUDA(cudaSetDevice(h->device));
-  const int warps = 4;
-  const size_t smem = ((size_t)((h->desc.s_total + 3) & ~3) + (size_t)warps * strip_floats(h->desc, num_steps, true)) * sizeof(float);
+  const int sf = strip_floats(h->desc, num_steps, true);
+  const int warps = warps_that_fit(h->desc, sf, 4);
+  const size_t smem = ((size_t)((h->desc.s_total + 3) & ~3) + (size_t)warps * sf) * sizeof(float);
   BORE_CHECK(smem <= 227 * 1024, "bore_lstm_value_and_grad: needs %zu B of shared memory", smem);
   const auto kernel = acts_ext(&h->desc.act, 1) ? lstm_value_grad_kernel<true> : lstm_value_grad_kernel<false>;
   BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -841,9 +852,12 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   for (int i = 0; i < 3 * LSTM_MAX_LAYERS + 2; ++i) { a.l2[i] = h->l2[i]; a.l1[i] = h->l1[i]; }
   a.loss_out = loss_dev;
   a.scratch = h->scratch;
+  // 256 threads whatever the number of sample warps: phase 2's GEMM mapping takes all of them
   const int warps = 8;
+  const int sf = strip_floats(h->desc, T, true);
+  a.sample_warps = warps_that_fit(h->desc, sf, warps);
   const int AW = (h->desc.D > h->desc.U ? h->desc.D : h->desc.U) + h->desc.U;
-  const size_t strips = (size_t)warps * strip_floats(h->desc, T, true);
+  const size_t strips = (size_t)a.sample_warps * sf;
   const size_t tiles = (size_t)LSTM_MAX_BATCH * (AW + 4 * h->desc.U);
   const size_t smem = ((size_t)((h->desc.s_total + 3) & ~3) + std::max(strips, tiles)) * sizeof(float);
   BORE_CHECK(smem <= 227 * 1024, "bore_lstm_fit: needs %zu B of shared memory", smem);

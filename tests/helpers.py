@@ -20,6 +20,32 @@ def synthetic_targets(X):
     return np.sum((X - 0.4) ** 2, axis=1) + 0.1 * np.sin(5.0 * X[:, 0]) * np.cos(3.0 * X[:, -1])
 
 
+def lstm_sequences(seed, N, T, D, mask_value):
+    """Padded per-rung sequences X (N, T, D), Y (N, T, 1) as the multi-fidelity record makes them: every
+    sequence stops at a random rung, every third may start one rung late, some have a masked gap."""
+    rs = np.random.RandomState(seed)
+    X = rs.uniform(size=(N, T, D))
+    Y = (rs.uniform(size=(N, T, 1)) < 0.4).astype(np.float64)
+    for n in range(N):
+        first = rs.randint(0, 2) if n % 3 == 0 and T > 1 else 0      # brackets that start at a higher budget
+        keep = rs.randint(first + 1, T + 1)
+        X[n, :first] = mask_value; Y[n, :first] = mask_value
+        X[n, keep:] = mask_value; Y[n, keep:] = mask_value
+        if n % 7 == 3 and keep - first > 2:
+            X[n, first + 1] = mask_value; Y[n, first + 1] = mask_value   # a gap
+    return X, Y
+
+
+def lstm_factory(D, U, L, activation, seed=0, l2f=None):
+    """StackedRecurrentFactory of L cells of U units on D inputs, l2(l2f) on the kernels and biases."""
+    from bore_b200.layers import l2
+    from bore_b200.models import StackedRecurrentFactory
+    reg = None if l2f is None else l2(l2f)
+    return StackedRecurrentFactory(D, 1, num_layers=L, num_units=U, seed=seed,
+                                   layer_kws=dict(activation=activation, kernel_regularizer=reg,
+                                                  bias_regularizer=reg))
+
+
 def trained_weights(dims, acts, seed=0, N=300, epochs=30, gamma=0.25):
     """Glorot init + a short oracle fit on quantile-labelled data: realistic, non-degenerate
     weights for value/gradient/argmax parity."""

@@ -10,31 +10,9 @@ import numpy as np
 import pytest
 
 from oracle import keras_lstm as kl
+from helpers import lstm_factory as _factory, lstm_sequences as _sequences
 
 pytestmark = pytest.mark.gpu
-
-
-def _sequences(seed, N, T, D, mask_value):
-    rs = np.random.RandomState(seed)
-    X = rs.uniform(size=(N, T, D))
-    Y = (rs.uniform(size=(N, T, 1)) < 0.4).astype(np.float64)
-    for n in range(N):
-        first = rs.randint(0, 2) if n % 3 == 0 else 0      # brackets that start at a higher budget
-        keep = rs.randint(first + 1, T + 1)
-        X[n, :first] = mask_value; Y[n, :first] = mask_value
-        X[n, keep:] = mask_value; Y[n, keep:] = mask_value
-        if n % 7 == 3 and keep - first > 2:
-            X[n, first + 1] = mask_value; Y[n, first + 1] = mask_value   # a gap
-    return X, Y
-
-
-def _factory(D, U, L, activation, seed=0, l2f=None):
-    from bore_b200.layers import l2
-    from bore_b200.models import StackedRecurrentFactory
-    reg = None if l2f is None else l2(l2f)
-    return StackedRecurrentFactory(D, 1, num_layers=L, num_units=U, seed=seed,
-                                   layer_kws=dict(activation=activation, kernel_regularizer=reg,
-                                                  bias_regularizer=reg))
 
 
 CASES = [(5, 8, 2, "tanh"), (8, 32, 2, "elu"), (3, 16, 1, "relu"), (32, 32, 3, "elu"), (6, 24, 4, "sigmoid")]

@@ -10,7 +10,7 @@ import pytest
 from oracle import keras_lstm as kl, keras_mlp as km
 import optimizer_oracle as oo
 import weighted_oracle as wo
-from helpers import synthetic_targets
+from helpers import lstm_factory, lstm_sequences, synthetic_targets
 from bore_b200 import layers
 
 pytestmark = pytest.mark.gpu
@@ -246,18 +246,17 @@ def test_reset_and_kind_change():
 def test_lstm(name):
     """The LSTM fit kernel under every kind against keras_lstm with the optimizer oracle, with the bars of
     tests/test_gpu_lstm.py; two fit calls, the state persists between them."""
-    import test_gpu_lstm as tgl
     from bore_b200.layers import BinaryCrossentropy
     o = make(name) if name != "adam_custom" else layers.Adam(learning_rate=3e-3, beta_1=0.8, beta_2=0.99,
                                                              epsilon=1e-6)
     D, U, L, N, B, T, mv, E = 8, 32, 2, 100, 64, 4, -1.0, 12
-    X, Y = tgl._sequences(4, N, T, D, mv)
+    X, Y = lstm_sequences(4, N, T, D, mv)
     rs = np.random.RandomState(5)
     perms = np.stack([rs.permutation(N) for _ in range(E)])
     w0 = kl.init_weights(D, U, L, seed=6)
     w64 = [a.astype(np.float64) for a in w0]
     h64, st = kl.fit(w64, "tanh", X, Y, E, B, perms, mv, adam=oo.state_for(w64, o, np.float64), dtype=np.float64)
-    net = tgl._factory(D, U, L, "tanh").build_many_to_many(mask_value=mv)
+    net = lstm_factory(D, U, L, "tanh").build_many_to_many(mask_value=mv)
     net.compile(optimizer=o, loss=BinaryCrossentropy(from_logits=True))
     net.set_weights(w0)
     ha = net.fit(X, Y, epochs=6, batch_size=B, permutations=perms[:6], verbose=0).history["loss"]

@@ -11,7 +11,7 @@ from oracle import keras_lstm as kl, keras_mlp as km
 import optimizer_oracle as oo
 import regularizer_oracle as ro
 import weighted_oracle as wo
-from helpers import synthetic_targets
+from helpers import lstm_factory, lstm_sequences, synthetic_targets
 from bore_b200 import layers
 
 pytestmark = pytest.mark.gpu
@@ -237,11 +237,10 @@ def _lstm_factors(L):
 
 
 def test_lstm_fit_and_evaluate():
-    import test_gpu_lstm as tgl
     from bore_b200.layers import BinaryCrossentropy
     from bore_b200.models import StackedRecurrentFactory
     D, U, L, N, B, T, mv, E = 8, 32, 2, 100, 64, 4, -1.0, 12
-    X, Y = tgl._sequences(4, N, T, D, mv)
+    X, Y = lstm_sequences(4, N, T, D, mv)
     rs = np.random.RandomState(5)
     perms = np.stack([rs.permutation(N) for _ in range(E)])
     w0 = kl.init_weights(D, U, L, seed=6)
@@ -313,12 +312,11 @@ def test_zero_l1_is_bit_identical():
         assert np.array_equal(ha, hb) and ea == eb, mode
         assert all(np.array_equal(a, b) for a, b in zip(wa, wb)), mode
         assert all(np.array_equal(a, b) for a, b in zip(sa[0] + sa[1], sb[0] + sb[1])) and sa[2] == sb[2], mode
-    import test_gpu_lstm as tgl
     D, U, L, T, mv = 8, 32, 2, 4, -1.0
-    Xs, Ys = tgl._sequences(4, 64, T, D, mv)
+    Xs, Ys = lstm_sequences(4, 64, T, D, mv)
     out = []
     for l1 in (None, [0.0] * (3 * L + 2)):
-        net = tgl._factory(D, U, L, "tanh")._engine()
+        net = lstm_factory(D, U, L, "tanh")._engine()
         net.set_weights(kl.init_weights(D, U, L, seed=6))
         net.set_regularizers([1e-3] * (3 * L + 2), l1)
         loss = net.fit_async(Xs, Ys, 3, 32, np.stack([np.arange(64)] * 3), mv).cpu().numpy()
@@ -353,8 +351,7 @@ def test_zero_bias_gets_no_l1_gradient(mode):
 def test_native_argument_checks(native_lib):
     lib = native_lib
     net = _net(DIMS, ACTS)
-    import test_gpu_lstm as tgl
-    lstm = tgl._factory(8, 16, 2, "tanh")._engine()
+    lstm = lstm_factory(8, 16, 2, "tanh")._engine()
     ok = (C.c_float * 8)(*([1e-3] * 8))
     for bad in (-1e-3, float("nan"), float("inf")):
         arr = (C.c_float * 8)(*([1e-3] * 7 + [bad]))
