@@ -4,6 +4,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/bore_b200.h"
@@ -99,6 +100,16 @@ struct bore_mlp {
 };
 
 static inline int round_up(int a, int b) { return (a + b - 1) / b * b; }
+
+// f(std::bool_constant<b0>{}, std::bool_constant<b1>{}, ...): picks the build of a kernel template for run-time
+// flags, e.g. with_flags([](auto w, auto o) { return kern<w, o>; }, weighted, opt) (every build is instantiated)
+template <class F>
+auto with_flags(F f) { return f(); }
+template <class F, class... Bs>
+auto with_flags(F f, bool b, Bs... bs) {
+  if (b) return with_flags([&](auto... c) { return f(std::true_type{}, c...); }, bs...);
+  return with_flags([&](auto... c) { return f(std::false_type{}, c...); }, bs...);
+}
 
 // Per-sample loss weights of a weighted fit / evaluate (bore_mlp_fit_weighted): the weight of sample i is
 // w[i] (1 when w is NULL) times cw1 if its label is 1, else cw0.  w has the layout of the labels.  on == 0:
@@ -201,13 +212,3 @@ int launch_mlp_eval_multi(const bore_mlp *h, int model0, int n_models, int per_m
 // it runs, else -1 with the shared memory needed and the limit in the error text.  Host only, no device.
 int mlp_eval_check_envelope(const MlpDesc &d);
 int fit_check_envelope(const MlpDesc &d);
-// K1t (fit_mma.cu): 1 launched, 0 shape not taken (caller falls back to the FFMA kernels), < 0 error.
-// `tab`: the launch's problems (a ragged fit; N is then the largest N_p) or no table (uniform).
-int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
-                   int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                   float *loss_out_dev, const FitWeights &fw, FitTable &tab, cudaStream_t stream);
-// K1u (fit_unit.cu): one cluster per model, hidden units split over the CTAs.  1 launched, 0 shape not
-// taken (caller falls back to the sample-split cluster kernel), < 0 error
-int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
-                    int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                    float *loss_out_dev, const FitWeights &fw, FitTable &tab, cudaStream_t stream);

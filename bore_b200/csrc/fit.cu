@@ -114,24 +114,8 @@ __host__ __device__ inline void make_fit_plan(const MlpDesc &d, int batch, int t
   p.total = r4(off);
 }
 
-struct FitArgs {
-  MlpDesc d;
+struct FitArgs : FitJob {
   FitPlan P;
-  float *params, *adam_m, *adam_v;
-  long long *adam_t;
-  int model0;
-  const float *X, *z;
-  int N, shared_data, batch, epochs;
-  const int *perm;
-  int shared_perm;
-  float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
-  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];
-  int any_reg;  // some l1 or l2 factor is non-zero
-  float *loss_out;
-  OptHyper opt;
-  FitWeights fw;
-  const FitProblem *probs;  // NULL: uniform launch
-  float *opt_cache;         // [n_models] Nadam's momentum cache
 };
 
 // acc[i][u] += sum_k A[k*lda + i] * B[k*ldb + u]: the 4 x 4 register tile of every GEMM below
@@ -780,24 +764,8 @@ __host__ __device__ inline void make_fitc_plan(const MlpDesc &d, int batch, FitC
   p.total = r4(off);
 }
 
-struct FitCArgs {
-  MlpDesc d;
+struct FitCArgs : FitJob {
   FitCPlan P;
-  float *params, *adam_m, *adam_v;
-  long long *adam_t;
-  int model0;
-  const float *X, *z;
-  int N, shared_data, batch, epochs;
-  const int *perm;
-  int shared_perm;
-  const FitProblem *probs;  // NULL: uniform launch (fit_problem)
-  float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
-  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];
-  int any_reg;  // some l1 or l2 factor is non-zero
-  float *loss_out;
-  OptHyper opt;
-  FitWeights fw;
-  float *opt_cache;  // [n_models] Nadam's momentum cache
 };
 
 __device__ __forceinline__ uint32_t cluster_rank() {
@@ -1228,12 +1196,6 @@ fit_cluster_kernel(const FitCArgs a) {
   cluster_wait();  // nobody exits while a peer may still read its shared memory
 }
 
-// the build of a kernel for an optimizer kind: OPT for every kind but Adam
-template <bool W, bool R, bool E>
-static auto fit_onecta_for(bool opt) { return opt ? fit_kernel<W, R, E, true> : fit_kernel<W, R, E, false>; }
-template <bool W, bool E>
-static auto fit_cluster_for(bool opt) { return opt ? fit_cluster_kernel<W, E, true> : fit_cluster_kernel<W, E, false>; }
-
 // ---------------------------------------------------------------- evaluate (loss, accuracy)
 __global__ void __launch_bounds__(256)
 evaluate_kernel(const MlpDesc d, const float *__restrict__ params, const float *__restrict__ logits,
@@ -1314,12 +1276,82 @@ int fit_check_envelope(const MlpDesc &d) {
   return 0;
 }
 
+// The handle's part of a fit job: the net, its training state and optimizer, and its l1 / l2 factors with the
+// gates any_reg and any_l1.  The caller fills in the launch's data.
+static FitJob fit_job(const bore_mlp *h) {
+  FitJob j{};
+  j.d = h->desc;
+  j.params = h->params; j.adam_m = h->adam_m; j.adam_v = h->adam_v; j.adam_t = h->adam_t;
+  j.opt_cache = h->opt_cache; j.opt = h->opt;
+  for (int l = 0; l < h->desc.n_layers; ++l) {
+    j.l2k[l] = h->l2k[l]; j.l2b[l] = h->l2b[l]; j.l1k[l] = h->l1k[l]; j.l1b[l] = h->l1b[l];
+    if (j.l1k[l] != 0.f || j.l1b[l] != 0.f) j.any_l1 = 1;
+    if (j.any_l1 || j.l2k[l] != 0.f || j.l2b[l] != 0.f) j.any_reg = 1;
+  }
+  return j;
+}
+
+// The sample-split cluster kernel (K1c), one cluster of FIT_CLUSTER CTAs per model.  A net whose plan does not fit
+// is an error in fit mode 2, else not taken.
+static int launch_fit_cluster(const bore_mlp *h, const FitJob &job, int count, FitTable &tab, cudaStream_t stream) {
+  FitCArgs a{job};
+  size_t smem;
+  if (!fitc_plan(job.d, job.batch < job.N ? job.batch : job.N, a.P, smem)) {
+    BORE_CHECK(h->fit_mode != 2, "bore_mlp_fit: cluster mode needs %zu B of shared memory", smem);
+    return 0;
+  }
+  BORE_CHECK_RC(tab.get(&a.probs));
+  const auto kern = with_flags([](auto w, auto e, auto o) { return fit_cluster_kernel<w, e, o>; }, job.fw.on,
+                               acts_ext(job.d.act, job.d.n_layers), job.opt.kind != BORE_OPT_ADAM);
+  BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<count * FIT_CLUSTER, FIT_CTHREADS, smem, stream>>>(a);
+  BORE_CUDA(cudaGetLastError());
+  return 1;
+}
+
+// The one-CTA kernel (K1): takes every net bore_mlp_create accepts, up to the shared memory of larger batches.
+static int launch_fit_onecta(const bore_mlp *h, const FitJob &job, int count, FitTable &tab, cudaStream_t stream) {
+  // threads per CTA: with more models than CTA slots the throughput is set by how many CTAs are
+  // resident -- smaller CTAs, more of them (BORE_FIT_THREADS overrides).  Measured with the first
+  // version of the kernel, cfg 4 (4,096 x Dense32x2 models, ms per BO iteration of all of them):
+  // 256 threads 462, 128 threads 314, 64 threads 332, 32 threads 397
+  int threads = count >= 2 * h->sm_count ? 128 : FIT_THREADS;
+  {
+    static int forced = -1;
+    if (forced < 0) {
+      const char *e = getenv("BORE_FIT_THREADS");
+      forced = e ? atoi(e) : 0;
+    }
+    if (forced == 32 || forced == 64 || forced == 128 || forced == 256) threads = forced;
+  }
+  FitArgs a{job};
+  const int B = job.batch < job.N ? job.batch : job.N;
+  size_t smem;
+  {
+    static int narrow = -1;
+    if (narrow < 0) {
+      const char *e = getenv("BORE_FIT_NARROW");
+      narrow = e ? atoi(e) : 1;
+    }
+    smem = fit_onecta_plan(job.d, B, threads, narrow, a.P);
+  }
+  BORE_CHECK(smem <= FIT_MAX_SMEM, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
+  BORE_CHECK_RC(tab.get(&a.probs));
+  const auto kern = with_flags([](auto w, auto r, auto e, auto o) { return fit_kernel<w, r, e, o>; }, job.fw.on,
+                               a.probs != nullptr, acts_ext(job.d.act, job.d.n_layers),
+                               job.opt.kind != BORE_OPT_ADAM || job.any_l1);
+  BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  kern<<<count, threads, smem, stream>>>(a);
+  BORE_CUDA(cudaGetLastError());
+  return 1;
+}
+
 // bore_mlp_fit, bore_mlp_fit_weighted and bore_mlp_fit_ragged: the same checks and the same choice of kernel;
 // fw.on == 0 runs every kernel with its unweighted arithmetic.  probs_host (ragged fits; NULL otherwise): the
 // `count` problems of the launch in launch order, N the largest N_p and epochs the largest epochs_p.
 static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
                    int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                   float *loss_out_dev, const FitWeights &fw, void *stream,
+                   float *loss_out_dev, const FitWeights &fw, void *stream_,
                    const FitProblem *probs_host = nullptr) {
   BORE_CHECK(h != nullptr, "NULL handle");
   BORE_CHECK(model0 >= 0 && count >= 1 && model0 + count <= h->n_models,
@@ -1332,23 +1364,16 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
              "bore_mlp_fit: binary cross-entropy needs a sigmoid or linear (from_logits) output layer");
   BORE_CUDA(cudaSetDevice(h->device));
   if (epochs == 0) return 0;
-  FitArgs a;
-  a.d = h->desc;
-  const int B = batch_size < N ? batch_size : N;
-  a.params = h->params; a.adam_m = h->adam_m; a.adam_v = h->adam_v; a.adam_t = h->adam_t;
-  a.model0 = model0;
-  a.X = X_dev; a.z = z_dev; a.N = N; a.shared_data = shared_data; a.batch = batch_size;
-  a.epochs = epochs; a.perm = perm_dev; a.shared_perm = shared_perm;
-  fit_regularizers(h, a);
-  a.loss_out = loss_out_dev;
-  a.opt = h->opt; a.opt_cache = h->opt_cache;
-  a.fw = fw;
+  const cudaStream_t stream = (cudaStream_t)stream_;
+  FitJob job = fit_job(h);
+  job.model0 = model0;
+  job.X = X_dev; job.z = z_dev; job.N = N; job.shared_data = shared_data; job.batch = batch_size;
+  job.epochs = epochs; job.perm = perm_dev; job.shared_perm = shared_perm;
+  job.loss_out = loss_out_dev;
+  job.fw = fw;
   // ragged fits: uploaded by the launch path that takes the net, after its refusals; freed on the stream after
   // the launch
-  FitTable table{h, probs_host, count, (cudaStream_t)stream, {}};
-  a.probs = nullptr;
-  const bool ext = acts_ext(a.d.act, a.d.n_layers);
-  bool opt = h->opt.kind != BORE_OPT_ADAM;
+  FitTable table{h, probs_host, count, stream, {}};
   // Tensor-pipe kernel (fit_mma.cu: 3xTF32 mma.sync GEMMs, one CTA per model) on request only (fit mode 3 or
   // BORE_FIT_MMA=1): measured SLOWER than both FFMA mappings below on B200 -- the legacy HMMA path gives
   // 3xTF32 only 1.3x the FFMA peak and every HMMA needs ~14 more instructions for fragments and splits
@@ -1360,8 +1385,7 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
       mma_env = e ? atoi(e) : 0;
     }
     if (h->fit_mode == 3 || (h->fit_mode == 0 && mma_env)) {
-      const int rc = launch_fit_mma(h, model0, count, X_dev, z_dev, N, shared_data, batch_size, epochs, perm_dev,
-                                    shared_perm, loss_out_dev, fw, table, (cudaStream_t)stream);
+      const int rc = launch_fit_mma(h, job, count, table, stream);
       if (rc != 0) return rc < 0 ? rc : 0;
       BORE_CHECK(h->fit_mode != 3, "bore_mlp_fit: the tensor-pipe kernel does not take this net / batch size");
     }
@@ -1377,74 +1401,17 @@ static int fit_run(bore_mlp *h, int model0, int count, const float *X_dev, const
       unit_env = e ? atoi(e) : 1;
     }
     if (h->fit_mode == 4 || (h->fit_mode == 0 && unit_env && count * FIT_CLUSTER <= h->sm_count)) {
-      const int rc = launch_fit_unit(h, model0, count, X_dev, z_dev, N, shared_data, batch_size, epochs, perm_dev,
-                                     shared_perm, loss_out_dev, fw, table, (cudaStream_t)stream);
+      const int rc = launch_fit_unit(h, job, count, table, stream);
       if (rc != 0) return rc < 0 ? rc : 0;
       BORE_CHECK(h->fit_mode != 4, "bore_mlp_fit: the unit-split cluster kernel does not take this net / batch size");
     }
   }
-  {
-    FitCPlan CP;
-    size_t csmem;
-    const bool fits = fitc_plan(a.d, B, CP, csmem);
-    const bool want = h->fit_mode == 2 || (h->fit_mode == 0 && count * FIT_CLUSTER <= h->sm_count);
-    BORE_CHECK(!(h->fit_mode == 2 && !fits), "bore_mlp_fit: cluster mode needs %zu B of shared memory", csmem);
-    if (want && fits) {
-      FitCArgs c;
-      BORE_CHECK_RC(table.get(&a.probs));
-      c.d = a.d; c.P = CP;
-      c.params = a.params; c.adam_m = a.adam_m; c.adam_v = a.adam_v; c.adam_t = a.adam_t;
-      c.model0 = a.model0; c.X = a.X; c.z = a.z; c.N = a.N; c.shared_data = a.shared_data;
-      c.batch = a.batch; c.epochs = a.epochs; c.perm = a.perm; c.shared_perm = a.shared_perm;
-      c.probs = a.probs;
-      fit_regularizers(h, c);
-      c.loss_out = a.loss_out;
-      c.opt = a.opt; c.opt_cache = a.opt_cache;
-      c.fw = a.fw;
-      const auto kern = ext ? (a.fw.on ? fit_cluster_for<true, true>(opt) : fit_cluster_for<false, true>(opt))
-                            : (a.fw.on ? fit_cluster_for<true, false>(opt) : fit_cluster_for<false, false>(opt));
-      BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)csmem));
-      kern<<<count * FIT_CLUSTER, FIT_CTHREADS, csmem, (cudaStream_t)stream>>>(c);
-      BORE_CUDA(cudaGetLastError());
-      return 0;
-    }
+  if (h->fit_mode == 2 || (h->fit_mode == 0 && count * FIT_CLUSTER <= h->sm_count)) {
+    const int rc = launch_fit_cluster(h, job, count, table, stream);
+    if (rc != 0) return rc < 0 ? rc : 0;
   }
-  // threads per CTA: with more models than CTA slots the throughput is set by how many CTAs are
-  // resident -- smaller CTAs, more of them (BORE_FIT_THREADS overrides).  Measured with the first
-  // version of the kernel, cfg 4 (4,096 x Dense32x2 models, ms per BO iteration of all of them):
-  // 256 threads 462, 128 threads 314, 64 threads 332, 32 threads 397
-  int threads = count >= 2 * h->sm_count ? 128 : FIT_THREADS;
-  {
-    static int forced = -1;
-    if (forced < 0) {
-      const char *e = getenv("BORE_FIT_THREADS");
-      forced = e ? atoi(e) : 0;
-    }
-    if (forced == 32 || forced == 64 || forced == 128 || forced == 256) threads = forced;
-  }
-  size_t smem;
-  {
-    static int narrow = -1;
-    if (narrow < 0) {
-      const char *e = getenv("BORE_FIT_NARROW");
-      narrow = e ? atoi(e) : 1;
-    }
-    smem = fit_onecta_plan(a.d, B, threads, narrow, a.P);
-  }
-  BORE_CHECK(smem <= FIT_MAX_SMEM, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
-  BORE_CHECK_RC(table.get(&a.probs));
-  // the l1 terms are in the OPT build only; with Adam its arithmetic is the default build's
-  bool any_l1 = false;
-  for (int l = 0; l < BORE_MAX_LAYERS; ++l) any_l1 = any_l1 || a.l1k[l] != 0.f || a.l1b[l] != 0.f;
-  opt = opt || any_l1;
-  const auto kern = ext ? (a.probs ? (a.fw.on ? fit_onecta_for<true, true, true>(opt) : fit_onecta_for<false, true, true>(opt))
-                                   : (a.fw.on ? fit_onecta_for<true, false, true>(opt) : fit_onecta_for<false, false, true>(opt)))
-                        : (a.probs ? (a.fw.on ? fit_onecta_for<true, true, false>(opt) : fit_onecta_for<false, true, false>(opt))
-                                   : (a.fw.on ? fit_onecta_for<true, false, false>(opt) : fit_onecta_for<false, false, false>(opt)));
-  BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  kern<<<count, threads, smem, (cudaStream_t)stream>>>(a);
-  BORE_CUDA(cudaGetLastError());
-  return 0;
+  const int rc = launch_fit_onecta(h, job, count, table, stream);
+  return rc < 0 ? rc : 0;
 }
 
 int FitTable::get(const FitProblem **out) {
@@ -1487,15 +1454,11 @@ static int evaluate_run(bore_mlp *h, int model, const float *X_dev, const float 
   float *logits = nullptr, *out2 = nullptr;
   BORE_CUDA(cudaMalloc(&logits, (size_t)N * sizeof(float)));
   BORE_CUDA(cudaMalloc(&out2, (2 + 4 * BORE_MAX_LAYERS) * sizeof(float)));
+  const FitJob job = fit_job(h);
   float reghost[4 * BORE_MAX_LAYERS];
-  bool any = false;
   for (int l = 0; l < BORE_MAX_LAYERS; ++l) {
-    const bool in = l < h->desc.n_layers;
-    reghost[4 * l] = in ? h->l2k[l] : 0.f;
-    reghost[4 * l + 1] = in ? h->l2b[l] : 0.f;
-    reghost[4 * l + 2] = in ? h->l1k[l] : 0.f;
-    reghost[4 * l + 3] = in ? h->l1b[l] : 0.f;
-    for (int q = 0; q < 4; ++q) any = any || reghost[4 * l + q] != 0.f;
+    reghost[4 * l] = job.l2k[l]; reghost[4 * l + 1] = job.l2b[l];
+    reghost[4 * l + 2] = job.l1k[l]; reghost[4 * l + 3] = job.l1b[l];
   }
   float *regdev = out2 + 2;
   cudaMemcpyAsync(regdev, reghost, sizeof(reghost), cudaMemcpyHostToDevice, stream);
@@ -1506,7 +1469,7 @@ static int evaluate_run(bore_mlp *h, int model, const float *X_dev, const float 
                            nullptr, nullptr, stream);
   if (!rc) {
     evaluate_kernel<<<1, 256, 0, stream>>>(h->desc, h->params + (size_t)model * h->desc.n_params,
-                                           logits, z_dev, N, any ? regdev : nullptr, fw, out2);
+                                           logits, z_dev, N, job.any_reg ? regdev : nullptr, fw, out2);
     cudaMemcpyAsync(out_host, out2, 2 * sizeof(float), cudaMemcpyDeviceToHost, stream);
     cudaError_t e = cudaStreamSynchronize(stream);
     if (e != cudaSuccess) { bore_set_error("bore_mlp_evaluate: %s", cudaGetErrorString(e)); rc = -2; }

@@ -1,8 +1,42 @@
-// Device helpers shared by the training kernels (fit.cu: FP32 FFMA; fit_mma.cu: 3xTF32 tensor pipe).
+// The job of an MLP fit launch and device helpers shared by the training kernels (fit.cu: FP32 FFMA;
+// fit_unit.cu: FFMA2; fit_mma.cu: 3xTF32 tensor pipe).
 #pragma once
 #include "common.cuh"
 #include "act.cuh"
 #include "opt.cuh"
+
+// What every MLP fit kernel reads besides its shared-memory plan: each kernel's arguments are a FitJob plus its
+// plan (FitArgs, FitCArgs, FuArgs, FitMArgs).  The l1 / l2 factors are zero past the net's last layer.
+// The build of a kernel (template flag OPT): every optimizer but Adam runs the OPT build.  fit_kernel (and
+// lstm_fit_kernel) also run it for Adam when any_l1 is set, since their l1 terms are in the OPT build only; the
+// cluster, unit-split and tensor-pipe kernels read l1 in every build.
+struct FitJob {
+  MlpDesc d;
+  float *params, *adam_m, *adam_v;
+  long long *adam_t;
+  int model0;
+  const float *X, *z;
+  int N, shared_data, batch, epochs;
+  const int *perm;
+  int shared_perm;
+  const FitProblem *probs;  // NULL: uniform launch (fit_problem)
+  float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
+  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];
+  int any_reg;  // some l1 or l2 factor is non-zero: the penalty is added to the reported loss
+  int any_l1;   // some l1 factor is non-zero
+  float *loss_out;
+  OptHyper opt;
+  FitWeights fw;
+  float *opt_cache;  // [n_models] Nadam's momentum cache
+};
+
+// The launchers of the fit kernels, tried in this order by fit_run (fit.cu): 1 launched, 0 shape not taken (the
+// next one is tried), < 0 error.  `tab`: the launch's problems (a ragged fit; job.N is then the largest N_p) or
+// no table (uniform); a launcher uploads it after its last refusal.
+// K1t (fit_mma.cu): tensor pipe, one CTA per model, on request only
+int launch_fit_mma(const bore_mlp *h, const FitJob &job, int count, FitTable &tab, cudaStream_t stream);
+// K1u (fit_unit.cu): one cluster per model, hidden units split over the CTAs
+int launch_fit_unit(const bore_mlp *h, const FitJob &job, int count, FitTable &tab, cudaStream_t stream);
 
 namespace {
 
@@ -27,20 +61,5 @@ __device__ __forceinline__ float block_sum(float v, float *red) {
 // e / n for 0 <= e < 2^20 through a precomputed reciprocal (inv = 1.f / n): exact, the offset .5
 // keeps the product away from integer boundaries
 __device__ __forceinline__ int fdiv(int e, float inv) { return __float2int_rz(((float)e + 0.5f) * inv); }
-
-// The handle's l1 / l2 factors into a fit kernel's arguments (zero past the net's last layer) and the gate
-// any_reg that adds the penalty to the reported loss.
-template <class Args>
-static void fit_regularizers(const bore_mlp *h, Args &a) {
-  a.any_reg = 0;
-  for (int l = 0; l < BORE_MAX_LAYERS; ++l) {
-    const bool in = l < h->desc.n_layers;
-    a.l2k[l] = in ? h->l2k[l] : 0.f;
-    a.l2b[l] = in ? h->l2b[l] : 0.f;
-    a.l1k[l] = in ? h->l1k[l] : 0.f;
-    a.l1b[l] = in ? h->l1b[l] : 0.f;
-    if (a.l2k[l] != 0.f || a.l2b[l] != 0.f || a.l1k[l] != 0.f || a.l1b[l] != 0.f) a.any_reg = 1;
-  }
-}
 
 }  // namespace

@@ -122,24 +122,8 @@ bool make_fitm_plan(const MlpDesc &d, int B, int nwarps, FitMPlan &p) {
   return true;
 }
 
-struct FitMArgs {
-  MlpDesc d;
+struct FitMArgs : FitJob {
   FitMPlan P;
-  float *params, *adam_m, *adam_v;
-  long long *adam_t;
-  int model0;
-  const float *X, *z;
-  int N, shared_data, batch, epochs;
-  const int *perm;
-  int shared_perm;
-  const FitProblem *probs;  // NULL: uniform launch (fit_problem)
-  float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
-  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];
-  int any_reg;  // some l1 or l2 factor is non-zero
-  float *loss_out;
-  OptHyper opt;
-  FitWeights fw;
-  float *opt_cache;  // [n_models] Nadam's momentum cache
 };
 
 // ------------------------------------------------------------------------------------ mma plumbing
@@ -662,9 +646,8 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
 
 template <int NW, int TPW>
 int launch_cfg(const FitMArgs &a, int count, size_t smem, cudaStream_t stream) {
-  const bool ext = acts_ext(a.d.act, a.d.n_layers), opt = a.opt.kind != BORE_OPT_ADAM;
-  const auto kern = ext ? (opt ? fit_mma_kernel<NW, TPW, true, true> : fit_mma_kernel<NW, TPW, true, false>)
-                        : (opt ? fit_mma_kernel<NW, TPW, false, true> : fit_mma_kernel<NW, TPW, false, false>);
+  const auto kern = with_flags([](auto e, auto o) { return fit_mma_kernel<NW, TPW, e, o>; },
+                               acts_ext(a.d.act, a.d.n_layers), a.opt.kind != BORE_OPT_ADAM);
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count, NW * 32, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());
@@ -681,11 +664,8 @@ int launch_nw(const FitMArgs &a, int count, size_t smem, cudaStream_t stream) {
 
 }  // namespace
 
-// 1: launched; 0: shape not taken by the tensor kernel (caller falls back); < 0: error
-int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
-                   int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                   float *loss_out_dev, const FitWeights &fw, FitTable &tab, cudaStream_t stream) {
-  const int B = batch_size < N ? batch_size : N;
+int launch_fit_mma(const bore_mlp *h, const FitJob &job, int count, FitTable &tab, cudaStream_t stream) {
+  const int B = job.batch < job.N ? job.batch : job.N;
   // few models: one 16-warp CTA per model (latency); many: 4-warp CTAs, several per SM (throughput)
   int nw = count * 2 <= h->sm_count ? 16 : (count <= 2 * h->sm_count ? 8 : 4);
   {
@@ -696,8 +676,7 @@ int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev,
     }
     if (forced == 4 || forced == 8 || forced == 16) nw = forced;
   }
-  FitMArgs a;
-  a.d = h->desc;
+  FitMArgs a{job};
   bool ok = false;
   for (; nw <= 16; nw *= 2) {  // a wide layer may need more warps to own its update tiles
     if (make_fitm_plan(a.d, B, nw, a.P)) { ok = true; break; }
@@ -705,18 +684,7 @@ int launch_fit_mma(const bore_mlp *h, int model0, int count, const float *X_dev,
   if (!ok) return 0;
   const size_t smem = (size_t)a.P.total * sizeof(float);
   if (smem > 227 * 1024) return 0;
-  a.params = h->params; a.adam_m = h->adam_m; a.adam_v = h->adam_v; a.adam_t = h->adam_t;
-  a.model0 = model0;
-  a.X = X_dev; a.z = z_dev; a.N = N; a.shared_data = shared_data; a.batch = batch_size;
-  a.epochs = epochs; a.perm = perm_dev; a.shared_perm = shared_perm;
-  fit_regularizers(h, a);
-  a.loss_out = loss_out_dev;
-  a.opt = h->opt; a.opt_cache = h->opt_cache;
-  a.fw = fw;
-  {
-    const int rc = tab.get(&a.probs);  // taken: the table goes up now
-    if (rc) return rc;
-  }
+  BORE_CHECK_RC(tab.get(&a.probs));  // taken: the table goes up now
   int rc;
   if (nw == 16) rc = launch_nw<16>(a, count, smem, stream);
   else if (nw == 8) rc = launch_nw<8>(a, count, smem, stream);

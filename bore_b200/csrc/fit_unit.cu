@@ -145,24 +145,8 @@ __host__ __device__ inline bool make_fu_plan(const MlpDesc &d, int batch, FuPlan
   return true;
 }
 
-struct FuArgs {
-  MlpDesc d;
+struct FuArgs : FitJob {
   FuPlan P;
-  float *params, *adam_m, *adam_v;
-  long long *adam_t;
-  int model0;
-  const float *X, *z;
-  int N, shared_data, batch, epochs;
-  const int *perm;
-  int shared_perm;
-  const FitProblem *probs;  // NULL: uniform launch (fit_problem)
-  float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];
-  float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];
-  int any_reg;  // some l1 or l2 factor is non-zero
-  float *loss_out;
-  OptHyper opt;
-  FitWeights fw;
-  float *opt_cache;  // [n_models] Nadam's momentum cache
 };
 
 // ---------------------------------------------------------------- cluster / packed-FMA primitives
@@ -868,20 +852,14 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
 #undef FU_U
 }
 
-template <int NH, int HW, int SPT, bool OPT>
+template <int NH, int HW, int SPT>
 static int fu_launch(const FuArgs &a, int count, size_t smem, cudaStream_t stream) {
-  const auto kern = acts_ext(a.d.act, a.d.n_layers)
-                        ? (a.fw.on ? fit_unit_kernel<NH, HW, SPT, true, true, OPT> : fit_unit_kernel<NH, HW, SPT, false, true, OPT>)
-                        : (a.fw.on ? fit_unit_kernel<NH, HW, SPT, true, false, OPT> : fit_unit_kernel<NH, HW, SPT, false, false, OPT>);
+  const auto kern = with_flags([](auto w, auto e, auto o) { return fit_unit_kernel<NH, HW, SPT, w, e, o>; }, a.fw.on,
+                               acts_ext(a.d.act, a.d.n_layers), a.opt.kind != BORE_OPT_ADAM);
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count * FU_C, FU_THREADS, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());
   return 1;
-}
-template <int NH, int HW, int SPT>
-static int fu_launch(const FuArgs &a, int count, size_t smem, cudaStream_t stream) {
-  return a.opt.kind != BORE_OPT_ADAM ? fu_launch<NH, HW, SPT, true>(a, count, smem, stream)
-                                     : fu_launch<NH, HW, SPT, false>(a, count, smem, stream);
 }
 
 }  // namespace
@@ -894,13 +872,9 @@ static bool fu_plan(const MlpDesc &d, int batch, FuPlan &p, size_t &smem) {
   return p.SP <= 64 && smem <= 226 * 1024;
 }
 
-// 1 launched, 0 shape not taken (the caller falls back to the sample-split cluster kernel), < 0 error
-int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev, const float *z_dev, int N,
-                    int shared_data, int batch_size, int epochs, const int32_t *perm_dev, int shared_perm,
-                    float *loss_out_dev, const FitWeights &fw, FitTable &tab, cudaStream_t stream) {
-  FuArgs a;
-  a.d = h->desc;
-  const int B = batch_size < N ? batch_size : N;
+int launch_fit_unit(const bore_mlp *h, const FitJob &job, int count, FitTable &tab, cudaStream_t stream) {
+  FuArgs a{job};
+  const int B = job.batch < job.N ? job.batch : job.N;
   // compile-time shapes: NH hidden layers of one width (16 / 32 / 64), padded batch 64; BORE_FIT_UNIT_GENERIC=1
   // forces the run-time-shape build (A/B timing, tests of both).  A smaller batch (the first iterations of a BO
   // run have fewer than 64 observations) is padded to 64 samples for them: zero rows, zero dL/dlogit.
@@ -912,18 +886,7 @@ int launch_fit_unit(const bore_mlp *h, int model0, int count, const float *X_dev
                            ((nh == 3 && (hw == 64 || hw == 32)) || (nh == 2 && (hw == 32 || hw == 16)));
   size_t smem;
   if (!fu_plan(a.d, fixed_shape ? 64 : B, a.P, smem)) return 0;
-  a.params = h->params; a.adam_m = h->adam_m; a.adam_v = h->adam_v; a.adam_t = h->adam_t;
-  a.model0 = model0;
-  a.X = X_dev; a.z = z_dev; a.N = N; a.shared_data = shared_data; a.batch = batch_size;
-  a.epochs = epochs; a.perm = perm_dev; a.shared_perm = shared_perm;
-  fit_regularizers(h, a);
-  a.loss_out = loss_out_dev;
-  a.opt = h->opt; a.opt_cache = h->opt_cache;
-  a.fw = fw;
-  {
-    const int rc = tab.get(&a.probs);  // taken: the table goes up now
-    if (rc) return rc;
-  }
+  BORE_CHECK_RC(tab.get(&a.probs));  // taken: the table goes up now
   if (fixed_shape) {
     if (nh == 3 && hw == 64) return fu_launch<3, 64, 64>(a, count, smem, stream);
     if (nh == 3 && hw == 32) return fu_launch<3, 32, 64>(a, count, smem, stream);

@@ -863,9 +863,8 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   BORE_CHECK(smem <= 227 * 1024, "bore_lstm_fit: needs %zu B of shared memory", smem);
   bool any_l1 = false;
   for (int i = 0; i < 3 * LSTM_MAX_LAYERS + 2; ++i) any_l1 = any_l1 || h->l1[i] != 0.f;
-  const bool ext = acts_ext(&h->desc.act, 1), opt = h->opt.kind != BORE_OPT_ADAM || any_l1;
-  const auto kernel = ext ? (opt ? lstm_fit_kernel<true, true> : lstm_fit_kernel<true, false>)
-                          : (opt ? lstm_fit_kernel<false, true> : lstm_fit_kernel<false, false>);
+  const auto kernel = with_flags([](auto e, auto o) { return lstm_fit_kernel<e, o>; }, acts_ext(&h->desc.act, 1),
+                                 h->opt.kind != BORE_OPT_ADAM || any_l1);
   BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kernel<<<1, warps * 32, smem, (cudaStream_t)stream>>>(a);
   BORE_CUDA(cudaGetLastError());

@@ -563,8 +563,7 @@ static int launch_variant(const bore_mlp *h, const MlpDesc &d, int model0, const
   // two give bit-identical results)
   static const bool f2 = [] { const char *e = getenv("BORE_K2_FFMA2"); return !(e && e[0] == '0'); }();
   const bool ext = acts_ext(d.act, d.n_layers);
-  const auto kernel = f2 ? (ext ? mlp_eval_kernel<GRAD, UGB, true, true> : mlp_eval_kernel<GRAD, UGB, true, false>)
-                         : (ext ? mlp_eval_kernel<GRAD, UGB, false, true> : mlp_eval_kernel<GRAD, UGB, false, false>);
+  const auto kernel = with_flags([](auto f, auto e) { return mlp_eval_kernel<GRAD, UGB, f, e>; }, f2, ext);
   static bool attr_done[2][2][64] = {};  // per device: the attribute belongs to the device's context
   if (h->device >= 64 || !attr_done[f2][ext][h->device]) {
     BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 256));
