@@ -68,6 +68,42 @@ int opt_from_array(int kind, const float *hp, OptHyper &o, const char *who) {
   return 0;
 }
 
+int lr_schedule_from_array(int kind, const float *sp, int n_sp, LrSchedule &o, const char *who) {
+  BORE_CHECK(kind >= BORE_LR_CONSTANT && kind <= BORE_LR_PIECEWISE,
+             "%s: unknown schedule kind %d (BORE_LR_CONSTANT .. BORE_LR_PIECEWISE)", who, kind);
+  static const int n_of[] = {0, 4, 4, 5};  // sp entries of the kinds before BORE_LR_PIECEWISE
+  BORE_CHECK(n_sp >= 0 && (n_sp == 0 || sp != nullptr), "%s: %d schedule parameters, array NULL", who, n_sp);
+  if (kind == BORE_LR_PIECEWISE)
+    BORE_CHECK(n_sp % 2 == 1 && n_sp >= 3 && n_sp <= 2 * BORE_LR_MAX_BOUNDARIES + 1,
+               "%s: PiecewiseConstantDecay takes n boundaries and n + 1 values, 1 <= n <= %d (got %d parameters)",
+               who, BORE_LR_MAX_BOUNDARIES, n_sp);
+  else
+    BORE_CHECK(n_sp == n_of[kind], "%s: schedule kind %d takes %d parameters, got %d", who, kind, n_of[kind], n_sp);
+  for (int i = 0; i < n_sp; ++i) BORE_CHECK(isfinite(sp[i]), "%s: schedule parameter %d is %g", who, i, (double)sp[i]);
+  o = LrSchedule{};
+  o.kind = kind;
+  if (kind == BORE_LR_PIECEWISE) {
+    o.n = n_sp / 2;
+    for (int i = 0; i < o.n; ++i) {
+      BORE_CHECK(i == 0 || sp[i] > sp[i - 1], "%s: boundaries must be strictly increasing (%g after %g)", who,
+                 (double)sp[i], (double)sp[i - 1]);
+      o.bound[i] = sp[i];
+    }
+    for (int i = 0; i <= o.n; ++i) o.value[i] = sp[o.n + i];
+  } else if (kind != BORE_LR_CONSTANT) {
+    o.initial = sp[0];
+    o.decay_steps = sp[1];
+    BORE_CHECK(o.decay_steps > 0.f, "%s: decay_steps must be > 0, got %g", who, (double)o.decay_steps);
+    const float flag = sp[n_sp - 1];
+    BORE_CHECK(flag == 0.f || flag == 1.f, "%s: %s must be 0 or 1, got %g", who,
+               kind == BORE_LR_POLYNOMIAL ? "cycle" : "staircase", (double)flag);
+    o.flag = flag != 0.f;
+    if (kind == BORE_LR_POLYNOMIAL) { o.end = sp[2]; o.power = sp[3]; }
+    else o.rate = sp[2];
+  }
+  return 0;
+}
+
 extern "C" {
 
 int bore_abi_version(void) { return BORE_ABI_VERSION; }
@@ -251,6 +287,14 @@ int bore_mlp_set_optimizer_kind(bore_mlp *h, int kind, const float *hp) {
   BORE_CHECK_RC(opt_from_array(kind, hp, o, "bore_mlp_set_optimizer_kind"));
   BORE_CHECK(h != nullptr, "NULL handle");
   return mlp_change_optimizer(h, o);
+}
+
+int bore_mlp_set_lr_schedule(bore_mlp *h, int kind, const float *sp, int n_sp) {
+  LrSchedule s;
+  BORE_CHECK_RC(lr_schedule_from_array(kind, sp, n_sp, s, "bore_mlp_set_lr_schedule"));
+  BORE_CHECK(h != nullptr, "NULL handle");
+  h->sched = s;  // the state is kept, as Keras keeps its slots under a new rate
+  return 0;
 }
 
 int bore_mlp_get_nadam_cache(bore_mlp *h, int model, float *cache_host) {

@@ -73,6 +73,16 @@ struct OptHyper {
   int centered;    // RMSprop
 };
 
+// Learning-rate schedule of a handle (bore_mlp_set_lr_schedule / bore_lstm_set_lr_schedule), passed by value to
+// the fit kernels and evaluated once per step (lr_at, opt.cuh).  All zeros: BORE_LR_CONSTANT.
+struct LrSchedule {
+  int kind;  // BORE_LR_*
+  int flag;  // staircase (exponential, inverse time) or cycle (polynomial)
+  float initial, decay_steps, rate, end, power;
+  int n;  // piecewise: boundaries
+  float bound[BORE_LR_MAX_BOUNDARIES], value[BORE_LR_MAX_BOUNDARIES + 1];
+};
+
 struct MlpPackCache {
   float *buf[4];
   size_t cap[4];  // floats allocated
@@ -90,6 +100,7 @@ struct bore_mlp {
   long long *adam_t;   // [n_models]   Keras `iterations`
   float *opt_cache;    // [n_models]   Nadam's momentum cache
   OptHyper opt;
+  LrSchedule sched;
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];  // l2 regularisers per layer
   float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];  // l1 regularisers per layer
   int fit_mode;  // 0 auto, 1 one CTA per model (FFMA), 2 one cluster per model, samples split (FFMA), 3 tensor
@@ -192,6 +203,13 @@ int opt_reset_state(const OptHyper &opt, float *s0, float *s1, size_t n_params, 
                     int count, cudaStream_t stream);
 // bore_*_set_optimizer_kind's check of (kind, hp); 0, or -1 with the error text set
 int opt_from_array(int kind, const float *hp, OptHyper &out, const char *who);
+// bore_*_set_lr_schedule's check of (kind, sp, n_sp); 0, or -1 with the error text set
+int lr_schedule_from_array(int kind, const float *sp, int n_sp, LrSchedule &out, const char *who);
+// The build of a fit kernel (template flag OPT, opt.cuh): every optimizer but Adam, and any schedule, run the OPT
+// build.  fit_kernel and lstm_fit_kernel also run it for Adam with an l1 factor (fit_common.cuh, FitJob).
+inline bool opt_build(const OptHyper &o, const LrSchedule &s) {
+  return o.kind != BORE_OPT_ADAM || s.kind != BORE_LR_CONSTANT;
+}
 
 // ---------------------------------------------------------------- launchers (one per .cu)
 // K0 / K2.  `list` (may be NULL) is a device array of row indices: point i of the launch

@@ -336,7 +336,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
       float loss = block_sum(lsum, red) * inv_nb;  // (also the barrier publishing dz)
 
       // ---- optimizer scalars for this step ----
-      const OptStep os = run.step(a.opt);
+      const OptStep os = run.step(a.opt, a.sched);
       float reg = 0.f;
 
       // ---- reverse + update, top layer first ----
@@ -1016,7 +1016,7 @@ fit_cluster_kernel(const FitCArgs a) {
       if (tid == 0) sm[P.slots + par] = lsum;
 
       // ---- optimizer scalars for this step ----
-      const OptStep os = run.step(a.opt);
+      const OptStep os = run.step(a.opt, a.sched);
 
       // ---- reverse: per layer, delta_{l-1} and this CTA's partial dW_l / db_l ----
       int cur = 0;
@@ -1276,13 +1276,13 @@ int fit_check_envelope(const MlpDesc &d) {
   return 0;
 }
 
-// The handle's part of a fit job: the net, its training state and optimizer, and its l1 / l2 factors with the
-// gates any_reg and any_l1.  The caller fills in the launch's data.
+// The handle's part of a fit job: the net, its training state, optimizer and learning-rate schedule, and its l1 / l2
+// factors with the gates any_reg and any_l1.  The caller fills in the launch's data.
 static FitJob fit_job(const bore_mlp *h) {
   FitJob j{};
   j.d = h->desc;
   j.params = h->params; j.adam_m = h->adam_m; j.adam_v = h->adam_v; j.adam_t = h->adam_t;
-  j.opt_cache = h->opt_cache; j.opt = h->opt;
+  j.opt_cache = h->opt_cache; j.opt = h->opt; j.sched = h->sched;
   for (int l = 0; l < h->desc.n_layers; ++l) {
     j.l2k[l] = h->l2k[l]; j.l2b[l] = h->l2b[l]; j.l1k[l] = h->l1k[l]; j.l1b[l] = h->l1b[l];
     if (j.l1k[l] != 0.f || j.l1b[l] != 0.f) j.any_l1 = 1;
@@ -1302,7 +1302,7 @@ static int launch_fit_cluster(const bore_mlp *h, const FitJob &job, int count, F
   }
   BORE_CHECK_RC(tab.get(&a.probs));
   const auto kern = with_flags([](auto w, auto e, auto o) { return fit_cluster_kernel<w, e, o>; }, job.fw.on,
-                               acts_ext(job.d.act, job.d.n_layers), job.opt.kind != BORE_OPT_ADAM);
+                               acts_ext(job.d.act, job.d.n_layers), opt_build(job.opt, job.sched));
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count * FIT_CLUSTER, FIT_CTHREADS, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());
@@ -1339,7 +1339,7 @@ static int launch_fit_onecta(const bore_mlp *h, const FitJob &job, int count, Fi
   BORE_CHECK_RC(tab.get(&a.probs));
   const auto kern = with_flags([](auto w, auto r, auto e, auto o) { return fit_kernel<w, r, e, o>; }, job.fw.on,
                                a.probs != nullptr, acts_ext(job.d.act, job.d.n_layers),
-                               job.opt.kind != BORE_OPT_ADAM || job.any_l1);
+                               opt_build(job.opt, job.sched) || job.any_l1);
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count, threads, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());

@@ -7,9 +7,10 @@
 
 // What every MLP fit kernel reads besides its shared-memory plan: each kernel's arguments are a FitJob plus its
 // plan (FitArgs, FitCArgs, FuArgs, FitMArgs).  The l1 / l2 factors are zero past the net's last layer.
-// The build of a kernel (template flag OPT): every optimizer but Adam runs the OPT build.  fit_kernel (and
-// lstm_fit_kernel) also run it for Adam when any_l1 is set, since their l1 terms are in the OPT build only; the
-// cluster, unit-split and tensor-pipe kernels read l1 in every build.
+// The build of a kernel (template flag OPT, opt_build in common.cuh): every optimizer but Adam, and every
+// learning-rate schedule, run the OPT build.  fit_kernel (and lstm_fit_kernel) also run it for Adam when any_l1 is
+// set, since their l1 terms are in the OPT build only; the cluster, unit-split and tensor-pipe kernels read l1 in
+// every build.
 struct FitJob {
   MlpDesc d;
   float *params, *adam_m, *adam_v;
@@ -28,6 +29,7 @@ struct FitJob {
   OptHyper opt;
   FitWeights fw;
   float *opt_cache;  // [n_models] Nadam's momentum cache
+  LrSchedule sched;  // last: the members above keep their offsets
 };
 
 // The launchers of the fit kernels, tried in this order by fit_run (fit.cu): 1 launched, 0 shape not taken (the

@@ -401,7 +401,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
     const int nmb = (nb + 15) >> 4, BP = nmb << 4;
     const float inv_nb = 1.f / (float)nb;
     reg = 0.f;
-    run.advance(a.opt, os);
+    run.advance(a.opt, a.sched, os);
 
     const int row_next = row_of(gs + 1);  // (consumed after the forward pass)
     cp_async_wait_all();
@@ -647,7 +647,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
 template <int NW, int TPW>
 int launch_cfg(const FitMArgs &a, int count, size_t smem, cudaStream_t stream) {
   const auto kern = with_flags([](auto e, auto o) { return fit_mma_kernel<NW, TPW, e, o>; },
-                               acts_ext(a.d.act, a.d.n_layers), a.opt.kind != BORE_OPT_ADAM);
+                               acts_ext(a.d.act, a.d.n_layers), opt_build(a.opt, a.sched));
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count, NW * 32, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());

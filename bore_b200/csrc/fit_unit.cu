@@ -585,7 +585,7 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
       // ---- optimizer scalars of this step ----
       FU_T();
       FU_T();
-      const OptStep os = run.step(a.opt);
+      const OptStep os = run.step(a.opt, a.sched);
       FU_T();
       __syncthreads();  // dz and the loss slots are in place
       FU_T();
@@ -855,7 +855,7 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
 template <int NH, int HW, int SPT>
 static int fu_launch(const FuArgs &a, int count, size_t smem, cudaStream_t stream) {
   const auto kern = with_flags([](auto w, auto e, auto o) { return fit_unit_kernel<NH, HW, SPT, w, e, o>; }, a.fw.on,
-                               acts_ext(a.d.act, a.d.n_layers), a.opt.kind != BORE_OPT_ADAM);
+                               acts_ext(a.d.act, a.d.n_layers), opt_build(a.opt, a.sched));
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count * FU_C, FU_THREADS, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());

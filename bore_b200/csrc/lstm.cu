@@ -49,6 +49,7 @@ struct bore_lstm {
   long long adam_t;
   float *opt_cache;  // (device, 1 float) Nadam's momentum cache
   OptHyper opt;
+  LrSchedule sched;
   float l2[3 * LSTM_MAX_LAYERS + 2];  // per array, Keras order
   float l1[3 * LSTM_MAX_LAYERS + 2];
   float *scratch;
@@ -303,10 +304,11 @@ struct LstmFitArgs {
   float *loss_out;      // [epochs]
   float *scratch;       // A [L][T][B][AW] | Z [L][T][B][4U] | HT [T][B][U] | DU [T][B]
   float *opt_cache;     // Nadam's momentum cache (1 float)
+  LrSchedule sched;
 };
 
-// OPT: the optimizers other than Adam (opt.cuh) and the l1 regulariser terms; the Adam build keeps its own IEEE
-// arithmetic
+// OPT: the optimizers other than Adam (opt.cuh), the learning-rate schedules and the l1 regulariser terms; the Adam
+// build keeps its own IEEE arithmetic
 template <bool EXT, bool OPT>
 __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
   extern __shared__ __align__(16) float sm[];
@@ -436,7 +438,7 @@ __global__ void __launch_bounds__(256) lstm_fit_kernel(const LstmFitArgs a) {
       OptStep os;
       float alpha = 0.f;
       if (OPT) {
-        os = run.step(a.opt);
+        os = run.step(a.opt, a.sched);
       } else {
         run.t += 1;
         run.p1 *= (double)a.opt.b1; run.p2 *= (double)a.opt.b2;
@@ -723,6 +725,14 @@ int bore_lstm_set_optimizer_kind(bore_lstm *h, int kind, const float *hp) {
   return 0;
 }
 
+int bore_lstm_set_lr_schedule(bore_lstm *h, int kind, const float *sp, int n_sp) {
+  LrSchedule s;
+  BORE_CHECK_RC(lr_schedule_from_array(kind, sp, n_sp, s, "bore_lstm_set_lr_schedule"));
+  BORE_CHECK(h != nullptr, "NULL handle");
+  h->sched = s;  // the state is kept, as Keras keeps its slots under a new rate
+  return 0;
+}
+
 int bore_lstm_get_nadam_cache(bore_lstm *h, float *cache_host) {
   BORE_CHECK(h && cache_host, "NULL argument");
   BORE_CUDA(cudaSetDevice(h->device));
@@ -848,7 +858,7 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   a.t0 = h->adam_t;
   a.X = X_dev; a.Y = Y_dev; a.N = N; a.T = T; a.batch = batch_size; a.epochs = epochs;
   a.perm = perm_dev; a.mask_value = mask_value;
-  a.opt = h->opt; a.opt_cache = h->opt_cache;
+  a.opt = h->opt; a.opt_cache = h->opt_cache; a.sched = h->sched;
   for (int i = 0; i < 3 * LSTM_MAX_LAYERS + 2; ++i) { a.l2[i] = h->l2[i]; a.l1[i] = h->l1[i]; }
   a.loss_out = loss_dev;
   a.scratch = h->scratch;
@@ -864,7 +874,7 @@ int bore_lstm_fit(bore_lstm *h, const float *X_dev, const float *Y_dev, int N, i
   bool any_l1 = false;
   for (int i = 0; i < 3 * LSTM_MAX_LAYERS + 2; ++i) any_l1 = any_l1 || h->l1[i] != 0.f;
   const auto kernel = with_flags([](auto e, auto o) { return lstm_fit_kernel<e, o>; }, acts_ext(&h->desc.act, 1),
-                                 h->opt.kind != BORE_OPT_ADAM || any_l1);
+                                 opt_build(h->opt, h->sched) || any_l1);
   BORE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kernel<<<1, warps * 32, smem, (cudaStream_t)stream>>>(a);
   BORE_CUDA(cudaGetLastError());

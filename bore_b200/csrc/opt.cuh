@@ -9,8 +9,9 @@
 // Padding parameters of the kernels have a zero gradient and zero slots: every rule leaves them exactly zero
 // as long as eps > 0, which bore_*_set_optimizer_kind demands of every kind but Adam.
 //
-// Every fit kernel comes in two builds, selected at launch from the kind: OPT = false is Adam only, with the
-// arithmetic and the instructions it always had; OPT = true adds the other kinds.
+// Every fit kernel comes in two builds, selected at launch (opt_build, common.cuh): OPT = false is Adam at a
+// constant learning rate, with the arithmetic and the instructions it always had; OPT = true adds the other kinds
+// and the learning-rate schedules (lr_at).
 #pragma once
 #include "common.cuh"
 
@@ -22,10 +23,38 @@ constexpr double kNadamDecayBase = 0.96, kNadamCacheDecay = 0.004;
 // scalars of one step, the same for every parameter of a model
 struct OptStep {
   float om1, om2;  // 1 - beta_1 (or 1 - rho), 1 - beta_2
+  float lr;        // the learning rate of the step (OPT only): the schedule's, else the optimizer's
   float alpha;     // Adam: lr sqrt(1 - beta_2^t) / (1 - beta_1^t); Adamax: lr / (1 - beta_1^t); else lr
   float cg, cm;    // Nadam: (1 - mu_t) / (1 - cache_t), mu_{t+1} / (1 - cache_t mu_{t+1})
   float vd;        // Nadam: 1 / (1 - beta_2^t)
 };
+
+// Keras learning-rate schedules (keras/optimizer_v2/learning_rate_schedule.py, TF 2.5) at `step`, fp32 as Keras
+// computes them on a float32 initial_learning_rate; `lr` for BORE_LR_CONSTANT.  __fmul_rn / __fadd_rn keep the
+// products and sums TF rounds separately from being contracted into one fma.
+__device__ __forceinline__ float lr_at(const LrSchedule &c, float lr, float step) {
+  switch (c.kind) {
+    case BORE_LR_EXPONENTIAL:
+    case BORE_LR_INVERSE_TIME: {
+      float p = step / c.decay_steps;
+      if (c.flag) p = floorf(p);  // staircase
+      return c.kind == BORE_LR_EXPONENTIAL ? __fmul_rn(c.initial, powf(c.rate, p))
+                                           : c.initial / __fadd_rn(1.f, __fmul_rn(c.rate, p));
+    }
+    case BORE_LR_POLYNOMIAL: {
+      float ds = c.decay_steps;
+      if (c.flag) ds = __fmul_rn(ds, step == 0.f ? 1.f : ceilf(step / c.decay_steps));  // cycle
+      else step = fminf(step, ds);
+      return __fadd_rn(__fmul_rn(c.initial - c.end, powf(1.f - step / ds, c.power)), c.end);
+    }
+    case BORE_LR_PIECEWISE: {  // values[i] for b_{i-1} < step <= b_i
+      int i = 0;
+      while (i < c.n && step > c.bound[i]) ++i;
+      return c.value[i];
+    }
+    default: return lr;
+  }
+}
 
 // The optimizer state of one model inside a fit kernel: Keras `iterations`, beta^t as fp64 running products
 // (one multiplication per step instead of two pow calls) and Nadam's momentum cache.
@@ -48,12 +77,14 @@ struct OptRun {
     OptStep s;
     s.om1 = 1.f - h.b1;
     s.om2 = 1.f - h.b2;
+    s.lr = h.lr;
     s.alpha = s.cg = s.cm = s.vd = 0.f;
     return s;
   }
 
-  // advance to the next step (Keras: t starts at 1): the scalars of s that depend on it
-  __device__ __forceinline__ void advance(const OptHyper &h, OptStep &s) {
+  // advance to the next step (Keras: t starts at 1): the scalars of s that depend on it.  Update t takes the
+  // schedule at step t - 1: Keras' _decayed_lr reads `iterations` before the increment.  Nadam has no schedule.
+  __device__ __forceinline__ void advance(const OptHyper &h, const LrSchedule &sch, OptStep &s) {
     t += 1;
     if (!OPT) {
       p1 *= (double)h.b1;
@@ -64,26 +95,27 @@ struct OptRun {
     }
     p1 *= f1;
     p2 *= (double)h.b2;
+    s.lr = h.kind == BORE_OPT_NADAM ? h.lr : lr_at(sch, h.lr, (float)(t - 1));
     switch (h.kind) {
-      case BORE_OPT_ADAM: s.alpha = h.lr * sqrtf(1.f - (float)p2) / (1.f - (float)p1); break;
-      case BORE_OPT_ADAMAX: s.alpha = h.lr / (1.f - (float)p1); break;
+      case BORE_OPT_ADAM: s.alpha = s.lr * sqrtf(1.f - (float)p2) / (1.f - (float)p1); break;
+      case BORE_OPT_ADAMAX: s.alpha = s.lr / (1.f - (float)p1); break;
       case BORE_OPT_NADAM: {
         const float mu = h.b1 * (1.f - 0.5f * (float)p1), mu_next = h.b1 * (1.f - 0.5f * (float)(p1 * f1));
         cache *= mu;  // fp32, as Keras keeps its m_cache variable
-        s.alpha = h.lr;
+        s.alpha = s.lr;
         s.cg = (1.f - mu) / (1.f - cache);
         s.cm = mu_next / (1.f - cache * mu_next);
         s.vd = 1.f / (1.f - (float)p2);
         break;
       }
-      default: s.alpha = h.lr; break;
+      default: s.alpha = s.lr; break;
     }
   }
 
   // advance to the next step and give all its scalars
-  __device__ __forceinline__ OptStep step(const OptHyper &h) {
+  __device__ __forceinline__ OptStep step(const OptHyper &h, const LrSchedule &sch) {
     OptStep s = consts(h);
-    advance(h, s);
+    advance(h, sch, s);
     return s;
   }
 
@@ -123,7 +155,7 @@ __device__ __forceinline__ float opt_update(const OptHyper &h, const OptStep &s,
       case BORE_OPT_RMSPROP:
         if (h.momentum > 0.f) {  // ResourceApplyRMSProp: eps inside the root
           s0 += (g * g - s0) * s.om1;
-          s1 = h.momentum * s1 + h.lr * g * rsqrtf(s0 + h.eps);
+          s1 = h.momentum * s1 + s.lr * g * rsqrtf(s0 + h.eps);
           return wv - s1;
         } else {
           s0 = h.b1 * s0 + s.om1 * (g * g);
@@ -132,16 +164,16 @@ __device__ __forceinline__ float opt_update(const OptHyper &h, const OptStep &s,
             s1 = h.b1 * s1 + s.om1 * g;
             den = s0 - s1 * s1;
           }
-          return wv - __fdividef(h.lr * g, sqrt_approx(den) + h.eps);
+          return wv - __fdividef(s.lr * g, sqrt_approx(den) + h.eps);
         }
       case BORE_OPT_ADAGRAD:  // ResourceApplyAdagradV2
         s0 += g * g;
-        return wv - __fdividef(h.lr * g, sqrt_approx(s0) + h.eps);
+        return wv - __fdividef(s.lr * g, sqrt_approx(s0) + h.eps);
       case BORE_OPT_ADADELTA: {  // ResourceApplyAdadelta
         s0 = s0 * h.b1 + (g * g) * s.om1;
         const float u = sqrt_approx(s1 + h.eps) * rsqrtf(s0 + h.eps) * g;
         s1 = s1 * h.b1 + (u * u) * s.om1;
-        return wv - u * h.lr;
+        return wv - u * s.lr;
       }
       case BORE_OPT_ADAMAX:  // ResourceApplyAdaMax
         s0 += (g - s0) * s.om1;
@@ -151,7 +183,7 @@ __device__ __forceinline__ float opt_update(const OptHyper &h, const OptStep &s,
         s0 = h.b1 * s0 + s.om1 * g;
         s1 = h.b2 * s1 + s.om2 * (g * g);
         const float mbar = s.cg * g + s.cm * s0;
-        return wv - __fdividef(h.lr * mbar, sqrt_approx(s1 * s.vd) + h.eps);
+        return wv - __fdividef(s.lr * mbar, sqrt_approx(s1 * s.vd) + h.eps);
       }
       default: break;
     }

@@ -215,9 +215,13 @@ class NativeMLP:
         self.opt_kind = 0
 
     def set_optimizer_kind(self, optimizer):
-        """Every model's optimizer: a ``bore_b200.layers`` optimizer.  A new kind resets every model's state."""
+        """Every model's optimizer and learning-rate schedule: a ``bore_b200.layers`` optimizer.  A new kind resets
+        every model's state; a schedule keeps it and continues from each model's ``iterations``."""
         kind, hp = optimizer.hyper()
         _lib.check(self.lib.bore_mlp_set_optimizer_kind(self.h, kind, _np_ptr(np.asarray(hp, np.float32))))
+        code, sp = optimizer.lr_schedule()
+        sp = np.asarray(sp, np.float32)
+        _lib.check(self.lib.bore_mlp_set_lr_schedule(self.h, code, _np_ptr(sp), sp.size))
         self.opt_kind = kind
 
     def get_optimizer_state(self, model=0):

@@ -6,6 +6,8 @@ the call sites README.rst:60-66 and bore/plugins/hpbandster/base.py:113-116,147-
 
 import numpy as np
 
+from . import schedules
+
 # Keras 2.5 element-wise activations whose derivative is a function of the layer output, the one value the
 # kernels keep (swish and gelu are not: DESIGN.md, "Activations")
 _ACTIVATIONS = ("linear", "relu", "elu", "sigmoid", "tanh", "selu", "softplus", "softsign", "hard_sigmoid",
@@ -131,8 +133,10 @@ _OPT_REFUSED = {
 
 
 class _Optimizer:
-    """Keras 2.5 ``optimizer_v2`` hyper-parameters.  ``decay``, ``clipnorm``, ``clipvalue``,
-    ``global_clipnorm`` and learning-rate schedules are not taken: the kernels apply the plain rule."""
+    """Keras 2.5 ``optimizer_v2`` hyper-parameters.  ``learning_rate`` is a number or an instance of one of the
+    four schedules of ``bore_b200.schedules``, which the kernels evaluate every step.  ``decay``, ``clipnorm``,
+    ``clipvalue``, ``global_clipnorm`` and other callables as the learning rate are not taken: the kernels apply
+    the plain rule."""
 
     kind = None
 
@@ -140,19 +144,35 @@ class _Optimizer:
         if kwargs:
             raise TypeError(f"{type(self).__name__}: unsupported arguments {sorted(kwargs)} (decay, gradient "
                             "clipping and the like are not in the training kernels)")
-        if callable(learning_rate):
-            raise NotImplementedError(f"{type(self).__name__}: learning-rate schedules are not in the training "
-                                      "kernels")
-        self.learning_rate = float(learning_rate)
+        if type(learning_rate) in schedules.SCHEDULES:
+            learning_rate.native()  # its arguments are refused here, not at the first fit
+            self.learning_rate = learning_rate
+        elif callable(learning_rate):
+            raise NotImplementedError(
+                f"{type(self).__name__}: the learning-rate schedules in the training kernels are "
+                f"bore_b200.schedules.{{{', '.join(c.__name__ for c in schedules.SCHEDULES)}}}; another callable "
+                f"(a function or a LearningRateSchedule subclass) runs Python, which the kernels cannot, got "
+                f"{learning_rate!r}")
+        else:
+            self.learning_rate = float(learning_rate)
         self.name = name
 
     def hyper(self):
-        """(BORE_OPT_* code, the BORE_OPT_NHP hyper-parameters of bore_mlp_set_optimizer_kind)."""
+        """(BORE_OPT_* code, the BORE_OPT_NHP hyper-parameters of bore_mlp_set_optimizer_kind).  Under a schedule
+        the learning-rate entry is 1, a stand-in the kernels do not read (lr_schedule gives the rate)."""
         g = lambda k: float(getattr(self, k, 0.0))  # noqa: E731
         rho = getattr(self, "rho", None)
-        return OPT_CODES[self.kind], [self.learning_rate, g("beta_1") if rho is None else float(rho), g("beta_2"),
+        lr = 1.0 if isinstance(self.learning_rate, schedules.LearningRateSchedule) else self.learning_rate
+        return OPT_CODES[self.kind], [lr, g("beta_1") if rho is None else float(rho), g("beta_2"),
                                       self.epsilon, g("momentum"), g("initial_accumulator_value"),
                                       float(bool(getattr(self, "centered", False)))]
+
+    def lr_schedule(self):
+        """(BORE_LR_* code, the parameters of bore_mlp_set_lr_schedule): BORE_LR_CONSTANT and none for a
+        constant learning rate."""
+        if isinstance(self.learning_rate, schedules.LearningRateSchedule):
+            return self.learning_rate.native()
+        return schedules.LR_CODES["constant"], []
 
 
 class Adam(_Optimizer):
@@ -217,11 +237,15 @@ class Adamax(_Optimizer):
 
 
 class Nadam(_Optimizer):
-    """``keras.optimizers.Nadam`` (its learning rate is not decayed; the momentum cache is per model)."""
+    """``keras.optimizers.Nadam`` (its learning rate is not decayed; the momentum cache is per model).  A
+    learning-rate schedule is a ValueError, as in Keras 2.5."""
 
     kind = "nadam"
 
     def __init__(self, learning_rate=1e-3, beta_1=0.9, beta_2=0.999, epsilon=1e-7, name="Nadam", **kwargs):
+        if isinstance(learning_rate, schedules.LearningRateSchedule):
+            raise ValueError("The Nadam optimizer does not support tf.keras.optimizers.LearningRateSchedules as "
+                             "the learning rate.")
         super().__init__(learning_rate, name, kwargs)
         self.beta_1, self.beta_2, self.epsilon = float(beta_1), float(beta_2), float(epsilon)
 

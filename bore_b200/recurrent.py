@@ -116,9 +116,13 @@ class NativeLSTM:
     opt_kind = 0  # BORE_OPT_* of the handle (Adam when created)
 
     def set_optimizer_kind(self, optimizer):
-        """The optimizer: a ``bore_b200.layers`` optimizer.  A new kind resets the state."""
+        """The optimizer and learning-rate schedule: a ``bore_b200.layers`` optimizer.  A new kind resets the
+        state; a schedule keeps it and continues from ``iterations``."""
         kind, hp = optimizer.hyper()
         _lib.check(self.lib.bore_lstm_set_optimizer_kind(self.h, kind, _np_ptr(np.asarray(hp, np.float32))))
+        code, sp = optimizer.lr_schedule()
+        sp = np.asarray(sp, np.float32)
+        _lib.check(self.lib.bore_lstm_set_lr_schedule(self.h, code, _np_ptr(sp), sp.size))
         self.opt_kind = kind
 
     def get_optimizer_state(self):

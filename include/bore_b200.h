@@ -42,6 +42,12 @@ enum { BORE_TRANSFORM_IDENTITY = 0, BORE_TRANSFORM_SIGMOID = 1, BORE_TRANSFORM_E
 enum { BORE_OPT_ADAM = 0, BORE_OPT_RMSPROP = 1, BORE_OPT_ADAGRAD = 2, BORE_OPT_ADADELTA = 3,
        BORE_OPT_ADAMAX = 4, BORE_OPT_NADAM = 5 };
 #define BORE_OPT_NHP 7
+/* learning-rate schedules of the training kernels (keras.optimizers.schedules: ExponentialDecay,
+ * InverseTimeDecay, PolynomialDecay, PiecewiseConstantDecay); bore_mlp_set_lr_schedule /
+ * bore_lstm_set_lr_schedule.  BORE_LR_CONSTANT: the optimizer's learning_rate at every step. */
+enum { BORE_LR_CONSTANT = 0, BORE_LR_EXPONENTIAL = 1, BORE_LR_INVERSE_TIME = 2, BORE_LR_POLYNOMIAL = 3,
+       BORE_LR_PIECEWISE = 4 };
+#define BORE_LR_MAX_BOUNDARIES 16
 /* per-start termination status, scipy.optimize.OptimizeResult.status for L-BFGS-B */
 enum { BORE_STATUS_CONVERGED = 0, BORE_STATUS_LIMIT = 1, BORE_STATUS_ABNORMAL = 2 };
 
@@ -104,6 +110,18 @@ int bore_mlp_set_optimizer(bore_mlp *h, float lr, float beta1, float beta2, floa
  * hyper-parameters.  bore_mlp_{get,set}_adam_state read and write slot 0 and slot 1 of any kind
  * (DESIGN.md, "Optimizers", has the slot of each kind).  Synchronous.                         */
 int bore_mlp_set_optimizer_kind(bore_mlp *h, int kind, const float *hp);
+/* The handle's learning-rate schedule: kind = BORE_LR_*, sp[n_sp] =
+ *   BORE_LR_CONSTANT      nothing (n_sp = 0, sp may be NULL): learning_rate of the optimizer, the state at create
+ *   BORE_LR_EXPONENTIAL   {initial_learning_rate, decay_steps, decay_rate, staircase (0 / 1)}
+ *   BORE_LR_INVERSE_TIME  {initial_learning_rate, decay_steps, decay_rate, staircase (0 / 1)}
+ *   BORE_LR_POLYNOMIAL    {initial_learning_rate, decay_steps, end_learning_rate, power, cycle (0 / 1)}
+ *   BORE_LR_PIECEWISE     {boundaries b_0 < .. < b_{n-1}, values v_0 .. v_n}: n_sp = 2 n + 1, 1 <= n <=
+ *                         BORE_LR_MAX_BOUNDARIES
+ * with the Keras 2.5 meaning; every value finite and decay_steps > 0, else refused.  Update number t (1-based)
+ * of a model uses the schedule at step t - 1, in fp32, as Keras' _decayed_lr evaluates it at `iterations`
+ * before the increment, so a later fit continues the schedule.  The optimizer state is kept.  Nadam takes
+ * no schedule (Keras 2.5 refuses one) and keeps its learning_rate.  Synchronous, host only.          */
+int bore_mlp_set_lr_schedule(bore_mlp *h, int kind, const float *sp, int n_sp);
 /* Nadam's momentum cache (Keras' m_cache, one fp32 scalar per model; 1 after a reset).  synchronous */
 int bore_mlp_get_nadam_cache(bore_mlp *h, int model, float *cache_host);
 int bore_mlp_set_nadam_cache(bore_mlp *h, int model, float cache);
@@ -435,6 +453,8 @@ int bore_lstm_set_adam_state(bore_lstm *h, const float *m_host, const float *v_h
 int bore_lstm_get_adam_state(bore_lstm *h, float *m_host, float *v_host, int64_t *iterations);
 /* the optimizer and Nadam's momentum cache, as bore_mlp_set_optimizer_kind / bore_mlp_{get,set}_nadam_cache */
 int bore_lstm_set_optimizer_kind(bore_lstm *h, int kind, const float *hp);
+/* the learning-rate schedule, as bore_mlp_set_lr_schedule */
+int bore_lstm_set_lr_schedule(bore_lstm *h, int kind, const float *sp, int n_sp);
 int bore_lstm_get_nadam_cache(bore_lstm *h, float *cache_host);
 int bore_lstm_set_nadam_cache(bore_lstm *h, float cache);
 /* l2 and l1 factors per weight array in Keras order (kernel, recurrent kernel, bias of every cell, then
