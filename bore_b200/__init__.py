@@ -5,7 +5,7 @@ Same Python surface as the reference for that path; hand-written CUDA kernels be
 """
 __version__ = "0.1.0"
 
-from .layers import (Dense, BinaryCrossentropy, Adam, RMSprop, Adagrad, Adadelta, Adamax, Nadam, L1, L2, L1L2,  # noqa: F401
+from .layers import (Dense, Dropout, BinaryCrossentropy, Adam, RMSprop, Adagrad, Adadelta, Adamax, Nadam, L1, L2, L1L2,  # noqa: F401
                      l1, l2, l1_l2)
 from .ops import identity, sigmoid, exp, TRANSFORMS  # noqa: F401
 from .base import convert, maybe_distort, maybe_distort_batch, truncated_normal  # noqa: F401

@@ -51,6 +51,7 @@ SIGNATURES = {
                                       vp, vp, vp]),
     "bore_mlp_set_regularizers": (C.c_int, [vp, vp, vp]),
     "bore_mlp_set_l1_regularizers": (C.c_int, [vp, vp, vp]),
+    "bore_mlp_set_dropout": (C.c_int, [vp, C.c_int, vp, vp]),
     "bore_lbfgsb_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "bore_lbfgsb_minimize_workspace_bytes": (C.c_size_t, [vp, C.c_int, C.c_int]),
     "bore_lbfgsb_set_mode": (C.c_int, [C.c_int]),

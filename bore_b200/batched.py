@@ -15,7 +15,7 @@ from sklearn.utils import check_random_state
 
 from . import ops
 from .engine import NativeMLP, lbfgsb_message
-from .layers import Dense, BinaryCrossentropy, optimizer_spec, regularizer_factors
+from .layers import BinaryCrossentropy, optimizer_spec, regularizer_factors, split_dropout, dropout_rates_seeds
 from .models import check_class_weight, sample_weights
 from .optimizers.utils import from_bounds
 from .ragged import ragged_inputs, ragged_rows
@@ -115,12 +115,14 @@ class BatchedResults:
 class BatchedMaximizableSequential:
 
     def __init__(self, layers, n_problems, transform=ops.identity, seed=None, device=None):
-        self.layers = list(layers)
-        assert self.layers and all(isinstance(l, Dense) for l in self.layers)
-        assert self.layers[0].input_dim is not None, "the first Dense layer needs input_dim"
+        self.layers = list(layers)  # Dense layers, each hidden one optionally followed by a Dropout
+        assert self.layers
+        dense, after = split_dropout(self.layers)
+        self._dense = dense
+        assert dense[0].input_dim is not None, "the first Dense layer needs input_dim"
         self.n_problems = int(n_problems)
-        dims = [self.layers[0].input_dim] + [l.units for l in self.layers]
-        acts = [l.activation for l in self.layers]
+        dims = [dense[0].input_dim] + [l.units for l in dense]
+        acts = [l.activation for l in dense]
         self.dims, self.acts = dims, acts
         e = transform(-ops.Expr(self, (1,), (1,)))
         if not isinstance(e, ops.Expr) or e.sign != -1:
@@ -136,6 +138,9 @@ class BatchedMaximizableSequential:
                 ws += [self._rs.uniform(-lim, lim, size=(fi, fo)).astype(np.float32),
                        np.zeros(fo, np.float32)]
             self._net.set_weights(ws, model=p)
+        drop = dropout_rates_seeds(after, self._rs)  # (seeds drawn after the initial weights; every problem has
+        if drop is not None:                          # its own masks through its model index)
+            self._net.set_dropout(*drop)
         self._last_stats = {}
 
     # ------------------------------------------------------------------ keras-shaped surface
@@ -150,7 +155,7 @@ class BatchedMaximizableSequential:
                                       "BinaryCrossentropy(from_logits=True)")
         self._net.set_optimizer_kind(optimizer)
         self._net.set_regularizers(*regularizer_factors(
-            r for lyr in self.layers for r in (lyr.kernel_regularizer, lyr.bias_regularizer)))
+            r for lyr in self._dense for r in (lyr.kernel_regularizer, lyr.bias_regularizer)))
         self._compiled = True
 
     def set_weights(self, weights_per_problem):

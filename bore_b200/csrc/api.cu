@@ -334,6 +334,24 @@ int bore_mlp_set_l1_regularizers(bore_mlp *h, const float *l1_kernel_host, const
   return 0;
 }
 
+int bore_mlp_set_dropout(bore_mlp *h, int n, const float *rates_host, const uint32_t *seeds_host) {
+  BORE_CHECK(n >= 0 && n < BORE_MAX_LAYERS, "bore_mlp_set_dropout: %d hidden layers, outside [0, %d]", n,
+             BORE_MAX_LAYERS - 1);
+  BORE_CHECK(n == 0 || (rates_host != nullptr && seeds_host != nullptr), "bore_mlp_set_dropout: NULL argument");
+  for (int l = 0; l < n; ++l)
+    BORE_CHECK(isfinite(rates_host[l]) && rates_host[l] >= 0.f && rates_host[l] < 1.f,
+               "bore_mlp_set_dropout: rate of hidden layer %d is %g: it must be finite and in [0, 1)", l,
+               (double)rates_host[l]);
+  BORE_CHECK(h != nullptr, "NULL handle");
+  BORE_CHECK(n == h->desc.n_layers - 1, "bore_mlp_set_dropout: the net has %d hidden layers, got %d",
+             h->desc.n_layers - 1, n);
+  for (int l = 0; l < BORE_MAX_LAYERS; ++l) {  // the weights and the optimizer state are kept
+    h->drop_rate[l] = l < n ? rates_host[l] : 0.f;
+    h->drop_seed[l] = l < n ? seeds_host[l] : 0u;
+  }
+  return 0;
+}
+
 int bore_mlp_params_dev(bore_mlp *h, float **params_dev) {
   BORE_CHECK(h != nullptr && params_dev != nullptr, "NULL argument");
   *params_dev = h->params;

@@ -103,6 +103,8 @@ struct bore_mlp {
   LrSchedule sched;
   float l2k[BORE_MAX_LAYERS], l2b[BORE_MAX_LAYERS];  // l2 regularisers per layer
   float l1k[BORE_MAX_LAYERS], l1b[BORE_MAX_LAYERS];  // l1 regularisers per layer
+  float drop_rate[BORE_MAX_LAYERS];                  // Dropout after hidden layer l (0: none)
+  uint32_t drop_seed[BORE_MAX_LAYERS];
   int fit_mode;  // 0 auto, 1 one CTA per model (FFMA), 2 one cluster per model, samples split (FFMA), 3 tensor
                  // pipe, 4 one cluster per model, units split (FFMA2)  (bore_mlp_set_fit_mode)
   void *tab_pinned;      // pinned staging buffer of the ragged fit's problem table (FitTable), tab_cap bytes
@@ -206,7 +208,8 @@ int opt_from_array(int kind, const float *hp, OptHyper &out, const char *who);
 // bore_*_set_lr_schedule's check of (kind, sp, n_sp); 0, or -1 with the error text set
 int lr_schedule_from_array(int kind, const float *sp, int n_sp, LrSchedule &out, const char *who);
 // The build of a fit kernel (template flag OPT, opt.cuh): every optimizer but Adam, and any schedule, run the OPT
-// build.  fit_kernel and lstm_fit_kernel also run it for Adam with an l1 factor (fit_common.cuh, FitJob).
+// build.  fit_kernel and lstm_fit_kernel also run it for Adam with an l1 factor (fit_common.cuh, FitJob, which
+// also has the dropout build of the MLP fit kernels).
 inline bool opt_build(const OptHyper &o, const LrSchedule &s) {
   return o.kind != BORE_OPT_ADAM || s.kind != BORE_LR_CONSTANT;
 }

@@ -184,7 +184,9 @@ __device__ __forceinline__ void narrow_tile(const float *__restrict__ Hin, const
 // expressions of before: deriving its problem through fit_problem() cost cfg 4 0.4 % (132.0 -> 132.5 ms)
 // EXT: the activation codes above BORE_ACT_TANH (act.cuh).  OPT: the optimizers other than Adam (opt.cuh) and the l1
 // regulariser terms, which cost the default build 1.8 % of the cfg-4 fit when they were in it (DESIGN.md, "Regularizers").
-template <bool WEIGHTED, bool RAGGED, bool EXT, bool OPT>
+// DROP (with OPT only): dropout after the hidden layers (dropout.cuh), kept out of the OPT build, whose registers it
+// raised into spills (DESIGN.md, "Dropout").
+template <bool WEIGHTED, bool RAGGED, bool EXT, bool OPT, bool DROP>
 __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
   extern __shared__ __align__(16) float sm[];
   const MlpDesc &d = a.d;
@@ -238,6 +240,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
       const int nb = min(a.batch, N - s0);
       const int BP = r4(nb), nchunk = BP >> 2;
       const float inv_nchunk = 1.f / (float)nchunk;
+      const long long tm = run.t;  // the dropout masks' step: `iterations` before this step's increment
       // ---- gather the minibatch (transposed) ----
       for (int p = tid; p < BP; p += NT) {
         const int row = p < nb ? perm[(size_t)ep * N + s0 + p] : -1;
@@ -262,6 +265,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
         const float *bs = sm + P.b[l];
         float *H = sm + P.h[l + 1];
         const int act = (l == L - 1) ? BORE_ACT_LINEAR : d.act[l];  // loss works on the logit
+        const bool drop = DROP && a.drop.rate[l] > 0.f;  // (0 for the output layer)
         if (out == 1) {
           // u[p] = b + sum_k h[k][p] w[k]: one 4-sample chunk per group of kf adjacent lanes,
           // k interleaved over the group, partial sums combined by shuffle
@@ -287,8 +291,10 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
             }
             if (valid && s == 0) {
               const float b = bs[0];
-              *reinterpret_cast<float4 *>(H + 4 * c) = make_float4(act_fwd<EXT>(act, acc.x + b), act_fwd<EXT>(act, acc.y + b),
-                                                                   act_fwd<EXT>(act, acc.z + b), act_fwd<EXT>(act, acc.w + b));
+              float4 o = make_float4(act_fwd<EXT>(act, acc.x + b), act_fwd<EXT>(act, acc.y + b),
+                                     act_fwd<EXT>(act, acc.z + b), act_fwd<EXT>(act, acc.w + b));
+              if (drop) o = drop_fwd_unit4(a.drop, l, tm, 4 * c, 0, model, o);
+              *reinterpret_cast<float4 *>(H + 4 * c) = o;
             }
           }
         } else {
@@ -297,6 +303,10 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
             const int tj = fdiv(tt, inv_nchunk), tp = tt - tj * nchunk;
             float acc[4][4] = {};
             tile_fma(A + tp * 4, BS, W + tj * 4, JP, in, acc);
+            uint32_t kb[4];  // keep bits of units tj*4 .. +3, per sample
+            if (drop)
+#pragma unroll
+              for (int i = 0; i < 4; ++i) kb[i] = drop_keep4(a.drop, l, tm, tp * 4 + i, tj, model);
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
               const int j = tj * 4 + u;
@@ -307,6 +317,13 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
                 o.y = act_fwd<EXT>(act, acc[1][u] + b);
                 o.z = act_fwd<EXT>(act, acc[2][u] + b);
                 o.w = act_fwd<EXT>(act, acc[3][u] + b);
+                if (drop) {
+                  const float sc = a.drop.scale[l];
+                  o.x = drop_fwd(o.x, (kb[0] >> u) & 1u, sc);
+                  o.y = drop_fwd(o.y, (kb[1] >> u) & 1u, sc);
+                  o.z = drop_fwd(o.z, (kb[2] >> u) & 1u, sc);
+                  o.w = drop_fwd(o.w, (kb[3] >> u) & 1u, sc);
+                }
                 *reinterpret_cast<float4 *>(H + j * BS + tp * 4) = o;
               }
             }
@@ -353,6 +370,7 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
           const float *WT = sm + P.wt[l];
           float *DN = sm + P.dl[cur ^ 1];
           const int actp = d.act[l - 1];
+          const bool drop = DROP && a.drop.rate[l - 1] > 0.f;  // Hin holds h~ of hidden layer l - 1
           if (out == 1) {
             for (int e = tid; e < in * nchunk; e += NT) {
               const int k = fdiv(e, inv_nchunk), c = e - k * nchunk;
@@ -360,8 +378,10 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
               const float4 hv = *reinterpret_cast<const float4 *>(Hin + k * BS + 4 * c);
               const float w = WT[k];
               *reinterpret_cast<float4 *>(DN + k * BS + 4 * c) =
-                  make_float4(dv.x * w * act_bwd<EXT>(actp, hv.x), dv.y * w * act_bwd<EXT>(actp, hv.y),
-                              dv.z * w * act_bwd<EXT>(actp, hv.z), dv.w * w * act_bwd<EXT>(actp, hv.w));
+                  drop ? drop_bwd_unit4<EXT>(a.drop, l - 1, tm, 4 * c, k, model, actp,
+                                             make_float4(dv.x * w, dv.y * w, dv.z * w, dv.w * w), hv)
+                       : make_float4(dv.x * w * act_bwd<EXT>(actp, hv.x), dv.y * w * act_bwd<EXT>(actp, hv.y),
+                                     dv.z * w * act_bwd<EXT>(actp, hv.z), dv.w * w * act_bwd<EXT>(actp, hv.w));
             }
           } else {
             const int ntile = nchunk * (r4(in) / 4);
@@ -369,16 +389,28 @@ __global__ void __launch_bounds__(FIT_THREADS, 2) fit_kernel(const FitArgs a) {
               const int tk = fdiv(tt, inv_nchunk), tp = tt - tk * nchunk;
               float acc[4][4] = {};
               tile_fma(DL + tp * 4, BS, WT + tk * 4, KP, out, acc);
+              uint32_t kb[4];  // keep bits of units tk*4 .. +3, per sample
+              if (drop)
+#pragma unroll
+                for (int i = 0; i < 4; ++i) kb[i] = drop_keep4(a.drop, l - 1, tm, tp * 4 + i, tk, model);
 #pragma unroll
               for (int u = 0; u < 4; ++u) {
                 const int k = tk * 4 + u;
                 if (k < in) {
                   const float4 hv = *reinterpret_cast<const float4 *>(Hin + k * BS + tp * 4);
                   float4 o;
-                  o.x = acc[0][u] * act_bwd<EXT>(actp, hv.x);
-                  o.y = acc[1][u] * act_bwd<EXT>(actp, hv.y);
-                  o.z = acc[2][u] * act_bwd<EXT>(actp, hv.z);
-                  o.w = acc[3][u] * act_bwd<EXT>(actp, hv.w);
+                  if (drop) {
+                    const float sc = a.drop.scale[l - 1], r = a.drop.rate[l - 1];
+                    o.x = drop_bwd<EXT>(actp, acc[0][u], hv.x, (kb[0] >> u) & 1u, sc, r);
+                    o.y = drop_bwd<EXT>(actp, acc[1][u], hv.y, (kb[1] >> u) & 1u, sc, r);
+                    o.z = drop_bwd<EXT>(actp, acc[2][u], hv.z, (kb[2] >> u) & 1u, sc, r);
+                    o.w = drop_bwd<EXT>(actp, acc[3][u], hv.w, (kb[3] >> u) & 1u, sc, r);
+                  } else {
+                    o.x = acc[0][u] * act_bwd<EXT>(actp, hv.x);
+                    o.y = acc[1][u] * act_bwd<EXT>(actp, hv.y);
+                    o.z = acc[2][u] * act_bwd<EXT>(actp, hv.z);
+                    o.w = acc[3][u] * act_bwd<EXT>(actp, hv.w);
+                  }
                   *reinterpret_cast<float4 *>(DN + k * BS + tp * 4) = o;
                 }
               }
@@ -862,7 +894,8 @@ __device__ __forceinline__ float4 f_act_bwd4(int a, float4 acc, float4 h) {
                      acc.w * act_bwd<EXT>(a, h.w));
 }
 
-template <bool WEIGHTED, bool EXT, bool OPT>
+// OPT, DROP: the builds of fit_kernel
+template <bool WEIGHTED, bool EXT, bool OPT, bool DROP>
 __global__ void __cluster_dims__(FIT_CLUSTER, 1, 1) __launch_bounds__(FIT_CTHREADS)
 fit_cluster_kernel(const FitCArgs a) {
   extern __shared__ __align__(16) float sm[];
@@ -979,6 +1012,8 @@ fit_cluster_kernel(const FitCArgs a) {
       const int nb = min(a.batch, N - s0);
       const int spc = (nb + FIT_CLUSTER - 1) / FIT_CLUSTER;  // samples per CTA
       const int mine = max(0, min(spc, nb - rank * spc));     // this CTA's samples
+      const long long tm = run.t;  // the dropout masks' step: `iterations` before this step's increment
+      const int pos0 = rank * spc;  // minibatch position of this CTA's sample 0
 
       // ---- forward (the minibatch slice is already in place) ----
       for (int l = 0; l < L; ++l) {
@@ -986,10 +1021,12 @@ fit_cluster_kernel(const FitCArgs a) {
         const float *bs = sm + P.b[l];
         float *H = sm + P.h[l + 1];
         const int act = (l == L - 1) ? BORE_ACT_LINEAR : d.act[l];  // loss works on the logit
+        const bool drop = DROP && a.drop.rate[l] > 0.f;
         dense_pass(sm + P.h[l], sm + P.w[l], in, ldo(out), out, SP, [&](int j, int q, float4 acc) {
           const float b = bs[j];
-          *reinterpret_cast<float4 *>(H + j * SP + 4 * q) =
-              f_act4<EXT>(act, make_float4(acc.x + b, acc.y + b, acc.z + b, acc.w + b));
+          float4 o = f_act4<EXT>(act, make_float4(acc.x + b, acc.y + b, acc.z + b, acc.w + b));
+          if (drop) o = drop_fwd_unit4(a.drop, l, tm, pos0 + 4 * q, j, model, o);
+          *reinterpret_cast<float4 *>(H + j * SP + 4 * q) = o;
         });
         __syncthreads();
       }
@@ -1027,9 +1064,12 @@ fit_cluster_kernel(const FitCArgs a) {
         if (l > 0) {
           float *DN = sm + P.dl[cur ^ 1];
           const int actp = d.act[l - 1];
+          const bool drop = DROP && a.drop.rate[l - 1] > 0.f;  // Hin holds h~ of hidden layer l - 1
           dense_pass(DL, sm + P.wt[l], out, ldo(in), in, SP, [&](int k, int q, float4 acc) {
             const float4 hv = *reinterpret_cast<const float4 *>(Hin + k * SP + 4 * q);
-            *reinterpret_cast<float4 *>(DN + k * SP + 4 * q) = f_act_bwd4<EXT>(actp, acc, hv);
+            *reinterpret_cast<float4 *>(DN + k * SP + 4 * q) =
+                drop ? drop_bwd_unit4<EXT>(a.drop, l - 1, tm, pos0 + 4 * q, k, model, actp, acc, hv)
+                     : f_act_bwd4<EXT>(actp, acc, hv);
           });
         }
         {
@@ -1276,8 +1316,8 @@ int fit_check_envelope(const MlpDesc &d) {
   return 0;
 }
 
-// The handle's part of a fit job: the net, its training state, optimizer and learning-rate schedule, and its l1 / l2
-// factors with the gates any_reg and any_l1.  The caller fills in the launch's data.
+// The handle's part of a fit job: the net, its training state, optimizer and learning-rate schedule, its l1 / l2
+// factors with the gates any_reg and any_l1, and its dropout.  The caller fills in the launch's data.
 static FitJob fit_job(const bore_mlp *h) {
   FitJob j{};
   j.d = h->desc;
@@ -1286,6 +1326,12 @@ static FitJob fit_job(const bore_mlp *h) {
   for (int l = 0; l < h->desc.n_layers; ++l) {
     j.l2k[l] = h->l2k[l]; j.l2b[l] = h->l2b[l]; j.l1k[l] = h->l1k[l]; j.l1b[l] = h->l1b[l];
     if (j.l1k[l] != 0.f || j.l1b[l] != 0.f) j.any_l1 = 1;
+    if (h->drop_rate[l] > 0.f) {
+      j.drop.rate[l] = h->drop_rate[l];
+      j.drop.scale[l] = (float)(1.0 / (1.0 - (double)h->drop_rate[l]));
+      j.drop.seed[l] = h->drop_seed[l];
+      j.drop.any = 1;
+    }
     if (j.any_l1 || j.l2k[l] != 0.f || j.l2b[l] != 0.f) j.any_reg = 1;
   }
   return j;
@@ -1301,8 +1347,9 @@ static int launch_fit_cluster(const bore_mlp *h, const FitJob &job, int count, F
     return 0;
   }
   BORE_CHECK_RC(tab.get(&a.probs));
-  const auto kern = with_flags([](auto w, auto e, auto o) { return fit_cluster_kernel<w, e, o>; }, job.fw.on,
-                               acts_ext(job.d.act, job.d.n_layers), opt_build(job.opt, job.sched));
+  const auto kern = with_build(opt_build(job.opt, job.sched), job.drop.any,
+                               [](auto w, auto e, auto o, auto dr) { return fit_cluster_kernel<w, e, o, dr>; },
+                               job.fw.on, acts_ext(job.d.act, job.d.n_layers));
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count * FIT_CLUSTER, FIT_CTHREADS, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());
@@ -1337,9 +1384,9 @@ static int launch_fit_onecta(const bore_mlp *h, const FitJob &job, int count, Fi
   }
   BORE_CHECK(smem <= FIT_MAX_SMEM, "bore_mlp_fit: model + batch of %d need %zu B of shared memory", B, smem);
   BORE_CHECK_RC(tab.get(&a.probs));
-  const auto kern = with_flags([](auto w, auto r, auto e, auto o) { return fit_kernel<w, r, e, o>; }, job.fw.on,
-                               a.probs != nullptr, acts_ext(job.d.act, job.d.n_layers),
-                               opt_build(job.opt, job.sched) || job.any_l1);
+  const auto kern = with_build(opt_build(job.opt, job.sched) || job.any_l1, job.drop.any,
+                               [](auto w, auto r, auto e, auto o, auto dr) { return fit_kernel<w, r, e, o, dr>; },
+                               job.fw.on, a.probs != nullptr, acts_ext(job.d.act, job.d.n_layers));
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count, threads, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());

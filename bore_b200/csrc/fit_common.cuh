@@ -4,13 +4,15 @@
 #include "common.cuh"
 #include "act.cuh"
 #include "opt.cuh"
+#include "dropout.cuh"
 
 // What every MLP fit kernel reads besides its shared-memory plan: each kernel's arguments are a FitJob plus its
 // plan (FitArgs, FitCArgs, FuArgs, FitMArgs).  The l1 / l2 factors are zero past the net's last layer.
-// The build of a kernel (template flag OPT, opt_build in common.cuh): every optimizer but Adam, and every
-// learning-rate schedule, run the OPT build.  fit_kernel (and lstm_fit_kernel) also run it for Adam when any_l1 is
+// The build of a kernel (template flags OPT and DROP, with_build below): every optimizer but Adam and every
+// learning-rate schedule run the OPT build.  fit_kernel (and lstm_fit_kernel) also run it for Adam when any_l1 is
 // set, since their l1 terms are in the OPT build only; the cluster, unit-split and tensor-pipe kernels read l1 in
-// every build.
+// every build.  Any dropout runs the build OPT = DROP = true, whatever the optimizer: the dropout code is in that
+// build only, so the OPT build without dropout keeps its registers and instructions.
 struct FitJob {
   MlpDesc d;
   float *params, *adam_m, *adam_v;
@@ -29,8 +31,17 @@ struct FitJob {
   OptHyper opt;
   FitWeights fw;
   float *opt_cache;  // [n_models] Nadam's momentum cache
-  LrSchedule sched;  // last: the members above keep their offsets
+  LrSchedule sched;
+  Dropout drop;  // last: the members above keep their offsets
 };
+
+// The kernel of a fit launch: f(flags..., OPT, DROP) over the run-time flags bs, in one of the three builds that are
+// instantiated -- (OPT = opt, DROP = false) without dropout, (true, true) with it (see FitJob).
+template <class F, class... Bs>
+auto with_build(bool opt, bool drop, F f, Bs... bs) {
+  if (drop) return with_flags([&](auto... c) { return f(c..., std::true_type{}, std::true_type{}); }, bs...);
+  return with_flags([&](auto... c) { return f(c..., std::false_type{}); }, bs..., opt);
+}
 
 // The launchers of the fit kernels, tried in this order by fit_run (fit.cu): 1 launched, 0 shape not taken (the
 // next one is tried), < 0 error.  `tab`: the launch's problems (a ragged fit; job.N is then the largest N_p) or

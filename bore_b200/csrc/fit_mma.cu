@@ -220,10 +220,17 @@ __device__ __forceinline__ void cp_async4(float *dst_smem, const float *src) {
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-// forward unit: NG tiles of H_l = act(A W_l + b_l), rows mb*16.., columns n0..
+// The dropout of one unit call: hidden layer dl of model m at step t (dl < 0: none)
+struct DropAt {
+  const Dropout &dp;
+  int dl, m;
+  long long t;
+};
+
+// forward unit: NG tiles of H_l = act(A W_l + b_l), rows mb*16.., columns n0..; dropout after it (dr)
 template <int NG, bool EXT>
 __device__ __forceinline__ void fwd_unit(const float *A, int a_rs, const float2 *Wp, int ldw, const float *bs, float *H,
-                                         int lda, int mb, int n0, int K, int act, int lane) {
+                                         int lda, int mb, int n0, int K, int act, int lane, const DropAt &dr) {
   const int g = lane >> 2, t = lane & 3;
   float acc[NG][4];
 #pragma unroll
@@ -234,15 +241,26 @@ __device__ __forceinline__ void fwd_unit(const float *A, int a_rs, const float2 
     const int n = n0 + q * 8 + 2 * t;
     const float2 b = *reinterpret_cast<const float2 *>(bs + n);
     float *h0 = H + (mb * 16 + g) * lda + n;
-    *reinterpret_cast<float2 *>(h0) = make_float2(act_fwd<EXT>(act, acc[q][0] + b.x), act_fwd<EXT>(act, acc[q][1] + b.y));
-    *reinterpret_cast<float2 *>(h0 + 8 * lda) = make_float2(act_fwd<EXT>(act, acc[q][2] + b.x), act_fwd<EXT>(act, acc[q][3] + b.y));
+    float2 o0 = make_float2(act_fwd<EXT>(act, acc[q][0] + b.x), act_fwd<EXT>(act, acc[q][1] + b.y));
+    float2 o1 = make_float2(act_fwd<EXT>(act, acc[q][2] + b.x), act_fwd<EXT>(act, acc[q][3] + b.y));
+    if (dr.dl >= 0) {  // units n, n + 1 (n even) of rows g and g + 8: one Philox call per row
+      const uint32_t k0 = drop_keep4(dr.dp, dr.dl, dr.t, mb * 16 + g, n >> 2, dr.m) >> (n & 3);
+      const uint32_t k1 = drop_keep4(dr.dp, dr.dl, dr.t, mb * 16 + g + 8, n >> 2, dr.m) >> (n & 3);
+      const float sc = dr.dp.scale[dr.dl];
+      o0 = make_float2(drop_fwd(o0.x, k0 & 1u, sc), drop_fwd(o0.y, (k0 >> 1) & 1u, sc));
+      o1 = make_float2(drop_fwd(o1.x, k1 & 1u, sc), drop_fwd(o1.y, (k1 >> 1) & 1u, sc));
+    }
+    *reinterpret_cast<float2 *>(h0) = o0;
+    *reinterpret_cast<float2 *>(h0 + 8 * lda) = o1;
   }
 }
 
-// reverse unit: NG tiles of D_{l-1} = (D_l W_l') . act'(H_{l-1}) and their column sums (bias gradient partials)
+// reverse unit: NG tiles of D_{l-1} = (D_l W_l') . act'(H_{l-1}) and their column sums (bias gradient partials);
+// H_{l-1} holds h~ when dr has the dropout of layer l - 1
 template <int NG, bool EXT>
 __device__ __forceinline__ void bwd_unit(const float *Dl, int lda, const float2 *Wp, int ldw, const float *Hin, int h_rs,
-                                         float *DN, float *cs, int mb, bool live, int n0, int K, int actp, int lane) {
+                                         float *DN, float *cs, int mb, bool live, int n0, int K, int actp, int lane,
+                                         const DropAt &dr) {
   const int g = lane >> 2, t = lane & 3;
   float acc[NG][4];
 #pragma unroll
@@ -256,8 +274,18 @@ __device__ __forceinline__ void bwd_unit(const float *Dl, int lda, const float2 
       const float *h0 = Hin + (mb * 16 + g) * h_rs + n;
       const float2 hv0 = *reinterpret_cast<const float2 *>(h0);
       const float2 hv1 = *reinterpret_cast<const float2 *>(h0 + 8 * h_rs);
-      d0 = make_float2(acc[q][0] * act_bwd<EXT>(actp, hv0.x), acc[q][1] * act_bwd<EXT>(actp, hv0.y));
-      d1 = make_float2(acc[q][2] * act_bwd<EXT>(actp, hv1.x), acc[q][3] * act_bwd<EXT>(actp, hv1.y));
+      if (dr.dl >= 0) {
+        const uint32_t k0 = drop_keep4(dr.dp, dr.dl, dr.t, mb * 16 + g, n >> 2, dr.m) >> (n & 3);
+        const uint32_t k1 = drop_keep4(dr.dp, dr.dl, dr.t, mb * 16 + g + 8, n >> 2, dr.m) >> (n & 3);
+        const float sc = dr.dp.scale[dr.dl], r = dr.dp.rate[dr.dl];
+        d0 = make_float2(drop_bwd<EXT>(actp, acc[q][0], hv0.x, k0 & 1u, sc, r),
+                         drop_bwd<EXT>(actp, acc[q][1], hv0.y, (k0 >> 1) & 1u, sc, r));
+        d1 = make_float2(drop_bwd<EXT>(actp, acc[q][2], hv1.x, k1 & 1u, sc, r),
+                         drop_bwd<EXT>(actp, acc[q][3], hv1.y, (k1 >> 1) & 1u, sc, r));
+      } else {
+        d0 = make_float2(acc[q][0] * act_bwd<EXT>(actp, hv0.x), acc[q][1] * act_bwd<EXT>(actp, hv0.y));
+        d1 = make_float2(acc[q][2] * act_bwd<EXT>(actp, hv1.x), acc[q][3] * act_bwd<EXT>(actp, hv1.y));
+      }
       float *o0 = DN + (mb * 16 + g) * lda + n;
       *reinterpret_cast<float2 *>(o0) = d0;
       *reinterpret_cast<float2 *>(o0 + 8 * lda) = d1;
@@ -273,7 +301,8 @@ __device__ __forceinline__ void bwd_unit(const float *Dl, int lda, const float2 
 }
 
 // ------------------------------------------------------------------------------------ the kernel
-template <int NW, int TPW, bool EXT, bool OPT>
+// OPT: the optimizers other than Adam (opt.cuh); DROP (with OPT only): dropout after the hidden layers (dropout.cuh)
+template <int NW, int TPW, bool EXT, bool OPT, bool DROP>
 __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit_mma_kernel(const FitMArgs a) {
   extern __shared__ __align__(16) float sm[];
   const MlpDesc &d = a.d;
@@ -401,6 +430,7 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
     const int nmb = (nb + 15) >> 4, BP = nmb << 4;
     const float inv_nb = 1.f / (float)nb;
     reg = 0.f;
+    const long long tm = run.t;  // the dropout masks' step: `iterations` before this step's increment
     run.advance(a.opt, a.sched, os);
 
     const int row_next = row_of(gs + 1);  // (consumed after the forward pass)
@@ -416,11 +446,12 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
       float *H = sm + P.h[l];
       const int ldw = P.ldw[l], ntn = P.np[l] >> 3, act = d.act[l], K = P.kp[l], ng = P.ngf[l];
       const int groups = ntn / ng;
+      const DropAt dr{a.drop, DROP && a.drop.rate[l] > 0.f ? l : -1, model, tm};
       for (int u = warp; u < nmb * groups; u += NW) {
         const int mb = u / groups, n0 = (u - mb * groups) * ng * 8;
-        if (ng == 4) fwd_unit<4, EXT>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane);
-        else if (ng == 2) fwd_unit<2, EXT>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane);
-        else fwd_unit<1, EXT>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane);
+        if (ng == 4) fwd_unit<4, EXT>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane, dr);
+        else if (ng == 2) fwd_unit<2, EXT>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane, dr);
+        else fwd_unit<1, EXT>(A, a_rs, Wp, ldw, bs, H, lda, mb, n0, K, act, lane, dr);
       }
       __syncthreads();
     }
@@ -468,13 +499,16 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
       const int npv = P.np[LH - 1], actp = d.act[LH - 1];
       // thread = one column j and every RG-th row (RG row groups)
       const int RG = NT / npv > 0 ? min(NT / npv, 4) : 1;
+      const bool drop = DROP && a.drop.rate[LH - 1] > 0.f;  // H holds h~ of the top hidden layer
       if (tid < npv * RG) {
         const int j = tid % npv, rg = tid / npv;
         const float wj = w[j];
         float csum = 0.f;
         for (int r = rg; r < BP; r += RG) {
           const float hv = H[r * lda + j];
-          const float dv = du[r] * wj * act_bwd<EXT>(actp, hv);
+          const float dv = drop ? drop_bwd<EXT>(actp, du[r] * wj, hv, drop_keep(a.drop, LH - 1, tm, r, j, model),
+                                                a.drop.scale[LH - 1], a.drop.rate[LH - 1])
+                                : du[r] * wj * act_bwd<EXT>(actp, hv);
           DN[r * lda + j] = dv;
           csum += dv;
         }
@@ -565,12 +599,13 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
         const int nti = P.np[l - 1] >> 3, actp = d.act[l - 1], K = P.np[l], ng = P.ngb[l];
         float *cs = sm + P.cs[csi ^ 1];
         const int groups = nti / ng;
+        const DropAt dr{a.drop, DROP && a.drop.rate[l - 1] > 0.f ? l - 1 : -1, model, tm};
         for (int u = warp; u < 4 * groups; u += NW) {  // all four row blocks: dead ones publish zero column sums
           const int mb = u / groups, n0 = (u - mb * groups) * ng * 8;
           const bool live = mb < nmb;
-          if (ng == 4) bwd_unit<4, EXT>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane);
-          else if (ng == 2) bwd_unit<2, EXT>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane);
-          else bwd_unit<1, EXT>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane);
+          if (ng == 4) bwd_unit<4, EXT>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane, dr);
+          else if (ng == 2) bwd_unit<2, EXT>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane, dr);
+          else bwd_unit<1, EXT>(dbuf, lda, Wp, ldw, Hin, h_rs, DN, cs, mb, live, n0, K, actp, lane, dr);
         }
       }
       // (4) dW_l = H_{l-1}' delta_l on the tiles this warp owns
@@ -646,8 +681,9 @@ __global__ void __launch_bounds__(NW * 32, NW >= 16 ? 1 : (NW >= 8 ? 2 : 4)) fit
 
 template <int NW, int TPW>
 int launch_cfg(const FitMArgs &a, int count, size_t smem, cudaStream_t stream) {
-  const auto kern = with_flags([](auto e, auto o) { return fit_mma_kernel<NW, TPW, e, o>; },
-                               acts_ext(a.d.act, a.d.n_layers), opt_build(a.opt, a.sched));
+  const auto kern = with_build(opt_build(a.opt, a.sched), a.drop.any,
+                               [](auto e, auto o, auto dr) { return fit_mma_kernel<NW, TPW, e, o, dr>; },
+                               acts_ext(a.d.act, a.d.n_layers));
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count, NW * 32, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());

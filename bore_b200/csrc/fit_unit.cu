@@ -353,7 +353,8 @@ __device__ __forceinline__ float fu_row_sum(const float *__restrict__ a, int SP)
 // compile-time shape, D stays a run-time value; NH == 0: everything from the descriptor and the plan.
 // WT: per-sample loss weights (FuArgs::fw); the unweighted build runs none of their code.
 // EXT: the activation codes above BORE_ACT_TANH (act.cuh).  OPT: the optimizers other than Adam (opt.cuh).
-template <int NH, int HW, int SPT, bool WT, bool EXT, bool OPT>
+// DROP (with OPT only): dropout after the hidden layers (dropout.cuh).
+template <int NH, int HW, int SPT, bool WT, bool EXT, bool OPT, bool DROP>
 __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_unit_kernel(const FuArgs a) {
   extern __shared__ __align__(16) float sm[];
   constexpr bool FIX = NH > 0;
@@ -507,6 +508,7 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
       if (nst == steps_per_epoch) { nst = 0; ++nep; }
       const bool more = nep < epochs;
       if (more) index_stage(nep, nst);  // read by gather_async in the gradient phase
+      const long long tm = run.t;  // the dropout masks' step: `iterations` before this step's increment
 #ifdef FU_TRACE
       ntr = 0;
 #endif
@@ -530,11 +532,13 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
         FU_T();
         const float *bs = W + P.bs[l];
         float *Hn = sm + P.h[l + 1][l == 0 ? par : 0] + rank * U * SPP;  // own rows of h_{l+1}
+        const bool drop = DROP && a.drop.rate[l] > 0.f;
         fu_reduce(sm + P.scratch, U, SP, inv_nq, wstride, [&](int u, int s, float4 sum) {
           if (rank * U + u < outd) {
             const float b = bs[u];
-            *reinterpret_cast<float4 *>(Hn + u * SPP + s) =
-                make_float4(act_fwd<EXT>(act, sum.x + b), act_fwd<EXT>(act, sum.y + b), act_fwd<EXT>(act, sum.z + b), act_fwd<EXT>(act, sum.w + b));
+            float4 o = make_float4(act_fwd<EXT>(act, sum.x + b), act_fwd<EXT>(act, sum.y + b), act_fwd<EXT>(act, sum.z + b), act_fwd<EXT>(act, sum.w + b));
+            if (drop) o = drop_fwd_unit4(a.drop, l, tm, s, rank * U + u, model, o);
+            *reinterpret_cast<float4 *>(Hn + u * SPP + s) = o;
           }
         });
         if (warp < FU_KS || U * (SP >> 2) > 32 * FU_KS) fu_fence_async();  // the slice's writers: generic-proxy stores -> visible to the bulk-copy engine
@@ -594,16 +598,22 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
       {
         float *DF = sm + (L - 1 >= 2 ? P.dg[L - 1] : P.dg[1]);
         const int nq = SP >> 2, actp = d.act[L - 2];
+        const bool drop = DROP && a.drop.rate[L - 2] > 0.f;
         for (int e = tid; e < HL * nq; e += FU_THREADS) {
           const int k = fdiv(e, inv_nq), q = e - k * nq;
           const float4 hv = *reinterpret_cast<const float4 *>(HLb + k * SPP + 4 * q);
           const float4 dz = *reinterpret_cast<const float4 *>(sm + P.dz + 4 * q);
           const float w = W[P.wl + k];
           float4 o;
-          o.x = dz.x * w * act_bwd<EXT>(actp, hv.x);
-          o.y = dz.y * w * act_bwd<EXT>(actp, hv.y);
-          o.z = dz.z * w * act_bwd<EXT>(actp, hv.z);
-          o.w = dz.w * w * act_bwd<EXT>(actp, hv.w);
+          if (drop) {
+            o = drop_bwd_unit4<EXT>(a.drop, L - 2, tm, 4 * q, k, model, actp,
+                                    make_float4(dz.x * w, dz.y * w, dz.z * w, dz.w * w), hv);
+          } else {
+            o.x = dz.x * w * act_bwd<EXT>(actp, hv.x);
+            o.y = dz.y * w * act_bwd<EXT>(actp, hv.y);
+            o.z = dz.z * w * act_bwd<EXT>(actp, hv.z);
+            o.w = dz.w * w * act_bwd<EXT>(actp, hv.w);
+          }
           *reinterpret_cast<float4 *>(DF + k * SPP + 4 * q) = o;
         }
       }
@@ -629,12 +639,14 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
         const int actp = d.act[i - 1];
         // delta_i slice: own rows of the complete buffer (i >= 2, pushed to the peers) or the local slice (i == 1)
         float *Dn = sm + (i >= 2 ? P.dg[i] + rank * U * SPP : P.d1);
+        const bool drop = DROP && a.drop.rate[i - 1] > 0.f;  // h_i holds h~ of hidden layer i - 1
         fu_reduce(sm + P.scratch, U, SP, inv_nq, wstride, [&](int u, int s, float4 sum) {
           if (rank * U + u < width) {
             const float4 hv = *reinterpret_cast<const float4 *>(Hi + u * SPP + s);
             *reinterpret_cast<float4 *>(Dn + u * SPP + s) =
-                make_float4(sum.x * act_bwd<EXT>(actp, hv.x), sum.y * act_bwd<EXT>(actp, hv.y), sum.z * act_bwd<EXT>(actp, hv.z),
-                            sum.w * act_bwd<EXT>(actp, hv.w));
+                drop ? drop_bwd_unit4<EXT>(a.drop, i - 1, tm, s, rank * U + u, model, actp, sum, hv)
+                     : make_float4(sum.x * act_bwd<EXT>(actp, hv.x), sum.y * act_bwd<EXT>(actp, hv.y), sum.z * act_bwd<EXT>(actp, hv.z),
+                                   sum.w * act_bwd<EXT>(actp, hv.w));
           }
         });
         if (i >= 2) {
@@ -854,8 +866,9 @@ __global__ void __cluster_dims__(FU_C, 1, 1) __launch_bounds__(FU_THREADS) fit_u
 
 template <int NH, int HW, int SPT>
 static int fu_launch(const FuArgs &a, int count, size_t smem, cudaStream_t stream) {
-  const auto kern = with_flags([](auto w, auto e, auto o) { return fit_unit_kernel<NH, HW, SPT, w, e, o>; }, a.fw.on,
-                               acts_ext(a.d.act, a.d.n_layers), opt_build(a.opt, a.sched));
+  const auto kern = with_build(opt_build(a.opt, a.sched), a.drop.any,
+                               [](auto w, auto e, auto o, auto dr) { return fit_unit_kernel<NH, HW, SPT, w, e, o, dr>; },
+                               a.fw.on, acts_ext(a.d.act, a.d.n_layers));
   BORE_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<count * FU_C, FU_THREADS, smem, stream>>>(a);
   BORE_CUDA(cudaGetLastError());

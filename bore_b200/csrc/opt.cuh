@@ -11,7 +11,8 @@
 //
 // Every fit kernel comes in two builds, selected at launch (opt_build, common.cuh): OPT = false is Adam at a
 // constant learning rate, with the arithmetic and the instructions it always had; OPT = true adds the other kinds
-// and the learning-rate schedules (lr_at).
+// and the learning-rate schedules (lr_at).  The MLP fit kernels have a third build for dropout (DROP, with_build in
+// fit_common.cuh).
 #pragma once
 #include "common.cuh"
 

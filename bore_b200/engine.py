@@ -238,6 +238,13 @@ class NativeMLP:
         if cache is not None:
             _lib.check(self.lib.bore_mlp_set_nadam_cache(self.h, model, float(cache)))
 
+    def set_dropout(self, rates, seeds):
+        """Dropout after each hidden layer in training: ``rates[l]`` in [0, 1) (0: none) and uint32 ``seeds[l]``, one
+        entry per hidden layer.  Keeps the weights and the optimizer state."""
+        r = np.ascontiguousarray(rates, np.float32)
+        sd = np.ascontiguousarray(seeds, np.uint32)
+        _lib.check(self.lib.bore_mlp_set_dropout(self.h, int(r.size), _np_ptr(r), _np_ptr(sd)))
+
     def set_fit_mode(self, mode):
         """0 automatic, 1 one CTA per model, 2 one thread-block cluster per model."""
         _lib.check(self.lib.bore_mlp_set_fit_mode(self.h, int(mode)))

@@ -116,6 +116,76 @@ class Dense:
         self.bias_regularizer = regularizer_get(bias_regularizer, "Dense")
 
 
+class Dropout:
+    """``keras.layers.Dropout(rate, noise_shape=None, seed=None)``: in training, each unit of the layer's input is
+    kept with probability 1 - rate and scaled by 1 / (1 - rate); ``predict`` and ``evaluate`` see no dropout.  Only
+    directly after a hidden ``Dense`` layer.  ``rate`` must be finite and in [0, 1), checked here rather than at the
+    first call as Keras does; ``seed`` is a uint32, or None for one drawn from the model's ``RandomState`` when its
+    weights are made.  The mask is the project's own (DESIGN.md, "Dropout"): TF's random stream is not reproduced."""
+
+    def __init__(self, rate, noise_shape=None, seed=None, **kwargs):
+        if kwargs:
+            raise TypeError(f"Dropout: unsupported arguments {sorted(kwargs)}")
+        if noise_shape is not None:
+            raise NotImplementedError("Dropout(noise_shape=...) is not in the training kernels: their masks are per "
+                                      "sample and unit")
+        r = float(rate)
+        if not (np.isfinite(r) and 0.0 <= r < 1.0):
+            raise ValueError(f"Dropout: rate must be finite and in [0, 1), got {rate!r}")
+        if seed is not None and not (int(seed) == seed and 0 <= int(seed) < 2 ** 32):
+            raise ValueError(f"Dropout: seed must be None or an integer in [0, 2**32), got {seed!r}")
+        self.rate = r
+        self.noise_shape = None
+        self.seed = None if seed is None else int(seed)
+
+
+def split_dropout(layers, final=True):
+    """(the Dense layers, the Dropout after each hidden layer or None) of a layer list.  A Dropout is taken only
+    directly after a hidden Dense layer; NotImplementedError says why for any other place.  ``final=False``: the list
+    may still grow (``add``), so its last Dense layer need not be the output layer, and ``after`` has an entry for it."""
+    dense, after = [], []
+    for lyr in layers:
+        check_layer_order(dense, after, lyr)
+        if isinstance(lyr, Dense):
+            dense.append(lyr)
+            after.append(None)
+        else:
+            after[-1] = lyr
+    if not final:
+        return dense, after
+    if after and after[-1] is not None:
+        raise NotImplementedError("a Dropout must be followed by a Dense layer: dropout after the output layer is "
+                                  "not taken, since the loss reaches through to its logit")
+    return dense, after[:-1]
+
+
+def check_layer_order(dense, after, layer):
+    """What ``add`` can check of appending ``layer`` to the Dense layers ``dense`` with their Dropouts ``after``."""
+    if isinstance(layer, Dense):
+        return
+    if not isinstance(layer, Dropout):
+        raise NotImplementedError("only Dense and Dropout layers are on the BORE-MLP path")
+    if not dense:
+        raise NotImplementedError("a Dropout as the first layer (input dropout) is not taken: the training kernels "
+                                  "gather the minibatch straight into their tiles")
+    if after[-1] is not None:
+        raise NotImplementedError("two Dropout layers in a row are not taken: a Dropout must follow a Dense layer")
+
+
+def dropout_rates_seeds(after, random_state):
+    """The (rates, seeds) of the hidden layers for ``NativeMLP.set_dropout``, or None when no rate is > 0.  A
+    Dropout with ``seed=None`` and rate > 0 draws its seed from ``random_state``, in layer order."""
+    if not any(d is not None and d.rate > 0 for d in after):
+        return None
+    rates, seeds = [], []
+    for d in after:
+        on = d is not None and d.rate > 0
+        rates.append(d.rate if on else 0.0)
+        seeds.append(0 if not on else d.seed if d.seed is not None else int(random_state.randint(0, 2 ** 32,
+                                                                                                  dtype=np.int64)))
+    return rates, seeds
+
+
 class BinaryCrossentropy:
     """``keras.losses.BinaryCrossentropy(from_logits=...)`` (plugins/hpbandster/base.py:157)."""
 

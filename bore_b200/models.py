@@ -12,7 +12,8 @@ parity testing: ``fit(..., permutations=...)`` and ``get/set_optimizer_state``.
 import numpy as np
 
 from . import ops
-from .layers import Dense, BinaryCrossentropy, optimizer_spec, regularizer_factors
+from .layers import (Dense, Dropout, BinaryCrossentropy, optimizer_spec, regularizer_factors, split_dropout,
+                     check_layer_order, dropout_rates_seeds)
 from .mixins import MaximizableMixin, BatchMaximizableMixin
 
 
@@ -70,7 +71,8 @@ class History:
 
 
 class Sequential:
-    """Stack of ``Dense`` layers with a scalar output."""
+    """Stack of ``Dense`` layers with a scalar output, with a ``Dropout`` after any hidden one.  ``layers`` holds
+    both kinds in order, as Keras' ``model.layers`` does."""
 
     def __init__(self, layers=None, seed=None, device=None):
         self.layers = []
@@ -84,11 +86,21 @@ class Sequential:
 
     # ------------------------------------------------------------------ construction
     def add(self, layer):
-        if not isinstance(layer, Dense):
-            raise NotImplementedError("only Dense layers are on the BORE-MLP path")
+        if not isinstance(layer, (Dense, Dropout)):
+            raise NotImplementedError("only Dense and Dropout layers are on the BORE-MLP path")
         if self._net is not None:
             raise RuntimeError("cannot add layers after the model was built")
+        dense, after = self._split(final=False)
+        check_layer_order(dense, after, layer)
         self.layers.append(layer)
+
+    def _split(self, final=True):
+        """(Dense layers, the Dropout after each Dense layer or None); ``final``: the whole model, whose last layer
+        must be a Dense layer (then one entry per hidden layer)."""
+        return split_dropout(self.layers, final)
+
+    def _dense(self):
+        return [lyr for lyr in self.layers if isinstance(lyr, Dense)]
 
     @property
     def input_dim(self):
@@ -97,7 +109,7 @@ class Sequential:
     def _factors(self):
         """Per-array (l2, l1) factors in Keras weight order [k0, b0, k1, b1, ...] (the plugin
         regularises its hidden layers only: plugins/hpbandster/base.py:113-116,152-155)."""
-        return regularizer_factors(r for lyr in self.layers for r in (lyr.kernel_regularizer, lyr.bias_regularizer))
+        return regularizer_factors(r for lyr in self._dense() for r in (lyr.kernel_regularizer, lyr.bias_regularizer))
 
     def _l2(self):
         return self._factors()[0]
@@ -115,8 +127,9 @@ class Sequential:
             raise RuntimeError("input dimension unknown: pass input_dim to the first Dense layer "
                                "or call fit/predict first")
         from .engine import NativeMLP
-        dims = [int(D)] + [lyr.units for lyr in self.layers]
-        acts = [lyr.activation for lyr in self.layers]
+        dense, after = self._split()
+        dims = [int(D)] + [lyr.units for lyr in dense]
+        acts = [lyr.activation for lyr in dense]
         net = NativeMLP(dims, acts, n_models=1, device=self._device)
         if self._pending_weights is not None:
             net.set_weights(self._pending_weights)
@@ -128,6 +141,9 @@ class Sequential:
                 ws.append(self._rs.uniform(-lim, lim, size=(fi, fo)).astype(np.float32))
                 ws.append(np.zeros(fo, np.float32))
             net.set_weights(ws)
+        drop = dropout_rates_seeds(after, self._rs)  # (seeds drawn after the initial weights)
+        if drop is not None:
+            net.set_dropout(*drop)
         if self._compiled is not None:
             net.set_optimizer_kind(self._compiled["optimizer"])
         self._net = net
@@ -135,7 +151,8 @@ class Sequential:
 
     def compile(self, optimizer="adam", loss=None, metrics=None, **kwargs):
         optimizer = optimizer_spec(optimizer)
-        final = self.layers[-1].activation if self.layers else None
+        dense = self._split()[0]
+        final = dense[-1].activation if dense else None
         if isinstance(loss, str):
             if loss != "binary_crossentropy":
                 raise NotImplementedError("only binary cross-entropy is on the BORE path")
@@ -173,16 +190,22 @@ class Sequential:
         self._engine().set_optimizer_state(m, v, iterations, cache)
 
     def count_params(self):
-        dims = [self.input_dim] + [lyr.units for lyr in self.layers]
+        dims = [self.input_dim] + [lyr.units for lyr in self._dense()]
         return sum(a * b + b for a, b in zip(dims[:-1], dims[1:]))
 
     def summary(self, print_fn=print):
         print_fn('Model: "sequential" (bore_b200 native, sm_100a)')
         fi = self.input_dim
-        for i, lyr in enumerate(self.layers):
+        i = k = 0
+        for lyr in self.layers:
+            if isinstance(lyr, Dropout):
+                print_fn(f"dropout_{k} (Dropout)  output=(None, {fi})  rate={lyr.rate}  params=0")
+                k += 1
+                continue
             n = "?" if fi is None else fi * lyr.units + lyr.units
             print_fn(f"dense_{i} (Dense)  output=(None, {lyr.units})  activation={lyr.activation}  params={n}")
             fi = lyr.units
+            i += 1
         if self.input_dim is not None:
             print_fn(f"Total params: {self.count_params()}")
 

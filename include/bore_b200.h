@@ -134,6 +134,15 @@ int bore_mlp_set_regularizers(bore_mlp *h, const float *l2_kernel_host, const fl
  * term is l1 * sign(w) with sign(0) = 0, as TF's Abs gradient.  n_layers floats each, finite and >= 0
  * (anything else is refused); zeros = none, the state at create.                                      */
 int bore_mlp_set_l1_regularizers(bore_mlp *h, const float *l1_kernel_host, const float *l1_bias_host);
+/* Dropout (keras.layers.Dropout) after each hidden layer, in training only: rates[l] and seeds[l] for the
+ * output of Dense layer l, l < n = n_layers - 1 hidden layers; rate 0 is no dropout, every rate finite and
+ * in [0, 1), else refused.  Arrays may be NULL when n = 0.  The mask of hidden layer l, unit j, minibatch
+ * position i, model m at the step whose Keras `iterations` is t before its increment is Philox4x32-10 with
+ * counter (t mod 2^32, t div 2^32, i, 65536 l + j div 4) and key (seeds[l], m): unit j is kept when output
+ * word j mod 4 gives (w >> 8) 2^-24 >= rates[l], and scaled by fp32(1 / (1 - rates[l])) (DESIGN.md,
+ * "Dropout").  evaluate, predict, value-and-gradient and the argmax see no dropout.  All rates are 0 at
+ * create; setting dropout keeps the weights and the optimizer state.  Synchronous, host only.           */
+int bore_mlp_set_dropout(bore_mlp *h, int n, const float *rates_host, const uint32_t *seeds_host);
 /* device pointer of the flat parameter block [n_models][n_params] (for NCCL broadcast) */
 int bore_mlp_params_dev(bore_mlp *h, float **params_dev);
 
